@@ -10,9 +10,11 @@ is missing or the tensors are not on a CUDA device.
 """
 import sys as _sys
 
-from . import _cabi, functional, gp, kernels, likelihoods, optim, synthetic, utilities  # noqa: F401
+from . import _cabi, counts, functional, gp, kernels, likelihoods, optim, synthetic, utilities  # noqa: F401
+from .counts import SparseCounts
 
-__all__ = ["kernels", "gp", "likelihoods", "utilities", "optim", "functional", "synthetic", "install_as_gpzoo"]
+__all__ = ["kernels", "gp", "likelihoods", "utilities", "optim", "functional", "synthetic", "counts", "SparseCounts",
+           "install_as_gpzoo"]
 
 
 def install_as_gpzoo():

@@ -40,6 +40,7 @@ def lib():
                 l.gpz_launch_count.restype = ctypes.c_longlong
                 for suf in ("f32", "f64"):
                     getattr(l, f"gpz_poisson_workspace_bytes_{suf}").restype = c_i64
+                    getattr(l, f"gpz_poisson_csc_workspace_bytes_{suf}").restype = c_i64
                 _lib = l
     return _lib
 

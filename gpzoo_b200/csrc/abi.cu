@@ -2,7 +2,7 @@
 #include "common.cuh"
 #include "gpzoo_b200.h"
 
-extern "C" int gpz_abi_version(void) { return 2; }      // 2: kernel_build_* take `kind`
+extern "C" int gpz_abi_version(void) { return 3; }      // 2: kernel_build_* take `kind`; 3: sparse-count K7 (poisson_*_csc_*)
 
 extern "C" const char* gpz_error_string(int rc) {
   if (rc == 0) return "success";

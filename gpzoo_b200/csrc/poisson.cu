@@ -1377,6 +1377,345 @@ __global__ void poisson_rate_kernel(const T* __restrict__ W, int w_softplus, con
   }
 }
 
+// ---- K7-CSC: the same outputs from sparse counts (spot-major compressed columns: indptr[N+1], genes[nnz], values[nnz]) --------
+// With s_n = softplus(V_n), w = softplus(W) (or raw W), c_f = sum_g w_gf, eps_efn = s_n exp(F_efn), r_egn = sum_f w_gf eps_efn and
+// t_egn = y_gn / (E r_egn) on the nonzeros only, the y = 0 entries contribute only -r, whose sums close through c_f:
+//   ll          = sum_nz [ (1/E) sum_e y log r - lgamma(y+1) ] - (1/E) sum_{e,n,f} c_f eps_efn
+//   d/dF_efn    = eps_efn ( sum_{g in nz(n)} t_egn w_gf - c_f / E )
+//   d/dw_gf     = sum_e sum_{n in nz(g)} t_egn eps_efn - u_f,          u_f = (1/E) sum_{e,n} eps_efn
+//   d/dV_n      = softplus'(V_n) / s_n ( sum_{g in nz(n)} y_gn - (1/E) sum_{e,f} c_f eps_efn )
+// so the work per step is O(nnz F + B F + G F) whatever the density.  The "-1" the dense kernels take per element is taken here
+// once per (spot, factor) and once per factor: near a fit the two sides nearly cancel, so c_f, u_f, ll, the per-spot
+// sum_g t w and the final combination of the per-CTA d/dw partials are all carried in double.
+// Mapping: one warp per spot (lanes stride over the spot's nonzeros; lane f owns factor f of the spot's per-spot terms), a fixed
+// range of spots per CTA.  d/dw is scattered into a per-CTA G x F shared-memory accumulator when it fits (summed afterwards by
+// csc_reduce_kernel in a fixed order), else into one G x F double accumulator in global memory by atomics.
+constexpr int CSC_MAX_WARPS = 16;
+// 512 threads; 256 for F > 12, whose F double accumulators per lane need more than the 128 registers a 512-thread CTA allows
+template <int FMAX> constexpr int csc_threads() { return FMAX > 12 ? 256 : 512; }
+constexpr size_t CSC_SMEM_MAX = 160 * 1024;      // per-CTA d/dw accumulator limit: G F <= 40960 in fp32 (config 2's 2000 x 20 fits)
+
+template <typename T> struct CscArgs {
+  const int64_t* indptr; const int32_t* genes; const void* values;
+  const int64_t* idx;
+  const T* W; int w_softplus; const T* V; const T* mean; const T* spread; const T* eps;
+  int G, F, B, E, n_var; T clamp_min; int with_lgamma;
+  // workspace
+  const T* w;                  // [G][FMAX] softplus(W) or W, factors >= F zero
+  const double* c;             // [F] column sums of w
+  double* ll_part;             // [nbx]
+  double* u_part;              // [nbx][F]
+  T* gw_part;                  // [nbx][G][F] (shared-memory path) or null
+  double* gw_acc;              // [G][F] (atomic path) or null
+  int spots_per_cta;
+  // outputs
+  T* gV; T* gmean; T* gspread;
+};
+
+// blocks [0, F): c_f = sum_g w_gf in double; blocks [F, ...): the padded rows of w
+template <typename T, int FMAX>
+__global__ void __launch_bounds__(256) csc_prep_kernel(const T* __restrict__ W, int w_softplus, int G, int F, T* __restrict__ w,
+                                                       double* __restrict__ c) {
+  __shared__ double red[32];
+  if ((int)blockIdx.x < F) {
+    const int f = blockIdx.x;
+    double s = 0.0;
+    for (int g = threadIdx.x; g < G; g += blockDim.x) {
+      const T v = W[(int64_t)g * F + f];
+      s += (double)(w_softplus ? softplus(v) : v);
+    }
+    s = block_sum<double>(s, red);
+    if (threadIdx.x == 0) c[f] = s;
+    return;
+  }
+  const int64_t i = (int64_t)(blockIdx.x - F) * blockDim.x + threadIdx.x;
+  if (i >= (int64_t)G * FMAX) return;
+  const int64_t g = i / FMAX;
+  const int f = (int)(i - g * FMAX);
+  T v = T(0);
+  if (f < F) {
+    v = W[g * F + f];
+    if (w_softplus) v = softplus(v);
+  }
+  w[i] = v;
+}
+
+template <typename YT, typename T> __device__ __forceinline__ T csc_value(const void* p, int64_t k) {
+  return (T)reinterpret_cast<const YT*>(p)[k];
+}
+// four consecutive elements of a 16-byte aligned row
+__device__ __forceinline__ void ld4(const float* p, float (&o)[4]) {
+  const float4 v = *reinterpret_cast<const float4*>(p);
+  o[0] = v.x; o[1] = v.y; o[2] = v.z; o[3] = v.w;
+}
+__device__ __forceinline__ void ld4(const double* p, double (&o)[4]) {
+  const double2 v0 = reinterpret_cast<const double2*>(p)[0], v1 = reinterpret_cast<const double2*>(p)[1];
+  o[0] = v0.x; o[1] = v0.y; o[2] = v1.x; o[3] = v1.y;
+}
+__device__ __forceinline__ void ld4_nc(const float* p, float (&o)[4]) {
+  const float4 v = __ldg(reinterpret_cast<const float4*>(p));
+  o[0] = v.x; o[1] = v.y; o[2] = v.z; o[3] = v.w;
+}
+__device__ __forceinline__ void ld4_nc(const double* p, double (&o)[4]) {
+  const double2 v0 = __ldg(reinterpret_cast<const double2*>(p)), v1 = __ldg(reinterpret_cast<const double2*>(p) + 1);
+  o[0] = v0.x; o[1] = v0.y; o[2] = v1.x; o[3] = v1.y;
+}
+
+template <typename T, typename YT, int FMAX, bool SMEM_ACC>
+__global__ void __launch_bounds__(csc_threads<FMAX>(), 1) poisson_csc_kernel(const CscArgs<T> a) {
+  constexpr int CSC_THREADS = csc_threads<FMAX>(), CSC_WARPS = CSC_THREADS / 32;
+  extern __shared__ __align__(16) unsigned char csc_smem[];
+  T* sAcc = reinterpret_cast<T*>(csc_smem);                     // [G][F] (SMEM_ACC)
+  __shared__ double red[32];
+  __shared__ double sU[CSC_MAX_WARPS][32];
+  __shared__ __align__(16) T sEf[CSC_MAX_WARPS][32];                  // eps_e[:] of the warp's current spot (read as broadcasts)
+  __shared__ T lfact[64];                                         // log(y!) for integer counts y < 64
+
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int F = a.F, GF = a.G * a.F;
+  if (tid < 64) lfact[tid] = Num<T>::lgamma(T(tid + 1));
+  if (SMEM_ACC)
+    for (int i = tid; i < GF; i += CSC_THREADS) sAcc[i] = T(0);
+  __syncthreads();
+
+  const T invE = T(1) / T(a.E);
+  const double cf = lane < F ? a.c[lane] : 0.0;
+  double ll = 0.0, u = 0.0;                                       // u: lane f's share of u_f
+  const int b_begin = blockIdx.x * a.spots_per_cta, b_end = min(a.B, b_begin + a.spots_per_cta);
+  for (int b = b_begin + warp; b < b_end; b += CSC_WARPS) {
+    const int64_t col = a.idx ? a.idx[b] : (int64_t)b;
+    const int64_t p0 = a.indptr[col], p1 = a.indptr[col + 1];
+    const T vraw = a.V[col];
+    const T spV = softplus(vraw);
+    // lane f: this spot's variational parameters of factor f
+    T mu = T(0), sd = T(0), sp = T(0);
+    if (lane < F) {
+      const int64_t o = (int64_t)lane * a.B + b;
+      mu = a.mean[o];
+      sp = a.spread[o];
+      sd = lane < a.n_var ? Num<T>::sqrt(sp > a.clamp_min ? sp : a.clamp_min) : sp;
+    }
+    T gm = T(0), gs = T(0);
+    double ysum = 0.0, rsum = 0.0;                                // sum_nz y;  sum_e sum_f c_f eps_ef
+    for (int e = 0; e < a.E; ++e) {
+      T epsv = T(0), ev = T(0);
+      if (lane < F) {
+        epsv = a.eps[((int64_t)e * F + lane) * a.B + b];
+        ev = spV * Num<T>::exp(fma(epsv, sd, mu));
+      }
+      const T* sE = sEf[warp];
+      __syncwarp();                                               // the previous spot / sample is done with sE
+      if (lane < FMAX) sEf[warp][lane] = ev;                      // lanes >= F hold 0
+      __syncwarp();
+      rsum += warp_sum<double>(cf * (double)ev);
+      u += (double)ev;
+      double acc[FMAX];                                           // sum over the lane's nonzeros of t w_f
+#pragma unroll
+      for (int f = 0; f < FMAX; ++f) acc[f] = 0.0;
+      double llc = 0.0;
+      for (int64_t k = p0 + lane; k < p1; k += 32) {
+        const int g = a.genes[k];
+        const T y = csc_value<YT, T>(a.values, k);
+        const T* wr = a.w + (int64_t)g * FMAX;
+        T r = T(0);
+#pragma unroll
+        for (int f4 = 0; f4 < FMAX; f4 += 4) {
+          T w4[4], e4[4];
+          ld4_nc(wr + f4, w4);
+          ld4(sE + f4, e4);
+#pragma unroll
+          for (int j = 0; j < 4; ++j) r = fma(w4[j], e4[j], r);
+        }
+        const T t = fast_div(y, r) * invE;
+        T lp = y * fast_log(r) * invE;
+        if (e == 0) {
+          if (a.with_lgamma) {
+            const int yi = (int)y;
+            lp -= (yi >= 0 && yi < 64 && T(yi) == y) ? lfact[yi] : Num<T>::lgamma(y + T(1));
+          }
+          ysum += (double)y;
+        }
+        llc += (double)lp;
+        // second pass over the row (reloaded from L1 rather than held: keeps the F double accumulators spill-free)
+#pragma unroll
+        for (int f4 = 0; f4 < FMAX; f4 += 4) {
+          T w4[4], e4[4];
+          ld4(wr + f4, w4);
+          ld4(sE + f4, e4);
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            const int f = f4 + j;
+            acc[f] += (double)(t * w4[j]);
+            if (f < F) {
+              const T gw = t * e4[j];
+              if (SMEM_ACC) atomicAdd(sAcc + g * F + f, gw);
+              else atomicAdd(a.gw_acc + (int64_t)g * F + f, (double)gw);
+            }
+          }
+        }
+      }
+      ll += llc;
+      // lane f: d ll / d F_ef = eps_ef (sum_g t w_f - c_f / E)
+      double mine = 0.0;
+#pragma unroll
+      for (int f = 0; f < FMAX; ++f) {
+        const double v = warp_sum<double>(acc[f]);
+        if (lane == f) mine = v;
+      }
+      if (lane < F) {
+        const T gF = (T)((double)ev * (mine - cf * (double)invE));
+        gm += gF;
+        gs = fma(gF, epsv, gs);
+      }
+    }
+    ysum = warp_sum<double>(ysum);
+    if (lane == 0) {
+      ll -= rsum * (double)invE;
+      a.gV[b] = (T)((double)(softplus_grad(vraw) / spV) * (ysum - rsum * (double)invE));
+    }
+    if (lane < F) {
+      const int64_t o = (int64_t)lane * a.B + b;
+      if (lane < a.n_var) gs = sp >= a.clamp_min ? gs / (T(2) * sd) : T(0);   // spread is a variance: d sd / d var = 1 / (2 sd)
+      a.gmean[o] = gm;
+      a.gspread[o] = gs;
+    }
+  }
+
+  // per-CTA partials: ll, u_f, and the d/dw accumulator
+  sU[warp][lane] = u;
+  const double tot = block_sum<double>(ll, red);                  // its barriers also publish sU and the shared atomics
+  if (tid == 0) a.ll_part[blockIdx.x] = tot;
+  if (tid < F) {
+    double s = 0.0;
+    for (int w8 = 0; w8 < CSC_WARPS; ++w8) s += sU[w8][tid];
+    a.u_part[(int64_t)blockIdx.x * F + tid] = s * (double)invE;
+  }
+  if (SMEM_ACC)
+    for (int i = tid; i < GF; i += CSC_THREADS) a.gw_part[(int64_t)blockIdx.x * GF + i] = sAcc[i];
+}
+
+// gW[g, f] = (softplus'(W) or 1) * (sum of the d/dw partials - u_f), all sums in double and in a fixed order; block 0 also sums ll
+template <typename T>
+__global__ void __launch_bounds__(256) csc_reduce_kernel(const CscArgs<T> a, int nbx, T* __restrict__ gW, double* __restrict__ ll_out) {
+  __shared__ double u[32];
+  __shared__ double red[32];
+  const int tid = threadIdx.x;
+  if (tid < a.F) {
+    double s = 0.0;
+    for (int b = 0; b < nbx; ++b) s += a.u_part[(int64_t)b * a.F + tid];
+    u[tid] = s;
+  }
+  if (blockIdx.x == 0) {
+    double s = 0.0;
+    for (int b = tid; b < nbx; b += blockDim.x) s += a.ll_part[b];
+    s = block_sum<double>(s, red);                                // also the barrier that publishes u
+    if (tid == 0) ll_out[0] = s;
+  } else {
+    __syncthreads();
+  }
+  // 64 outputs per block; thread (o, p) adds the partials of the CTAs b = p, p + 4, ... with four independent accumulators
+  __shared__ double part[4][64];
+  const int64_t GF = (int64_t)a.G * a.F, i = (int64_t)blockIdx.x * 64 + (tid & 63);
+  const int p = tid >> 6;
+  double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
+  if (i < GF && a.gw_part) {
+    int b = p;
+    for (; b + 12 < nbx; b += 16) {
+      s0 += (double)a.gw_part[(int64_t)b * GF + i];
+      s1 += (double)a.gw_part[(int64_t)(b + 4) * GF + i];
+      s2 += (double)a.gw_part[(int64_t)(b + 8) * GF + i];
+      s3 += (double)a.gw_part[(int64_t)(b + 12) * GF + i];
+    }
+    for (; b < nbx; b += 4) s0 += (double)a.gw_part[(int64_t)b * GF + i];
+  }
+  part[p][tid & 63] = (s0 + s1) + (s2 + s3);
+  __syncthreads();
+  if (tid >= 64 || i >= GF) return;
+  const double s = a.gw_part ? (part[0][tid] + part[1][tid]) + (part[2][tid] + part[3][tid]) : a.gw_acc[i];
+  const T d = (T)(s - u[i % a.F]);
+  gW[i] = a.w_softplus ? d * softplus_grad(a.W[i]) : d;
+}
+
+static int csc_fmax(int F) { return F <= 4 ? 4 : F <= 12 ? 12 : F <= 20 ? 20 : 32; }
+static int csc_nbx(int B) {                   // one CTA per SM (the per-CTA d/dw partials are G F each), at least 16 spots per CTA
+  static int nsm = 0;
+  if (nsm == 0) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) nsm = 148;
+  }
+  return (int)max((int64_t)1, min(cdiv(B, 16), (int64_t)nsm));
+}
+static bool csc_smem_acc(int G, int F, size_t elt) { return elt * (size_t)G * F <= CSC_SMEM_MAX; }
+static size_t align16(size_t b) { return (b + 15) / 16 * 16; }
+// workspace: ll_part [nbx] | u_part [nbx][F] | c [F] (doubles) | w [G][FMAX] | d/dw partials [nbx][G][F] T or accumulator [G][F] double
+static size_t csc_ws_bytes(int G, int F, int B, size_t elt) {
+  const int nbx = csc_nbx(B);
+  size_t b = align16(sizeof(double) * ((size_t)nbx * (F + 1) + F)) + align16(elt * (size_t)G * csc_fmax(F));
+  b += csc_smem_acc(G, F, elt) ? align16(elt * (size_t)nbx * G * F) : align16(sizeof(double) * (size_t)G * F);
+  return b;
+}
+
+template <typename T, typename YT, int FMAX> int csc_launch_main(const CscArgs<T>& a, int nbx, cudaStream_t st) {
+  if (a.gw_part) {
+    const size_t smem = sizeof(T) * (size_t)a.G * a.F;
+    GPZ_CUDA(cudaFuncSetAttribute(poisson_csc_kernel<T, YT, FMAX, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    poisson_csc_kernel<T, YT, FMAX, true><<<nbx, csc_threads<FMAX>(), smem, st>>>(a);
+  } else {
+    poisson_csc_kernel<T, YT, FMAX, false><<<nbx, csc_threads<FMAX>(), 0, st>>>(a);
+  }
+  GPZ_CHECK_LAUNCH();
+  return GPZ_OK;
+}
+template <typename T, int FMAX> int csc_launch(CscArgs<T> a, int count_kind, int nbx, double* wbase_c, cudaStream_t st) {
+  csc_prep_kernel<T, FMAX><<<(unsigned)(a.F + cdiv((int64_t)a.G * FMAX, 256)), 256, 0, st>>>(a.W, a.w_softplus, a.G, a.F,
+                                                                                              const_cast<T*>(a.w), wbase_c);
+  GPZ_CHECK_LAUNCH();
+  switch (count_kind) {
+    case 1: return csc_launch_main<T, uint8_t, FMAX>(a, nbx, st);
+    case 2: return csc_launch_main<T, int16_t, FMAX>(a, nbx, st);
+    case 3: return csc_launch_main<T, int32_t, FMAX>(a, nbx, st);
+    default: return csc_launch_main<T, T, FMAX>(a, nbx, st);
+  }
+}
+
+template <typename T>
+int poisson_fwdbwd_csc(CscArgs<T> a, int count_kind, int64_t n_total, T* gW, double* ll_out, void* ws, size_t ws_bytes, cudaStream_t st) {
+  if (a.F < 1 || a.F > 32 || a.E < 1 || a.G < 1) return GPZ_ERR_UNSUPPORTED;
+  if (count_kind < 0 || count_kind > 3 || a.B < 0 || (!a.idx && a.B != n_total)) return GPZ_ERR_BADARG;
+  if (a.B == 0) {                       // empty minibatch: ll = 0, no gradient
+    GPZ_CUDA(cudaMemsetAsync(ll_out, 0, sizeof(double), st));
+    GPZ_CUDA(cudaMemsetAsync(gW, 0, sizeof(T) * (size_t)a.G * a.F, st));
+    return GPZ_OK;
+  }
+  if (ws_bytes < csc_ws_bytes(a.G, a.F, a.B, sizeof(T))) return GPZ_ERR_BADARG;
+  const int nbx = csc_nbx(a.B), fmax = csc_fmax(a.F);
+  unsigned char* p = reinterpret_cast<unsigned char*>(ws);
+  a.ll_part = reinterpret_cast<double*>(p);
+  a.u_part = a.ll_part + nbx;
+  double* c = a.u_part + (size_t)nbx * a.F;
+  a.c = c;
+  p += align16(sizeof(double) * ((size_t)nbx * (a.F + 1) + a.F));
+  a.w = reinterpret_cast<T*>(p);
+  p += align16(sizeof(T) * (size_t)a.G * fmax);
+  a.gw_part = nullptr; a.gw_acc = nullptr;
+  if (csc_smem_acc(a.G, a.F, sizeof(T))) {
+    a.gw_part = reinterpret_cast<T*>(p);
+  } else {
+    a.gw_acc = reinterpret_cast<double*>(p);
+    GPZ_CUDA(cudaMemsetAsync(a.gw_acc, 0, sizeof(double) * (size_t)a.G * a.F, st));
+  }
+  a.spots_per_cta = (int)cdiv(a.B, nbx);
+  int rc;
+  if (fmax == 4) rc = csc_launch<T, 4>(a, count_kind, nbx, c, st);
+  else if (fmax == 12) rc = csc_launch<T, 12>(a, count_kind, nbx, c, st);
+  else if (fmax == 20) rc = csc_launch<T, 20>(a, count_kind, nbx, c, st);
+  else rc = csc_launch<T, 32>(a, count_kind, nbx, c, st);
+  if (rc) return rc;
+  csc_reduce_kernel<T><<<(unsigned)max((int64_t)1, cdiv((int64_t)a.G * a.F, 64)), 256, 0, st>>>(a, nbx, gW, ll_out);
+  GPZ_CHECK_LAUNCH();
+  return GPZ_OK;
+}
+
 }  // namespace gpz
 
 using namespace gpz;
@@ -1420,3 +1759,25 @@ extern "C" int gpz_poisson_fwdbwd_yt_f32(const void* y, int y_kind, int64_t y_ld
   a.with_lgamma = with_lgamma; a.gV = gV; a.gmean = gmean; a.gspread = gspread;
   return poisson_fwdbwd<float>(a, gW, ll, ws, (size_t)ws_bytes, (cudaStream_t)stream, y_kind);
 }
+
+// sparse counts (K7-CSC): count_kind 0 = T, 1 = uint8, 2 = int16, 3 = int32
+#define GPZ_POISSON_CSC_IMPL(SUF, T)                                                                                    \
+  extern "C" int64_t gpz_poisson_csc_workspace_bytes_##SUF(int G, int F, int B, int E) {                                \
+    (void)E;                                                                                                            \
+    return (int64_t)csc_ws_bytes(G, F, B, sizeof(T));                                                                   \
+  }                                                                                                                     \
+  extern "C" int gpz_poisson_fwdbwd_csc_##SUF(const int64_t* indptr, const int32_t* genes, const void* counts,          \
+                                              int count_kind, int64_t n_total, const int64_t* idx, const T* W,           \
+                                              int w_softplus, const T* V, const T* mean, const T* spread, const T* eps,  \
+                                              int G, int F, int B, int E, int n_var, T clamp_min, int with_lgamma,       \
+                                              double* ll, T* gW, T* gV, T* gmean, T* gspread, void* ws, int64_t ws_bytes, \
+                                              void* stream) {                                                            \
+    CscArgs<T> a;                                                                                                       \
+    a.indptr = indptr; a.genes = genes; a.values = counts; a.idx = idx; a.W = W; a.w_softplus = w_softplus; a.V = V;   \
+    a.mean = mean; a.spread = spread; a.eps = eps; a.G = G; a.F = F; a.B = B; a.E = E; a.n_var = n_var;                 \
+    a.clamp_min = clamp_min; a.with_lgamma = with_lgamma; a.gV = gV; a.gmean = gmean; a.gspread = gspread;              \
+    return poisson_fwdbwd_csc<T>(a, count_kind, n_total, gW, ll, ws, (size_t)ws_bytes, (cudaStream_t)stream);          \
+  }
+
+GPZ_POISSON_CSC_IMPL(f32, float)
+GPZ_POISSON_CSC_IMPL(f64, double)

@@ -16,6 +16,7 @@ from torch.autograd.function import once_differentiable
 
 from . import _cabi
 from ._cabi import c_f, c_i, c_i64, c_p, call, ptr, scalar
+from .counts import SparseCounts
 
 # When True (default) a non-positive-definite Kzz raises torch.linalg.LinAlgError right away like the
 # reference's torch.linalg.cholesky (one device sync).  Throughput runs may turn it off and call
@@ -1072,7 +1073,8 @@ class MvnKL(Function):
 # ------------------------------------------------------------------------------------------------
 class PoissonLL(Function):
     """mean_E sum_{g,n} Poisson log-lik of y under rate = softplus(V) (w(W) @ exp(mean + eps*sd)),
-    with all gradients produced by the same pass (csrc/poisson.cu)."""
+    with all gradients produced by the same pass (csrc/poisson.cu).  y is a dense G x N tensor or a `SparseCounts`
+    (read by the K7-CSC kernel, whose work scales with the nonzeros)."""
 
     Y_KINDS = {torch.uint8: 1, torch.int16: 2, torch.int32: 3}     # counts stored as integers (gpz_poisson_fwdbwd_yt_f32)
 
@@ -1081,6 +1083,11 @@ class PoissonLL(Function):
         W, V, mean, spread, eps = _c(W), _c(V), _c(mean), _c(spread), _c(eps)
         dt = W.dtype
         G, F = W.shape
+        if isinstance(y, SparseCounts):
+            gW, gV, gmean, gspread, ll, idx = _poisson_csc(y, idx, W, V, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma)
+            ctx.save_for_backward(gW, gV, gmean, gspread, idx)
+            ctx.nV = V.shape[0]
+            return ll.to(dt).reshape(())
         # y: the reference passes floats; integer counts (uint8 / int16 / int32) are read as stored by the fp32 tensor-core kernel
         # (F <= 16), any other combination is converted on the device
         y_kind = PoissonLL.Y_KINDS.get(y.dtype, 0) if (dt == torch.float32 and F <= 16 and POISSON_NARROW_Y) else 0
@@ -1123,6 +1130,36 @@ class PoissonLL(Function):
             full.index_add_(0, idx, gV)
             gV = full
         return None, None, g * gW, g * gV, g * gmean, g * gspread, None, None, None, None, None
+
+
+_CSC_KINDS = {torch.uint8: 1, torch.int16: 2, torch.int32: 3}      # count_kind of gpz_poisson_fwdbwd_csc_* (0 = the compute type)
+
+
+def _poisson_csc(y, idx, W, V, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma):
+    """K7 on sparse counts: gpz_poisson_fwdbwd_csc_*.  Same outputs as the dense call."""
+    dt = W.dtype
+    G, F = W.shape
+    B, E = mean.shape[1], eps.shape[0]
+    N = y.shape[1]
+    assert y.shape[0] == G and mean.shape[0] == F and eps.shape[1] == F and eps.shape[2] == B
+    if idx is not None:
+        idx = _c(idx.to(device=W.device, dtype=torch.int64))
+    else:
+        assert N == B
+    vals = y.values
+    kind = _CSC_KINDS.get(vals.dtype, 0)
+    if kind == 0 and vals.dtype != dt:
+        vals = vals.to(dt)
+    ws_bytes = int(getattr(_cabi.lib(), "gpz_poisson_csc_workspace_bytes_" + ("f32" if dt == torch.float32 else "f64"))(
+        c_i(G), c_i(F), c_i(B), c_i(E)))
+    ws = torch.empty(ws_bytes // 8 + 1, dtype=torch.float64, device=W.device)
+    ll = torch.empty(1, dtype=torch.float64, device=W.device)
+    gW, gV = torch.empty_like(W), torch.empty(B, dtype=dt, device=W.device)
+    gmean, gspread = torch.empty_like(mean), torch.empty_like(spread)
+    call("poisson_fwdbwd_csc", dt, ptr(y.indptr), ptr(y.genes), ptr(_c(vals)), c_i(kind), c_i64(N), ptr(idx), ptr(W),
+         c_i(int(w_softplus)), ptr(V), ptr(mean), ptr(spread), ptr(eps), c_i(G), c_i(F), c_i(B), c_i(E), c_i(int(n_var)),
+         scalar(dt, clamp_min), c_i(int(with_lgamma)), ptr(ll), ptr(gW), ptr(gV), ptr(gmean), ptr(gspread), ptr(ws), c_i64(ws_bytes))
+    return gW, gV, gmean, gspread, ll, idx
 
 
 def poisson_rate(W, V, idx, F, w_softplus=True):

@@ -197,6 +197,25 @@ int gpz_poisson_fwdbwd_yt_f32(const void* y, int y_kind, int64_t y_ld, const int
                               const float* mean, const float* spread, const float* eps, int G, int F, int B, int E, int n_var,
                               float clamp_min, int with_lgamma, double* ll, float* gW, float* gV, float* gmean, float* gspread,
                               void* ws, int64_t ws_bytes, void* stream);
+/* K7-CSC: the same call on sparse counts, whose work scales with the nonzeros instead of G x N.  The count matrix is stored as
+ * spot-major compressed columns (AnnData's N x G CSR): spot n owns entries indptr[n] .. indptr[n+1] (int64, n_total + 1 of them)
+ * of genes (int32, in [0, G), ascending and unique within a spot) and counts (count_kind 0 = T, 1 = uint8, 2 = int16,
+ * 3 = int32; non-negative, no explicit zeros needed).  idx (B or NULL; NULL requires B == n_total) picks the columns of the
+ * resident matrix, no gather copy.  The y = 0 entries enter in closed form through the column sums of the loadings; c_f, u_f,
+ * ll and the final combination of the d/dW partials are carried in double.  Outputs and conventions as gpz_poisson_fwdbwd_*;
+ * F <= 32 (GPZ_ERR_UNSUPPORTED otherwise), any E.  ws sized by gpz_poisson_csc_workspace_bytes_*. */
+int64_t gpz_poisson_csc_workspace_bytes_f32(int G, int F, int B, int E);
+int64_t gpz_poisson_csc_workspace_bytes_f64(int G, int F, int B, int E);
+int gpz_poisson_fwdbwd_csc_f32(const int64_t* indptr, const int32_t* genes, const void* counts, int count_kind, int64_t n_total,
+                               const int64_t* idx, const float* W, int w_softplus, const float* V, const float* mean,
+                               const float* spread, const float* eps, int G, int F, int B, int E, int n_var, float clamp_min,
+                               int with_lgamma, double* ll, float* gW, float* gV, float* gmean, float* gspread, void* ws,
+                               int64_t ws_bytes, void* stream);
+int gpz_poisson_fwdbwd_csc_f64(const int64_t* indptr, const int32_t* genes, const void* counts, int count_kind, int64_t n_total,
+                               const int64_t* idx, const double* W, int w_softplus, const double* V, const double* mean,
+                               const double* spread, const double* eps, int G, int F, int B, int E, int n_var, double clamp_min,
+                               int with_lgamma, double* ll, double* gW, double* gV, double* gmean, double* gspread, void* ws,
+                               int64_t ws_bytes, void* stream);
 int gpz_poisson_rate_f32(const float* W, int w_softplus, const float* V, const int64_t* idx, const float* F, float* rate,
                          int G, int nF, int B, int E, void* stream);
 int gpz_poisson_rate_f64(const double* W, int w_softplus, const double* V, const int64_t* idx, const double* F, double* rate,
