@@ -2,7 +2,9 @@
 #include "common.cuh"
 #include "gpzoo_b200.h"
 
-extern "C" int gpz_abi_version(void) { return 3; }      // 2: kernel_build_* take `kind`; 3: sparse-count K7 (poisson_*_csc_*)
+// 2: kernel_build_* take `kind`; 3: sparse-count K7 (poisson_*_csc_*); 4: the separate Cholesky and triangular-inverse entry
+// points are gone (gpz_chol_inv_* computes both), gpz_svgp_predict_bwd_h_f32 lost its Lc argument
+extern "C" int gpz_abi_version(void) { return 4; }
 
 extern "C" const char* gpz_error_string(int rc) {
   if (rc == 0) return "success";

@@ -253,8 +253,7 @@ extern "C" int gpz_svgp_chain_bwd_f32(const float* Lc, const float* Linv, const 
 //     Y = T T^T ;  V = (S1 + gkl I) T ;  gLu = tril(Linv^T V) - gkl / diag(Lu)  (+ incoming)
 //     G2 = Y S1 + S1 Y - S1 + gkl Y + q gqp^T
 //     gLc = gkl / diag(Lc) - tril(Linv^T G2) - tril(gmu q^T)  (+ incoming) ;  P = Phi(Lc^T gLc) ;  gKzz = Linv^T P Linv
-// i.e. 8 M x M x M products and ONE reduction over the spots, instead of 11 products and two reductions, and without the
-// multiply-by-Lc-then-by-Linv round trip of the un-merged regrouping (which costs accuracy on ill-conditioned Kzz).
+// i.e. 8 M x M x M products and ONE reduction over the spots, where the predictive backward alone needs two (gT and gLinv).
 // ws: 13 L M M + 2 L M floats.
 extern "C" int gpz_svgp_chain_bwd_s1_f32(const float* Lc, const float* Linv, const float* Lu, const float* T, const float* q,
                                          const float* mu, const float* aux, const float* S1, const float* S1_lo, const float* gqp,

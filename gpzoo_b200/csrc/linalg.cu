@@ -1,15 +1,13 @@
-// K2: batched blocked right-looking Cholesky (gp.py:213,360,55 -> torch.linalg.cholesky) and the
-// blocked triangular inverse used to turn the two triangular solves of torch.cholesky_solve
-// (gp.py:218,365) into triangular matrix products, plus the small O(M^2) element-wise helpers of the
-// variational parameters (lower-Cholesky transform gp.py:220, KL reductions torch kl.py MVN||MVN).
+// K2: batched Cholesky fused with the triangular inverse (gp.py:213,360,55 -> torch.linalg.cholesky; the inverse turns the
+// two triangular solves of torch.cholesky_solve, gp.py:218,365, into triangular matrix products), plus the small O(M^2)
+// element-wise helpers of the variational parameters (lower-Cholesky transform gp.py:220, KL reductions torch kl.py MVN||MVN).
 //
-// Blocked right-looking factorisation, panel width NB: for each panel k
-//   (1) potf2: factor the NB x NB diagonal block in shared memory (one CTA per factor l)
-//   (2) trsm : L21 = A21 L11^-T, one thread per row, panel staged through shared memory
-//   (3) syrk : A22 -= L21 L21^T  -- the only O(M^3) part; a GEMM (gemm_simt.cuh / tcgen05 path)
+// Right-looking blocked factorisation, panel width NB: for each panel k the NB x NB diagonal block is factored AND inverted
+// (leaf_body), then the panel L21 = A21 X11^T and the trailing update A22 -= L21 L21^T; X = Lc^-1 follows by recursive
+// doubling, X21 = -X22 (L21 X11).  chol_inv runs it as one cluster kernel per factor (M <= 1536) or as a sweep of GEMM launches;
+// chol_inv_hybrid (fp32, large M) runs 256-wide panels on the cluster kernel and every larger product on tcgen05.
 #include <cooperative_groups.h>
 
-#include <cstdlib>
 #include <type_traits>
 
 #include "gemm_simt.cuh"
@@ -20,160 +18,7 @@ namespace gpz {
 
 constexpr int NB = 64;
 
-// ---- (1) diagonal block ---------------------------------------------------------------------------
-template <typename T>
-__global__ void __launch_bounds__(256) potf2_kernel(T* __restrict__ Aall, int M, int k0, int nb, int* __restrict__ info) {
-  __shared__ T s[NB][NB + 1];
-  T* A = Aall + (int64_t)blockIdx.x * M * M;
-  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-  for (int e = tid; e < nb * nb; e += 256) {
-    const int i = e / nb, j = e % nb;
-    s[i][j] = j <= i ? A[(int64_t)(k0 + i) * M + k0 + j] : T(0);
-  }
-  for (int j = 0; j < nb; ++j) {
-    __syncthreads();
-    const T d = s[j][j];
-    if (!(d > T(0))) {                       // not positive definite (also catches NaN), LAPACK-style info
-      if (tid == 0 && info[blockIdx.x] == 0) info[blockIdx.x] = k0 + j + 1;
-    }
-    const T inv = T(1) / d;
-    for (int i = j + 1 + ty; i < nb; i += 16)
-      for (int k = j + 1 + tx; k <= i; k += 16) s[i][k] -= s[i][j] * s[k][j] * inv;
-    __syncthreads();
-    const T rs = Num<T>::rsqrt(d);
-    if (tid > j && tid < nb) s[tid][j] *= rs;
-    if (tid == j) s[j][j] = Num<T>::sqrt(d);
-  }
-  __syncthreads();
-  for (int e = tid; e < nb * nb; e += 256) {
-    const int i = e / nb, j = e % nb;
-    A[(int64_t)(k0 + i) * M + k0 + j] = s[i][j];     // upper part of the block written as 0
-  }
-}
-
-// ---- (2) panel solve:  X L11^T = A21  ------------------------------------------------------------
-template <typename T> struct PanelRows { static constexpr int R = sizeof(T) == 8 ? 16 : 64; };
-template <typename T>
-__global__ void __launch_bounds__(NB) trsm_panel_kernel(T* __restrict__ Aall, int M, int k0, int nb) {
-  constexpr int RB = PanelRows<T>::R;
-  __shared__ T l11[NB][NB + 1];
-  __shared__ T rows[RB][NB + 1];
-  T* A = Aall + (int64_t)blockIdx.y * M * M;
-  const int tid = threadIdx.x;
-  const int r0 = k0 + nb + blockIdx.x * RB;
-  const int nr = min(RB, M - r0);
-  for (int e = tid; e < nb * nb; e += NB) {
-    const int i = e / nb, j = e % nb;
-    l11[i][j] = A[(int64_t)(k0 + i) * M + k0 + j];
-  }
-  for (int e = tid; e < nr * nb; e += NB) {
-    const int i = e / nb, j = e % nb;
-    rows[i][j] = A[(int64_t)(r0 + i) * M + k0 + j];
-  }
-  __syncthreads();
-  if (tid < nr) {
-    for (int c = 0; c < nb; ++c) {
-      T v = rows[tid][c];
-      for (int t = 0; t < c; ++t) v -= rows[tid][t] * l11[c][t];
-      rows[tid][c] = v / l11[c][c];
-    }
-  }
-  __syncthreads();
-  for (int e = tid; e < nr * nb; e += NB) {
-    const int i = e / nb, j = e % nb;
-    A[(int64_t)(r0 + i) * M + k0 + j] = rows[i][j];
-  }
-}
-
-template <typename T> __global__ void zero_upper_kernel(T* __restrict__ A, int M, int64_t total) {
-  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= total) return;
-  const int64_t r = e % ((int64_t)M * M);
-  const int i = (int)(r / M), j = (int)(r % M);
-  if (j > i) A[e] = T(0);
-}
-
-template <typename T> int potrf(T* A, int M, int L, int* info, cudaStream_t st) {
-  GPZ_CUDA(cudaMemsetAsync(info, 0, sizeof(int) * L, st));
-  const int64_t sL = (int64_t)M * M;
-  for (int k0 = 0; k0 < M; k0 += NB) {
-    const int nb = min(NB, M - k0);
-    potf2_kernel<T><<<L, 256, 0, st>>>(A, M, k0, nb, info);
-    GPZ_CHECK_LAUNCH();
-    const int rem = M - k0 - nb;
-    if (rem > 0) {
-      trsm_panel_kernel<T><<<dim3((unsigned)cdiv(rem, PanelRows<T>::R), L), NB, 0, st>>>(A, M, k0, nb);
-      GPZ_CHECK_LAUNCH();
-      T* L21 = A + (int64_t)(k0 + nb) * M + k0;
-      T* A22 = A + (int64_t)(k0 + nb) * M + (k0 + nb);
-      int rc = gemm<T>(st, false, true, rem, rem, nb, T(-1), L21, M, sL, L21, M, sL, T(1), A22, M, sL, L, 0, 0, 1);
-      if (rc) return rc;
-    }
-  }
-  const int64_t total = sL * L;
-  zero_upper_kernel<T><<<(unsigned)cdiv(total, 256), 256, 0, st>>>(A, M, total);
-  GPZ_CHECK_LAUNCH();
-  return GPZ_OK;
-}
-
-// ---- triangular inverse ---------------------------------------------------------------------------
-// diagonal blocks: X_ii = L_ii^-1 by forward substitution, one thread per column
-template <typename T>
-__global__ void __launch_bounds__(NB) trtri_diag_kernel(const T* __restrict__ Lall, T* __restrict__ Xall, int M) {
-  // s holds L_ii in its lower triangle (incl. diagonal) and the strictly-lower part of X transposed in its
-  // strictly-upper triangle (x[r][c], r > c, lives at s[c][r]); the diagonal of X lives in xd.
-  __shared__ T s[NB][NB + 1];
-  __shared__ T xd[NB];
-  const T* Lm = Lall + (int64_t)blockIdx.y * M * M;
-  T* X = Xall + (int64_t)blockIdx.y * M * M;
-  const int k0 = blockIdx.x * NB, nb = min(NB, M - k0), tid = threadIdx.x;
-  for (int e = tid; e < nb * nb; e += NB) {
-    const int i = e / nb, j = e % nb;
-    if (j <= i) s[i][j] = Lm[(int64_t)(k0 + i) * M + k0 + j];
-  }
-  __syncthreads();
-  if (tid < nb) {
-    const int c = tid;
-    const T xc = T(1) / s[c][c];
-    xd[c] = xc;
-    for (int r = c + 1; r < nb; ++r) {
-      T v = -s[r][c] * xc;
-      for (int t = c + 1; t < r; ++t) v -= s[r][t] * s[c][t];
-      s[c][r] = v / s[r][r];
-    }
-  }
-  __syncthreads();
-  for (int e = tid; e < nb * nb; e += NB) {
-    const int i = e / nb, j = e % nb;
-    X[(int64_t)(k0 + i) * M + k0 + j] = j < i ? s[j][i] : (j == i ? xd[i] : T(0));
-  }
-}
-
-// X = L^-1 for lower-triangular L (L x M x M).  `tmp` is an L x NB x M scratch panel.
-// Block row i:  X[i, 0:i] = -X_ii * (L[i, 0:i] * X[0:i, 0:i]),  X_ii from trtri_diag_kernel.
-template <typename T> int trtri(const T* Lc, T* X, T* tmp, int M, int L, cudaStream_t st) {
-  const int64_t sL = (int64_t)M * M;
-  GPZ_CUDA(cudaMemsetAsync(X, 0, sizeof(T) * sL * L, st));
-  const int nblk = (int)cdiv(M, NB);
-  trtri_diag_kernel<T><<<dim3(nblk, L), NB, 0, st>>>(Lc, X, M);
-  GPZ_CHECK_LAUNCH();
-  for (int i = 1; i < nblk; ++i) {
-    const int r0 = i * NB, nb = min(NB, M - r0);
-    int rc = gemm<T>(st, false, false, nb, r0, r0, T(-1), Lc + (int64_t)r0 * M, M, sL, X, M, sL, T(0), tmp, M,
-                     (int64_t)NB * M, L, 0, 1, 0);
-    if (rc) return rc;
-    rc = gemm<T>(st, false, false, nb, r0, nb, T(1), X + (int64_t)r0 * M + r0, M, sL, tmp, M, (int64_t)NB * M, T(0),
-                 X + (int64_t)r0 * M, M, sL, L, 1, 0, 0);
-    if (rc) return rc;
-  }
-  return GPZ_OK;
-}
-
-// ---- fused recursive Cholesky + inverse -------------------------------------------------------------
-// (Lc, X = Lc^-1) by divide and conquer: for A = [A11 .; A21 A22]
-//     (L11, X11) = rec(A11);  L21 = A21 X11^T;  A22 -= L21 L21^T;  (L22, X22) = rec(A22);  X21 = -X22 (L21 X11)
-// so all O(M^3) work is GEMMs (4 per internal node) and the only sequential kernel is the 64 x 64 leaf below, which
-// factors AND inverts its block.
+// ---- leaf: Cholesky + inverse of one 64 x 64 diagonal block -----------------------------------------
 // Factor and invert the n x n (n <= 64) diagonal block at (r0, r0) of one factor: W (input, lower), Lm and X (outputs), all with
 // row stride ld.  `a`, `x`: two [NB][NB+1] shared-memory tiles.  256 threads; contains block barriers.
 //
@@ -600,35 +445,6 @@ chol_inv_cluster_kernel(T* __restrict__ Wall, T* __restrict__ Lall, T* __restric
 long long* g_chol_dbg = nullptr;
 extern "C" void gpz_chol_debug_(long long* p) { g_chol_dbg = p; }
 
-template <typename T>
-static int chol_inv_rec(T* W, T* Lc, T* X, T* tmp, int M, int L, int r0, int n, int* info, cudaStream_t st) {
-  const int64_t sL = (int64_t)M * M;
-  if (n <= NB) {
-    constexpr int smem = (int)(2 * NB * (NB + 1) * sizeof(T));
-    GPZ_CUDA(cudaFuncSetAttribute(chol_inv_leaf_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    chol_inv_leaf_kernel<T><<<L, 256, smem, st>>>(W, Lc, X, M, r0, n, info);
-    GPZ_CHECK_LAUNCH();
-    return GPZ_OK;
-  }
-  const int nb = (int)cdiv(n, NB);
-  const int n1 = (nb / 2) * NB, n2 = n - n1;
-  int rc = chol_inv_rec<T>(W, Lc, X, tmp, M, L, r0, n1, info, st);
-  if (rc) return rc;
-  const int64_t o11 = (int64_t)r0 * M + r0, o21 = (int64_t)(r0 + n1) * M + r0, o22 = (int64_t)(r0 + n1) * M + r0 + n1;
-  // L21 = A21 X11^T
-  rc = gemm<T>(st, false, true, n2, n1, n1, T(1), W + o21, M, sL, X + o11, M, sL, T(0), Lc + o21, M, sL, L, 0, 2, 0);
-  if (rc) return rc;
-  // A22 -= L21 L21^T  (lower)
-  rc = gemm<T>(st, false, true, n2, n2, n1, T(-1), Lc + o21, M, sL, Lc + o21, M, sL, T(1), W + o22, M, sL, L, 0, 0, 1);
-  if (rc) return rc;
-  rc = chol_inv_rec<T>(W, Lc, X, tmp, M, L, r0 + n1, n2, info, st);
-  if (rc) return rc;
-  // tmp = L21 X11 ;  X21 = -X22 tmp
-  rc = gemm<T>(st, false, false, n2, n1, n1, T(1), Lc + o21, M, sL, X + o11, M, sL, T(0), tmp, M, sL, L, 0, 1, 0);
-  if (rc) return rc;
-  return gemm<T>(st, false, false, n2, n1, n2, T(-1), X + o22, M, sL, tmp, M, sL, T(0), X + o21, M, sL, L, 1, 0, 0);
-}
-
 // batched (outer = factor, inner = block pair) GEMM on sub-blocks of L x M x M matrices
 template <typename T>
 static int gemm_pairs(cudaStream_t st, int m, int n, int k, T alpha, const T* A, const T* B, T beta, T* D, int M, int L, int npairs,
@@ -652,11 +468,9 @@ template <typename T> int chol_inv(T* W, T* Lc, T* X, T* tmp, int M, int L, int*
   GPZ_CUDA(cudaMemsetAsync(Lc, 0, sizeof(T) * sL * L, st));
   GPZ_CUDA(cudaMemsetAsync(X, 0, sizeof(T) * sL * L, st));
   constexpr int smem = (int)(2 * NB * (NB + 1) * sizeof(T));
-  static int use_cluster = -1;
-  if (use_cluster < 0) { const char* e = getenv("GPZ_CHOL_CLUSTER"); use_cluster = e ? atoi(e) : 1; }
   // one cluster kernel while the chain is latency-bound (M <= 1536); beyond that the O(M^3) trailing updates dominate and
   // the multi-launch path below, whose GEMMs use the whole GPU, is faster (measured: M = 2048 23.8 vs 26.7 ms/step)
-  if (use_cluster && M <= 1536) {
+  if (M <= 1536) {
     constexpr int csmem = (int)(2 * NB * TLD * sizeof(T));
     GPZ_CUDA(cudaFuncSetAttribute(chol_inv_cluster_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, csmem));
     chol_inv_cluster_kernel<T><<<L * CL, 256, csmem, st>>>(W, Lc, X, tmp, M, 0, M, info, g_chol_dbg);
@@ -702,18 +516,17 @@ template <typename T> int chol_inv(T* W, T* Lc, T* X, T* tmp, int M, int L, int*
   return GPZ_OK;
 }
 
-// ---- large M (fp32): the same divide and conquer with the O(M^3) products on the tcgen05 split-TF32 GEMM ---------------
-// For M > 1536 the right-looking sweep above is dominated by its rank-64 trailing updates (each a memory-bound read-modify-write
-// of the whole trailing matrix on the CUDA cores: 29 ms at M = 4096, L = 10).  Here the recursion of chol_inv_rec is cut off at
-// 256 x 256 diagonal blocks (factored + inverted by the CUDA-core recursion) and every product above that size is ONE batched
-// tensor-core GEMM on sub-blocks in place (row stride M): 4 GEMMs per internal node, half of the flops in the top node.
-// The split-TF32 kernel needs the lo plane (x - tf32(x)) of each operand: Wlo / Llo / Xlo / Tlo shadow W / Lc / X / tmp with
-// the same layout; GEMM epilogues write the lo plane of what they produce, leaf blocks get theirs from a small strided pass.
-static int tc_leaf() {            // diagonal blocks up to this size stay on the CUDA-core recursion (GPZ_CHOL_TC_LEAF overrides)
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPZ_CHOL_TC_LEAF"); v = e ? atoi(e) : 256; if (v < 64) v = 64; }
-  return v;
-}
+// ---- large M (fp32): right-looking with 256-wide panels; diagonal blocks on the cluster kernel, everything else on tcgen05 -------
+// The cluster kernel above is bound by its serial chain of 64 x 64 leaves and by CUDA-core tile products, the sweep by its rank-64
+// trailing updates (each a memory-bound read-modify-write of the whole trailing matrix on the CUDA cores: 29 ms at M = 4096, L = 10).
+// Here the cluster kernel only factors and inverts the HYB_NB x HYB_NB diagonal blocks (4 leaves each), and every product that
+// involves more than one such block is one batched tcgen05 split-TF32 GEMM on sub-blocks in place (row stride M):
+//     for each panel k:   (L11, X11) = cluster(W11);   L21 = W21 X11^T;   W22 -= L21 L21^T        (trailing update, lower)
+//     then X = Lc^-1 by recursive doubling over the panels:   X21 = -X22 (L21 X11)
+// 12 GEMM launches at M = 1024.  The split-TF32 kernel needs the lo plane (x - tf32(x)) of each operand: Wlo / Llo / Xlo / Tlo
+// shadow W / Lc / X / tmp with the same layout; GEMM epilogues write the lo plane of what they produce, diagonal blocks get theirs
+// from a small strided pass (lo_block).
+constexpr int HYB_NB = 256;
 
 __global__ void tf32_lo_block_kernel(const float* __restrict__ x, float* __restrict__ lo, int n, int M) {
   // one n x n block (row stride M) per blockIdx.z; blockIdx.y = row, threads over the columns
@@ -729,68 +542,6 @@ static int lo_block(const float* x, float* lo, int n, int M, int L, cudaStream_t
   return GPZ_OK;
 }
 
-static int chol_inv_rec_tc(float* W, float* Lc, float* X, float* tmp, float* Wlo, float* Llo, float* Xlo, float* Tlo, int M, int L,
-                           int r0, int n, int* info, cudaStream_t st) {
-  const int64_t sL = (int64_t)M * M;
-  const int64_t o11 = (int64_t)r0 * M + r0;
-  if (n <= tc_leaf()) {
-    int rc = chol_inv_rec<float>(W, Lc, X, tmp, M, L, r0, n, info, st);
-    if (rc) return rc;
-    rc = lo_block(Lc + o11, Llo + o11, n, M, L, st);
-    if (rc) return rc;
-    return lo_block(X + o11, Xlo + o11, n, M, L, st);
-  }
-  const int nb = (int)cdiv(n, 128);
-  const int n1 = (nb / 2) * 128, n2 = n - n1;
-  int rc = chol_inv_rec_tc(W, Lc, X, tmp, Wlo, Llo, Xlo, Tlo, M, L, r0, n1, info, st);
-  if (rc) return rc;
-  const int64_t o21 = (int64_t)(r0 + n1) * M + r0, o22 = (int64_t)(r0 + n1) * M + r0 + n1;
-  // L21 = A21 X11^T            (B = X11 stored n x k: K-major; op(B) = X11^T is upper triangular)
-  rc = umma_gemm_ex(1, n2, n1, n1, 1.0f, W + o21, Wlo + o21, M, sL, X + o11, Xlo + o11, M, sL, nullptr, Lc + o21, Llo + o21, M, sL, L,
-                    0, 2, 0, 1, 3, nullptr, (void*)st);
-  if (rc) return rc;
-  // A22 -= L21 L21^T  (lower triangle, in place)
-  rc = umma_gemm_ex(1, n2, n2, n1, -1.0f, Lc + o21, Llo + o21, M, sL, Lc + o21, Llo + o21, M, sL, W + o22, W + o22, Wlo + o22, M, sL,
-                    L, 0, 0, 1, 1, 3, nullptr, (void*)st);
-  if (rc) return rc;
-  rc = chol_inv_rec_tc(W, Lc, X, tmp, Wlo, Llo, Xlo, Tlo, M, L, r0 + n1, n2, info, st);
-  if (rc) return rc;
-  // tmp21 = L21 X11  (X11 lower triangular, stored k x n) ;  X21 = -X22 tmp21  (X22 lower triangular)
-  rc = umma_gemm_ex(0, n2, n1, n1, 1.0f, Lc + o21, Llo + o21, M, sL, X + o11, Xlo + o11, M, sL, nullptr, tmp + o21, Tlo + o21, M, sL, L,
-                    0, 1, 0, 1, 3, nullptr, (void*)st);
-  if (rc) return rc;
-  return umma_gemm_ex(0, n2, n1, n2, -1.0f, X + o22, Xlo + o22, M, sL, tmp + o21, Tlo + o21, M, sL, nullptr, X + o21, Xlo + o21, M, sL,
-                      L, 1, 0, 0, 1, 3, nullptr, (void*)st);
-}
-
-// lo_ws: 4 L M M floats (shadow lo planes of W, Lc, X, tmp)
-static int chol_inv_tc(float* W, float* Lc, float* X, float* tmp, float* lo_ws, int M, int L, int* info, cudaStream_t st) {
-  const int64_t sL = (int64_t)M * M, tot = sL * L;
-  GPZ_CUDA(cudaMemsetAsync(info, 0, sizeof(int) * L, st));
-  GPZ_CUDA(cudaMemsetAsync(Lc, 0, sizeof(float) * tot, st));
-  GPZ_CUDA(cudaMemsetAsync(X, 0, sizeof(float) * tot, st));
-  float* Wlo = lo_ws; float* Llo = lo_ws + tot; float* Xlo = lo_ws + 2 * tot; float* Tlo = lo_ws + 3 * tot;
-  // the triangular GEMMs read whole k-blocks of Lc / X, i.e. also entries above the diagonal of a diagonal block's row: those
-  // are zero in Lc / X (memset above) and must be zero in their lo planes too (only the lower blocks are ever written)
-  GPZ_CUDA(cudaMemsetAsync(Llo, 0, sizeof(float) * 2 * tot, st));
-  int rc = gpz_tf32_lo_f32(W, Wlo, tot, (void*)st);
-  if (rc) return rc;
-  return chol_inv_rec_tc(W, Lc, X, tmp, Wlo, Llo, Xlo, Tlo, M, L, 0, M, info, st);
-}
-
-// ---- hybrid: right-looking with 256-wide panels; diagonal blocks on the cluster kernel, everything else on tcgen05 -------------
-// The cluster kernel above is bound by its serial chain of 64 x 64 leaves and by CUDA-core tile products; here it only factors
-// and inverts the nbo x nbo (256) diagonal blocks (4 leaves each), and every product that involves more than one such block is
-// one batched tcgen05 split-TF32 GEMM on sub-blocks in place:
-//     for each panel k:   (L11, X11) = cluster(W11);   L21 = W21 X11^T;   W22 -= L21 L21^T        (trailing update, lower)
-//     then X = Lc^-1 by recursive doubling over the panels:   X21 = -X22 (L21 X11)
-// 12 GEMM launches at M = 1024.  lo planes as in chol_inv_rec_tc.
-static int hyb_nb() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPZ_CHOL_HYB_NB"); v = e ? atoi(e) : 256; if (v < 64) v = 64; v = (v / 64) * 64; }
-  return v;
-}
-
 static int chol_inv_hybrid(float* W, float* Lc, float* X, float* tmp, float* lo_ws, int M, int L, int* info, cudaStream_t st) {
   const int64_t sL = (int64_t)M * M, tot = sL * L;
   float* Wlo = lo_ws; float* Llo = lo_ws + tot; float* Xlo = lo_ws + 2 * tot; float* Tlo = lo_ws + 3 * tot;
@@ -802,9 +553,8 @@ static int chol_inv_hybrid(float* W, float* Lc, float* X, float* tmp, float* lo_
   if (rc) return rc;
   constexpr int csmem = (int)(2 * NB * TLD * sizeof(float));
   GPZ_CUDA(cudaFuncSetAttribute(chol_inv_cluster_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, csmem));
-  const int nbo = hyb_nb();
-  for (int r0 = 0; r0 < M; r0 += nbo) {
-    const int n = min(nbo, M - r0), rem = M - r0 - n;
+  for (int r0 = 0; r0 < M; r0 += HYB_NB) {
+    const int n = min(HYB_NB, M - r0), rem = M - r0 - n;
     const int64_t o11 = (int64_t)r0 * M + r0, o21 = (int64_t)(r0 + n) * M + r0, o22 = (int64_t)(r0 + n) * M + r0 + n;
     chol_inv_cluster_kernel<float><<<L * CL, 256, csmem, st>>>(W, Lc, X, tmp, M, r0, n, info, nullptr);
     GPZ_CHECK_LAUNCH();
@@ -823,7 +573,7 @@ static int chol_inv_hybrid(float* W, float* Lc, float* X, float* tmp, float* lo_
       if (rc) return rc;
     }
   }
-  for (int b = nbo; b < M; b *= 2) {
+  for (int b = HYB_NB; b < M; b *= 2) {
     for (int f0 = 0; f0 + b < M; f0 += 2 * b) {
       const int n1 = b, n2 = min(b, M - f0 - b);
       const int64_t o11 = (int64_t)f0 * M + f0, o21 = (int64_t)(f0 + b) * M + f0, o22 = (int64_t)(f0 + b) * M + f0 + b;
@@ -929,14 +679,6 @@ using namespace gpz;
 #define ST(s) ((cudaStream_t)(s))
 
 #define GPZ_LINALG_IMPL(SUF, T)                                                                                   \
-  extern "C" int gpz_potrf_##SUF(T* A, int M, int L, int* info, void* stream) {                                  \
-    if (M <= 0 || L <= 0) return GPZ_ERR_BADARG;                                                                  \
-    return potrf<T>(A, M, L, info, ST(stream));                                                                  \
-  }                                                                                                               \
-  extern "C" int gpz_trtri_##SUF(const T* Lc, T* X, T* tmp, int M, int L, void* stream) {                        \
-    if (M <= 0 || L <= 0) return GPZ_ERR_BADARG;                                                                  \
-    return trtri<T>(Lc, X, tmp, M, L, ST(stream));                                                               \
-  }                                                                                                               \
   extern "C" int gpz_chol_inv_##SUF(T* W, T* Lc, T* X, T* tmp, int M, int L, int* info, void* stream) {          \
     if (M <= 0 || L <= 0) return GPZ_ERR_BADARG;                                                                  \
     return chol_inv<T>(W, Lc, X, tmp, M, L, info, ST(stream));                                                   \
@@ -987,13 +729,10 @@ using namespace gpz;
 GPZ_LINALG_IMPL(f32, float)
 GPZ_LINALG_IMPL(f64, double)
 
-// fp32 Cholesky + inverse for large M with the O(M^3) products on the tensor cores (see chol_inv_rec_tc); lo_ws: 4 L M M floats.
+// fp32 Cholesky + inverse for large M with the O(M^3) products on the tensor cores (see chol_inv_hybrid); lo_ws: 4 L M M floats.
 // Same outputs and info convention as gpz_chol_inv_f32.  M % 4 == 0.
 extern "C" int gpz_chol_inv_tc_f32(float* W, float* Lc, float* X, float* tmp, float* lo_ws, int M, int L, int* info, void* stream) {
   if (M <= 0 || L <= 0) return GPZ_ERR_BADARG;
   if (M % 4) return GPZ_ERR_UNSUPPORTED;
-  static int mode = -1;                 // GPZ_CHOL_TC_MODE=rec: the divide-and-conquer recursion instead of the panel hybrid
-  if (mode < 0) { const char* e = getenv("GPZ_CHOL_TC_MODE"); mode = (e && e[0] == 'r') ? 1 : 0; }
-  if (mode == 1) return chol_inv_tc(W, Lc, X, tmp, lo_ws, M, L, info, ST(stream));
   return chol_inv_hybrid(W, Lc, X, tmp, lo_ws, M, L, info, ST(stream));
 }

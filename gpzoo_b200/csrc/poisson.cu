@@ -7,12 +7,8 @@
 // and autograd's backward through all of it.  Here nothing of size G x B is ever written: one pass over
 // y (G x B floats, the algorithmic HBM traffic) produces ll and the gradients w.r.t. mean, spread, W, V.
 //
-// Mapping: a CTA owns 128 spots (thread = spot, so y rows are read coalesced) and walks the genes in
-// chunks of 32.  Phase A (thread = spot): zr, log-lik, t = d ll/d zr, accumulates d/dF in registers and
-// parks t in shared memory.  Phase B (lane = gene, warp = quarter of the spots): the gW[g,f] partial
-// sum_n t[g,n] exp(F)[f,n] from shared memory.  Per-CTA gW partials go to a workspace slice and are
-// summed by a second tiny kernel (deterministic, no atomics on the G x F output).
-#include <cstdlib>
+// Dense counts: fp32 with F <= 16 runs the contractions on the tensor cores (poisson_prep4 / kernel4 / post4); fp64 and
+// F > 16 run poisson_kernel2 on the CUDA cores.  Sparse counts run the K7-CSC kernels at the end of the file.
 #include <type_traits>
 
 #include "common.cuh"
@@ -20,7 +16,6 @@
 
 namespace gpz {
 
-constexpr int PZ_SPOTS = 128;
 constexpr int PZ_GCH = 32;
 
 template <typename T> struct PoissonArgs {
@@ -58,177 +53,11 @@ template <int FMAX> __device__ __forceinline__ void load_row(const double* p, do
   }
 }
 
-template <typename T, int FMAX>
-__global__ void __launch_bounds__(PZ_SPOTS, sizeof(T) == 4 ? 3 : 1) poisson_kernel(const PoissonArgs<T> a) {
-  extern __shared__ __align__(16) unsigned char pz_smem[];
-  typedef T RowT[PZ_SPOTS + 1];
-  typedef T RowE[FMAX];
-  typedef T RowW[FMAX];
-  typedef T AccW[PZ_GCH][FMAX];
-  RowT* tS = reinterpret_cast<RowT*>(pz_smem);                         // [PZ_GCH][PZ_SPOTS+1]
-  RowE* efS = reinterpret_cast<RowE*>(tS + PZ_GCH);                    // [PZ_SPOTS][FMAX]  (spot-major)
-  RowW* sW = reinterpret_cast<RowW*>(efS + PZ_SPOTS);                  // [PZ_GCH][FMAX]
-  AccW* sAcc = reinterpret_cast<AccW*>(sW + PZ_GCH);                   // [4][PZ_GCH][FMAX]
-  __shared__ double red[32];
-
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int n = blockIdx.x * PZ_SPOTS + tid;
-  const bool active = n < a.B;
-  const bool block_full = (blockIdx.x + 1) * PZ_SPOTS <= a.B;      // uniform: every thread of the CTA has a spot
-  const int64_t col = active ? (a.idx ? a.idx[n] : (int64_t)n) : 0;
-  const T invE = T(1) / T(a.E);
-
-  T mu[FMAX], sd[FMAX], gm[FMAX], gs[FMAX];
-#pragma unroll
-  for (int f = 0; f < FMAX; ++f) {
-    gm[f] = T(0); gs[f] = T(0); mu[f] = T(0); sd[f] = T(0);
-    if (f < a.F && active) {
-      mu[f] = a.mean[(int64_t)f * a.B + n];
-      const T s = a.spread[(int64_t)f * a.B + n];
-      sd[f] = f < a.n_var ? Num<T>::sqrt(s > a.clamp_min ? s : a.clamp_min) : s;
-    }
-  }
-  const T vraw = active ? a.V[col] : T(0);
-  const T spV = active ? softplus(vraw) : T(0);
-  T gVacc = T(0);
-  double ll = 0.0;
-
-  const int g_begin = blockIdx.y * a.genes_per_cta;
-  const int g_end = min(a.G, g_begin + a.genes_per_cta);
-  // software pipeline over groups of 8 genes: the y values of the NEXT group are in flight while the current group is
-  // being processed (the sequence of groups is chunk -> sample e -> group, so with E > 1 a chunk is re-read E times)
-  T ynext[8];
-#pragma unroll
-  for (int u = 0; u < 8; ++u)
-    ynext[u] = (active && g_begin + u < g_end) ? __ldcs(a.y + (int64_t)(g_begin + u) * a.y_ld + col) : T(0);
-  for (int g0 = g_begin; g0 < g_end; g0 += PZ_GCH) {
-    T acc[FMAX];
-#pragma unroll
-    for (int f = 0; f < FMAX; ++f) acc[f] = T(0);
-    __syncthreads();
-    for (int e = tid; e < PZ_GCH * FMAX; e += PZ_SPOTS) {
-      const int gi = e / FMAX, f = e % FMAX;
-      T w = T(0);
-      if (g0 + gi < g_end && f < a.F) {
-        w = a.W[(int64_t)(g0 + gi) * a.F + f];
-        if (a.w_softplus) w = softplus(w);
-      }
-      sW[gi][f] = w;
-    }
-    for (int e = 0; e < a.E; ++e) {
-      T ef[FMAX], pg[FMAX];
-#pragma unroll
-      for (int f = 0; f < FMAX; ++f) {
-        pg[f] = T(0);
-        T v = T(0);
-        if (f < a.F && active) v = Num<T>::exp(fma(a.eps[((int64_t)e * a.F + f) * a.B + n], sd[f], mu[f]));
-        ef[f] = v;
-      }
-      __syncthreads();               // previous phase B finished with tS / efS; sW visible
-#pragma unroll
-      for (int f = 0; f < FMAX; ++f) efS[tid][f] = ef[f];
-      // ---- phase A: thread = spot ----
-      T llc = T(0);
-#pragma unroll 1
-      for (int gb = 0; gb < PZ_GCH; gb += 8) {
-        T yv[8];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) yv[u] = ynext[u];
-        {
-          // first gene of the group after this one
-          int gn = g0 + gb + 8;
-          if (gb + 8 == PZ_GCH) gn = (e + 1 < a.E) ? g0 : g0 + PZ_GCH;
-#pragma unroll
-          for (int u = 0; u < 8; ++u)
-            ynext[u] = (active && gn + u < g_end) ? __ldcs(a.y + (int64_t)(gn + u) * a.y_ld + col) : T(0);
-        }
-        // per-gene body; GUARD=false is the interior case (all 128 spots and all 32 genes of the chunk valid): no branches
-        auto body = [&](auto guard, int u) {
-          constexpr bool GUARD = decltype(guard)::value;
-          const int gi = gb + u;
-          T t = T(0);
-          if (!GUARD || (active && g0 + gi < g_end)) {
-            const T y = yv[u];
-            T wrow[FMAX];
-            load_row<FMAX>(&sW[gi][0], wrow);
-            T zr = T(0);
-#pragma unroll
-            for (int f = 0; f < FMAX; ++f) zr = fma(wrow[f], ef[f], zr);
-            const T r = spV * zr;
-            const T ylog = y * fast_log(r);
-            T lp = (y == T(0) ? T(0) : ylog) - r;
-            if (a.with_lgamma && y > T(1.5)) lp -= Num<T>::lgamma(y + T(1));   // lgamma(1) = lgamma(2) = 0
-            llc += lp;
-            t = (fast_div(y, zr) - spV) * invE;
-            gVacc += y - r;
-#pragma unroll
-            for (int f = 0; f < FMAX; ++f) pg[f] = fma(wrow[f], t, pg[f]);
-          }
-          tS[gi][tid] = t;
-        };
-        if (block_full && g0 + PZ_GCH <= g_end) {
-#pragma unroll
-          for (int u = 0; u < 8; ++u) body(std::false_type{}, u);
-        } else {
-#pragma unroll
-          for (int u = 0; u < 8; ++u) body(std::true_type{}, u);
-        }
-      }
-      ll += (double)(llc * invE);
-#pragma unroll
-      for (int f = 0; f < FMAX; ++f) {
-        if (f < a.F && active) {
-          const T gF = ef[f] * pg[f];
-          gm[f] += gF;
-          gs[f] = fma(gF, a.eps[((int64_t)e * a.F + f) * a.B + n], gs[f]);
-        }
-      }
-      __syncthreads();
-      // ---- phase B: lane = gene, warp = quarter of the spots ----
-      const int nb = warp * 32;
-#pragma unroll 4
-      for (int k = 0; k < 32; ++k) {
-        const T t = tS[lane][nb + k];
-        T erow[FMAX];
-        load_row<FMAX>(&efS[nb + k][0], erow);
-#pragma unroll
-        for (int f = 0; f < FMAX; ++f) acc[f] = fma(t, erow[f], acc[f]);
-      }
-    }
-#pragma unroll
-    for (int f = 0; f < FMAX; ++f) sAcc[warp][lane][f] = acc[f];
-    __syncthreads();
-    for (int e = tid; e < PZ_GCH * a.F; e += PZ_SPOTS) {
-      const int gi = e / a.F, f = e % a.F;
-      if (g0 + gi < g_end)
-        a.gW_part[((int64_t)blockIdx.x * a.G + g0 + gi) * a.F + f] =
-            sAcc[0][gi][f] + sAcc[1][gi][f] + sAcc[2][gi][f] + sAcc[3][gi][f];
-    }
-  }
-
-  if (active) {
-    const T gv = softplus_grad(vraw) * gVacc * invE / spV;
-    if (a.atomic_out) atomicAdd(a.gV + n, gv); else a.gV[n] = gv;
-#pragma unroll
-    for (int f = 0; f < FMAX; ++f) {
-      if (f < a.F) {
-        T gsp = gs[f];
-        if (f < a.n_var) {                        // spread is a variance: d sd/d var = 1/(2 sd) where not clamped
-          const T s = a.spread[(int64_t)f * a.B + n];
-          gsp = s >= a.clamp_min ? gsp / (T(2) * sd[f]) : T(0);
-        }
-        const int64_t o = (int64_t)f * a.B + n;
-        if (a.atomic_out) { atomicAdd(a.gmean + o, gm[f]); atomicAdd(a.gspread + o, gsp); }
-        else { a.gmean[o] = gm[f]; a.gspread[o] = gsp; }
-      }
-    }
-  }
-  const double tot = block_sum<double>(ll, red);
-  if (tid == 0) a.ll_part[blockIdx.y * gridDim.x + blockIdx.x] = tot;
-}
-
-// ---- v2: two spots per thread (256 spots per CTA), sample loop outermost ---------------------------------------------
-// Same two-phase scheme, restructured for instruction count and occupancy (the kernel is FMA-issue bound, not HBM bound):
+// ---- poisson_kernel2 (fp64, fp32 with F > 16): two spots per thread (256 spots per CTA), sample loop outermost ----------------
+// A CTA walks its gene range in chunks of 32.  Phase A (thread = two spots, so y rows are read coalesced): rate, log-lik,
+// t = d ll / d zr, d/dF accumulated in registers, t parked in shared memory.  Phase B (lane = gene, warp = a quarter of the spots):
+// the gW[g, f] partial sum_n t[g, n] exp(F)[f, n] from shared memory.  Per-CTA gW partials go to a workspace slice and are summed
+// by poisson_gw_reduce_kernel (deterministic, no atomics on the G x F output).  The kernel is FMA-issue bound, not HBM bound:
 // each softplus(W) row fetched from shared memory serves two spots; per-thread state is only exp(F) and the d/dF
 // accumulator of the current sample (the E samples are an outer loop; y is re-read per sample, from L2 when it fits).
 constexpr int P2_THREADS = 128, P2_SPOTS = 256;
@@ -421,269 +250,9 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
   if (tid == 0) a.ll_part[blockIdx.y * gridDim.x + blockIdx.x] = tot;
 }
 
-// ---- v3 (fp32): the v2 scheme on packed fp32x2 FMAs -------------------------------------------------------------------------
-// The kernel is bound by instruction issue, not by HBM (v2: 113 instructions per (gene, spot) element, 232 M warp instructions
-// per launch at config 2).  Blackwell issues one 3-register FFMA per two cycles and scheduler, but FFMA2 (fma.rn.f32x2) does
-// two fp32 FMAs per instruction, so the three F-long contractions per element (rate, d/dF, d/dW) run on pairs of factors:
-// F = 10 -> 5 FFMA2 each, no padding to 12.  On top of that
-//   * ef' = softplus(V_n) exp(F) is formed once per spot, so the rate is the contraction itself and t' = (y / r - 1) / E;
-//   * sum_g r (for the log-likelihood and for d/dV) is sum_f ef'_f * (sum_g w_gf): one short contraction per 32-gene chunk
-//     instead of two adds per element;
-//   * log(y!) comes from a 64-entry table for integer counts (anything else takes the exact lgamma).
-// Same outputs, workspace layout and grid as v2.
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-  unsigned long long ra = *reinterpret_cast<unsigned long long*>(&a), rb = *reinterpret_cast<unsigned long long*>(&b),
-                     rc = *reinterpret_cast<unsigned long long*>(&c), rd;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(rd) : "l"(ra), "l"(rb), "l"(rc));
-  return *reinterpret_cast<float2*>(&rd);
-}
-
-template <int FP>       // FP = pairs of factors held per thread (F <= 2 FP)
-__global__ void __launch_bounds__(P2_THREADS, 4) poisson_kernel3(const PoissonArgs<float> a) {
-  constexpr int FPP = (FP + 1) & ~1;      // pairs per shared-memory row, padded to 16-byte multiples
-  extern __shared__ __align__(16) unsigned char pz_smem[];
-  typedef float RowT[P2_SPOTS + 1];
-  typedef float2 RowP[FPP];
-  RowT* tS = reinterpret_cast<RowT*>(pz_smem);                                           // [PZ_GCH][P2_SPOTS+1]  t' = (y/r - 1)/E
-  RowP* efS = reinterpret_cast<RowP*>(pz_smem + ((sizeof(float) * PZ_GCH * (P2_SPOTS + 1) + 15) / 16) * 16);   // [P2_SPOTS][FPP]
-  RowP* sW = efS + P2_SPOTS;                                                             // [PZ_GCH][FPP]
-  RowP* sAcc = sW + PZ_GCH;                                                              // [4 * PZ_GCH][FPP]
-  float2* sWsum = reinterpret_cast<float2*>(sAcc + 4 * PZ_GCH);                          // [FPP]  sum over the chunk's genes
-  __shared__ double red[32];
-  __shared__ float lfact[64];                   // log(y!) for integer counts y < 64
-
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid < 64) lfact[tid] = lgammaf((float)(tid + 1));
-  const int n0 = blockIdx.x * P2_SPOTS;
-  int nn[2]; bool act[2]; int64_t col[2]; float spV[2], vraw[2], ysum[2], rsum[2];
-#pragma unroll
-  for (int s2 = 0; s2 < 2; ++s2) {
-    nn[s2] = n0 + s2 * P2_THREADS + tid;
-    act[s2] = nn[s2] < a.B;
-    col[s2] = act[s2] ? (a.idx ? a.idx[nn[s2]] : (int64_t)nn[s2]) : 0;
-    vraw[s2] = act[s2] ? a.V[col[s2]] : 0.f;
-    spV[s2] = act[s2] ? softplus(vraw[s2]) : 0.f;
-    ysum[s2] = 0.f; rsum[s2] = 0.f;
-  }
-  const bool block_full = n0 + P2_SPOTS <= a.B;
-  const float invE = 1.f / (float)a.E;
-  const int g_begin = blockIdx.y * a.genes_per_cta;
-  const int g_end = min(a.G, g_begin + a.genes_per_cta);
-  double ll = 0.0;
-  constexpr float LN2 = 0.69314718055994530942f;
-
-  float ynext[PZ_GRP][2];
-  auto prefetch = [&](int gfirst) {
-#pragma unroll
-    for (int u = 0; u < PZ_GRP; ++u)
-#pragma unroll
-      for (int s2 = 0; s2 < 2; ++s2)
-        ynext[u][s2] = (act[s2] && gfirst + u < g_end) ? __ldcs(a.y + (int64_t)(gfirst + u) * a.y_ld + col[s2]) : 0.f;
-  };
-  prefetch(g_begin);
-
-  for (int e = 0; e < a.E; ++e) {
-    float2 ef[2][FP], pg[2][FP];
-#pragma unroll
-    for (int s2 = 0; s2 < 2; ++s2)
-#pragma unroll
-      for (int fp = 0; fp < FP; ++fp) {
-        pg[s2][fp] = make_float2(0.f, 0.f);
-        float v[2] = {0.f, 0.f};
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int f = 2 * fp + h;
-          if (f < a.F && act[s2]) {
-            const int64_t o = (int64_t)f * a.B + nn[s2];
-            const float sp = a.spread[o];
-            const float sd = f < a.n_var ? sqrtf(sp > a.clamp_min ? sp : a.clamp_min) : sp;
-            v[h] = spV[s2] * expf(fmaf(a.eps[((int64_t)e * a.F + f) * a.B + nn[s2]], sd, a.mean[o]));
-          }
-        }
-        ef[s2][fp] = make_float2(v[0], v[1]);
-      }
-    __syncthreads();                               // phase B of the previous sample finished with efS
-#pragma unroll
-    for (int s2 = 0; s2 < 2; ++s2) {
-#pragma unroll
-      for (int fp = 0; fp < FP; ++fp) efS[s2 * P2_THREADS + tid][fp] = ef[s2][fp];
-      if (FPP > FP) efS[s2 * P2_THREADS + tid][FPP - 1] = make_float2(0.f, 0.f);
-    }
-
-    for (int g0 = g_begin; g0 < g_end; g0 += PZ_GCH) {
-      __syncthreads();                             // previous chunk's phase B / flush finished with sW, tS, sAcc
-      for (int i = tid; i < PZ_GCH * FPP; i += P2_THREADS) {
-        const int gi = i / FPP, fp = i % FPP;
-        float w[2] = {0.f, 0.f};
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int f = 2 * fp + h;
-          if (g0 + gi < g_end && f < a.F) {
-            w[h] = a.W[(int64_t)(g0 + gi) * a.F + f];
-            if (a.w_softplus) w[h] = softplus(w[h]);
-          }
-        }
-        sW[gi][fp] = make_float2(w[0], w[1]);
-      }
-      __syncthreads();
-      if (tid < FPP) {                             // column sums of the chunk's loadings
-        float2 sacc = make_float2(0.f, 0.f);
-        for (int gi = 0; gi < PZ_GCH; ++gi) { const float2 w = sW[gi][tid]; sacc.x += w.x; sacc.y += w.y; }
-        sWsum[tid] = sacc;
-      }
-      // ---- phase A: thread = two spots ----
-      float llc = 0.f;
-#pragma unroll 1
-      for (int gb = 0; gb < PZ_GCH; gb += PZ_GRP) {
-        float yv[PZ_GRP][2];
-#pragma unroll
-        for (int u = 0; u < PZ_GRP; ++u) { yv[u][0] = ynext[u][0]; yv[u][1] = ynext[u][1]; }
-        {
-          int gn = g0 + gb + PZ_GRP;               // first gene of the next group in (sample, chunk, group) order
-          if (gb + PZ_GRP == PZ_GCH && g0 + PZ_GCH >= g_end) gn = (e + 1 < a.E) ? g_begin : g_end;
-          prefetch(gn);
-        }
-        auto body = [&](auto guard, int u) {
-          constexpr bool GUARD = decltype(guard)::value;
-          const int gi = gb + u;
-          float2 wrow[FPP];
-#pragma unroll
-          for (int i = 0; i < FPP / 2; ++i) {
-            const float4 v = reinterpret_cast<const float4*>(&sW[gi][0])[i];
-            wrow[2 * i] = make_float2(v.x, v.y); wrow[2 * i + 1] = make_float2(v.z, v.w);
-          }
-#pragma unroll
-          for (int s2 = 0; s2 < 2; ++s2) {
-            float t = 0.f;
-            if (!GUARD || (act[s2] && g0 + gi < g_end)) {
-              const float y = yv[u][s2];
-              float2 z = make_float2(0.f, 0.f);
-#pragma unroll
-              for (int fp = 0; fp < FP; ++fp) z = ffma2(wrow[fp], ef[s2][fp], z);
-              const float r = z.x + z.y;                                  // rate (softplus(V) is inside ef)
-              const float ylog = (y * LN2) * __log2f(r);
-              float lp = y == 0.f ? 0.f : ylog;
-              if (a.with_lgamma) {
-                const int yi = (int)y;
-                lp -= (yi >= 0 && yi < 64 && (float)yi == y) ? lfact[yi] : lgammaf(y + 1.f);
-              }
-              llc += lp;
-              ysum[s2] += y;
-              t = fmaf(y * invE, __frcp_rn(r), -invE);                    // (y / r - 1) / E
-              const float2 t2 = make_float2(t, t);
-#pragma unroll
-              for (int fp = 0; fp < FP; ++fp) pg[s2][fp] = ffma2(wrow[fp], t2, pg[s2][fp]);
-            }
-            tS[gi][s2 * P2_THREADS + tid] = t;
-          }
-        };
-        if (block_full && g0 + PZ_GCH <= g_end) {
-#pragma unroll
-          for (int u = 0; u < PZ_GRP; ++u) body(std::false_type{}, u);
-        } else {
-#pragma unroll 1
-          for (int u = 0; u < PZ_GRP; ++u) body(std::true_type{}, u);
-        }
-      }
-      __syncthreads();
-      // sum over the chunk's genes of the rate, per spot: sum_f ef'_f * Wsum_f
-#pragma unroll
-      for (int s2 = 0; s2 < 2; ++s2) {
-        float2 z = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int fp = 0; fp < FP; ++fp) z = ffma2(sWsum[fp], ef[s2][fp], z);
-        rsum[s2] += z.x + z.y;
-        llc -= act[s2] ? (z.x + z.y) : 0.f;
-      }
-      ll += (double)(llc * invE);
-      // ---- phase B: lane = gene, warp = a quarter (64) of the spots ----
-      float2 acc[FP];
-#pragma unroll
-      for (int fp = 0; fp < FP; ++fp) acc[fp] = make_float2(0.f, 0.f);
-      const int nb = warp * 64;
-#pragma unroll 4
-      for (int k = 0; k < 64; ++k) {
-        const float t = tS[lane][nb + k];
-        const float2 t2 = make_float2(t, t);
-        float2 erow[FPP];
-#pragma unroll
-        for (int i = 0; i < FPP / 2; ++i) {
-          const float4 v = reinterpret_cast<const float4*>(&efS[nb + k][0])[i];
-          erow[2 * i] = make_float2(v.x, v.y); erow[2 * i + 1] = make_float2(v.z, v.w);
-        }
-#pragma unroll
-        for (int fp = 0; fp < FP; ++fp) acc[fp] = ffma2(t2, erow[fp], acc[fp]);
-      }
-#pragma unroll
-      for (int fp = 0; fp < FP; ++fp) sAcc[warp * PZ_GCH + lane][fp] = acc[fp];
-      __syncthreads();
-      for (int i = tid; i < PZ_GCH * a.F; i += P2_THREADS) {
-        const int gi = i / a.F, f = i % a.F;
-        if (g0 + gi < g_end) {
-          float* dst = a.gW_part + ((int64_t)blockIdx.x * a.G + g0 + gi) * a.F + f;
-          float v = 0.f;
-#pragma unroll
-          for (int w4 = 0; w4 < 4; ++w4) {
-            const float2 pr = sAcc[w4 * PZ_GCH + gi][f >> 1];
-            v += (f & 1) ? pr.y : pr.x;
-          }
-          *dst = e == 0 ? v : *dst + v;
-        }
-      }
-    }
-    // ---- per-sample epilogue: d ll / d mean, d ll / d spread ----
-#pragma unroll
-    for (int s2 = 0; s2 < 2; ++s2) {
-      if (!act[s2]) continue;
-#pragma unroll
-      for (int fp = 0; fp < FP; ++fp) {
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int f = 2 * fp + h;
-          if (f < a.F) {
-            const int64_t o = (int64_t)f * a.B + nn[s2];
-            const float gF = h ? ef[s2][fp].y * pg[s2][fp].y : ef[s2][fp].x * pg[s2][fp].x;
-            float gsp = gF * a.eps[((int64_t)e * a.F + f) * a.B + nn[s2]];
-            if (f < a.n_var) {                       // spread is a variance: d sd / d var = 1 / (2 sd) where not clamped
-              const float sp = a.spread[o];
-              gsp = sp >= a.clamp_min ? gsp / (2.f * sqrtf(sp)) : 0.f;
-            }
-            if (a.atomic_out) { atomicAdd(a.gmean + o, gF); atomicAdd(a.gspread + o, gsp); }
-            else if (e == 0) { a.gmean[o] = gF; a.gspread[o] = gsp; }
-            else { a.gmean[o] += gF; a.gspread[o] += gsp; }
-          }
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int s2 = 0; s2 < 2; ++s2) {
-    if (act[s2]) {
-      // d ll / d V = softplus'(V) / softplus(V) * mean_e sum_g (y - r);  ysum was accumulated once per sample
-      const float gv = softplus_grad(vraw[s2]) * (ysum[s2] - rsum[s2]) * invE / spV[s2];
-      if (a.atomic_out) atomicAdd(a.gV + nn[s2], gv); else a.gV[nn[s2]] = gv;
-    }
-  }
-  const double tot = block_sum<double>(ll, red);
-  if (tid == 0) a.ll_part[blockIdx.y * gridDim.x + blockIdx.x] = tot;
-}
-
-template <int FP> constexpr size_t poisson_smem3() {
-  constexpr int FPP = (FP + 1) & ~1;
-  return ((sizeof(float) * PZ_GCH * (P2_SPOTS + 1) + 15) / 16) * 16 + sizeof(float2) * FPP * (P2_SPOTS + PZ_GCH + 4 * PZ_GCH + 1);
-}
-template <int FP> int poisson_launch3(const PoissonArgs<float>& a, dim3 grid, cudaStream_t st) {
-  constexpr size_t smem = poisson_smem3<FP>();
-  GPZ_CUDA(cudaFuncSetAttribute(poisson_kernel3<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  poisson_kernel3<FP><<<grid, P2_THREADS, smem, st>>>(a);
-  GPZ_CHECK_LAUNCH();
-  return GPZ_OK;
-}
-
-
 // ---- v4 (fp32, F <= 16): the three F-long contractions on the tensor cores ------------------------------------------------
-// v2 / v3 are bound by instruction issue (3.3 warp instructions per (gene, spot) element, 36 of the 105 thread instructions being
-// the FMAs of the contractions); HBM sits at 12 %.  Here the contractions are warp-level MMAs (mma.sync m16n8k16, bf16 operands,
+// poisson_kernel2 is bound by instruction issue (3.3 warp instructions per (gene, spot) element, 36 of the 105 thread instructions
+// being the FMAs of the contractions); HBM sits at 12 %.  Here the contractions are warp-level MMAs (mma.sync m16n8k16, bf16 operands,
 // fp32 accumulation) chained in registers the way a fused attention kernel chains QK^T -> P -> PV:
 //   C1[n, g] = EF'^T[n, :] Wm[g, :]^T                      rate tile (16 spots x 8 genes), EF' = softplus(V) exp(F)
 //   t'       = (y / C1 - 1) / E,  ll += y log2 C1          element-wise on the accumulator fragment, y read straight into that layout
@@ -696,7 +265,7 @@ template <int FP> int poisson_launch3(const PoissonArgs<float>& a, dim3 grid, cu
 //         planes [E][B][16]; zeroes the D2 accumulator.  Everything that is per gene or per spot is done ONCE here, not once per CTA.
 //   main  grid (256-spot blocks) x (gene ranges).  A warp owns 32 spots (two 16-spot sub-tiles, D2 resident in registers over the
 //         CTA's gene range) and walks the range in 16-gene blocks; D3 is summed over the sub-tiles in registers, over the warps through
-//         shared memory once per 64-gene chunk, and leaves as per-CTA partials (same workspace layout as v2).  D2 leaves by vector
+//         shared memory once per 64-gene chunk, and leaves as per-CTA partials (same workspace layout as kernel2).  D2 leaves by vector
 //         atomics into [E][B][16].  ~0.6 warp instructions per element instead of 3.3.
 //   post  gW = softplus'(W) * sum of the partials; per spot: gF = EF' D2 -> d/dmean, d/dspread, d/dV, and the terms that never needed
 //         the G x B elements: sum_g r = sum_l EF'_l (sum_g Wm_gl), d ll / d V = softplus'(V) / softplus(V) sum_l EF'_l D2_l; the last
@@ -1213,29 +782,14 @@ __global__ void sum_double_kernel(const double* __restrict__ part, int n, double
   if (threadIdx.x == 0) out[0] = s;
 }
 
-template <typename T, int FMAX> constexpr size_t poisson_smem() {
-  return sizeof(T) * (PZ_GCH * (PZ_SPOTS + 1) + FMAX * PZ_SPOTS + PZ_GCH * FMAX + 4 * PZ_GCH * FMAX);
-}
 template <typename T, int FMAX> constexpr size_t poisson_smem2() {
   return ((sizeof(T) * PZ_GCH * (P2_SPOTS + 1) + 15) / 16) * 16 + sizeof(T) * (FMAX * P2_SPOTS + PZ_GCH * FMAX + 4 * PZ_GCH * FMAX);
 }
-static int poisson_version() {          // GPZ_POISSON_V: 1 = thread-per-spot kernel, 2 = two spots per thread, 3 = 2 on packed fp32x2 FMAs (fp32 only; measured equal to 2: both are bound by bookkeeping instructions), 4 (default) = tensor-core contractions (fp32, F <= 16; anything else runs 2)
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("GPZ_POISSON_V"); v = e ? atoi(e) : 4; }
-  return v;
-}
-static bool poisson_use_v4(int F, bool is_f32) { return is_f32 && F <= 16 && poisson_version() >= 4; }
-static bool poisson_v2_forced() { return poisson_version() == 2; }
+static bool poisson_use_v4(int F, bool is_f32) { return is_f32 && F <= 16; }     // tensor-core kernels; anything else runs kernel2
 template <typename T, int FMAX> int poisson_launch(const PoissonArgs<T>& a, dim3 grid, cudaStream_t st) {
-  if (poisson_version() >= 2) {
-    constexpr size_t smem = poisson_smem2<T, FMAX>();
-    GPZ_CUDA(cudaFuncSetAttribute(poisson_kernel2<T, FMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    poisson_kernel2<T, FMAX><<<grid, P2_THREADS, smem, st>>>(a);
-  } else {
-    constexpr size_t smem = poisson_smem<T, FMAX>();
-    GPZ_CUDA(cudaFuncSetAttribute(poisson_kernel<T, FMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    poisson_kernel<T, FMAX><<<grid, PZ_SPOTS, smem, st>>>(a);
-  }
+  constexpr size_t smem = poisson_smem2<T, FMAX>();
+  GPZ_CUDA(cudaFuncSetAttribute(poisson_kernel2<T, FMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  poisson_kernel2<T, FMAX><<<grid, P2_THREADS, smem, st>>>(a);
   GPZ_CHECK_LAUNCH();
   return GPZ_OK;
 }
@@ -1251,7 +805,7 @@ static void poisson_grid(int G, int F, int B, bool is_f32, int* nbx, int* nby, i
     *nby = (int)cdiv(G, *gpc);
     return;
   }
-  *nbx = (int)cdiv(B, poisson_version() >= 2 ? P2_SPOTS : PZ_SPOTS);
+  *nbx = (int)cdiv(B, P2_SPOTS);
   const int chunks = (int)cdiv(G, PZ_GCH);
   int by = 1;
   if (*nbx < 1184) by = (int)min((int64_t)chunks, cdiv(1184, *nbx > 0 ? *nbx : 1));
@@ -1325,20 +879,6 @@ int poisson_fwdbwd(PoissonArgs<T> a, T* gW, double* ll_out, void* ws, size_t ws_
 #undef GPZ_P4_LAUNCH
       GPZ_CHECK_LAUNCH();
       poisson_post4_kernel<<<gw_blocks + spot_blocks, 256, 0, st>>>(a, w, gW, nbx, nby, gw_blocks, spot_blocks, ll_out);
-      GPZ_CHECK_LAUNCH();
-      return GPZ_OK;
-    }
-    if (poisson_version() == 3) {          // fp32: the packed-FMA kernel
-      if (a.F <= 4) rc = poisson_launch3<2>(a, grid, st);
-      else if (a.F <= 10) rc = poisson_launch3<5>(a, grid, st);
-      else if (a.F <= 12) rc = poisson_launch3<6>(a, grid, st);
-      else if (a.F <= 20) rc = poisson_launch3<10>(a, grid, st);
-      else rc = poisson_launch3<16>(a, grid, st);
-      if (rc) return rc;
-      const int64_t GF3 = (int64_t)a.G * a.F;
-      poisson_gw_reduce_kernel<T><<<(unsigned)cdiv(GF3, 256), 256, 0, st>>>(a.gW_part, a.W, gW, GF3, nbx, a.w_softplus);
-      GPZ_CHECK_LAUNCH();
-      sum_double_kernel<<<1, 256, 0, st>>>(a.ll_part, nbx * nby, ll_out);
       GPZ_CHECK_LAUNCH();
       return GPZ_OK;
     }

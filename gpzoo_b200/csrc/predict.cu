@@ -328,20 +328,6 @@ __global__ void __launch_bounds__(256) sym_lo_kernel(float* __restrict__ S, floa
     S_lo[mat + (int64_t)i * M + j] = v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
   }
 }
-// R = tril(R0 - S1 + q gq^T) in place, with its lo plane (zeros above the diagonal)
-__global__ void __launch_bounds__(256) regroup_r_kernel(float* __restrict__ R, float* __restrict__ R_lo, const float* __restrict__ S1,
-                                                         const float* __restrict__ q, const float* __restrict__ gq, int M) {
-  const int i = blockIdx.x, l = blockIdx.y;
-  const int64_t row = ((int64_t)l * M + i) * M;
-  const float qi = q[(int64_t)l * M + i];
-  for (int j = threadIdx.x; j < M; j += blockDim.x) {
-    float v = 0.f;
-    if (j <= i) v = R[row + j] - S1[row + j] + qi * gq[(int64_t)l * M + j];
-    R[row + j] = v;
-    R_lo[row + j] = v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
-  }
-}
-
 static Umma16Args h_args(int bk, int m, int n, int k, const __half* Ah, const __half* Al, int64_t lda, int64_t sA, const float* sa,
                          const __half* Bh, const __half* Bl, int64_t ldb, int64_t sB, const float* sb, int64_t ldd, int64_t sD,
                          int batch, int a_tri, int d_tri, int splitk) {
@@ -396,7 +382,8 @@ static int predict_fwd_h(const __half* Kh, const __half* Kl, const float* sK, co
 static int predict_bwd_h(const __half* Kh, const __half* Kl, const float* sK, const float* Tm, const float* q, const __half* Ah,
                          const __half* Al, const __half* Ch, const __half* Cl, const float* gm, const float* gv, __half* AWh,
                          __half* AWl, __half* gAh, __half* gAl, float* gKzx, float* gLinv, float* gT, float* gq, __half* ws_h,
-                         float* ws_f, const float* Lc, float* ws_m, int M, int N, int L, cudaStream_t st) {
+                         float* ws_f, float* ws_m, int M, int N, int L, cudaStream_t st) {
+  if (ws_m != nullptr && (gT != nullptr || gLinv != nullptr)) return GPZ_ERR_BADARG;
   const int64_t sMM = (int64_t)M * M, sMN = (int64_t)M * N, W = sMM * L, LN = (int64_t)L * N;
   __half* LinvT_h = ws_h + 2 * W; __half* LinvT_l = ws_h + 3 * W;
   __half* T_h = ws_h + 4 * W; __half* T_l = ws_h + 5 * W;
@@ -443,12 +430,9 @@ static int predict_bwd_h(const __half* Kh, const __half* Kl, const float* sK, co
     g6.D = gLinv;
     return umma_gemm16_ex(g6, (void*)st);
   }
-  // Regrouped: ONE reduction over the N spots,  S1 = A diag(2 gv) A^T  (symmetric, lower triangle computed), and the identities
-  //     C = T^T A   =>  gT    = tril(AW C^T)    = tril(S1 T)
-  //     Kzx = Lc A  =>  gLinv = tril(gA Kzx^T)  = tril(((T T^T - I) S1 + q gq^T) Lc^T)       (gq = A gm)
-  // turn the second one into four M x M x M products (tcgen05 split-TF32, ~0.07 ms each at M = 1024) instead of 0.85 ms.
-  float* S1 = ws_m; float* S1_lo = ws_m + W; float* Y = ws_m + 2 * W; float* Y_lo = ws_m + 3 * W; float* R = ws_m + 4 * W;
-  float* R_lo = ws_m + 5 * W; float* T_lo = ws_m + 6 * W; float* Lc_lo = ws_m + 7 * W;
+  // merged backward (csrc/chain.cu takes S1 and gq from here): ONE reduction over the N spots, S1 = A diag(2 gv) A^T (symmetric,
+  // lower triangle computed, then mirrored with its lo plane), instead of the two above
+  float* S1 = ws_m; float* S1_lo = ws_m + W;
   GPZ_CUDA(cudaMemsetAsync(S1, 0, sizeof(float) * W, st));
   Umma16Args g4 = h_args(1, M, M, N, AWh, AWl, N, sMN, sAW, Ah, Al, N, sMN, sA, M, sMM, L, 0, 1, splitk);
   g4.D = S1;
@@ -461,26 +445,7 @@ static int predict_bwd_h(const __half* Kh, const __half* Kl, const float* sK, co
   if (rc) return rc;
   sym_lo_kernel<<<dim3(M, L), 256, 0, st>>>(S1, S1_lo, M);
   GPZ_CHECK_LAUNCH();
-  if (gT == nullptr && gLinv == nullptr) return GPZ_OK;       // the caller (csrc/chain.cu, merged backward) takes S1 and gq from here
-  GPZ_CUDA(cudaMemsetAsync(R, 0, sizeof(float) * W, st));
-  rc = gpz_tf32_lo_f32(Tm, T_lo, W, (void*)st);
-  if (rc) return rc;
-  rc = gpz_tf32_lo_f32(Lc, Lc_lo, W, (void*)st);
-  if (rc) return rc;
-  auto mm = [&](int bk, float alpha, const float* A_, const float* Alo_, const float* B_, const float* Blo_, float* D_, float* Dlo_,
-                int a_tri, int b_tri, int d_tri) {
-    return umma_gemm_ex(bk, M, M, M, alpha, A_, Alo_, M, sMM, B_, Blo_, M, sMM, nullptr, D_, Dlo_, M, sMM, L, a_tri, b_tri, d_tri, 1, 3,
-                        nullptr, (void*)st);
-  };
-  rc = mm(1, 1.0f, Tm, T_lo, Tm, T_lo, Y, Y_lo, 1, 2, 0);            // Y = T T^T  (full; op(B) = T^T from T stored n x k)
-  if (rc) return rc;
-  rc = mm(0, 1.0f, S1, S1_lo, Tm, T_lo, gT, nullptr, 0, 1, 1);       // gT = tril(S1 T)
-  if (rc) return rc;
-  rc = mm(0, 1.0f, Y, Y_lo, S1, S1_lo, R, nullptr, 0, 0, 1);         // R0 = tril(Y S1)   (only the lower part of R is used below)
-  if (rc) return rc;
-  regroup_r_kernel<<<dim3(M, L), 256, 0, st>>>(R, R_lo, S1, q, gq, M);
-  GPZ_CHECK_LAUNCH();
-  return mm(1, 1.0f, R, R_lo, Lc, Lc_lo, gLinv, nullptr, 1, 2, 1);   // gLinv = tril(R Lc^T)
+  return GPZ_OK;
 }
 
 }  // namespace gpz
@@ -529,12 +494,12 @@ extern "C" int gpz_svgp_predict_fwd_h_f32(const void* Kh, const void* Kl, const 
 extern "C" int gpz_svgp_predict_bwd_h_f32(const void* Kh, const void* Kl, const float* sK, const float* T, const float* q,
                                           const void* Ah, const void* Al, const void* Ch, const void* Cl, const float* gm,
                                           const float* gv, void* AWh, void* AWl, void* gAh, void* gAl, float* gKzx, float* gLinv,
-                                          float* gT, float* gq, void* ws_h, float* ws_f, const float* Lc, float* ws_m, int M, int N,
-                                          int L, void* stream) {
+                                          float* gT, float* gq, void* ws_h, float* ws_f, float* ws_m, int M, int N, int L,
+                                          void* stream) {
   if (!gpz_svgp_predict_h_supported(M, N) || L <= 0) return GPZ_ERR_UNSUPPORTED;
   return predict_bwd_h((const __half*)Kh, (const __half*)Kl, sK, T, q, (const __half*)Ah, (const __half*)Al, (const __half*)Ch,
                        (const __half*)Cl, gm, gv, (__half*)AWh, (__half*)AWl, (__half*)gAh, (__half*)gAl, gKzx, gLinv, gT, gq,
-                       (__half*)ws_h, ws_f, Lc, ws_m, M, N, L, (cudaStream_t)stream);
+                       (__half*)ws_h, ws_f, ws_m, M, N, L, (cudaStream_t)stream);
 }
 
 #define GPZ_PREDICT_IMPL(SUF, T)                                                                                      \

@@ -25,7 +25,6 @@
 #include <cuda_fp16.h>
 
 #include <atomic>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "gpzoo_b200.h"
@@ -1069,9 +1068,7 @@ int umma_gemm_ex(int b_kmajor, int m, int n, int k, float alpha, const float* A,
     if (rc) return rc;
     rc = make_map_kmajor(&mBlo, Blo ? Blo : B, n, k, ldb, sB, batch, BN);
   } else {
-    static int use4d = -1;
-    if (use4d < 0) { const char* e = getenv("GPZ_UMMA_MAP4D"); use4d = e ? atoi(e) : 1; }
-    b_map4d = (use4d && n % 32 == 0) ? 1 : 0;
+    b_map4d = n % 32 == 0 ? 1 : 0;
     if (b_map4d) {
       rc = make_map_mnmajor4d(&mB, B, k, n, ldb, sB, batch);
       if (rc == GPZ_OK) rc = make_map_mnmajor4d(&mBlo, Blo ? Blo : B, k, n, ldb, sB, batch);

@@ -28,10 +28,6 @@ USE_TENSOR_CORES = True      # fp32: route large contractions through the tcgen0
 TENSOR_CORE_ARITH = os.environ.get("GPZ_TC_ARITH", "fp16x3")
 # fp32 models: up to this many inducing points the O(M^3) chain runs in fp64 (gp.py `_chain_dtype`); GPZ_CHAIN_FP64_MAX_M=0 turns it off
 CHAIN_FP64_MAX_M = int(os.environ.get("GPZ_CHAIN_FP64_MAX_M", "256"))
-# two-node path only: split-FP16 predict backward with one N-reduction + four M^3 products instead of two N-reductions
-# (csrc/predict.cu).  Off by default: its multiply-by-Lc / multiply-by-Linv round trip costs accuracy on ill-conditioned Kzz
-# (d lengthscale 1.2e-4 instead of 4e-5 at cond 600); the one-node path (SvgpMomentsH) merges the algebra instead.
-REGROUP_PREDICT_BWD = os.environ.get("GPZ_REGROUP", "0") != "0"
 FUSED_CHAIN = os.environ.get("GPZ_FUSED_CHAIN", "1") != "0"
 # chain + predict as one autograd node with the merged backward (SvgpMomentsH); GPZ_FUSED_MOMENTS=0: the two-node path
 FUSED_MOMENTS = os.environ.get("GPZ_FUSED_MOMENTS", "1") != "0"       # csrc/chain.cu instead of the Function-per-op chain
@@ -195,7 +191,6 @@ def gemm(A, B, ta=False, tb=False, alpha=1.0, beta=0.0, out=None, a_tri=0, b_tri
     return out
 
 
-POISSON_NARROW_Y = os.environ.get("GPZ_POISSON_V", "4") == "4"     # integer-typed counts are read as stored (K7 tensor-core kernel only)
 GEMM16_MIN_DIM = 2048        # M x M x M products at least this large go to the split-FP16 kernel
 
 
@@ -687,7 +682,7 @@ class SvgpMomentsH(Function):
         gqp = torch.empty((L, M), dtype=dt, device=dev)
         S = _workspace("moments_bwd_S", (2, L, M, M), dt, dev)              # S1 and its lo plane
         call("svgp_predict_bwd_h", dt, ptr(Kh), ptr(Kl), ptr(sK), ptr(T), ptr(q), ptr(Ah), ptr(Al), ptr(Ch), ptr(Cl), ptr(gm), ptr(gv),
-             ptr(AWh), ptr(AWl), ptr(gAh), ptr(gAl), ptr(gKzx), ptr(None), ptr(None), ptr(gqp), ptr(ws_h), ptr(ws_f), ptr(Lc), ptr(S),
+             ptr(AWh), ptr(AWl), ptr(gAh), ptr(gAl), ptr(gKzx), ptr(None), ptr(None), ptr(gqp), ptr(ws_h), ptr(ws_f), ptr(S),
              c_i(M), c_i(N), c_i(L))
         stt = ws_f[2 * L * N:].view(-1, L)
         _track_amax(stt[_stat_row(4)].unsqueeze(0), stt[_stat_row(3)].unsqueeze(0), ("dL/dA",))
@@ -842,10 +837,8 @@ class PredictH(Function):
     `Kzx` is KernelBuildH's stand-in (it only routes dL/dKzx); (Kh, Kl, sK) are the planes it wrote."""
 
     @staticmethod
-    def forward(ctx, Kxx, Kzx, Linv, T, q, Kh, Kl, sK, Lc=None):
-        """Lc: the Cholesky factor whose inverse `Linv` is (a constant of the backward's regrouping Kzx = Lc A; optional)."""
+    def forward(ctx, Kxx, Kzx, Linv, T, q, Kh, Kl, sK):
         Kxx, Linv, T, q, Kh, Kl, sK = _c(Kxx), _c(Linv), _c(T), _c(q), _c(Kh), _c(Kl), _c(sK)
-        ctx.Lc = _c(Lc.detach()) if (Lc is not None and REGROUP_PREDICT_BWD) else None
         dt = Linv.dtype
         L, M, N = Kh.shape
         dev = Kh.device
@@ -879,14 +872,12 @@ class PredictH(Function):
         gLinv = torch.zeros_like(Linv)
         gT = torch.zeros_like(T)
         gq = torch.empty_like(q)
-        Lc = ctx.Lc
-        ws_m = torch.empty(8 * L * M * M, dtype=dt, device=dev) if Lc is not None else None
         call("svgp_predict_bwd_h", dt, ptr(Kh), ptr(Kl), ptr(sK), ptr(T), ptr(q), ptr(Ah), ptr(Al), ptr(Ch), ptr(Cl), ptr(gm), ptr(gv),
-             ptr(AWh), ptr(AWl), ptr(gAh), ptr(gAl), ptr(gKzx), ptr(gLinv), ptr(gT), ptr(gq), ptr(ws_h), ptr(ws_f), ptr(Lc), ptr(ws_m),
+             ptr(AWh), ptr(AWl), ptr(gAh), ptr(gAl), ptr(gKzx), ptr(gLinv), ptr(gT), ptr(gq), ptr(ws_h), ptr(ws_f), ptr(None),
              c_i(M), c_i(N), c_i(L))
         st = ws_f[2 * L * N:].view(-1, L)
         _track_amax(st[_stat_row(4)].unsqueeze(0), st[_stat_row(3)].unsqueeze(0), ("dL/dA",))   # max |gA| vs its scale
-        return gv, gKzx, gLinv, gT, gq, None, None, None, None
+        return gv, gKzx, gLinv, gT, gq, None, None, None
 
 
 def umma_gemm(A, B, b_kmajor, Alo=None, Blo=None, Cin=None, alpha=1.0, want_lo=False, a_tri=0, b_tri=0, d_tri=0, splitk=1,
@@ -1090,7 +1081,7 @@ class PoissonLL(Function):
             return ll.to(dt).reshape(())
         # y: the reference passes floats; integer counts (uint8 / int16 / int32) are read as stored by the fp32 tensor-core kernel
         # (F <= 16), any other combination is converted on the device
-        y_kind = PoissonLL.Y_KINDS.get(y.dtype, 0) if (dt == torch.float32 and F <= 16 and POISSON_NARROW_Y) else 0
+        y_kind = PoissonLL.Y_KINDS.get(y.dtype, 0) if (dt == torch.float32 and F <= 16) else 0
         if y_kind == 0 and y.dtype != dt:
             y = y.to(dt)
         y = _c(y)

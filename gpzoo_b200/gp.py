@@ -190,8 +190,7 @@ class _SparseGPBase(nn.Module):
             Kzx, Kh, Kl, sK = Kzx
             if Kh.shape[0] != L:
                 Kzx, Kh, Kl, sK = Kzx.expand(L, -1, -1), Kh.expand(L, -1, -1), Kl.expand(L, -1, -1), sK.expand(L)
-            Lc_true = getattr(self, "_true_Lc", None) if getattr(self, "_true_Lc", None) is not None else Lc
-            mean, var = F.PredictH.apply(Kxx, Kzx, Linv, T, q, Kh, Kl, sK, Lc_true.to(dt))
+            mean, var = F.PredictH.apply(Kxx, Kzx, Linv, T, q, Kh, Kl, sK)
             return dict(out, mean=mean, var=var)
         Kzx_lo = None
         if want_lo:
@@ -308,8 +307,7 @@ class WSVGP(_SparseGPBase):
         Lu_raw = _as3(self.Lu)
         L = max(Kzz.shape[0], mu.shape[0], Lu_raw.shape[0])
         ex = lambda t: t if t.shape[0] == L else t.expand(L, *t.shape[1:])
-        Lc, Linv = F.CholeskyInverse.apply(Kzz)
-        self._true_Lc = ex(Lc.detach())                                  # (the predictive backward regroups with Kzx = Lc A)
+        _, Linv = F.CholeskyInverse.apply(Kzz)
         Lu = ex(F.LowerCholesky.apply(Lu_raw.to(Kzz.dtype)))
         eye = torch.eye(Kzz.shape[-1], dtype=Kzz.dtype, device=Kzz.device).expand(L, -1, -1).contiguous()
         return eye, ex(Linv), Lu, Lu, ex(mu.to(Kzz.dtype)), L          # (Lc := I for the KL, Linv, Lu, T := Lu, q := mu)

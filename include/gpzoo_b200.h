@@ -56,20 +56,14 @@ int gpz_kernel_build_bwd_f64(const double* x1, const double* x2, const double* s
 int gpz_cdist_f32(const float* x1, const float* x2, float* out, int n1, int n2, int D, void* stream);
 int gpz_cdist_f64(const double* x1, const double* x2, double* out, int n1, int n2, int D, void* stream);
 
-/* ---- K2 batched Cholesky: gp.py:213, 360, 55, 270 (torch.linalg.cholesky).  A (L x M x M) is overwritten by
- *      its lower factor (upper triangle zeroed); info[l] = 0 or (1-based) index of the first non-positive pivot. */
-int gpz_potrf_f32(float* A, int M, int L, int* info, void* stream);
-int gpz_potrf_f64(double* A, int M, int L, int* info, void* stream);
-/* X = Lc^-1 (lower).  With it the two triangular solves of gp.py:218 (torch.cholesky_solve) and the solves
- * inside kl_divergence(qU,pU) (torch kl.py) become triangular products.  tmp: L x 64 x M scratch. */
-int gpz_trtri_f32(const float* Lc, float* X, float* tmp, int M, int L, void* stream);
-int gpz_trtri_f64(const double* Lc, double* X, double* tmp, int M, int L, void* stream);
-/* fused recursive Cholesky + inverse (the path the GP modules use): W = copy of Kzz (destroyed), outputs Lc and X = Lc^-1
- * (both lower, upper triangle zero), tmp = L x M x M scratch, info as gpz_potrf.  All O(M^3) work is GEMMs. */
+/* ---- K2 batched Cholesky fused with the triangular inverse: gp.py:213, 360, 55, 270 (torch.linalg.cholesky).  With
+ *      X = Lc^-1 the two triangular solves of gp.py:218 (torch.cholesky_solve) and the solves inside kl_divergence(qU,pU)
+ *      (torch kl.py) become triangular products.  W = copy of Kzz (destroyed), outputs Lc and X = Lc^-1 (both lower, upper
+ *      triangle zero), tmp = L x M x M scratch; info[l] = 0 or (1-based) index of the first non-positive pivot of factor l. */
 int gpz_chol_inv_f32(float* W, float* Lc, float* X, float* tmp, int M, int L, int* info, void* stream);
 int gpz_chol_inv_f64(double* W, double* Lc, double* X, double* tmp, int M, int L, int* info, void* stream);
-/* the same for large M in fp32 (M % 4 == 0; used for M > 1536): divide and conquer whose products above 256 x 256 run on the
- * tcgen05 split-TF32 GEMM in place; lo_ws: 4 L M M floats of scratch (lo planes shadowing W, Lc, X, tmp) */
+/* the same for large M in fp32 (M % 4 == 0): 256-wide panels whose diagonal blocks run on the cluster kernel of gpz_chol_inv and
+ * every larger product on the tcgen05 split-TF32 GEMM in place; lo_ws: 4 L M M floats of scratch (lo planes shadowing W, Lc, X, tmp) */
 int gpz_chol_inv_tc_f32(float* W, float* Lc, float* X, float* tmp, float* lo_ws, int M, int L, int* info, void* stream);
 /* strided-batched D = alpha op(A) op(B) + beta D with triangular-structure skipping (see csrc/gemm_simt.cuh):
  * S = Lu Lu^T (gp.py:221), W@(S-Kzz) (utilities.py:395) and the O(M^3) backward products are built from it. */
@@ -266,11 +260,10 @@ int gpz_svgp_predict_fwd_h_f32(const void* Kh, const void* Kl, const float* sK, 
 int gpz_svgp_predict_bwd_h_f32(const void* Kh, const void* Kl, const float* sK, const float* T, const float* q, const void* Ah,
                                const void* Al, const void* Ch, const void* Cl, const float* gm, const float* gv, void* AWh, void* AWl,
                                void* gAh, void* gAl, float* gKzx, float* gLinv, float* gT, float* gq, void* ws_h, float* ws_f,
-                               const float* Lc, float* ws_m, int M, int N, int L, void* stream);
-/*      Lc (the Cholesky factor whose inverse Linv is) + ws_m (8 L M M floats; may be NULL): with ws_m given the backward runs ONE
- *      reduction over the N spots, S1 = A diag(2 gv) A^T, and gets gT = tril(S1 T) and gLinv = tril(((T T^T - I) S1 + q gq^T) Lc^T)
- *      from four M x M x M products (C = T^T A and Kzx = Lc A); without them it runs the two reductions gT = tril(AW C^T),
- *      gLinv = tril(gA Kzx^T). */
+                               float* ws_m, int M, int N, int L, void* stream);
+/*      ws_m NULL: the backward runs the two reductions over the N spots gT = tril(AW C^T), gLinv = tril(gA Kzx^T).
+ *      ws_m = [S1 | S1_lo] (2 L M M floats), which requires gT = gLinv = NULL (GPZ_ERR_BADARG otherwise): it runs ONE reduction,
+ *      S1 = A diag(2 gv) A^T, for gpz_svgp_chain_bwd_s1_f32. */
 
 /* ---- training-step update (SURVEY §8(f) row 1): multi-tensor Adam in one launch (torch.optim.Adam without weight decay /
  *      amsgrad; utilities.py:621 optimizer.step()) with the reference's post-step clamp W.clamp_(min=0) (utilities.py:623) fused in

@@ -135,7 +135,7 @@ def test_package_exports_and_abi():
     if not os.path.exists(_cabi.LIB_PATH):
         build.build()
     lib = _cabi.lib()
-    assert lib.gpz_abi_version() == 3
+    assert lib.gpz_abi_version() == 4
     syms = _cabi.exported_symbols()
     for s in ("gpz_poisson_csc_workspace_bytes_f32", "gpz_poisson_csc_workspace_bytes_f64", "gpz_poisson_fwdbwd_csc_f32",
               "gpz_poisson_fwdbwd_csc_f64"):

@@ -1,6 +1,6 @@
-"""K7 alone: the fp32 kernel selected by GPZ_POISSON_V against the fp64 instantiation on the same inputs, plus its time.
-usage: GPZ_POISSON_V=4 python tools/k7_check.py [G F B E with_lgamma use_idx y_kind]   (y_kind 1 / 2 / 3: counts as uint8 / int16 / int32)"""
-import os, sys, torch
+"""K7 alone: the default fp32 call against the fp64 call on the same inputs, plus its time.
+usage: python tools/k7_check.py [G F B E with_lgamma use_idx y_kind]   (y_kind 1 / 2 / 3: counts as uint8 / int16 / int32)"""
+import sys, torch
 sys.path.insert(0, '.')
 from gpzoo_b200 import functional as F
 
@@ -30,7 +30,7 @@ def run(dt):
 ref, gref = run(torch.float64)
 out, gout = run(torch.float32)
 rel = lambda x, r: float((x - r).norm() / r.norm())
-print(f"V={os.environ.get('GPZ_POISSON_V', 'default')} G={G} F={Fn} B={B} E={E} lgamma={lg} idx={use_idx}: ll {float(out):.6f} ref {float(ref):.6f} rel {rel(out, ref):.2e}  "
+print(f"G={G} F={Fn} B={B} E={E} lgamma={lg} idx={use_idx}: ll {float(out):.6f} ref {float(ref):.6f} rel {rel(out, ref):.2e}  "
       + "  ".join(f"d{n} {rel(g, r):.2e}" for n, g, r in zip(("W", "V", "mean", "var"), gout, gref)))
 y32, W32, V32, m32, v32, e32 = (t.float() for t in (y, W, V, mean, var, eps))
 if YDT is not None:
