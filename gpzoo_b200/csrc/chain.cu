@@ -20,8 +20,6 @@
 
 namespace gpz {
 
-__device__ __forceinline__ float tf32_lo_part(float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); }
-
 // forward prep, one 32 x 32 tile per CTA: Linv_lo ; LinvT, LinvT_lo ; LcT, LcT_lo ; Lu = lct(raw), Lu_lo
 __global__ void __launch_bounds__(256) chain_prep_kernel(const float* __restrict__ Linv, const float* __restrict__ Lc,
                                                           const float* __restrict__ raw, float* __restrict__ Linv_lo,

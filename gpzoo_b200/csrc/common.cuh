@@ -26,6 +26,9 @@ namespace gpz {
 
 __host__ __device__ inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// the split-TF32 lo plane of x: x - tf32(x), tf32(x) being x with the 13 low mantissa bits cleared
+__device__ __forceinline__ float tf32_lo_part(float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); }
+
 template <typename T> struct Num;
 template <> struct Num<float> {
   __device__ static float exp(float x) { return expf(x); }

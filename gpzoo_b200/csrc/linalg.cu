@@ -5,9 +5,12 @@
 // Right-looking blocked factorisation, panel width NB: for each panel k the NB x NB diagonal block is factored AND inverted
 // (leaf_body), then the panel L21 = A21 X11^T and the trailing update A22 -= L21 L21^T; X = Lc^-1 follows by recursive
 // doubling, X21 = -X22 (L21 X11).  chol_inv runs it as one cluster kernel per factor (M <= 1536) or as a sweep of GEMM launches;
-// chol_inv_hybrid (fp32, large M) runs 256-wide panels on the cluster kernel and every larger product on tcgen05.
+// chol_inv_hybrid (fp32, large M) runs 256-wide diagonal blocks on the cluster kernel and every larger product on tcgen05, with
+// only the look-ahead (next panel block, next diagonal update) on the caller's stream and the rest of each panel, the rest of the
+// trailing update and the inverse, one block row at a time (X[k,0:k] = -X[k,k] L[k,0:k] X[0:k,0:k]), on a side stream.
 #include <cooperative_groups.h>
 
+#include <mutex>
 #include <type_traits>
 
 #include "gemm_simt.cuh"
@@ -37,22 +40,39 @@ template <typename T> __device__ __forceinline__ T shfl_t(T v, int src) { return
 // Out: column j of L to Ls[lane][j], 1 / L[j][j] to rd[j].
 // No division ever sees a zero numerator (an IEEE division resolves 0 / x through FCHK + a slow-path call, which makes the warp
 // diverge in the middle of the shuffle sequence; the previous leaf lost 25 % on config 2's mostly-zero Kzz to exactly that).
+// Software-pipelined by one column: slot 0 (the next column's entry) is updated first, the next pivot is shuffled out and its
+// square root and reciprocal are issued before the other 30 updates, so their latency hides under those shuffles instead of
+// starting the next column's dependent chain.
+template <typename T>
+__device__ __forceinline__ void pivot_sqrt_recip(T d, T& s, T& r) {
+  if constexpr (std::is_same<T, float>::value) {
+    // one MUFU rsqrt and a Newton step (~1 ulp) instead of sqrt followed by an IEEE division (fp64 keeps the exact path)
+    const float y = rsqrtf(d);
+    r = y * fmaf(-0.5f * d * y, y, 1.5f);
+    s = d * r;
+  } else {
+    s = Num<T>::sqrt(d);
+    r = T(1) / s;
+  }
+}
 template <typename T, int LDS>
 __device__ __forceinline__ void warp_chol32(T (&a)[32], T* __restrict__ Ls, T* __restrict__ rd, int lane, int* __restrict__ info_l,
                                             int base) {
   int bad = 0;                                       // first non-positive pivot (uniform)
+  T d = shfl_t(a[0], 0), s, r;                       // pivot of the current column, uniform over the warp
+  pivot_sqrt_recip(d, s, r);
   auto column = [&](int j, auto nslots) {
     constexpr int NS = decltype(nslots)::value;
-    const T d = shfl_t(a[0], j);                     // pivot, uniform over the warp
     bad = (bad == 0 && !(d > T(0))) ? base + j + 1 : bad;           // not positive definite (also catches NaN)
-    const T s = Num<T>::sqrt(d);
-    const T r = T(1) / s;
     const T lij = lane > j ? a[0] * r : (lane == j ? s : T(0));     // L[lane][j]
     Ls[lane * LDS + j] = lij;
     if (lane == 0) rd[j] = r;
     const T lsub = lane > j ? lij : T(0);
+    a[0] = fma(-lsub, shfl_t(lij, (j + 1) & 31), a[1]);
+    d = shfl_t(a[0], (j + 1) & 31);                  // next pivot (garbage after the last column, never used)
+    pivot_sqrt_recip(d, s, r);
 #pragma unroll
-    for (int k = 1; k < NS; ++k) a[k - 1] = fma(-lsub, shfl_t(lij, (j + k) & 31), a[k]);
+    for (int k = 2; k < NS; ++k) a[k - 1] = fma(-lsub, shfl_t(lij, (j + k) & 31), a[k]);
   };
 #pragma unroll 1
   for (int j = 0; j < 16; ++j) column(j, std::integral_constant<int, 32>{});
@@ -92,9 +112,17 @@ __device__ void leaf_body(T (*a)[NB + 1], T (*x)[NB + 1], const T* __restrict__ 
   long long tc0 = clock64();
   auto mark = [&](int slot) { if (dbg != nullptr && tid == 0) { const long long t = clock64(); dbg[slot] = t - tc0; tc0 = t; } };
   // identity padding beyond n keeps the routine free of size tests; the padding never reaches global memory
-  for (int e = tid; e < NB * NB; e += 256) {
-    const int i = e >> 6, j = e & (NB - 1);
-    a[i][j] = (i < n && j <= i) ? W[(int64_t)(r0 + i) * ld + r0 + j] : ((i == j && i >= n) ? T(1) : T(0));
+  // all 16 loads of a thread are issued before the first shared-memory store (one round trip instead of 16 dependent ones)
+  T w[NB * NB / 256];
+#pragma unroll
+  for (int u = 0; u < NB * NB / 256; ++u) {
+    const int i = (tid >> 6) + 4 * u, j = tid & (NB - 1);
+    w[u] = (i < n && j <= i) ? W[(int64_t)(r0 + i) * ld + r0 + j] : ((i == j && i >= n) ? T(1) : T(0));
+  }
+#pragma unroll
+  for (int u = 0; u < NB * NB / 256; ++u) {
+    const int i = (tid >> 6) + 4 * u, j = tid & (NB - 1);
+    a[i][j] = w[u];
     x[i][j] = T(0);
   }
   __syncthreads();
@@ -170,8 +198,9 @@ __device__ void leaf_body(T (*a)[NB + 1], T (*x)[NB + 1], const T* __restrict__ 
     __syncthreads();
     mark(4);
   }
-  for (int e = tid; e < NB * NB; e += 256) {
-    const int i = e >> 6, j = e & (NB - 1);
+#pragma unroll
+  for (int u = 0; u < NB * NB / 256; ++u) {
+    const int i = (tid >> 6) + 4 * u, j = tid & (NB - 1);
     if (i < n && j < n) {
       Lm[(int64_t)(r0 + i) * ld + r0 + j] = j <= i ? a[i][j] : T(0);
       X[(int64_t)(r0 + i) * ld + r0 + j] = j <= i ? x[i][j] : T(0);
@@ -194,7 +223,7 @@ __global__ void __launch_bounds__(256) chol_inv_leaf_kernel(const T* __restrict_
 // ---- the whole Cholesky + inverse of one factor in ONE kernel: a thread-block cluster of 8 CTAs per factor --------
 // Same right-looking algorithm as chol_inv() below, but the ~60 dependent launches become phases separated by
 // hardware cluster barriers (barrier.cluster, ~0.2 us): leaf on CTA 0 -> panel row blocks over the 8 CTAs -> trailing
-// 64 x 64 tiles over the 8 CTAs; then the doubling inverse tile by tile.  All tile products are 64 x 64 x 64 from
+// 64 x 64 tiles over the 8 CTAs, while the inverse grows one block row per step on the CTAs that do not run the leaf.  All tile products are 64 x 64 x 64 from
 // shared memory; matrices stay in global memory (L2-resident: 3 x 4 MB per factor).
 constexpr int CL = 8;     // CTAs per cluster
 
@@ -337,9 +366,11 @@ __device__ void run_steps(T (*tA)[TLD], T (*tB)[TLD], const int4* __restrict__ s
 template <typename T>
 __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(256)
 chol_inv_cluster_kernel(T* __restrict__ Wall, T* __restrict__ Lall, T* __restrict__ Xall, T* __restrict__ Tall, int M, int blk0,
-                        int nsz, int* __restrict__ info, long long* __restrict__ dbg) {
+                        int nsz, int* __restrict__ info, long long* __restrict__ dbg, float* __restrict__ Xlo_all = nullptr) {
   // factors + inverts the nsz x nsz diagonal block starting at row / column blk0 of every M x M matrix (blk0 = 0, nsz = M: all
-  // of it); block coordinates below are relative to that block, M is the row stride
+  // of it); block coordinates below are relative to that block, M is the row stride.
+  // Xlo_all (fp32 only, the hybrid's diagonal blocks): finally write the tf32 lo plane of the X block and zeros above the diagonal
+  // of the Lc, X and Xlo blocks, so that nothing has to be zeroed or split before or after this launch.
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   extern __shared__ __align__(16) unsigned char cl_smem[];
@@ -363,85 +394,90 @@ chol_inv_cluster_kernel(T* __restrict__ Wall, T* __restrict__ Lall, T* __restric
   if (rank == 0) leaf_body<T>(la, lx, W, Lm, X, (int64_t)M, 0, bsz(0), info + l, blk0, (dbg != nullptr && blockIdx.x == 0) ? dbg + 4 : nullptr);
   cluster.sync();
   t1 = clock64(); t_leaf += t1 - t0; t0 = t1;
-  for (int k = 0; k < nblk - 1; ++k) {
-    const int nrb = nblk - k - 1;                       // row blocks below the diagonal block (>= 1 here)
-    // panel: L21 = W21 X11^T      (A = W[gi][k], B = X[k][k], out = Lc[gi][k])
-    if (threadIdx.x == 0) {
-      int ns = 0;
-      for (int rb = rank; rb < nrb; rb += CL) steps[ns++] = make_int4(k + 1 + rb, k, k, 3);
-      nsteps_s = ns;
-    }
-    __syncthreads();
-    run_steps<T>(tA, tB, steps, nsteps_s, W, X, Lm, false, T(1), T(0), M, nsz);
-    cluster.sync();
-    t1 = clock64(); t_panel += t1 - t0; t0 = t1;
-    // trailing update of the lower triangle: W[gi][gj] -= Lc[gi][k] Lc[gj][k]^T   (in rounds of at most MAX_STEPS tiles).
-    // Tile 0 (the next diagonal block) belongs to CTA 0, which then runs the next leaf; tiles 1.. go round-robin to CTAs 1..7.
+  // The inverse is built one block row at a time, X[k][0:k] = -X[k][k] tmp[k][0:k] with tmp[k][0:k] = Lc[k][0:k] X[0:k][0:k]:
+  // tmp row k+1 needs nothing of leaf k+1, so CTAs 1..7 compute it while CTA 0 runs that leaf, and block row k joins the panel
+  // phase of step k.  Only the last block row is left after the factorisation.
+  // Runs one list of tile-product steps; tile q of the list (nq tiles) with `cost(q)` steps goes to CTA `owner(q)`; `emit(q, t,
+  // flags)` writes the t-th step of tile q.  The per-CTA list is processed in rounds of at most MAX_STEPS steps.
+  auto run_list = [&](int nq, auto owner, auto cost, auto emit, const T* MA, const T* MB, T* MO, bool b_tr, T alpha, T beta) {
     for (int q_start = 0; q_start >= 0;) {
       if (threadIdx.x == 0) {
-        int ns = 0, q = 0, q_next = -1;
-        for (int bi = 0; bi < nrb && q_next < 0; ++bi)
-          for (int bj = 0; bj <= bi; ++bj, ++q) {
-            const int owner = q == 0 ? 0 : 1 + (q - 1) % (CL - 1);
-            if (q < q_start || owner != rank) continue;
-            if (ns == MAX_STEPS) { q_next = q; break; }
-            steps[ns++] = make_int4(k + 1 + bi, k + 1 + bj, k, 3);
-          }
+        int ns = 0, q_next = -1;
+        for (int q = q_start; q < nq; ++q) {
+          if (owner(q) != rank) continue;
+          const int c = cost(q);
+          if (ns + c > MAX_STEPS) { q_next = q; break; }
+          for (int t = 0; t < c; ++t) steps[ns++] = emit(q, t, (t == 0 ? 1 : 0) | (t == c - 1 ? 2 : 0));
+        }
         nsteps_s = ns;
         q_next_s = q_next;
       }
       __syncthreads();
       const int ns = nsteps_s, qn = q_next_s;
-      run_steps<T>(tA, tB, steps, ns, Lm, Lm, W, false, T(-1), T(1), M, nsz);
+      run_steps<T>(tA, tB, steps, ns, MA, MB, MO, b_tr, alpha, beta, M, nsz);
       __syncthreads();
       q_start = qn;
     }
-    if (rank == 0) leaf_body<T>(la, lx, W, Lm, X, (int64_t)M, (k + 1) * NB, bsz(k + 1), info + l, blk0);
+  };
+  // X[k][j] = -X[k][k] tmp[k][j], j < k   (one step per tile; owners from the top rank down, the panel's start at rank 0)
+  auto inverse_row = [&](int k) {
+    run_list(k, [&](int j) { return CL - 1 - j % CL; }, [](int) { return 1; },
+             [&](int j, int, int f) { return make_int4(k, j, k, f); }, X, Tm, X, true, T(-1), T(0));
+  };
+  for (int k = 0; k < nblk - 1; ++k) {
+    const int nrb = nblk - k - 1;                       // row blocks below the diagonal block (>= 1 here)
+    // panel: L21 = W21 X11^T      (A = W[gi][k], B = X[k][k], out = Lc[gi][k]); block row k of the inverse
+    run_list(nrb, [](int rb) { return rb % CL; }, [](int) { return 1; },
+             [&](int rb, int, int f) { return make_int4(k + 1 + rb, k, k, f); }, W, X, Lm, false, T(1), T(0));
+    inverse_row(k);
+    cluster.sync();
+    t1 = clock64(); t_panel += t1 - t0; t0 = t1;
+    // trailing update of the lower triangle: W[gi][gj] -= Lc[gi][k] Lc[gj][k]^T.
+    // Tile 0 (the next diagonal block) belongs to CTA 0, which then runs the next leaf; tiles 1.. go round-robin to CTAs 1..7.
+    run_list(nrb * (nrb + 1) / 2, [](int q) { return q == 0 ? 0 : 1 + (q - 1) % (CL - 1); }, [](int) { return 1; },
+             [&](int q, int, int f) {
+               int bi = 0;
+               while ((bi + 1) * (bi + 2) / 2 <= q) ++bi;
+               return make_int4(k + 1 + bi, k + 1 + q - bi * (bi + 1) / 2, k, f);
+             }, Lm, Lm, W, false, T(-1), T(1));
+    if (rank == 0) {
+      leaf_body<T>(la, lx, W, Lm, X, (int64_t)M, (k + 1) * NB, bsz(k + 1), info + l, blk0);
+    } else {
+      // tmp[k+1][j] = sum_{t=j}^{k} Lc[k+1][t] X[t][j]   (k - j + 1 steps; X rows 0..k are final after the panel phase)
+      run_list(k + 1, [](int j) { return 1 + j % (CL - 1); }, [&](int j) { return k - j + 1; },
+               [&](int j, int t, int f) { return make_int4(k + 1, j, j + t, f); }, Lm, X, Tm, true, T(1), T(0));
+    }
     cluster.sync();
     t1 = clock64(); t_trail += t1 - t0; t0 = t1;
   }
-  // ---- inverse by recursive doubling, tile by tile:  tmp21 = L21 X11 ;  X21 = -X22 tmp21 ----
-  for (int b = 1; b < nblk; b *= 2) {                      // b = blocks per half
-    const int npair = (nblk + 2 * b - 1) / (2 * b);
-    for (int stage = 0; stage < 2; ++stage) {
-      // the per-CTA step list can exceed MAX_STEPS at large M: process it in rounds
-      for (int q_start = 0; q_start >= 0;) {
-        if (threadIdx.x == 0) {
-          int ns = 0, q = 0, q_next = -1;
-          for (int p = 0; p < npair && q_next < 0; ++p) {
-            const int f0 = p * 2 * b;
-            const int n2 = min(b, nblk - f0 - b);
-            if (n2 <= 0) continue;
-            for (int ti = 0; ti < n2 && q_next < 0; ++ti)
-              for (int tj = 0; tj < b; ++tj, ++q) {
-                // owner rotates with (ti + tj): the cost of a tile is b - tj (stage 0) or ti + 1 (stage 1), so a plain
-                // q % CL would hand one CTA all the expensive tiles
-                if (q < q_start || (ti + tj + p) % CL != rank) continue;
-                // stage 0: sum_{tk=tj}^{b-1} L[gi][f0+tk] X[f0+tk][gj];  stage 1: sum_{tk=0}^{ti} X[gi][f0+b+tk] tmp[f0+b+tk][gj]
-                const int t_lo = stage == 0 ? tj : 0, t_hi = stage == 0 ? b - 1 : ti;
-                if (ns + (t_hi - t_lo + 1) > MAX_STEPS) { q_next = q; break; }
-                for (int tk = t_lo; tk <= t_hi; ++tk)
-                  steps[ns++] = make_int4(f0 + b + ti, f0 + tj, stage == 0 ? f0 + tk : f0 + b + tk,
-                                          (tk == t_lo ? 1 : 0) | (tk == t_hi ? 2 : 0));
-              }
+  if (nblk > 1) {
+    inverse_row(nblk - 1);
+    cluster.sync();
+  }
+  if constexpr (std::is_same<T, float>::value) {
+    if (Xlo_all != nullptr) {                              // X is final everywhere after the last cluster barrier
+      float* Xlo = Xlo_all + off;
+      for (int q = rank; q < nblk * nblk; q += CL) {
+        const int bi = q / nblk, bj = q % nblk, nr = bsz(bi), nc = bsz(bj);
+        for (int e = threadIdx.x; e < NB * NB; e += 256) {
+          const int i = e >> 6, j = e & (NB - 1);
+          if (i >= nr || j >= nc) continue;
+          const int64_t o = (int64_t)(bi * NB + i) * M + bj * NB + j;
+          if (bi >= bj) {
+            Xlo[o] = tf32_lo_part(X[o]);
+          } else {
+            Lm[o] = 0.f; X[o] = 0.f; Xlo[o] = 0.f;
           }
-          nsteps_s = ns;
-          q_next_s = q_next;
         }
-        __syncthreads();
-        const int ns = nsteps_s, qn = q_next_s;
-        if (stage == 0) run_steps<T>(tA, tB, steps, ns, Lm, X, Tm, true, T(1), T(0), M, nsz);
-        else run_steps<T>(tA, tB, steps, ns, X, Tm, X, true, T(-1), T(0), M, nsz);
-        __syncthreads();
-        q_start = qn;
       }
-      cluster.sync();
     }
   }
   t1 = clock64(); t_inv = t1 - t0;
   if (dbg != nullptr && blockIdx.x == 0 && threadIdx.x == 0) { dbg[0] = t_leaf; dbg[1] = t_panel; dbg[2] = t_trail; dbg[3] = t_inv; }
 }
 
+// profiling hook (tools/prof_chol.py): when set, the first cluster launch of a call writes 10 clock64 counts there, its four phases
+// (leaf, panel, trailing update + leaves, inverse) and the six phases of its first leaf
 long long* g_chol_dbg = nullptr;
 extern "C" void gpz_chol_debug_(long long* p) { g_chol_dbg = p; }
 
@@ -520,72 +556,156 @@ template <typename T> int chol_inv(T* W, T* Lc, T* X, T* tmp, int M, int L, int*
 // The cluster kernel above is bound by its serial chain of 64 x 64 leaves and by CUDA-core tile products, the sweep by its rank-64
 // trailing updates (each a memory-bound read-modify-write of the whole trailing matrix on the CUDA cores: 29 ms at M = 4096, L = 10).
 // Here the cluster kernel only factors and inverts the HYB_NB x HYB_NB diagonal blocks (4 leaves each), and every product that
-// involves more than one such block is one batched tcgen05 split-TF32 GEMM on sub-blocks in place (row stride M):
-//     for each panel k:   (L11, X11) = cluster(W11);   L21 = W21 X11^T;   W22 -= L21 L21^T        (trailing update, lower)
-//     then X = Lc^-1 by recursive doubling over the panels:   X21 = -X22 (L21 X11)
-// 12 GEMM launches at M = 1024.  The split-TF32 kernel needs the lo plane (x - tf32(x)) of each operand: Wlo / Llo / Xlo / Tlo
-// shadow W / Lc / X / tmp with the same layout; GEMM epilogues write the lo plane of what they produce, diagonal blocks get theirs
-// from a small strided pass (lo_block).
+// involves more than one such block is a batched tcgen05 split-TF32 GEMM on sub-blocks in place (row stride M).  The split-TF32
+// kernel needs the lo plane (x - tf32(x)) of each operand: Wlo / Llo / Xlo / Tlo shadow W / Lc / X / tmp with the same layout; GEMM
+// epilogues write the lo plane of what they produce, the cluster kernel that of its X block.
+//
+// Only part of the work lies on the path from one diagonal block to the next.  That part runs on the caller's stream (the critical
+// stream), everything else on a side stream owned by the library, where it overlaps the next cluster launch.  P = ceil(M / 256)
+// panels, block indices in units of 256:
+//   critical, k = 0 .. P-1:  [wait T]  cluster(k): (Lc, X, Xlo)[k,k] = chol / inv of W[k,k]
+//                                      L[k+1,k] = W[k+1,k] X[k,k]^T                 (look-ahead panel, one 256^3 product)
+//                            [record C]  W[k+1,k+1] -= L[k+1,k] L[k+1,k]^T          (look-ahead SYRK)
+//   side, first:             zero the upper off-diagonal blocks of Lc and X; Wlo of block column 0; [record T]
+//   side, k = 0 .. P-1:      [wait C]  L[k+2:,k] = W[k+2:,k] X[k,k]^T
+//                                      W[k+2:,k+1] -= L[k+2:,k] L[k+1,k]^T;  W[k+2:,k+2:] -= L[k+2:,k] L[k+2:,k]^T  (lower)
+//                            [record T]  X[k,0:k] = -X[k,k] tmp[k,0:k]               (block row k of the inverse)
+//                                      tmp[k+1,0:k+1] = L[k+1,0:k+1] X[0:k+1,0:k+1]  (needs nothing of cluster(k+1))
+// The critical stream waits for T(k-1) before its look-ahead of step k (the side's trailing update of k-1 last wrote W[k+1,k] and
+// W[k+1,k+1]; one in-order side stream, so one event covers every earlier update), and finally for the side stream's last work.
+// So the critical path is P cluster launches, P-1 pairs of 256^3 products and the last block row of the inverse.
+// Ownership at step k, which keeps the regions the two streams write disjoint: the critical stream owns the diagonal blocks
+// W / Lc / X / Xlo / tmp [k,k] (tmp[k,k] is the cluster kernel's scratch), Lc / Llo [k+1,k] and W [k+1,k+1]; the side stream owns
+// Lc / Llo [k+2:,k], W / Wlo [k+2:,k+1:] except the diagonal block [k+1,k+1], X / Xlo [k,0:k], tmp / Tlo [k+1,0:k+1] and the upper
+// off-diagonal blocks of Lc and X.  The GEMMs never read above the diagonal of a block (their 256-wide tiles start on block
+// boundaries), so those blocks of Llo / Xlo / Tlo are never written.
 constexpr int HYB_NB = 256;
 
-__global__ void tf32_lo_block_kernel(const float* __restrict__ x, float* __restrict__ lo, int n, int M) {
-  // one n x n block (row stride M) per blockIdx.z; blockIdx.y = row, threads over the columns
+// lo plane of a rows x cols block (row stride M) of every factor: blockIdx.z = factor, blockIdx.y = row
+__global__ void tf32_lo_block_kernel(const float* __restrict__ x, float* __restrict__ lo, int cols, int M) {
   const int64_t base = (int64_t)blockIdx.z * M * M + (int64_t)blockIdx.y * M;
-  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) {
-    const float v = x[base + j];
-    lo[base + j] = v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
-  }
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < cols; j += gridDim.x * blockDim.x) lo[base + j] = tf32_lo_part(x[base + j]);
 }
-static int lo_block(const float* x, float* lo, int n, int M, int L, cudaStream_t st) {
-  tf32_lo_block_kernel<<<dim3((unsigned)cdiv(n, 256), n, L), 256, 0, st>>>(x, lo, n, M);
-  GPZ_CHECK_LAUNCH();
+// zeros in the blocks of Lc and X above the diagonal blocks (the cluster kernel clears the upper part of the diagonal blocks)
+__global__ void zero_upper_blocks_kernel(float* __restrict__ Lc, float* __restrict__ X, int M) {
+  const int i = blockIdx.x;
+  const int64_t row = ((int64_t)blockIdx.y * M + i) * M;
+  for (int j = (i / HYB_NB + 1) * HYB_NB + threadIdx.x; j < M; j += blockDim.x) { Lc[row + j] = 0.f; X[row + j] = 0.f; }
+}
+
+// the side stream of chol_inv_hybrid and its two events, created once per device and reused by every call
+struct HybridStreams {
+  cudaStream_t side = nullptr;
+  cudaEvent_t crit = nullptr, done = nullptr;      // recorded on the critical / the side stream
+};
+static int hybrid_streams(HybridStreams** out) {
+  constexpr int MAX_DEV = 64;
+  static HybridStreams per_dev[MAX_DEV];
+  static std::mutex mu;
+  int dev = 0;
+  GPZ_CUDA(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= MAX_DEV) return GPZ_ERR_UNSUPPORTED;
+  std::lock_guard<std::mutex> lock(mu);
+  HybridStreams& h = per_dev[dev];
+  if (h.side == nullptr) {
+    GPZ_CUDA(cudaStreamCreateWithFlags(&h.side, cudaStreamNonBlocking));
+    GPZ_CUDA(cudaEventCreateWithFlags(&h.crit, cudaEventDisableTiming));
+    GPZ_CUDA(cudaEventCreateWithFlags(&h.done, cudaEventDisableTiming));
+  }
+  *out = &h;
   return GPZ_OK;
 }
 
 static int chol_inv_hybrid(float* W, float* Lc, float* X, float* tmp, float* lo_ws, int M, int L, int* info, cudaStream_t st) {
   const int64_t sL = (int64_t)M * M, tot = sL * L;
   float* Wlo = lo_ws; float* Llo = lo_ws + tot; float* Xlo = lo_ws + 2 * tot; float* Tlo = lo_ws + 3 * tot;
-  GPZ_CUDA(cudaMemsetAsync(info, 0, sizeof(int) * L, st));
-  GPZ_CUDA(cudaMemsetAsync(Lc, 0, sizeof(float) * tot, st));
-  GPZ_CUDA(cudaMemsetAsync(X, 0, sizeof(float) * tot, st));
-  GPZ_CUDA(cudaMemsetAsync(Llo, 0, sizeof(float) * 2 * tot, st));       // Llo, Xlo: zero above the diagonal like Lc, X
-  int rc = gpz_tf32_lo_f32(W, Wlo, tot, (void*)st);
+  HybridStreams* hs = nullptr;
+  int rc = hybrid_streams(&hs);
   if (rc) return rc;
+  cudaStream_t side = hs->side;
+  static int num_sms = 0;
+  if (num_sms == 0) {
+    int dev = 0;
+    GPZ_CUDA(cudaGetDevice(&dev));
+    GPZ_CUDA(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
+  }
+  // the side GEMMs are persistent: capped, they leave the SMs for the next cluster launch (L clusters of CL CTAs) free
+  const int side_ctas = max(16, num_sms - L * CL);
+  const int P = (M + HYB_NB - 1) / HYB_NB;
+  auto nb = [&](int k) { return min(HYB_NB, M - k * HYB_NB); };
+  auto off = [&](int bi, int bj) { return (int64_t)bi * HYB_NB * M + (int64_t)bj * HYB_NB; };
+
+  GPZ_CUDA(cudaMemsetAsync(info, 0, sizeof(int) * L, st));
+  GPZ_CUDA(cudaEventRecord(hs->crit, st));                  // fork: the side stream sees W as the caller left it
+  GPZ_CUDA(cudaStreamWaitEvent(side, hs->crit, 0));
+  zero_upper_blocks_kernel<<<dim3(M, L), 256, 0, side>>>(Lc, X, M);
+  GPZ_CHECK_LAUNCH();
+  if (P > 1) {                                              // the first panel product reads W[1:,0] with its lo plane
+    tf32_lo_block_kernel<<<dim3(1, M - HYB_NB, L), 256, 0, side>>>(W + off(1, 0), Wlo + off(1, 0), HYB_NB, M);
+    GPZ_CHECK_LAUNCH();
+  }
+  GPZ_CUDA(cudaEventRecord(hs->done, side));
+
   constexpr int csmem = (int)(2 * NB * TLD * sizeof(float));
   GPZ_CUDA(cudaFuncSetAttribute(chol_inv_cluster_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, csmem));
-  for (int r0 = 0; r0 < M; r0 += HYB_NB) {
-    const int n = min(HYB_NB, M - r0), rem = M - r0 - n;
-    const int64_t o11 = (int64_t)r0 * M + r0, o21 = (int64_t)(r0 + n) * M + r0, o22 = (int64_t)(r0 + n) * M + r0 + n;
-    chol_inv_cluster_kernel<float><<<L * CL, 256, csmem, st>>>(W, Lc, X, tmp, M, r0, n, info, nullptr);
+  for (int k = 0; k < P; ++k) {
+    const int n = nb(k);
+    // ---- critical stream ----
+    chol_inv_cluster_kernel<float><<<L * CL, 256, csmem, st>>>(W, Lc, X, tmp, M, k * HYB_NB, n, info, k == 0 ? g_chol_dbg : nullptr,
+                                                                Xlo);
     GPZ_CHECK_LAUNCH();
-    rc = lo_block(Lc + o11, Llo + o11, n, M, L, st);
-    if (rc) return rc;
-    rc = lo_block(X + o11, Xlo + o11, n, M, L, st);
-    if (rc) return rc;
-    if (rem > 0) {
-      // L21 = W21 X11^T            (B = X11 stored n x k: K-major; op(B) = X11^T is upper triangular)
-      rc = umma_gemm_ex(1, rem, n, n, 1.0f, W + o21, Wlo + o21, M, sL, X + o11, Xlo + o11, M, sL, nullptr, Lc + o21, Llo + o21, M, sL,
-                        L, 0, 2, 0, 1, 3, nullptr, (void*)st);
+    if (k + 1 < P) {
+      const int n1 = nb(k + 1);
+      GPZ_CUDA(cudaStreamWaitEvent(st, hs->done, 0));      // the side's trailing update of k-1 (or its set-up)
+      // L[k+1,k] = W[k+1,k] X[k,k]^T      (B = X[k,k] stored n x k: K-major; op(B) = X^T is upper triangular)
+      rc = umma_gemm_ex(1, n1, n, n, 1.0f, W + off(k + 1, k), Wlo + off(k + 1, k), M, sL, X + off(k, k), Xlo + off(k, k), M, sL,
+                        nullptr, Lc + off(k + 1, k), Llo + off(k + 1, k), M, sL, L, 0, 2, 0, 1, 3, nullptr, (void*)st);
       if (rc) return rc;
-      // W22 -= L21 L21^T  (lower triangle, in place): the trailing update
-      rc = umma_gemm_ex(1, rem, rem, n, -1.0f, Lc + o21, Llo + o21, M, sL, Lc + o21, Llo + o21, M, sL, W + o22, W + o22, Wlo + o22, M,
-                        sL, L, 0, 0, 1, 1, 3, nullptr, (void*)st);
+      GPZ_CUDA(cudaEventRecord(hs->crit, st));
+      // W[k+1,k+1] -= L[k+1,k] L[k+1,k]^T  (lower, in place; its lo plane is never read: the cluster kernel works in fp32)
+      rc = umma_gemm_ex(1, n1, n1, n, -1.0f, Lc + off(k + 1, k), Llo + off(k + 1, k), M, sL, Lc + off(k + 1, k), Llo + off(k + 1, k),
+                        M, sL, W + off(k + 1, k + 1), W + off(k + 1, k + 1), nullptr, M, sL, L, 0, 0, 1, 1, 3, nullptr, (void*)st);
+      if (rc) return rc;
+    } else {
+      GPZ_CUDA(cudaEventRecord(hs->crit, st));
+    }
+    // ---- side stream ----
+    GPZ_CUDA(cudaStreamWaitEvent(side, hs->crit, 0));
+    if (k + 2 < P) {
+      const int r2 = (k + 2) * HYB_NB, m2 = M - r2;
+      // L[k+2:,k] = W[k+2:,k] X[k,k]^T
+      rc = umma_gemm_ex(1, m2, n, n, 1.0f, W + off(k + 2, k), Wlo + off(k + 2, k), M, sL, X + off(k, k), Xlo + off(k, k), M, sL,
+                        nullptr, Lc + off(k + 2, k), Llo + off(k + 2, k), M, sL, L, 0, 2, 0, 1, 3, nullptr, (void*)side, side_ctas);
+      if (rc) return rc;
+      // W[k+2:,k+1] -= L[k+2:,k] L[k+1,k]^T
+      rc = umma_gemm_ex(1, m2, HYB_NB, n, -1.0f, Lc + off(k + 2, k), Llo + off(k + 2, k), M, sL, Lc + off(k + 1, k), Llo + off(k + 1, k),
+                        M, sL, W + off(k + 2, k + 1), W + off(k + 2, k + 1), Wlo + off(k + 2, k + 1), M, sL, L, 0, 0, 0, 1, 3, nullptr,
+                        (void*)side, side_ctas);
+      if (rc) return rc;
+      // W[k+2:,k+2:] -= L[k+2:,k] L[k+2:,k]^T  (lower)
+      rc = umma_gemm_ex(1, m2, m2, n, -1.0f, Lc + off(k + 2, k), Llo + off(k + 2, k), M, sL, Lc + off(k + 2, k), Llo + off(k + 2, k),
+                        M, sL, W + off(k + 2, k + 2), W + off(k + 2, k + 2), Wlo + off(k + 2, k + 2), M, sL, L, 0, 0, 1, 1, 3, nullptr,
+                        (void*)side, side_ctas);
+      if (rc) return rc;
+    }
+    GPZ_CUDA(cudaEventRecord(hs->done, side));
+    if (k > 0) {
+      // X[k,0:k] = -X[k,k] tmp[k,0:k]      (X[k,k] lower triangular; the last block row's lo plane is never read)
+      rc = umma_gemm_ex(0, n, k * HYB_NB, n, -1.0f, X + off(k, k), Xlo + off(k, k), M, sL, tmp + off(k, 0), Tlo + off(k, 0), M, sL,
+                        nullptr, X + off(k, 0), k + 1 < P ? Xlo + off(k, 0) : nullptr, M, sL, L, 1, 0, 0, 1, 3, nullptr, (void*)side,
+                        side_ctas);
+      if (rc) return rc;
+    }
+    if (k + 1 < P) {
+      // tmp[k+1,0:k+1] = L[k+1,0:k+1] X[0:k+1,0:k+1]      (X lower triangular, stored k x n)
+      const int c = (k + 1) * HYB_NB;
+      rc = umma_gemm_ex(0, nb(k + 1), c, c, 1.0f, Lc + off(k + 1, 0), Llo + off(k + 1, 0), M, sL, X, Xlo, M, sL, nullptr,
+                        tmp + off(k + 1, 0), Tlo + off(k + 1, 0), M, sL, L, 0, 1, 0, 1, 3, nullptr, (void*)side, side_ctas);
       if (rc) return rc;
     }
   }
-  for (int b = HYB_NB; b < M; b *= 2) {
-    for (int f0 = 0; f0 + b < M; f0 += 2 * b) {
-      const int n1 = b, n2 = min(b, M - f0 - b);
-      const int64_t o11 = (int64_t)f0 * M + f0, o21 = (int64_t)(f0 + b) * M + f0, o22 = (int64_t)(f0 + b) * M + f0 + b;
-      // tmp21 = L21 X11  (X11 lower triangular, stored k x n) ;  X21 = -X22 tmp21  (X22 lower triangular)
-      rc = umma_gemm_ex(0, n2, n1, n1, 1.0f, Lc + o21, Llo + o21, M, sL, X + o11, Xlo + o11, M, sL, nullptr, tmp + o21, Tlo + o21, M, sL,
-                        L, 0, 1, 0, 1, 3, nullptr, (void*)st);
-      if (rc) return rc;
-      rc = umma_gemm_ex(0, n2, n1, n2, -1.0f, X + o22, Xlo + o22, M, sL, tmp + o21, Tlo + o21, M, sL, nullptr, X + o21, Xlo + o21, M, sL,
-                        L, 1, 0, 0, 1, 3, nullptr, (void*)st);
-      if (rc) return rc;
-    }
-  }
+  GPZ_CUDA(cudaEventRecord(hs->done, side));                // join: everything is final on the caller's stream
+  GPZ_CUDA(cudaStreamWaitEvent(st, hs->done, 0));
   return GPZ_OK;
 }
 

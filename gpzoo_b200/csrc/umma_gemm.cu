@@ -995,7 +995,7 @@ using namespace gpz::umma;
 // common launch: persistent grid, dynamic tile scheduler (one counter per in-flight launch, taken round-robin from a small
 // device array)
 static int launch_gemm(bool b_kmajor, bool f16, const CUtensorMap& mA, const CUtensorMap& mAlo, const CUtensorMap& mB,
-                       const CUtensorMap& mBlo, const Params& p, cudaStream_t st) {
+                       const CUtensorMap& mBlo, const Params& p, cudaStream_t st, int max_ctas = 0) {
   const int mtiles = (int)cdiv(p.m, BM), ntiles = (int)cdiv(p.n, BN);
   const int64_t total64 = (int64_t)mtiles * ntiles * p.batch * p.splitk;
   if (total64 > 0x7fffffff) return GPZ_ERR_UNSUPPORTED;
@@ -1017,7 +1017,8 @@ static int launch_gemm(bool b_kmajor, bool f16, const CUtensorMap& mA, const CUt
   }
   unsigned int* counter = counters + (next_slot.fetch_add(1) % NUM_COUNTERS);
   GPZ_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned int), st));
-  const int grid = total < num_sms ? total : num_sms;
+  int grid = total < num_sms ? total : num_sms;
+  if (max_ctas > 0 && grid > max_ctas) grid = max_ctas;
   if (f16) {
     if (b_kmajor) umma_gemm_kernel<true, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(mA, mAlo, mB, mBlo, p, counter, total, mtiles, ntiles);
     else umma_gemm_kernel<false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(mA, mAlo, mB, mBlo, p, counter, total, mtiles, ntiles);
@@ -1049,7 +1050,7 @@ extern "C" int gpz_umma_gemm_f32(int b_kmajor, int m, int n, int k, float alpha,
 int umma_gemm_ex(int b_kmajor, int m, int n, int k, float alpha, const float* A, const float* Alo, int64_t lda, int64_t sA,
                  const float* B, const float* Blo, int64_t ldb, int64_t sB, const float* Cin, float* D, float* Dlo, int64_t ldd,
                  int64_t sD, int batch, int a_tri, int b_tri, int d_tri, int splitk, int n_terms, const UmmaEpilogue* epi,
-                 void* stream) {
+                 void* stream, int max_ctas) {
   if (!gpz_umma_gemm_supported(b_kmajor, m, n, k, lda, ldb, ldd)) return GPZ_ERR_UNSUPPORTED;
   if (n_terms != 1 && n_terms != 3) return GPZ_ERR_BADARG;
   if (n_terms == 3 && (!Alo || !Blo)) return GPZ_ERR_BADARG;
@@ -1093,7 +1094,7 @@ int umma_gemm_ex(int b_kmajor, int m, int n, int k, float alpha, const float* A,
   p.bk = BK; p.sa = nullptr; p.sb = nullptr; p.Dh = nullptr; p.Dl = nullptr; p.sd = nullptr; p.amax = nullptr;
   p.AuxH = nullptr; p.AuxL = nullptr; p.saux = nullptr; p.D2h = nullptr; p.D2l = nullptr; p.sd2 = nullptr;
   if (p.epi_mode == 4) return GPZ_ERR_BADARG;            // split-FP16 only
-  return launch_gemm(b_kmajor != 0, false, mA, mAlo, mB, mBlo, p, (cudaStream_t)stream);
+  return launch_gemm(b_kmajor != 0, false, mA, mAlo, mB, mBlo, p, (cudaStream_t)stream, max_ctas);
 }
 
 // split-FP16 GEMM: every operand is a pair of fp16 planes (hi, lo) of x * s[b]; three kind::f16 MMAs per k-step

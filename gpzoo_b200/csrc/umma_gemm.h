@@ -13,7 +13,7 @@ struct UmmaEpilogue {
 int umma_gemm_ex(int b_kmajor, int m, int n, int k, float alpha, const float* A, const float* Alo, int64_t lda, int64_t sA,
                  const float* B, const float* Blo, int64_t ldb, int64_t sB, const float* Cin, float* D, float* Dlo, int64_t ldd,
                  int64_t sD, int batch, int a_tri, int b_tri, int d_tri, int splitk, int n_terms, const UmmaEpilogue* epi,
-                 void* stream);
+                 void* stream, int max_ctas = 0);     // max_ctas > 0: at most that many persistent CTAs (leaves SMs to other streams)
 
 // split-FP16 arithmetic: operands are fp16 planes (hi, lo) of x * s[b], s[b] a per-batch power of two kept in device memory
 struct Umma16Args {
