@@ -41,6 +41,7 @@ def lib():
                 for suf in ("f32", "f64"):
                     getattr(l, f"gpz_poisson_workspace_bytes_{suf}").restype = c_i64
                     getattr(l, f"gpz_poisson_csc_workspace_bytes_{suf}").restype = c_i64
+                    getattr(l, f"gpz_negbin_workspace_bytes_{suf}").restype = c_i64
                 _lib = l
     return _lib
 

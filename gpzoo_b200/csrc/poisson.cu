@@ -37,6 +37,16 @@ template <typename T> struct PoissonArgs {
   int atomic_out;                      // gridDim.y > 1
 };
 
+// K7-NB: the same call with the negative-binomial likelihood, theta_g = softplus(D_g) per gene (see the NB section below)
+template <typename T> struct NegBinArgs : PoissonArgs<T> {
+  const T* D;                          // G raw dispersion
+  const T* nbg;                        // [G][2] theta, 1 / theta                                          (negbin_tables_kernel)
+  const T* tab;                        // [G][64][2] Lambda_g[k] - k log theta (- log k! with_lgamma), Psi_g[k] (negbin_tables_kernel)
+  T* gD_part;                          // gridDim.x x G: sum over the CTA's spots and the samples of d log NB / d theta
+  T* gD;                               // G output: d ll / d D
+};
+template <typename T, bool NB> using K7Args = typename std::conditional<NB, NegBinArgs<T>, PoissonArgs<T>>::type;
+
 // 16-byte vector loads of an FMAX-long shared-memory row (FMAX is a multiple of 4, rows are 16-byte aligned)
 template <int FMAX> __device__ __forceinline__ void load_row(const float* p, float (&o)[FMAX]) {
 #pragma unroll
@@ -53,6 +63,46 @@ template <int FMAX> __device__ __forceinline__ void load_row(const double* p, do
   }
 }
 
+// ---- negative-binomial helpers ----------------------------------------------------------------------------------------------
+// log1p(q) for q >= 0.  fp32: the series to q^5 below 1/32 (truncation < 5e-9 relative; 1 + q would lose q's low bits),
+// __log2f(1 + q) above; fp64: the exact function.
+__device__ __forceinline__ float nb_log1p(float q) {
+  const float s = q * fmaf(q, fmaf(q, fmaf(q, fmaf(q, 0.2f, -0.25f), 0.333333343f), -0.5f), 1.f);
+  return q < 0.03125f ? s : __log2f(1.f + q) * 0.69314718055994530942f;
+}
+__device__ __forceinline__ double nb_log1p(double q) { return ::log1p(q); }
+
+// digamma for x > 0 (CUDA's math library has none): the recurrence psi(x) = psi(x + 1) - 1 / x up to x >= 10, then the asymptotic
+// series log x - 1 / (2x) - sum_k B_2k / (2k x^2k) through x^-16 (the next term is below 1e-17 at x = 10).  The recurrence's sum
+// is subtracted last: near the root at 1.4616 that order keeps the cancellation to a few ulp of the two sides.
+__device__ __forceinline__ double nb_digamma(double x) {
+  double acc = 0.0;
+  while (x < 10.0) { acc += 1.0 / x; x += 1.0; }
+  const double r = 1.0 / x, r2 = r * r;
+  const double ser = r2 * (1.0 / 12 - r2 * (1.0 / 120 - r2 * (1.0 / 252 - r2 * (1.0 / 240 - r2 * (1.0 / 132 - r2 * (691.0 / 32760 -
+                     r2 * (1.0 / 12 - r2 * (3617.0 / 8160))))))));
+  return (::log(x) - 0.5 * r - ser) - acc;
+}
+// lgamma for x > 0, written like nb_digamma (the library's lgamma is large code: called from the NB kernels' rare path it made them
+// spill): the product x (x + 1) ... up to x + n >= 10, then Stirling's series through x^-15 (next term below 1e-17 at x = 10)
+__device__ __forceinline__ double nb_lgamma(double x) {
+  double prod = 1.0;
+  while (x < 10.0) { prod *= x; x += 1.0; }
+  const double r = 1.0 / x, r2 = r * r;
+  const double ser = r * (1.0 / 12 - r2 * (1.0 / 360 - r2 * (1.0 / 1260 - r2 * (1.0 / 1680 - r2 * (1.0 / 1188 - r2 * (691.0 / 360360 -
+                     r2 * (1.0 / 156 - r2 * (3617.0 / 122400))))))));
+  return ((x - 0.5) * ::log(x) - x + 0.91893853320467274178 + ser) - ::log(prod);
+}
+
+// The table entries for counts >= 64 and non-integer y, in double: lgamma(y + theta) - lgamma(theta) - y log theta
+// (- lgamma(y + 1) with_lgamma) and psi(y + theta) - psi(theta).  Rare: the kernels zero these elements' table terms and add this
+// afterwards, in a pass of their own, so the call sits where few registers are live.
+__device__ __noinline__ double2 nb_slow(double y, double th, int with_lgamma) {
+  double l = nb_lgamma(y + th) - nb_lgamma(th) - y * ::log(th);
+  if (with_lgamma) l -= nb_lgamma(y + 1.0);
+  return make_double2(l, nb_digamma(y + th) - nb_digamma(th));
+}
+
 // ---- poisson_kernel2 (fp64, fp32 with F > 16): two spots per thread (256 spots per CTA), sample loop outermost ----------------
 // A CTA walks its gene range in chunks of 32.  Phase A (thread = two spots, so y rows are read coalesced): rate, log-lik,
 // t = d ll / d zr, d/dF accumulated in registers, t parked in shared memory.  Phase B (lane = gene, warp = a quarter of the spots):
@@ -63,8 +113,10 @@ template <int FMAX> __device__ __forceinline__ void load_row(const double* p, do
 constexpr int P2_THREADS = 128, P2_SPOTS = 256;
 constexpr int PZ_GRP = 4;        // genes per prefetch group
 
-template <typename T, int FMAX>
-__global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_kernel2(const PoissonArgs<T> a) {
+// NB = true is K7-NB: only the element-wise step, the staging of the per-gene dispersion terms and the d/dD partials differ.
+template <typename T, int FMAX, bool NB>
+// NB, fp32: two CTAs per SM instead of four, so that the heavier element step and the out-of-line call fit in registers.
+__global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? (NB ? 2 : 4) : 1) poisson_kernel2(const K7Args<T, NB> a) {
   extern __shared__ __align__(16) unsigned char pz_smem[];
   typedef T RowT[P2_SPOTS + 1];
   typedef T RowF[FMAX];
@@ -76,6 +128,8 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
   AccW* sAcc = reinterpret_cast<AccW*>(sW + PZ_GCH);                   // [4][PZ_GCH][FMAX]
   __shared__ double red[32];
   __shared__ T lfact[64];                     // log(y!) for integer counts y < 64 (lgamma(y+1) of torch poisson.py log_prob)
+  __shared__ __align__(16) T nbS[NB ? PZ_GCH : 1][2];           // NB: theta, 1 / theta of the chunk's genes
+  __shared__ T dS[NB ? P2_THREADS / 32 : 1][PZ_GCH];            // NB: per-warp d ll / d theta of the chunk's genes
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (tid < 64) lfact[tid] = Num<T>::lgamma(T(tid + 1));
@@ -139,6 +193,12 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
         }
         sW[gi][f] = w;
       }
+      if constexpr (NB) {
+        if (tid < PZ_GCH) {
+#pragma unroll
+          for (int j = 0; j < 2; ++j) nbS[tid][j] = g0 + tid < g_end ? a.nbg[(int64_t)(g0 + tid) * 2 + j] : T(1);
+        }
+      }
       __syncthreads();
       // ---- phase A: thread = two spots ----
       T llc = T(0);
@@ -152,11 +212,14 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
           if (gb + PZ_GRP == PZ_GCH && g0 + PZ_GCH >= g_end) gn = (e + 1 < a.E) ? g_begin : g_end;
           prefetch(gn);
         }
+        T dth[PZ_GRP];                             // NB: d ll / d theta of the group's genes, summed over the thread's two spots
+        unsigned slow = 0u;                        // NB: elements (bit 2u + s2) whose table terms nb_slow supplies
         auto body = [&](auto guard, int u) {
           constexpr bool GUARD = decltype(guard)::value;
           const int gi = gb + u;
           T wrow[FMAX];
           load_row<FMAX>(&sW[gi][0], wrow);
+          if constexpr (NB) dth[u] = T(0);
 #pragma unroll
           for (int s2 = 0; s2 < 2; ++s2) {
             T t = T(0);
@@ -167,16 +230,34 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
               for (int f = 0; f < FMAX; f += 2) { z0 = fma(wrow[f], ef[s2][f], z0); z1 = fma(wrow[f + 1], ef[s2][f + 1], z1); }
               const T zr = z0 + z1;
               const T r = spV[s2] * zr;
-              const T ylog = y * fast_log(r);
-              T lp = (y == T(0) ? T(0) : ylog) - r;
-              if (a.with_lgamma) {
+              if constexpr (NB) {
+                const T th = nbS[gi][0], q = r * nbS[gi][1];
+                const T l1p = nb_log1p(q);
+                const T ud = fast_div(y - r, fma(r, q, r));                 // (y - r) / (r (1 + r / theta)) = d log NB / d r
                 const int yi = (int)y;
-                // counts: table lookup (no divergent lgamma call); anything else: the real thing
-                lp -= (yi >= 0 && yi < 64 && T(yi) == y) ? lfact[yi] : Num<T>::lgamma(y + T(1));
+                T lam = T(0), psi = T(0);                                   // table entries; anything else: the slow pass below
+                if (yi >= 0 && yi < 64 && T(yi) == y) {
+                  const T* tv = a.tab + ((int64_t)(g0 + gi) * 64 + yi) * 2;
+                  lam = tv[0]; psi = tv[1];
+                } else {
+                  slow |= 1u << (2 * u + s2);
+                }
+                llc += (y == T(0) ? T(0) : y * fast_log(r)) - (y + th) * l1p + lam;
+                t = ud * spV[s2] * invE;
+                gVacc[s2] += ud * r;
+                dth[u] += psi - l1p - ud * q;
+              } else {
+                const T ylog = y * fast_log(r);
+                T lp = (y == T(0) ? T(0) : ylog) - r;
+                if (a.with_lgamma) {
+                  const int yi = (int)y;
+                  // counts: table lookup (no divergent lgamma call); anything else: the real thing
+                  lp -= (yi >= 0 && yi < 64 && T(yi) == y) ? lfact[yi] : Num<T>::lgamma(y + T(1));
+                }
+                llc += lp;
+                t = (fast_div(y, zr) - spV[s2]) * invE;
+                gVacc[s2] += y - r;
               }
-              llc += lp;
-              t = (fast_div(y, zr) - spV[s2]) * invE;
-              gVacc[s2] += y - r;
 #pragma unroll
               for (int f = 0; f < FMAX; ++f) pg[s2][f] = fma(wrow[f], t, pg[s2][f]);
             }
@@ -187,8 +268,39 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
 #pragma unroll
           for (int u = 0; u < PZ_GRP; ++u) body(std::false_type{}, u);
         } else {
+          if constexpr (NB) {                      // unrolled: dth stays in registers
+#pragma unroll
+            for (int u = 0; u < PZ_GRP; ++u) body(std::true_type{}, u);
+          } else {
 #pragma unroll 1
-          for (int u = 0; u < PZ_GRP; ++u) body(std::true_type{}, u);
+            for (int u = 0; u < PZ_GRP; ++u) body(std::true_type{}, u);
+          }
+        }
+        if constexpr (NB) {
+#pragma unroll 1
+          while (slow) {                           // one call site, not unrolled: it keeps the call's register cost off the hot path
+            const int b = __ffs(slow) - 1, u = b >> 1;
+            slow &= slow - 1u;
+            T y = T(0);
+#pragma unroll
+            for (int k = 0; k < 2 * PZ_GRP; ++k) y = k == b ? yv[k >> 1][k & 1] : y;
+            const double2 sl = nb_slow((double)y, (double)nbS[gb + u][0], a.with_lgamma);
+            llc += (T)sl.x;
+#pragma unroll
+            for (int k = 0; k < PZ_GRP; ++k) dth[k] += k == u ? (T)sl.y : T(0);
+          }
+          // sum the four genes' values over the warp's 32 lanes in 6 shuffles (halve, halve, then a plain tree): lane bits 4 and 3
+          // end up naming the gene; lanes 0, 8, 16, 24 hold the totals
+          const bool hi16 = lane & 16, hi8 = lane & 8;
+          T k0 = hi16 ? dth[2] : dth[0], k1 = hi16 ? dth[3] : dth[1];
+          k0 += __shfl_xor_sync(0xffffffffu, hi16 ? dth[0] : dth[2], 16);
+          k1 += __shfl_xor_sync(0xffffffffu, hi16 ? dth[1] : dth[3], 16);
+          T k = hi8 ? k1 : k0;
+          k += __shfl_xor_sync(0xffffffffu, hi8 ? k0 : k1, 8);
+          k += __shfl_xor_sync(0xffffffffu, k, 4);
+          k += __shfl_xor_sync(0xffffffffu, k, 2);
+          k += __shfl_xor_sync(0xffffffffu, k, 1);
+          if ((lane & 7) == 0) dS[warp][gb + (lane >> 3)] = k;
         }
       }
       ll += (double)(llc * invE);
@@ -214,6 +326,13 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
         if (g0 + gi < g_end) {
           T* dst = a.gW_part + ((int64_t)blockIdx.x * a.G + g0 + gi) * a.F + f;
           const T v = sAcc[0][gi][f] + sAcc[1][gi][f] + sAcc[2][gi][f] + sAcc[3][gi][f];
+          *dst = e == 0 ? v : *dst + v;
+        }
+      }
+      if constexpr (NB) {
+        if (tid < PZ_GCH && g0 + tid < g_end) {
+          T* dst = a.gD_part + (int64_t)blockIdx.x * a.G + g0 + tid;
+          const T v = (dS[0][tid] + dS[1][tid]) + (dS[2][tid] + dS[3][tid]);
           *dst = e == 0 ? v : *dst + v;
         }
       }
@@ -249,6 +368,7 @@ __global__ void __launch_bounds__(P2_THREADS, sizeof(T) == 4 ? 4 : 1) poisson_ke
   const double tot = block_sum<double>(ll, red);
   if (tid == 0) a.ll_part[blockIdx.y * gridDim.x + blockIdx.x] = tot;
 }
+
 
 // ---- v4 (fp32, F <= 16): the three F-long contractions on the tensor cores ------------------------------------------------
 // poisson_kernel2 is bound by instruction issue (3.3 warp instructions per (gene, spot) element, 36 of the 105 thread instructions
@@ -417,13 +537,17 @@ template <> __device__ __forceinline__ void y_load2<int32_t>(const int32_t* p, f
 
 __device__ __noinline__ float lfact_slow(float y) { return lgammaf(y + 1.f); }     // counts >= 64 or non-integer y: rare, kept out of line
 
-template <bool HAS_IDX, typename YT>
-__global__ void __launch_bounds__(P4_THREADS, 2) poisson_kernel4(const PoissonArgs<float> a, const Poisson4Ws w) {
+// NB = true is K7-NB (the NB element step, the per-gene dispersion terms and the d/dD partials).
+template <bool HAS_IDX, typename YT, bool NB>
+// NB: one CTA per SM.  With two, the NB step needs more than the 128 registers a thread then gets and spills to local memory.
+__global__ void __launch_bounds__(P4_THREADS, NB ? 1 : 2) poisson_kernel4(const K7Args<float, NB> a, const Poisson4Ws w) {
   __shared__ __align__(16) uint16_t sWh[P4_GCH][P4_WLD];      // softplus(W) chunk, bf16 hi / lo, [gene][factor]
   __shared__ __align__(16) uint16_t sWl[P4_GCH][P4_WLD];
   __shared__ __align__(16) float sAcc[P4_WARPS][16][P4_ALD];  // per-warp D3[l][gene of the chunk]
   __shared__ double red[32];
   __shared__ float lfact[64];                                 // log(y!) for integer counts y < 64
+  __shared__ float2 nbS[NB ? P4_GCH : 1];                     // NB: theta, 1 / theta of the chunk's genes
+  __shared__ float dS[NB ? P4_WARPS : 1][P4_GCH];             // NB: per-warp d ll / d theta of the chunk's genes
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int r = lane >> 2, c = lane & 3;                      // fragment coordinates (groupID, threadID_in_group)
@@ -528,6 +652,10 @@ __global__ void __launch_bounds__(P4_THREADS, 2) poisson_kernel4(const PoissonAr
         }
         *reinterpret_cast<uint2*>(&sWh[gi][lq]) = vh;
         *reinterpret_cast<uint2*>(&sWl[gi][lq]) = vl;
+        if constexpr (NB) {
+          if (tid < P4_GCH)
+            nbS[tid] = g0 + tid < g_end ? reinterpret_cast<const float2*>(a.nbg)[g0 + tid] : make_float2(1.f, 1.f);
+        }
       }
       __syncthreads();
       const int nblk = min(P4_GCH / 16, (g_end - g0 + 15) >> 4);
@@ -573,6 +701,59 @@ __global__ void __launch_bounds__(P4_THREADS, 2) poisson_kernel4(const PoissonAr
           }
           // element-wise on the rate fragment
           float t[8];
+          if constexpr (NB) {
+            // d log NB / d r = (y - r) / (r (1 + q)), q = r / theta; llg collects the natural-log terms with the opposite sign.
+            // The table terms of counts >= 64 and non-integer y are zero here and come from nb_slow in the pass below.
+            // dth: d ll / d theta of the thread's four genes over its two spots of the sub-tile; slot j <-> gene
+            // gblk + 8 (j >> 1) + 2c + (j & 1) (register q of a fragment is slot 2 (q >> 2) + (q & 1))
+            float dth[4] = {0.f, 0.f, 0.f, 0.f};
+            unsigned slow = 0u;
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+              const float y = yreg[s][q];
+              const float2 nb = nbS[16 * jb + 8 * (q >> 2) + 2 * c + (q & 1)];
+              const int yi = (int)min((unsigned)__float2int_rz(y), 63u);     // negative or huge -> 63, which fails the comparison
+              const bool ok = (float)yi == y;
+              const int g = min(gblk + 8 * (q >> 2) + 2 * c + (q & 1), g_end - 1);
+              float2 tv = __ldg(reinterpret_cast<const float2*>(a.tab) + (int64_t)g * 64 + yi);
+              if (!ok) { tv = make_float2(0.f, 0.f); slow |= 1u << q; }
+              const float rate = fmaxf(c1[q >> 2][q & 3], 1e-30f);
+              const float qq = rate * nb.y;
+              const float l1p = nb_log1p(qq);
+              float rd;
+              asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rd) : "f"(fmaf(rate, qq, rate)));
+              const float ud = (y - rate) * rd;
+              llc = fmaf(y, __log2f(rate), llc);
+              llg += fmaf(y + nb.x, l1p, -tv.x);
+              t[q] = ud * invE;
+              dth[2 * (q >> 2) + (q & 1)] += tv.y - fmaf(ud, qq, l1p);
+            }
+#pragma unroll 1
+            while (slow) {                          // one call site, not unrolled: it keeps the call's register cost off the hot path
+              const int q = __ffs(slow) - 1, j = 2 * (q >> 2) + (q & 1);
+              slow &= slow - 1u;
+              float y = 0.f;
+#pragma unroll
+              for (int k = 0; k < 8; ++k) y = k == q ? yreg[s][k] : y;
+              const double2 sl = nb_slow((double)y, (double)nbS[16 * jb + 8 * (j >> 1) + 2 * c + (j & 1)].x, a.with_lgamma);
+              llg -= (float)sl.x;
+#pragma unroll
+              for (int k = 0; k < 4; ++k) dth[k] += k == j ? (float)sl.y : 0.f;
+            }
+            // sum the four slots over the 8 lanes of equal c (lane bits 2-4) in 4 shuffles; lane bits 4 and 3 end up naming the
+            // slot.  Summed per sub-tile (the first one writes), so the four accumulators live only through this element step.
+            const bool hi16 = lane & 16, hi8 = lane & 8;
+            float k0 = hi16 ? dth[2] : dth[0], k1 = hi16 ? dth[3] : dth[1];
+            k0 += __shfl_xor_sync(0xffffffffu, hi16 ? dth[0] : dth[2], 16);
+            k1 += __shfl_xor_sync(0xffffffffu, hi16 ? dth[1] : dth[3], 16);
+            float k = hi8 ? k1 : k0;
+            k += __shfl_xor_sync(0xffffffffu, hi8 ? k0 : k1, 8);
+            k += __shfl_xor_sync(0xffffffffu, k, 4);
+            if ((lane & 4) == 0) {
+              float* d = &dS[warp][16 * jb + 8 * (lane >> 4) + 2 * c + ((lane >> 3) & 1)];
+              *d = s == 0 ? k : *d + k;
+            }
+          } else {
 #pragma unroll
           for (int q = 0; q < 8; ++q) {
             const float y = yreg[s][q];
@@ -582,7 +763,8 @@ __global__ void __launch_bounds__(P4_THREADS, 2) poisson_kernel4(const PoissonAr
             llc = fmaf(y, __log2f(rate), llc);
             t[q] = fmaf(y * invE, rinv, -invE);
           }
-          if (a.with_lgamma) {
+          }
+          if (!NB && a.with_lgamma) {
             // log(y!) from the table, branch-free: the entry of min(trunc(y), 63), exact whenever y is an integer count below 64
             // (lfact[0] = lfact[1] = 0); anything else (y >= 64, non-integer y) is detected by comparing back and redone exactly.
             bool exact = true;
@@ -651,6 +833,15 @@ __global__ void __launch_bounds__(P4_THREADS, 2) poisson_kernel4(const PoissonAr
         float* dst = a.gW_part + ((int64_t)blockIdx.x * a.G + g0 + gi) * a.F + f;
         *dst = e == 0 ? v : *dst + v;
       }
+      if constexpr (NB) {
+        if (tid < min(P4_GCH, g_end - g0)) {
+          float v = 0.f;
+#pragma unroll
+          for (int w8 = 0; w8 < P4_WARPS; ++w8) v += dS[w8][tid];
+          float* dst = a.gD_part + (int64_t)blockIdx.x * a.G + g0 + tid;
+          *dst = e == 0 ? v : *dst + v;
+        }
+      }
     }
     // D2[n][l] of the sample leaves the registers: (n = r + 8 (i >> 1), l = 8 lt + 2c + (i & 1)) pairs as float2
 #pragma unroll
@@ -671,15 +862,29 @@ __global__ void __launch_bounds__(P4_THREADS, 2) poisson_kernel4(const PoissonAr
   if (tid == 0) a.ll_part[blockIdx.y * gridDim.x + blockIdx.x] = tot;
 }
 
+
 // blocks [0, gw_blocks): gW[g, f] = (softplus'(W[g, f]) or 1) * sum_b gW_part[b, g, f]; blocks [gw_blocks, ...): 64 spots each, all samples:
 // gF = EF' D2 -> d/dmean, d/dspread, d/dV and sum_g r.  The last block to finish sums the log-likelihood partials (fixed order).
-__global__ void __launch_bounds__(256) poisson_post4_kernel(const PoissonArgs<float> a, const Poisson4Ws w, float* __restrict__ gW, int nbx,
+// NB: blocks [gw_blocks + spot_blocks, ...) reduce the d/dD partials, 256 genes each; ll has no sum_g r term.
+template <bool NB>
+__global__ void __launch_bounds__(256) poisson_post4_kernel(const K7Args<float, NB> a, const Poisson4Ws w, float* __restrict__ gW, int nbx,
                                                             int nby, int gw_blocks, int spot_blocks, double* __restrict__ ll_out) {
   __shared__ double red[32];
   __shared__ float wsum[16];
   __shared__ bool last;
   const int tid = threadIdx.x;
-  if ((int)blockIdx.x < gw_blocks) {
+  if (NB && (int)blockIdx.x >= gw_blocks + spot_blocks) {
+    if constexpr (NB) {                     // gD[g] = softplus'(D[g]) / E * sum_b gD_part[b, g], in a fixed order
+      const int g = (blockIdx.x - gw_blocks - spot_blocks) * 256 + tid;
+      if (g < a.G) {
+        float s0 = 0.f, s1 = 0.f;
+        int b = 0;
+        for (; b + 1 < nbx; b += 2) { s0 += a.gD_part[(int64_t)b * a.G + g]; s1 += a.gD_part[(int64_t)(b + 1) * a.G + g]; }
+        if (b < nbx) s0 += a.gD_part[(int64_t)b * a.G + g];
+        a.gD[g] = softplus_grad(a.D[g]) * (s0 + s1) / (float)a.E;
+      }
+    }
+  } else if ((int)blockIdx.x < gw_blocks) {
     // 64 outputs per block; thread (o, p) adds the partials of the CTAs b = p, p + 4, ... (independent loads, 256-byte rows)
     __shared__ float part[4][64];
     const int64_t GF = (int64_t)a.G * a.F, i = (int64_t)blockIdx.x * 64 + (tid & 63);
@@ -702,7 +907,7 @@ __global__ void __launch_bounds__(256) poisson_post4_kernel(const PoissonArgs<fl
       gW[i] = a.w_softplus ? s * softplus_grad(a.W[i]) : s;
     }
   } else {
-    if (tid < 16) {
+    if (!NB && tid < 16) {
       float v = 0.f;
       for (int by = 0; by < nby; ++by) v += w.wsum[by * 16 + tid];
       wsum[tid] = v;
@@ -725,7 +930,7 @@ __global__ void __launch_bounds__(256) poisson_post4_kernel(const PoissonArgs<fl
           gm[j] += gF;
           gs[j] = fmaf(gF, epsv[j], gs[j]);
           gsum += gF;
-          rs = fmaf(ev[j], wsum[lq + j], rs);
+          if constexpr (!NB) rs = fmaf(ev[j], wsum[lq + j], rs);
         }
       }
 #pragma unroll
@@ -744,8 +949,10 @@ __global__ void __launch_bounds__(256) poisson_post4_kernel(const PoissonArgs<fl
     gsum += __shfl_xor_sync(0xffffffffu, gsum, 1);
     gsum += __shfl_xor_sync(0xffffffffu, gsum, 2);
     if (n < a.B && (tid & 3) == 0) a.gV[n] = softplus_grad(vraw) * gsum / spV;
-    const double tot = block_sum<double>((double)rs, red);
-    if (tid == 0) w.rs_part[sb] = tot;
+    if constexpr (!NB) {
+      const double tot = block_sum<double>((double)rs, red);
+      if (tid == 0) w.rs_part[sb] = tot;
+    }
   }
   // last block done: ll = sum(main partials) - sum(rate sums) / E
   __threadfence();
@@ -756,12 +963,15 @@ __global__ void __launch_bounds__(256) poisson_post4_kernel(const PoissonArgs<fl
   __threadfence();
   double s = 0.0;
   for (int i = tid; i < nbx * nby; i += 256) s += __ldcg(a.ll_part + i);
-  double rsum = 0.0;
-  for (int i = tid; i < spot_blocks; i += 256) rsum += __ldcg(w.rs_part + i);
-  s -= rsum / (double)a.E;
+  if constexpr (!NB) {
+    double rsum = 0.0;
+    for (int i = tid; i < spot_blocks; i += 256) rsum += __ldcg(w.rs_part + i);
+    s -= rsum / (double)a.E;
+  }
   s = block_sum<double>(s, red);
   if (tid == 0) ll_out[0] = s;
 }
+
 
 // gW[g,f] = (softplus'(W[g,f]) or 1) * sum_b gW_part[b,g,f]
 template <typename T>
@@ -782,14 +992,47 @@ __global__ void sum_double_kernel(const double* __restrict__ part, int n, double
   if (threadIdx.x == 0) out[0] = s;
 }
 
+// K7-NB per-gene terms, in double: theta = softplus(D), 1 / theta, and for k < 64
+//   Lambda_g[k] = sum_{j<k} log1p(j / theta) = lgamma(k + theta) - lgamma(theta) - k log theta   (minus log k! with_lgamma)
+//   Psi_g[k]    = sum_{j<k} 1 / (theta + j)  = psi(k + theta) - psi(theta)
+// Four genes per 256-thread block, thread <-> (gene, k); each prefix is summed in the same order by its own thread.
+template <typename T>
+__global__ void __launch_bounds__(256) negbin_tables_kernel(const T* __restrict__ D, int G, int with_lgamma, T* __restrict__ nbg,
+                                                            T* __restrict__ tab) {
+  __shared__ double sl[4][64], sp[4][64];
+  const int k = threadIdx.x & 63, gl = threadIdx.x >> 6, g = blockIdx.x * 4 + gl;
+  const double th = g < G ? softplus((double)D[g]) : 1.0;
+  sl[gl][k] = ::log1p(k / th);                      // log(theta + k) - log theta, without the cancellation
+  sp[gl][k] = 1.0 / (th + k);
+  __syncthreads();
+  if (g >= G) return;
+  double lam = 0.0, psi = 0.0;
+  for (int j = 0; j < k; ++j) { lam += sl[gl][j]; psi += sp[gl][j]; }
+  if (with_lgamma) lam -= ::lgamma(k + 1.0);
+  tab[((int64_t)g * 64 + k) * 2] = (T)lam;
+  tab[((int64_t)g * 64 + k) * 2 + 1] = (T)psi;
+  if (k < 2) nbg[(int64_t)g * 2 + k] = (T)(k == 0 ? th : 1.0 / th);
+}
+
+// gD[g] = softplus'(D[g]) / E * sum_b part[b, g] (poisson_kernel2 path; the tensor-core path does this in poisson_post4_kernel<true>)
+template <typename T>
+__global__ void negbin_gd_reduce_kernel(const T* __restrict__ part, const T* __restrict__ D, T* __restrict__ gD, int G, int nb, int E) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= G) return;
+  T s = T(0);
+  for (int b = 0; b < nb; ++b) s += part[(int64_t)b * G + g];
+  gD[g] = softplus_grad(D[g]) * s / T(E);
+}
+
 template <typename T, int FMAX> constexpr size_t poisson_smem2() {
   return ((sizeof(T) * PZ_GCH * (P2_SPOTS + 1) + 15) / 16) * 16 + sizeof(T) * (FMAX * P2_SPOTS + PZ_GCH * FMAX + 4 * PZ_GCH * FMAX);
 }
 static bool poisson_use_v4(int F, bool is_f32) { return is_f32 && F <= 16; }     // tensor-core kernels; anything else runs kernel2
-template <typename T, int FMAX> int poisson_launch(const PoissonArgs<T>& a, dim3 grid, cudaStream_t st) {
+template <typename T, int FMAX, typename A> int poisson_launch(const A& a, dim3 grid, cudaStream_t st) {
   constexpr size_t smem = poisson_smem2<T, FMAX>();
-  GPZ_CUDA(cudaFuncSetAttribute(poisson_kernel2<T, FMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  poisson_kernel2<T, FMAX><<<grid, P2_THREADS, smem, st>>>(a);
+  void (*kern)(const A) = poisson_kernel2<T, FMAX, std::is_same<A, NegBinArgs<T>>::value>;
+  GPZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<grid, P2_THREADS, smem, st>>>(a);
   GPZ_CHECK_LAUNCH();
   return GPZ_OK;
 }
@@ -825,25 +1068,43 @@ static size_t poisson_ws_bytes(int G, int F, int B, int E, bool is_f32, size_t e
   }
   return b;
 }
+// K7-NB appends: gD partials [nbx][G] | per-gene terms [G][2] | tables [G][64][2]
+static size_t negbin_extra_bytes(int G, size_t elt, int nbx) { return (elt * (size_t)nbx * G + 15) / 16 * 16 + elt * 130 * (size_t)G; }
+static size_t negbin_ws_bytes(int G, int F, int B, int E, bool is_f32, size_t elt, int nbx, int nby) {
+  return (poisson_ws_bytes(G, F, B, E, is_f32, elt, nbx, nby) + 15) / 16 * 16 + negbin_extra_bytes(G, elt, nbx);
+}
 
-// y_kind: element type of y — 0 = T (the reference's format), 1 = uint8, 2 = int16, 3 = int32 (fp32 tensor-core kernel only)
-template <typename T>
-int poisson_fwdbwd(PoissonArgs<T> a, T* gW, double* ll_out, void* ws, size_t ws_bytes, cudaStream_t st, int y_kind = 0) {
+// y_kind: element type of y — 0 = T (the reference's format), 1 = uint8, 2 = int16, 3 = int32 (fp32 tensor-core kernel only).
+// A = PoissonArgs<T> runs K7; A = NegBinArgs<T> runs K7-NB (same grid and kernels' structure, plus the per-gene tables and gD).
+template <typename T, typename A>
+int poisson_fwdbwd(A a, T* gW, double* ll_out, void* ws, size_t ws_bytes, cudaStream_t st, int y_kind = 0) {
+  constexpr bool NB = std::is_same<A, NegBinArgs<T>>::value;
   if (a.F < 1 || a.F > 32 || a.E < 1 || a.G < 1) return GPZ_ERR_UNSUPPORTED;
   if (y_kind < 0 || y_kind > 3 || (y_kind != 0 && !poisson_use_v4(a.F, std::is_same<T, float>::value))) return GPZ_ERR_UNSUPPORTED;
   if (a.B == 0) {                       // empty minibatch: ll = 0, no gradient
     GPZ_CUDA(cudaMemsetAsync(ll_out, 0, sizeof(double), st));
     GPZ_CUDA(cudaMemsetAsync(gW, 0, sizeof(T) * (size_t)a.G * a.F, st));
+    if constexpr (NB) GPZ_CUDA(cudaMemsetAsync(a.gD, 0, sizeof(T) * (size_t)a.G, st));
     return GPZ_OK;
   }
   int nbx, nby, gpc;
   poisson_grid(a.G, a.F, a.B, std::is_same<T, float>::value, &nbx, &nby, &gpc);
-  const size_t need = poisson_ws_bytes(a.G, a.F, a.B, a.E, std::is_same<T, float>::value, sizeof(T), nbx, nby);
+  const size_t base = poisson_ws_bytes(a.G, a.F, a.B, a.E, std::is_same<T, float>::value, sizeof(T), nbx, nby);
+  const size_t need = NB ? negbin_ws_bytes(a.G, a.F, a.B, a.E, std::is_same<T, float>::value, sizeof(T), nbx, nby) : base;
   if (ws_bytes < need) return GPZ_ERR_BADARG;
   a.ll_part = reinterpret_cast<double*>(ws);
   a.gW_part = reinterpret_cast<T*>(a.ll_part + poisson_ll_slots(nbx, nby));
   a.genes_per_cta = gpc;
   a.atomic_out = nby > 1;
+  if constexpr (NB) {
+    unsigned char* pn = reinterpret_cast<unsigned char*>(ws) + (base + 15) / 16 * 16;
+    a.gD_part = reinterpret_cast<T*>(pn); pn += (sizeof(T) * (size_t)nbx * a.G + 15) / 16 * 16;
+    T* nbg = reinterpret_cast<T*>(pn);
+    T* tab = nbg + 2 * (size_t)a.G;
+    a.nbg = nbg; a.tab = tab;
+    negbin_tables_kernel<T><<<(unsigned)cdiv(a.G, 4), 256, 0, st>>>(a.D, a.G, a.with_lgamma, nbg, tab);
+    GPZ_CHECK_LAUNCH();
+  }
   if (a.atomic_out && !poisson_use_v4(a.F, std::is_same<T, float>::value)) {
     GPZ_CUDA(cudaMemsetAsync(a.gV, 0, sizeof(T) * a.B, st));
     GPZ_CUDA(cudaMemsetAsync(a.gmean, 0, sizeof(T) * a.B * a.F, st));
@@ -869,8 +1130,8 @@ int poisson_fwdbwd(PoissonArgs<T> a, T* gW, double* ll_out, void* ws, size_t ws_
       GPZ_CHECK_LAUNCH();
 #define GPZ_P4_LAUNCH(YT)                                                              \
   do {                                                                                 \
-    if (a.idx) poisson_kernel4<true, YT><<<grid, P4_THREADS, 0, st>>>(a, w);           \
-    else poisson_kernel4<false, YT><<<grid, P4_THREADS, 0, st>>>(a, w);                \
+    if (a.idx) poisson_kernel4<true, YT, NB><<<grid, P4_THREADS, 0, st>>>(a, w);       \
+    else poisson_kernel4<false, YT, NB><<<grid, P4_THREADS, 0, st>>>(a, w);            \
   } while (0)
       if (y_kind == 1) GPZ_P4_LAUNCH(uint8_t);
       else if (y_kind == 2) GPZ_P4_LAUNCH(int16_t);
@@ -878,7 +1139,8 @@ int poisson_fwdbwd(PoissonArgs<T> a, T* gW, double* ll_out, void* ws, size_t ws_
       else GPZ_P4_LAUNCH(float);
 #undef GPZ_P4_LAUNCH
       GPZ_CHECK_LAUNCH();
-      poisson_post4_kernel<<<gw_blocks + spot_blocks, 256, 0, st>>>(a, w, gW, nbx, nby, gw_blocks, spot_blocks, ll_out);
+      const int gd_blocks = NB ? (int)cdiv(a.G, 256) : 0;       // NB: the d/dD reduction
+      poisson_post4_kernel<NB><<<gw_blocks + spot_blocks + gd_blocks, 256, 0, st>>>(a, w, gW, nbx, nby, gw_blocks, spot_blocks, ll_out);
       GPZ_CHECK_LAUNCH();
       return GPZ_OK;
     }
@@ -891,6 +1153,10 @@ int poisson_fwdbwd(PoissonArgs<T> a, T* gW, double* ll_out, void* ws, size_t ws_
   const int64_t GF = (int64_t)a.G * a.F;
   poisson_gw_reduce_kernel<T><<<(unsigned)cdiv(GF, 256), 256, 0, st>>>(a.gW_part, a.W, gW, GF, nbx, a.w_softplus);
   GPZ_CHECK_LAUNCH();
+  if constexpr (NB) {
+    negbin_gd_reduce_kernel<T><<<(unsigned)cdiv(a.G, 256), 256, 0, st>>>(a.gD_part, a.D, a.gD, a.G, nbx, a.E);
+    GPZ_CHECK_LAUNCH();
+  }
   sum_double_kernel<<<1, 256, 0, st>>>(a.ll_part, nbx * nby, ll_out);
   GPZ_CHECK_LAUNCH();
   return GPZ_OK;
@@ -1298,6 +1564,72 @@ extern "C" int gpz_poisson_fwdbwd_yt_f32(const void* y, int y_kind, int64_t y_ld
   a.spread = spread; a.eps = eps; a.G = G; a.F = F; a.B = B; a.E = E; a.n_var = n_var; a.clamp_min = clamp_min;
   a.with_lgamma = with_lgamma; a.gV = gV; a.gmean = gmean; a.gspread = gspread;
   return poisson_fwdbwd<float>(a, gW, ll, ws, (size_t)ws_bytes, (cudaStream_t)stream, y_kind);
+}
+
+// K7-NB: the Poisson arguments plus D (G, raw dispersion) and the output gD (G)
+template <typename T>
+static NegBinArgs<T> negbin_args(const T* y, int64_t y_ld, const int64_t* idx, const T* W, int w_softplus, const T* V, const T* D,
+                                 const T* mean, const T* spread, const T* eps, int G, int F, int B, int E, int n_var, T clamp_min,
+                                 int with_lgamma, T* gV, T* gD, T* gmean, T* gspread) {
+  NegBinArgs<T> a;
+  a.y = y; a.y_ld = y_ld; a.idx = idx; a.W = W; a.w_softplus = w_softplus; a.V = V; a.mean = mean;
+  a.spread = spread; a.eps = eps; a.G = G; a.F = F; a.B = B; a.E = E; a.n_var = n_var; a.clamp_min = clamp_min;
+  a.with_lgamma = with_lgamma; a.gV = gV; a.gmean = gmean; a.gspread = gspread;
+  a.D = D; a.gD = gD;
+  return a;
+}
+
+#define GPZ_NEGBIN_IMPL(SUF, T)                                                                                        \
+  extern "C" int64_t gpz_negbin_workspace_bytes_##SUF(int G, int F, int B, int E) {                                    \
+    int nbx, nby, gpc;                                                                                                 \
+    poisson_grid(G, F, B, sizeof(T) == 4, &nbx, &nby, &gpc);                                                           \
+    return (int64_t)negbin_ws_bytes(G, F, B, E, sizeof(T) == 4, sizeof(T), nbx, nby);                                  \
+  }                                                                                                                    \
+  extern "C" int gpz_negbin_fwdbwd_##SUF(const T* y, int64_t y_ld, const int64_t* idx, const T* W, int w_softplus,     \
+                                         const T* V, const T* D, const T* mean, const T* spread, const T* eps, int G,  \
+                                         int F, int B, int E, int n_var, T clamp_min, int with_lgamma, double* ll,     \
+                                         T* gW, T* gV, T* gD, T* gmean, T* gspread, void* ws, int64_t ws_bytes,        \
+                                         void* stream) {                                                               \
+    const NegBinArgs<T> a = negbin_args<T>(y, y_ld, idx, W, w_softplus, V, D, mean, spread, eps, G, F, B, E, n_var,    \
+                                           clamp_min, with_lgamma, gV, gD, gmean, gspread);                            \
+    return poisson_fwdbwd<T>(a, gW, ll, ws, (size_t)ws_bytes, (cudaStream_t)stream);                                   \
+  }
+
+GPZ_NEGBIN_IMPL(f32, float)
+GPZ_NEGBIN_IMPL(f64, double)
+
+extern "C" int gpz_negbin_fwdbwd_yt_f32(const void* y, int y_kind, int64_t y_ld, const int64_t* idx, const float* W, int w_softplus,
+                                        const float* V, const float* D, const float* mean, const float* spread, const float* eps, int G,
+                                        int F, int B, int E, int n_var, float clamp_min, int with_lgamma, double* ll, float* gW,
+                                        float* gV, float* gD, float* gmean, float* gspread, void* ws, int64_t ws_bytes, void* stream) {
+  const NegBinArgs<float> a = negbin_args<float>(reinterpret_cast<const float*>(y), y_ld, idx, W, w_softplus, V, D, mean, spread, eps,
+                                                 G, F, B, E, n_var, clamp_min, with_lgamma, gV, gD, gmean, gspread);
+  return poisson_fwdbwd<float>(a, gW, ll, ws, (size_t)ws_bytes, (cudaStream_t)stream, y_kind);
+}
+
+namespace gpz {
+__global__ void digamma_kernel(const double* __restrict__ x, double* __restrict__ out, int64_t n) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = nb_digamma(x[i]);
+}
+__global__ void lgamma_kernel(const double* __restrict__ x, double* __restrict__ out, int64_t n) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = nb_lgamma(x[i]);
+}
+}  // namespace gpz
+
+// the NB kernels' own digamma / lgamma (x > 0), element-wise, for testing them against a reference
+extern "C" int gpz_digamma_f64(const double* x, double* out, int64_t n, void* stream) {
+  if (n <= 0) return GPZ_OK;
+  digamma_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>(x, out, n);
+  GPZ_CHECK_LAUNCH();
+  return GPZ_OK;
+}
+extern "C" int gpz_lgamma_f64(const double* x, double* out, int64_t n, void* stream) {
+  if (n <= 0) return GPZ_OK;
+  lgamma_kernel<<<(unsigned)cdiv(n, 256), 256, 0, (cudaStream_t)stream>>>(x, out, n);
+  GPZ_CHECK_LAUNCH();
+  return GPZ_OK;
 }
 
 // sparse counts (K7-CSC): count_kind 0 = T, 1 = uint8, 2 = int16, 3 = int32

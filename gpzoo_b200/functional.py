@@ -1073,41 +1073,12 @@ class PoissonLL(Function):
     def forward(ctx, y, idx, W, V, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma):
         W, V, mean, spread, eps = _c(W), _c(V), _c(mean), _c(spread), _c(eps)
         dt = W.dtype
-        G, F = W.shape
         if isinstance(y, SparseCounts):
             gW, gV, gmean, gspread, ll, idx = _poisson_csc(y, idx, W, V, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma)
             ctx.save_for_backward(gW, gV, gmean, gspread, idx)
             ctx.nV = V.shape[0]
             return ll.to(dt).reshape(())
-        # y: the reference passes floats; integer counts (uint8 / int16 / int32) are read as stored by the fp32 tensor-core kernel
-        # (F <= 16), any other combination is converted on the device
-        y_kind = PoissonLL.Y_KINDS.get(y.dtype, 0) if (dt == torch.float32 and F <= 16) else 0
-        if y_kind == 0 and y.dtype != dt:
-            y = y.to(dt)
-        y = _c(y)
-        B = mean.shape[1]
-        E = eps.shape[0]
-        assert y.shape[0] == G and mean.shape[0] == F and eps.shape[1] == F and eps.shape[2] == B
-        if idx is not None:
-            idx = _c(idx.to(device=W.device, dtype=torch.int64))
-        else:
-            assert y.shape[1] == B
-        lib = _cabi.lib()
-        suf = "f32" if dt == torch.float32 else "f64"
-        ws_bytes = int(getattr(lib, f"gpz_poisson_workspace_bytes_{suf}")(c_i(G), c_i(F), c_i(B), c_i(E)))
-        ws = torch.empty(ws_bytes // 8 + 1, dtype=torch.float64, device=W.device)
-        ll = torch.empty(1, dtype=torch.float64, device=W.device)
-        gW = torch.empty_like(W)
-        gV = torch.empty(B, dtype=dt, device=W.device)
-        gmean = torch.empty_like(mean)
-        gspread = torch.empty_like(spread)
-        tail = (c_i64(y.shape[1]), ptr(idx), ptr(W), c_i(int(w_softplus)), ptr(V), ptr(mean), ptr(spread), ptr(eps), c_i(G), c_i(F),
-                c_i(B), c_i(E), c_i(int(n_var)), scalar(dt, clamp_min), c_i(int(with_lgamma)), ptr(ll), ptr(gW), ptr(gV), ptr(gmean),
-                ptr(gspread), ptr(ws), c_i64(ws_bytes))
-        if y_kind:
-            call("poisson_fwdbwd_yt", dt, ptr(y), c_i(y_kind), *tail)
-        else:
-            call("poisson_fwdbwd", dt, ptr(y), *tail)
+        gW, gV, gmean, gspread, ll, idx, _ = _k7_dense(y, idx, W, V, None, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma)
         ctx.save_for_backward(gW, gV, gmean, gspread, idx)
         ctx.nV = V.shape[0]
         return ll.to(dt).reshape(())
@@ -1116,11 +1087,83 @@ class PoissonLL(Function):
     @once_differentiable
     def backward(ctx, g):
         gW, gV, gmean, gspread, idx = ctx.saved_tensors
-        if idx is not None:
-            full = torch.zeros(ctx.nV, dtype=gV.dtype, device=gV.device)
-            full.index_add_(0, idx, gV)
-            gV = full
-        return None, None, g * gW, g * gV, g * gmean, g * gspread, None, None, None, None, None
+        return None, None, g * gW, g * _scatter_gV(ctx.nV, gV, idx), g * gmean, g * gspread, None, None, None, None, None
+
+
+class NegBinLL(Function):
+    """mean_E sum_{g,n} negative-binomial log-lik of dense counts y under the same rate as PoissonLL and the per-gene dispersion
+    theta = softplus(D) (D: G, raw), with every gradient, dD included, from one pass (K7-NB, csrc/poisson.cu):
+    log NB = lgamma(y + theta) - lgamma(theta) - lgamma(y + 1) + y log(r / (theta + r)) - theta log1p(r / theta)."""
+
+    @staticmethod
+    def forward(ctx, y, idx, W, V, D, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma):
+        if isinstance(y, SparseCounts):
+            raise NotImplementedError(
+                "the negative-binomial likelihood needs dense counts: its zero counts each contribute -theta log1p(r / theta), "
+                "which has no closed form through the loadings' column sums the way the Poisson zeros' -r does, so the work is "
+                "G x N whatever the density; pass y.to_dense()")
+        W, V, D, mean, spread, eps = _c(W), _c(V), _c(D), _c(mean), _c(spread), _c(eps)
+        assert D.shape == (W.shape[0],) and D.dtype == W.dtype
+        gW, gV, gmean, gspread, ll, idx, gD = _k7_dense(y, idx, W, V, D, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma)
+        ctx.save_for_backward(gW, gV, gD, gmean, gspread, idx)
+        ctx.nV = V.shape[0]
+        return ll.to(W.dtype).reshape(())
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        gW, gV, gD, gmean, gspread, idx = ctx.saved_tensors
+        return (None, None, g * gW, g * _scatter_gV(ctx.nV, gV, idx), g * gD, g * gmean, g * gspread, None, None, None, None,
+                None)
+
+
+def _scatter_gV(nV, gV, idx):
+    """d/dV of the resident V from the minibatch's d/dV[idx] (a spot listed twice gets both contributions)."""
+    if idx is None:
+        return gV
+    full = torch.zeros(nV, dtype=gV.dtype, device=gV.device)
+    full.index_add_(0, idx, gV)
+    return full
+
+
+def _k7_dense(y, idx, W, V, D, mean, spread, eps, n_var, clamp_min, w_softplus, with_lgamma):
+    """K7 on a dense G x N count matrix: gpz_poisson_fwdbwd_* (D None) or gpz_negbin_fwdbwd_* (D the raw dispersion).
+    Returns gW, gV (minibatch), gmean, gspread, ll (one double), idx (int64 on the device or None) and gD (None for Poisson)."""
+    dt = W.dtype
+    G, F = W.shape
+    # y: the reference passes floats; integer counts (uint8 / int16 / int32) are read as stored by the fp32 tensor-core kernel
+    # (F <= 16), any other combination is converted on the device
+    y_kind = PoissonLL.Y_KINDS.get(y.dtype, 0) if (dt == torch.float32 and F <= 16) else 0
+    if y_kind == 0 and y.dtype != dt:
+        y = y.to(dt)
+    y = _c(y)
+    B = mean.shape[1]
+    E = eps.shape[0]
+    assert y.shape[0] == G and mean.shape[0] == F and eps.shape[1] == F and eps.shape[2] == B
+    if idx is not None:
+        idx = _c(idx.to(device=W.device, dtype=torch.int64))
+    else:
+        assert y.shape[1] == B
+    lib = _cabi.lib()
+    suf = "f32" if dt == torch.float32 else "f64"
+    name = "poisson" if D is None else "negbin"
+    ws_bytes = int(getattr(lib, f"gpz_{name}_workspace_bytes_{suf}")(c_i(G), c_i(F), c_i(B), c_i(E)))
+    ws = torch.empty(ws_bytes // 8 + 1, dtype=torch.float64, device=W.device)
+    ll = torch.empty(1, dtype=torch.float64, device=W.device)
+    gW = torch.empty_like(W)
+    gV = torch.empty(B, dtype=dt, device=W.device)
+    gD = None if D is None else torch.empty_like(D)
+    gmean = torch.empty_like(mean)
+    gspread = torch.empty_like(spread)
+    nb_in, nb_out = ((), ()) if D is None else ((ptr(D),), (ptr(gD),))
+    tail = (c_i64(y.shape[1]), ptr(idx), ptr(W), c_i(int(w_softplus)), ptr(V), *nb_in, ptr(mean), ptr(spread), ptr(eps), c_i(G),
+            c_i(F), c_i(B), c_i(E), c_i(int(n_var)), scalar(dt, clamp_min), c_i(int(with_lgamma)), ptr(ll), ptr(gW), ptr(gV), *nb_out,
+            ptr(gmean), ptr(gspread), ptr(ws), c_i64(ws_bytes))
+    if y_kind:
+        call(f"{name}_fwdbwd_yt", dt, ptr(y), c_i(y_kind), *tail)
+    else:
+        call(f"{name}_fwdbwd", dt, ptr(y), *tail)
+    return gW, gV, gmean, gspread, ll, idx, gD
 
 
 _CSC_KINDS = {torch.uint8: 1, torch.int16: 2, torch.int32: 3}      # count_kind of gpz_poisson_fwdbwd_csc_* (0 = the compute type)

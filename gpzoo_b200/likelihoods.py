@@ -11,6 +11,8 @@ Two ways to use them:
 """
 from __future__ import annotations
 
+import math
+
 import torch
 import torch.nn as nn
 from torch import distributions
@@ -77,7 +79,18 @@ class ExactLikelihood(nn.Module):
 # ------------------------------------------------------------------------------------------------
 # Poisson family
 # ------------------------------------------------------------------------------------------------
-class PoissonFactorization(nn.Module):
+class _PoissonCounts:
+    """The count model of the Poisson family: the fused likelihood call of `elbo` and the distribution `forward` returns.
+    The negative-binomial models override both (`_NegBinCounts`)."""
+
+    def _count_ll(self, y, idx, W, V, *args):
+        return F.PoissonLL.apply(y, idx, W, V, *args)
+
+    def _pY(self, rate):
+        return _poisson(rate)
+
+
+class PoissonFactorization(_PoissonCounts, nn.Module):
     """Base of PNMF / NSF2: loadings W (G x L), rate contraction softplus(W) @ exp(F) (likelihoods.py:39-53)."""
 
     _w_softplus = True
@@ -101,7 +114,7 @@ def _poisson(rate):
     return distributions.Poisson(rate, validate_args=False)
 
 
-class _FusedPoissonMixin:
+class _FusedPoissonMixin(_PoissonCounts):
     """Fused ELBO for models with one SVGP-family prior (NSF2 / NSF / MGGP_NSF)."""
 
     def _gp(self):
@@ -121,8 +134,8 @@ class _FusedPoissonMixin:
         if eps is None:
             eps = torch.randn((E,) + tuple(mean.shape), dtype=mean.dtype, device=mean.device)
         W = self.W.to(mean.dtype)
-        ll = F.PoissonLL.apply(y, idx, W, self.V.to(mean.dtype), mean, var, eps, mean.shape[0], gp.clamp_min,
-                               self._w_softplus, with_lgamma)
+        ll = self._count_ll(y, idx, W, self.V.to(mean.dtype), mean, var, eps, mean.shape[0], gp.clamp_min, self._w_softplus,
+                            with_lgamma)
         kl = _kl_of(m).to(mean.dtype)
         out = ll - kl_weight * kl.sum()
         if return_parts:
@@ -143,14 +156,14 @@ class PNMF(PoissonFactorization):
         qF, pF = self.prior()
         Fs = _sample(qF, E, eps)
         rate = F.poisson_rate(self.W, self.V, None, Fs, True)
-        return _poisson(rate), qF, pF
+        return self._pY(rate), qF, pF
 
     def elbo(self, y, idx=None, E=10, eps=None, with_lgamma=True):
         """mean_E sum log p(y|F) - sum KL(qF || pF), fused likelihood kernel (sd-mode factors)."""
         qF, pF = self.prior() if idx is None else self.prior.forward_batched(idx)
         if eps is None:
             eps = torch.randn((E,) + tuple(qF.loc.shape), dtype=qF.loc.dtype, device=qF.loc.device)
-        ll = F.PoissonLL.apply(y, idx, self.W, self.V, qF.loc, qF.scale, eps, 0, 0.0, True, with_lgamma)
+        ll = self._count_ll(y, idx, self.W, self.V, qF.loc, qF.scale, eps, 0, 0.0, True, with_lgamma)
         return ll - distributions.kl_divergence(qF, pF).sum()
 
 
@@ -166,13 +179,13 @@ class NSF2(_FusedPoissonMixin, PoissonFactorization):
         qF, qU, pU = _gp_call(self.prior, X, verbose, kwargs)
         Fs = _sample(qF, E, eps)
         rate = F.poisson_rate(self.W.to(Fs.dtype), self.V.to(Fs.dtype), None, Fs, True)
-        return _poisson(rate), qF, qU, pU
+        return self._pY(rate), qF, qU, pU
 
     def forward_batched(self, X, idx, E=10, verbose=False, eps=None, **kwargs):
         qF, qU, pU = _gp_call(self.prior, X[idx], verbose, kwargs)
         Fs = _sample(qF, E, eps)
         rate = F.poisson_rate(self.W.to(Fs.dtype), self.V.to(Fs.dtype), idx, Fs, True)
-        return _poisson(rate), qF, qU, pU
+        return self._pY(rate), qF, qU, pU
 
 
 class NSF(_FusedPoissonMixin, nn.Module):
@@ -208,7 +221,7 @@ class MGGP_NSF(NSF):
         return super().forward_batched(X, idx, E=E, verbose=verbose, eps=eps, groupsX=groupsX[idx])
 
 
-class Hybrid_NSF2(nn.Module):
+class Hybrid_NSF2(_PoissonCounts, nn.Module):
     """Spatial (GP) + non-spatial (GaussianPrior) factors (likelihoods.py:100-163)."""
 
     def __init__(self, gp, prior, y, L=10, T=10):
@@ -223,7 +236,7 @@ class Hybrid_NSF2(nn.Module):
         F2 = _sample(qF2, E, eps2)
         Fs = torch.cat((F1, F2), dim=1)
         W = torch.cat((self.sf.W, self.cf.W), dim=1).to(Fs.dtype)
-        return _poisson(F.poisson_rate(W, self.V.to(Fs.dtype), idx, Fs, True))
+        return self._pY(F.poisson_rate(W, self.V.to(Fs.dtype), idx, Fs, True))
 
     def forward(self, X, E=10, verbose=False, eps=None, eps2=None, **kwargs):
         qF1, qU, pU = _gp_call(self.sf.prior, X, verbose, kwargs)
@@ -261,8 +274,7 @@ class Hybrid_NSF2(nn.Module):
         mean = torch.cat((mean1, qF2.loc.to(dt)), 0)
         spread = torch.cat((var1, qF2.scale.to(dt)), 0)
         W = torch.cat((self.sf.W, self.cf.W), dim=1).to(dt)
-        ll = F.PoissonLL.apply(y, idx, W, self.V.to(dt), mean, spread, torch.cat((eps, eps2), 1), L, gp.clamp_min,
-                               True, with_lgamma)
+        ll = self._count_ll(y, idx, W, self.V.to(dt), mean, spread, torch.cat((eps, eps2), 1), L, gp.clamp_min, True, with_lgamma)
         kl = _kl_of(m).to(dt)
         return ll - kl_weight * kl.sum() - distributions.kl_divergence(qF2, pF2).sum()
 
@@ -330,3 +342,47 @@ class Hybrid_NSF(NSF):
                                with_lgamma)
         kl = _kl_of(m).to(dt)
         return ll - kl_weight * kl.sum() - distributions.kl_divergence(qF2, pF2).sum()
+
+
+# ------------------------------------------------------------------------------------------------
+# Negative binomial: the Poisson models with one dispersion per gene
+# ------------------------------------------------------------------------------------------------
+class _NegBinCounts:
+    """NB(y | r, theta_g) with theta = softplus(dispersion) (G, initialised to log(e - 1): theta = 1) in place of Poisson(r):
+    `elbo` runs the fused K7-NB call (functional.NegBinLL), `forward` returns
+    NegativeBinomial(total_count=theta[:, None], logits=log r - log theta[:, None]), whose mean is r.  In data-parallel training
+    `dispersion` is a shared gradient like W: include it in distributed.FlatGradReducer's list."""
+
+    def _init_dispersion(self, G):
+        self.dispersion = nn.Parameter(torch.full((G,), math.log(math.e - 1.0)))
+
+    def _count_ll(self, y, idx, W, V, *args):
+        return F.NegBinLL.apply(y, idx, W, V, self.dispersion.to(W.dtype), *args)      # SparseCounts: NotImplementedError
+
+    def _pY(self, rate):
+        theta = torch.nn.functional.softplus(self.dispersion.to(rate.dtype))[:, None]
+        return distributions.NegativeBinomial(total_count=theta, logits=rate.log() - theta.log(), validate_args=False)
+
+
+class NSF2_NB(_NegBinCounts, NSF2):
+    """NSF2 with a negative-binomial likelihood: any prior NSF2 takes (SVGP, VNNGP, MGGP_SVGP with groupsX, WSVGP)."""
+
+    def __init__(self, gp, y, L=10):
+        super().__init__(gp, y, L=L)
+        self._init_dispersion(y.shape[0])
+
+
+class PNMF_NB(_NegBinCounts, PNMF):
+    """PNMF with a negative-binomial likelihood."""
+
+    def __init__(self, prior, y, L=10):
+        super().__init__(prior, y, L=L)
+        self._init_dispersion(y.shape[0])
+
+
+class Hybrid_NSF2_NB(_NegBinCounts, Hybrid_NSF2):
+    """Hybrid_NSF2 with a negative-binomial likelihood."""
+
+    def __init__(self, gp, prior, y, L=10, T=10):
+        super().__init__(gp, prior, y, L=L, T=T)
+        self._init_dispersion(y.shape[0])

@@ -210,6 +210,28 @@ int gpz_poisson_fwdbwd_csc_f64(const int64_t* indptr, const int32_t* genes, cons
                                const double* spread, const double* eps, int G, int F, int B, int E, int n_var, double clamp_min,
                                int with_lgamma, double* ll, double* gW, double* gV, double* gmean, double* gspread, void* ws,
                                int64_t ws_bytes, void* stream);
+/* K7-NB: the same call with a negative-binomial likelihood, one dispersion per gene, theta_g = softplus(D_g):
+ *   log NB(y | r, theta) = lgamma(y + theta) - lgamma(theta) - lgamma(y + 1) + y log(r / (theta + r)) - theta log1p(r / theta)
+ *   ll = mean_e sum_{g,n} log NB; with_lgamma = 0 drops only lgamma(y + 1).  D (G, raw) is an input, gD = d ll / d D (G) an
+ *   output; every other argument and output as gpz_poisson_fwdbwd_*.  Dense counts only.  ws sized by gpz_negbin_workspace_bytes_*. */
+int64_t gpz_negbin_workspace_bytes_f32(int G, int F, int B, int E);
+int64_t gpz_negbin_workspace_bytes_f64(int G, int F, int B, int E);
+int gpz_negbin_fwdbwd_f32(const float* y, int64_t y_ld, const int64_t* idx, const float* W, int w_softplus, const float* V,
+                          const float* D, const float* mean, const float* spread, const float* eps, int G, int F, int B, int E,
+                          int n_var, float clamp_min, int with_lgamma, double* ll, float* gW, float* gV, float* gD, float* gmean,
+                          float* gspread, void* ws, int64_t ws_bytes, void* stream);
+int gpz_negbin_fwdbwd_f64(const double* y, int64_t y_ld, const int64_t* idx, const double* W, int w_softplus, const double* V,
+                          const double* D, const double* mean, const double* spread, const double* eps, int G, int F, int B, int E,
+                          int n_var, double clamp_min, int with_lgamma, double* ll, double* gW, double* gV, double* gD,
+                          double* gmean, double* gspread, void* ws, int64_t ws_bytes, void* stream);
+/* counts stored as integers (y_kind as gpz_poisson_fwdbwd_yt_f32; fp32, F <= 16) */
+int gpz_negbin_fwdbwd_yt_f32(const void* y, int y_kind, int64_t y_ld, const int64_t* idx, const float* W, int w_softplus,
+                             const float* V, const float* D, const float* mean, const float* spread, const float* eps, int G, int F,
+                             int B, int E, int n_var, float clamp_min, int with_lgamma, double* ll, float* gW, float* gV, float* gD,
+                             float* gmean, float* gspread, void* ws, int64_t ws_bytes, void* stream);
+/* the digamma and lgamma of the K7-NB kernels (x > 0), element-wise over n doubles on the device */
+int gpz_digamma_f64(const double* x, double* out, int64_t n, void* stream);
+int gpz_lgamma_f64(const double* x, double* out, int64_t n, void* stream);
 int gpz_poisson_rate_f32(const float* W, int w_softplus, const float* V, const int64_t* idx, const float* F, float* rate,
                          int G, int nF, int B, int E, void* stream);
 int gpz_poisson_rate_f64(const double* W, int w_softplus, const double* V, const int64_t* idx, const double* F, double* rate,
