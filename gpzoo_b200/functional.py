@@ -15,7 +15,7 @@ from torch.autograd import Function
 from torch.autograd.function import once_differentiable
 
 from . import _cabi
-from ._cabi import c_f, c_i, c_i64, c_p, call, ptr, scalar
+from ._cabi import call
 from .counts import SparseCounts
 
 # When True (default) a non-positive-definite Kzz raises torch.linalg.LinAlgError right away like the
@@ -179,15 +179,14 @@ def gemm(A, B, ta=False, tb=False, alpha=1.0, beta=0.0, out=None, a_tri=0, b_tri
             Ae, Ae_lo = transpose_lo(A)
         else:
             Ae, Ae_lo = A, tf32_lo(A)
-        call("umma_gemm", dt, c_i(int(tb)), c_i(m), c_i(n), c_i(k), c_f(alpha), ptr(Ae), ptr(Ae_lo), c_i64(k), c_i64(m * k),
-             ptr(B), ptr(tf32_lo(B)), c_i64(B.shape[2]), c_i64(B.shape[1] * B.shape[2]), ptr(out if beta == 1.0 else None),
-             ptr(out), ptr(None), c_i64(n), c_i64(m * n), c_i(bsz), c_i(a_tri), c_i(b_tri), c_i(d_tri), c_i(1), c_i(3))
+        call("umma_gemm", dt, int(tb), m, n, k, alpha, Ae, Ae_lo, k, m * k, B, tf32_lo(B), B.shape[2], B.shape[1] * B.shape[2],
+             out if beta == 1.0 else None, out, None, n, m * n, bsz, a_tri, b_tri, d_tri, 1, 3)
         return out
-    call("gemm", dt, c_i(int(ta)), c_i(int(tb)), c_i(m), c_i(n), c_i(k), scalar(dt, alpha),
-         ptr(A), c_i64(A.shape[2]), c_i64(A.shape[1] * A.shape[2]),
-         ptr(B), c_i64(B.shape[2]), c_i64(B.shape[1] * B.shape[2]),
-         scalar(dt, beta), ptr(out), c_i64(out.shape[2]), c_i64(out.shape[1] * out.shape[2]),
-         c_i(bsz), c_i(a_tri), c_i(b_tri), c_i(d_tri), c_i(splitk))
+    call("gemm", dt, int(ta), int(tb), m, n, k, alpha,
+         A, A.shape[2], A.shape[1] * A.shape[2],
+         B, B.shape[2], B.shape[1] * B.shape[2],
+         beta, out, out.shape[2], out.shape[1] * out.shape[2],
+         bsz, a_tri, b_tri, d_tri, splitk)
     return out
 
 
@@ -214,7 +213,7 @@ def transpose_lo(x):
 
     def make():
         xt, xt_lo = torch.empty_like(x), torch.empty_like(x)
-        call("transpose_lo", torch.float32, ptr(x), ptr(xt), ptr(xt_lo), c_i(x.shape[-1]), c_i(x.shape[0]))
+        call("transpose_lo", torch.float32, x, xt, xt_lo, x.shape[-1], x.shape[0])
         return xt, xt_lo
     return _cached("T", x, make)
 
@@ -280,14 +279,14 @@ def gemv(A, v, trans=False):
     A, v = _c(A), _c(v)
     L, rows, cols = A.shape
     out = torch.empty((L, cols if trans else rows), dtype=A.dtype, device=A.device)
-    call("gemv", A.dtype, c_i(int(trans)), ptr(A), ptr(v), ptr(out), c_i(rows), c_i(cols), c_i(L))
+    call("gemv", A.dtype, int(trans), A, v, out, rows, cols, L)
     return out
 
 
 def tri_op(X, mode, out=None):
     if out is None:
         out = torch.empty_like(X)
-    call("tri_op", X.dtype, ptr(X), ptr(out), c_i(X.shape[-1]), c_i(X.shape[0]), c_i(mode))
+    call("tri_op", X.dtype, X, out, X.shape[-1], X.shape[0], mode)
     return out
 
 
@@ -333,9 +332,8 @@ class KernelBuild(Function):
         out = torch.empty((L, n1, n2), dtype=dt, device=x1.device)
         want_lo = bool(want_lo) and dt == torch.float32
         out_lo = torch.empty_like(out) if want_lo else None
-        call("kernel_build_fwd", dt, ptr(x1), ptr(x2), ptr(sigma), ptr(ls), ptr(a if mg else None),
-             ptr(r2 if mg else None), ptr(g1 if mg else None), ptr(g2 if mg else None), c_i(n1), c_i(n2), c_i(D), c_i(L),
-             c_i(r2.shape[0] if mg else 0), c_i(int(kind)), scalar(dt, p_half), scalar(dt, jitter), ptr(out), ptr(out_lo))
+        call("kernel_build_fwd", dt, x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
+             g2 if mg else None, n1, n2, D, L, r2.shape[0] if mg else 0, int(kind), p_half, jitter, out, out_lo)
         ctx.save_for_backward(x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
                               g2 if mg else None)
         ctx.p_half = p_half
@@ -371,10 +369,8 @@ def _kernel_build_bwd(x1, x2, sigma, ls, a, r2, g1, g2, p_half, kind, need, G):
     g_ls = torch.empty_like(ls)
     g_a = torch.empty_like(a) if mg else None
     ws = torch.empty(3 * L + n1 * D, dtype=torch.float64, device=x1.device)
-    call("kernel_build_bwd", dt, ptr(x1), ptr(x2), ptr(sigma), ptr(ls), ptr(a), ptr(r2), ptr(g1), ptr(g2),
-         c_i(n1), c_i(n2), c_i(D), c_i(L), c_i(r2.shape[0] if mg else 0), c_i(int(kind)), scalar(dt, p_half),
-         ptr(G),
-         ptr(g_x1), ptr(g_x2), ptr(g_sigma), ptr(g_ls), ptr(g_a), ptr(ws))
+    call("kernel_build_bwd", dt, x1, x2, sigma, ls, a, r2, g1, g2, n1, n2, D, L, r2.shape[0] if mg else 0, int(kind), p_half, G,
+         g_x1, g_x2, g_sigma, g_ls, g_a, ws)
     return g_x1, g_x2, g_sigma, g_ls, g_a
 
 
@@ -409,9 +405,8 @@ class KernelBuildH(Function):
             a, r2, g1, g2 = _c(a), _c(r2), _c(g1), _c(g2)
         Kh, Kl = _plane_pair(L, n1, n2, x1.device)
         sK = torch.empty(L, dtype=dt, device=x1.device)
-        call("kernel_build_fwd_h", dt, ptr(x1), ptr(x2), ptr(sigma), ptr(ls), ptr(a if mg else None),
-             ptr(r2 if mg else None), ptr(g1 if mg else None), ptr(g2 if mg else None), c_i(n1), c_i(n2), c_i(D), c_i(L),
-             c_i(r2.shape[0] if mg else 0), c_i(int(kind)), scalar(dt, p_half), scalar(dt, jitter), ptr(Kh), ptr(Kl), ptr(sK))
+        call("kernel_build_fwd_h", dt, x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
+             g2 if mg else None, n1, n2, D, L, r2.shape[0] if mg else 0, int(kind), p_half, jitter, Kh, Kl, sK)
         ctx.save_for_backward(x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
                               g2 if mg else None)
         ctx.p_half = p_half
@@ -445,7 +440,7 @@ def cdist(x1, x2):
     """Euclidean distance matrix by direct differences (kernels.py:118 torch.cdist; no gradient)."""
     x1, x2 = _c(x1.detach()), _c(x2.detach())
     out = torch.empty((x1.shape[0], x2.shape[0]), dtype=x1.dtype, device=x1.device)
-    call("cdist", x1.dtype, ptr(x1), ptr(x2), ptr(out), c_i(x1.shape[0]), c_i(x2.shape[0]), c_i(x1.shape[1]))
+    call("cdist", x1.dtype, x1, x2, out, x1.shape[0], x2.shape[0], x1.shape[1])
     return out
 
 
@@ -465,9 +460,9 @@ class CholeskyInverse(Function):
         Lc, Linv, tmp = torch.empty_like(W), torch.empty_like(W), torch.empty_like(W)
         if USE_TENSOR_CORES and dt == torch.float32 and M > CHOL_TC_MIN_M and M % 4 == 0:
             lo_ws = torch.empty((4,) + tuple(W.shape), dtype=dt, device=W.device)      # lo planes shadowing W, Lc, Linv, tmp
-            call("chol_inv_tc", dt, ptr(W), ptr(Lc), ptr(Linv), ptr(tmp), ptr(lo_ws), c_i(M), c_i(L), ptr(info))
+            call("chol_inv_tc", dt, W, Lc, Linv, tmp, lo_ws, M, L, info)
         else:
-            call("chol_inv", dt, ptr(W), ptr(Lc), ptr(Linv), ptr(tmp), c_i(M), c_i(L), ptr(info))
+            call("chol_inv", dt, W, Lc, Linv, tmp, M, L, info)
         _track_info(info)
         if SYNC_CHECKS:
             check_cholesky_info()
@@ -494,7 +489,7 @@ class CholeskyInverse(Function):
 def chain_ok(dtype, M):
     """fp32 chains large enough for the fused two-call implementation (csrc/chain.cu)."""
     return (USE_TENSOR_CORES and FUSED_CHAIN and dtype == torch.float32
-            and bool(_cabi.lib().gpz_svgp_chain_supported(c_i(int(M)))))
+            and bool(_cabi.lib().gpz_svgp_chain_supported(int(M))))
 
 
 class SvgpChain(Function):
@@ -519,8 +514,7 @@ class SvgpChain(Function):
         aux = torch.empty((6, L, M, M), dtype=dt, device=dev)
         ws = torch.empty(((5 if chol_tc else 1) * L * M * M + 4 * L,), dtype=dt, device=dev)
         info = torch.empty(L, dtype=torch.int32, device=dev)
-        call("svgp_chain_fwd", dt, ptr(W), ptr(Lu_raw), ptr(mu), ptr(Lc), ptr(Linv), ptr(Lu), ptr(T), ptr(q), ptr(kl), ptr(aux),
-             ptr(ws), c_i(M), c_i(L), c_i(chol_tc), ptr(info))
+        call("svgp_chain_fwd", dt, W, Lu_raw, mu, Lc, Linv, Lu, T, q, kl, aux, ws, M, L, chol_tc, info)
         _track_info(info)
         if SYNC_CHECKS:
             check_cholesky_info()
@@ -543,8 +537,7 @@ class SvgpChain(Function):
         if grp is not None and torch.distributed.get_world_size(grp) > 1 and gLc is None and gLu is None:
             return SvgpChain._backward_sharded(grp, ctx.saved_tensors, gLinv, gT, gq, gkl, gKzz, gLu_raw, gmu) + (None,)
         ws = torch.empty((12 * L * M * M + 2 * L * M,), dtype=dt, device=dev)
-        call("svgp_chain_bwd", dt, ptr(Lc), ptr(Linv), ptr(Lu), ptr(T), ptr(q), ptr(mu), ptr(aux), ptr(gLc), ptr(gLinv), ptr(gLu),
-             ptr(gT), ptr(gq), ptr(gkl), ptr(gKzz), ptr(gLu_raw), ptr(gmu), ptr(ws), c_i(M), c_i(L))
+        call("svgp_chain_bwd", dt, Lc, Linv, Lu, T, q, mu, aux, gLc, gLinv, gLu, gT, gq, gkl, gKzz, gLu_raw, gmu, ws, M, L)
         return gKzz, gLu_raw, gmu, None
 
     @staticmethod
@@ -590,9 +583,8 @@ class SvgpChain(Function):
             gLu_o = torch.empty_like(gK_o)
             gmu_o = torch.empty((own, M), dtype=dt, device=dev)
             ws = torch.empty((12 * own * M * M + 2 * own * M,), dtype=dt, device=dev)
-            call("svgp_chain_bwd", dt, ptr(sl(Lc)), ptr(sl(Linv)), ptr(sl(Lu)), ptr(sl(T)), ptr(sl(q)), ptr(sl(mu)), ptr(aux_o),
-                 ptr(None), ptr(gLinv_o), ptr(None), ptr(gT_o), ptr(gq_o), ptr(gkl_o), ptr(gK_o), ptr(gLu_o), ptr(gmu_o), ptr(ws),
-                 c_i(M), c_i(own))
+            call("svgp_chain_bwd", dt, sl(Lc), sl(Linv), sl(Lu), sl(T), sl(q), sl(mu), aux_o, None, gLinv_o, None, gT_o, gq_o,
+                 gkl_o, gK_o, gLu_o, gmu_o, ws, M, own)
             gKzz[l0:l1], gLu_raw[l0:l1], gmu[l0:l1] = gK_o, gLu_o, gmu_o
         return gKzz, gLu_raw, gmu
 
@@ -636,16 +628,14 @@ class SvgpMomentsH(Function):
         aux = torch.empty((6, L, M, M), dtype=dt, device=dev)
         ws = torch.empty(((5 if chol_tc else 1) * L * M * M + 4 * L,), dtype=dt, device=dev)
         info = torch.empty(L, dtype=torch.int32, device=dev)
-        call("svgp_chain_fwd", dt, ptr(W), ptr(Lu_raw), ptr(mu), ptr(Lc), ptr(Linv), ptr(Lu), ptr(T), ptr(q), ptr(kl), ptr(aux),
-             ptr(ws), c_i(M), c_i(L), c_i(chol_tc), ptr(info))
+        call("svgp_chain_fwd", dt, W, Lu_raw, mu, Lc, Linv, Lu, T, q, kl, aux, ws, M, L, chol_tc, info)
         _track_info(info)
         (Ah, Al), (Ch, Cl) = _plane_pair(L, M, N, dev), _plane_pair(L, M, N, dev)
         mean = torch.empty((L, N), dtype=dt, device=dev)
         var = torch.empty_like(mean)
         ws_h = torch.empty(8 * L * M * M, dtype=torch.float16, device=dev)
         ws_f = torch.empty(2 * L * N + 16 * L, dtype=dt, device=dev)
-        call("svgp_predict_fwd_h", dt, ptr(Kh), ptr(Kl), ptr(sK), ptr(Linv), ptr(T), ptr(q), ptr(Kxx), ptr(Ah), ptr(Al), ptr(Ch),
-             ptr(Cl), ptr(mean), ptr(var), ptr(ws_h), ptr(ws_f), c_i(M), c_i(N), c_i(L))
+        call("svgp_predict_fwd_h", dt, Kh, Kl, sK, Linv, T, q, Kxx, Ah, Al, Ch, Cl, mean, var, ws_h, ws_f, M, N, L)
         st = ws_f[2 * L * N:].view(-1, L)
         r_sA, r_aA, r_aC, r_sC = (_stat_row(i) for i in (0, 1, 2, 5))
         _track_amax(torch.stack((st[r_aA], st[r_aC])), torch.stack((st[r_sA], st[r_sC])), ("A", "C"))
@@ -681,9 +671,8 @@ class SvgpMomentsH(Function):
                 "moments_gKzx", (L, M, N), dt, dev)
         gqp = torch.empty((L, M), dtype=dt, device=dev)
         S = _workspace("moments_bwd_S", (2, L, M, M), dt, dev)              # S1 and its lo plane
-        call("svgp_predict_bwd_h", dt, ptr(Kh), ptr(Kl), ptr(sK), ptr(T), ptr(q), ptr(Ah), ptr(Al), ptr(Ch), ptr(Cl), ptr(gm), ptr(gv),
-             ptr(AWh), ptr(AWl), ptr(gAh), ptr(gAl), ptr(gKzx), ptr(None), ptr(None), ptr(gqp), ptr(ws_h), ptr(ws_f), ptr(S),
-             c_i(M), c_i(N), c_i(L))
+        call("svgp_predict_bwd_h", dt, Kh, Kl, sK, T, q, Ah, Al, Ch, Cl, gm, gv, AWh, AWl, gAh, gAl, gKzx, None, None, gqp, ws_h,
+             ws_f, S, M, N, L)
         stt = ws_f[2 * L * N:].view(-1, L)
         _track_amax(stt[_stat_row(4)].unsqueeze(0), stt[_stat_row(3)].unsqueeze(0), ("dL/dA",))
         if early:
@@ -701,8 +690,7 @@ class SvgpMomentsH(Function):
         gLu_raw = torch.empty_like(gKzz)
         gmu = torch.empty((L, M), dtype=dt, device=dev)
         ws = _workspace("chain_bwd_s1_ws", (13 * L * M * M + 2 * L * M,), dt, dev)
-        call("svgp_chain_bwd_s1", dt, ptr(Lc), ptr(Linv), ptr(Lu), ptr(T), ptr(q), ptr(mu), ptr(aux), ptr(S[0]), ptr(S[1]), ptr(gqp),
-             ptr(gkl), ptr(gLc), ptr(gLu), ptr(gKzz), ptr(gLu_raw), ptr(gmu), ptr(ws), c_i(M), c_i(L))
+        call("svgp_chain_bwd_s1", dt, Lc, Linv, Lu, T, q, mu, aux, S[0], S[1], gqp, gkl, gLc, gLu, gKzz, gLu_raw, gmu, ws, M, L)
         return gKzz, gLu_raw, gmu, gv, g_handle, None, None, None, None, None
 
 
@@ -713,7 +701,7 @@ class LowerCholesky(Function):
     def forward(ctx, raw):
         raw = _c(raw)
         out = torch.empty_like(raw)
-        call("lower_cholesky_fwd", raw.dtype, ptr(raw), ptr(out), c_i(raw.shape[-1]), c_i(raw.shape[0]))
+        call("lower_cholesky_fwd", raw.dtype, raw, out, raw.shape[-1], raw.shape[0])
         ctx.save_for_backward(out)
         return out
 
@@ -723,7 +711,7 @@ class LowerCholesky(Function):
         (out,) = ctx.saved_tensors
         g = _c(g)
         graw = torch.empty_like(g)
-        call("lower_cholesky_bwd", g.dtype, ptr(g), ptr(out), ptr(graw), c_i(g.shape[-1]), c_i(g.shape[0]))
+        call("lower_cholesky_bwd", g.dtype, g, out, graw, g.shape[-1], g.shape[0])
         return graw
 
 
@@ -761,7 +749,7 @@ class Whiten(Function):
 # ------------------------------------------------------------------------------------------------
 def tensor_core_predict_ok(dtype, M, N):
     return (USE_TENSOR_CORES and dtype == torch.float32
-            and bool(_cabi.lib().gpz_svgp_predict_tc_supported(c_i(int(M)), c_i(int(N)))))
+            and bool(_cabi.lib().gpz_svgp_predict_tc_supported(int(M), int(N))))
 
 
 class Predict(Function):
@@ -783,12 +771,10 @@ class Predict(Function):
             Kzx_lo = _c(Kzx_lo)
             A_lo = torch.empty_like(Kzx)
             ws = torch.empty(6 * L * M * M + 2 * L * N, dtype=dt, device=Kzx.device)
-            call("svgp_predict_fwd_tc", dt, ptr(Kzx), ptr(Kzx_lo), ptr(Linv), ptr(T), ptr(q), ptr(Kxx), ptr(A), ptr(A_lo), ptr(C),
-                 ptr(mean), ptr(var), ptr(ws), c_i(M), c_i(N), c_i(L))
+            call("svgp_predict_fwd_tc", dt, Kzx, Kzx_lo, Linv, T, q, Kxx, A, A_lo, C, mean, var, ws, M, N, L)
             ctx.save_for_backward(Kzx, Linv, T, q, A, C, Kzx_lo, A_lo, ws)
         else:
-            call("svgp_predict_fwd", dt, ptr(Kzx), ptr(Linv), ptr(T), ptr(q), ptr(Kxx), ptr(A), ptr(C), ptr(mean), ptr(var),
-                 c_i(M), c_i(N), c_i(L))
+            call("svgp_predict_fwd", dt, Kzx, Linv, T, q, Kxx, A, C, mean, var, M, N, L)
             ctx.save_for_backward(Kzx, Linv, T, q, A, C)
         return mean, var
 
@@ -814,22 +800,21 @@ class Predict(Function):
         if ctx.tc:
             C_lo = torch.empty_like(Kzx)
             gA_lo = torch.empty_like(Kzx)
-            call("svgp_predict_bwd_tc", dt, ptr(Kzx), ptr(Kzx_lo), ptr(Linv), ptr(T), ptr(q), ptr(A), ptr(A_lo), ptr(C), ptr(C_lo),
-                 ptr(gm), ptr(gv), ptr(gA), ptr(gA_lo), ptr(gKzx), ptr(gLinv), ptr(gT), ptr(gq), ptr(ws), c_i(M), c_i(N), c_i(L))
+            call("svgp_predict_bwd_tc", dt, Kzx, Kzx_lo, Linv, T, q, A, A_lo, C, C_lo, gm, gv, gA, gA_lo, gKzx, gLinv, gT, gq, ws,
+                 M, N, L)
         else:
-            call("svgp_predict_bwd", dt, ptr(Kzx), ptr(Linv), ptr(T), ptr(q), ptr(A), ptr(C), ptr(gm), ptr(gv), ptr(gA),
-                 ptr(gKzx), ptr(gLinv), ptr(gT), ptr(gq), c_i(M), c_i(N), c_i(L))
+            call("svgp_predict_bwd", dt, Kzx, Linv, T, q, A, C, gm, gv, gA, gKzx, gLinv, gT, gq, M, N, L)
         return gv, gKzx, gLinv, gT, gq, None
 
 
 def predict_h_ok(dtype, M, N):
     """fp32 problems large and aligned enough for the split-FP16 tcgen05 path."""
     return (USE_TENSOR_CORES and TENSOR_CORE_ARITH == "fp16x3" and dtype == torch.float32
-            and bool(_cabi.lib().gpz_svgp_predict_h_supported(c_i(int(M)), c_i(int(N)))))
+            and bool(_cabi.lib().gpz_svgp_predict_h_supported(int(M), int(N))))
 
 
 def _stat_row(which):
-    return int(_cabi.lib().gpz_svgp_predict_h_stat_row(c_i(which)))
+    return int(_cabi.lib().gpz_svgp_predict_h_stat_row(which))
 
 
 class PredictH(Function):
@@ -847,8 +832,7 @@ class PredictH(Function):
         var = torch.empty_like(mean)
         ws_h = torch.empty(8 * L * M * M, dtype=torch.float16, device=dev)
         ws_f = torch.empty(2 * L * N + 16 * L, dtype=dt, device=dev)
-        call("svgp_predict_fwd_h", dt, ptr(Kh), ptr(Kl), ptr(sK), ptr(Linv), ptr(T), ptr(q), ptr(Kxx), ptr(Ah), ptr(Al), ptr(Ch),
-             ptr(Cl), ptr(mean), ptr(var), ptr(ws_h), ptr(ws_f), c_i(M), c_i(N), c_i(L))
+        call("svgp_predict_fwd_h", dt, Kh, Kl, sK, Linv, T, q, Kxx, Ah, Al, Ch, Cl, mean, var, ws_h, ws_f, M, N, L)
         ctx.save_for_backward(Kh, Kl, sK, Linv, T, q, Ah, Al, Ch, Cl, ws_h, ws_f)
         # tracked max |A|, max |C| (slots 7, 8 of the stats block, csrc/predict.cu): examined lazily with the Cholesky info
         st = ws_f[2 * L * N:].view(-1, L)
@@ -872,9 +856,8 @@ class PredictH(Function):
         gLinv = torch.zeros_like(Linv)
         gT = torch.zeros_like(T)
         gq = torch.empty_like(q)
-        call("svgp_predict_bwd_h", dt, ptr(Kh), ptr(Kl), ptr(sK), ptr(T), ptr(q), ptr(Ah), ptr(Al), ptr(Ch), ptr(Cl), ptr(gm), ptr(gv),
-             ptr(AWh), ptr(AWl), ptr(gAh), ptr(gAl), ptr(gKzx), ptr(gLinv), ptr(gT), ptr(gq), ptr(ws_h), ptr(ws_f), ptr(None),
-             c_i(M), c_i(N), c_i(L))
+        call("svgp_predict_bwd_h", dt, Kh, Kl, sK, T, q, Ah, Al, Ch, Cl, gm, gv, AWh, AWl, gAh, gAl, gKzx, gLinv, gT, gq, ws_h,
+             ws_f, None, M, N, L)
         st = ws_f[2 * L * N:].view(-1, L)
         _track_amax(st[_stat_row(4)].unsqueeze(0), st[_stat_row(3)].unsqueeze(0), ("dL/dA",))   # max |gA| vs its scale
         return gv, gKzx, gLinv, gT, gq, None, None, None
@@ -891,9 +874,8 @@ def umma_gemm(A, B, b_kmajor, Alo=None, Blo=None, Cin=None, alpha=1.0, want_lo=F
         Blo = lo(B) if Blo is None else Blo
     D = torch.zeros((bsz, m, n), dtype=torch.float32, device=A.device)
     Dlo = torch.empty_like(D) if want_lo else None
-    call("umma_gemm", torch.float32, c_i(int(b_kmajor)), c_i(m), c_i(n), c_i(k), c_f(alpha), ptr(A), ptr(Alo), c_i64(A.shape[2]),
-         c_i64(A.shape[1] * A.shape[2]), ptr(B), ptr(Blo), c_i64(B.shape[2]), c_i64(B.shape[1] * B.shape[2]), ptr(Cin), ptr(D),
-         ptr(Dlo), c_i64(n), c_i64(m * n), c_i(bsz), c_i(a_tri), c_i(b_tri), c_i(d_tri), c_i(splitk), c_i(n_terms))
+    call("umma_gemm", torch.float32, int(b_kmajor), m, n, k, alpha, A, Alo, A.shape[2], A.shape[1] * A.shape[2], B, Blo,
+         B.shape[2], B.shape[1] * B.shape[2], Cin, D, Dlo, n, m * n, bsz, a_tri, b_tri, d_tri, splitk, n_terms)
     return (D, Dlo) if want_lo else D
 
 
@@ -909,7 +891,7 @@ def split16(x, transpose=False):
     lT = torch.empty_like(hT) if transpose else None
     scale = torch.empty(bsz, dtype=torch.float32, device=x.device)
     ws = torch.empty(bsz, dtype=torch.int32, device=x.device)
-    call("split16", torch.float32, ptr(x), c_i(rows), c_i(cols), c_i(bsz), ptr(h), ptr(l), ptr(hT), ptr(lT), ptr(scale), ptr(ws))
+    call("split16", torch.float32, x, rows, cols, bsz, h, l, hT, lT, scale, ws)
     return (h, l, hT, lT, scale) if transpose else (h, l, scale)
 
 
@@ -926,10 +908,9 @@ def umma_gemm16(A, B, b_kmajor, a_tri=0, b_tri=0, d_tri=0, splitk=1, n_terms=3, 
     Dh = torch.zeros((bsz, m, n), dtype=torch.float16, device=dev) if out_planes else None
     Dl = torch.zeros_like(Dh) if out_planes else None
     amax = torch.zeros(bsz, dtype=torch.int32, device=dev) if want_amax else None
-    call("umma_gemm16", torch.float32, c_i(int(b_kmajor)), c_i(m), c_i(n), c_i(k), c_f(alpha), ptr(Ah), ptr(Al), c_i64(Ah.shape[2]),
-         c_i64(Ah.shape[1] * Ah.shape[2]), ptr(sa), ptr(Bh), ptr(Bl), c_i64(Bh.shape[2]), c_i64(Bh.shape[1] * Bh.shape[2]), ptr(sb),
-         ptr(Cin), ptr(D), ptr(Dh), ptr(Dl), ptr(out_scale), ptr(amax), c_i64(n), c_i64(m * n), c_i(bsz), c_i(a_tri), c_i(b_tri),
-         c_i(d_tri), c_i(splitk), c_i(n_terms))
+    call("umma_gemm16", torch.float32, int(b_kmajor), m, n, k, alpha, Ah, Al, Ah.shape[2], Ah.shape[1] * Ah.shape[2], sa, Bh, Bl,
+         Bh.shape[2], Bh.shape[1] * Bh.shape[2], sb, Cin, D, Dh, Dl, out_scale, amax, n, m * n, bsz, a_tri, b_tri, d_tri, splitk,
+         n_terms)
     res = (Dh, Dl) if out_planes else D
     return (res, amax.view(torch.float32)) if want_amax else res
 
@@ -960,7 +941,7 @@ def tf32_lo(x):
 
     def make():
         lo = torch.empty_like(x)
-        call("tf32_lo", torch.float32, ptr(x), ptr(lo), c_i64(x.numel()))
+        call("tf32_lo", torch.float32, x, lo, x.numel())
         return lo
     return _cached("lo", x, make) if x.dim() == 3 and x.shape[-1] == x.shape[-2] else make()
 
@@ -972,7 +953,7 @@ def vnngp_neighbors(X, Z, K):
     """K nearest inducing points of every x (ascending distance, ties to the lower index) — gp.py:64."""
     X, Z = _c(X.detach()), _c(Z.detach())
     idx = torch.empty((X.shape[0], K), dtype=torch.int64, device=X.device)
-    call("vnngp_neighbors", X.dtype, ptr(X), ptr(Z), ptr(idx), c_i(X.shape[0]), c_i(Z.shape[0]), c_i(X.shape[1]), c_i(K))
+    call("vnngp_neighbors", X.dtype, X, Z, idx, X.shape[0], Z.shape[0], X.shape[1], K)
     return idx
 
 
@@ -1007,8 +988,7 @@ class VnngpPredict(Function):
         K = nn.shape[1]
         mean = torch.empty((L, N), dtype=dt, device=X.device)
         var = torch.empty_like(mean)
-        call("vnngp_fwd", dt, ptr(X), ptr(Z), ptr(sigma), ptr(ls), ptr(Kzz), ptr(S), ptr(mu), ptr(Kxx), ptr(nn), c_i(N), c_i(M),
-             c_i(D), c_i(L), c_i(K), scalar(dt, jitter), ptr(mean), ptr(var))
+        call("vnngp_fwd", dt, X, Z, sigma, ls, Kzz, S, mu, Kxx, nn, N, M, D, L, K, jitter, mean, var)
         ctx.save_for_backward(X, Z, sigma, ls, Kzz, S, mu, Kxx, nn)
         ctx.jitter = jitter
         return mean, var
@@ -1026,8 +1006,7 @@ class VnngpPredict(Function):
         gKzz, gS = torch.empty_like(Kzz), torch.empty_like(S)
         gmu, gZ = torch.empty_like(mu), torch.empty_like(Z)
         gsl = torch.empty(2 * L, dtype=torch.float64, device=X.device)
-        call("vnngp_bwd", dt, ptr(X), ptr(Z), ptr(sigma), ptr(ls), ptr(Kzz), ptr(S), ptr(mu), ptr(Kxx), ptr(nn), c_i(N), c_i(M),
-             c_i(D), c_i(L), c_i(K), scalar(dt, ctx.jitter), ptr(gm), ptr(gv), ptr(gKzz), ptr(gS), ptr(gmu), ptr(gZ), ptr(gsl))
+        call("vnngp_bwd", dt, X, Z, sigma, ls, Kzz, S, mu, Kxx, nn, N, M, D, L, K, ctx.jitter, gm, gv, gKzz, gS, gmu, gZ, gsl)
         return None, gZ, gsl[:L].to(dt), gsl[L:].to(dt), gKzz, gS, gmu, gv, None, None
 
 
@@ -1043,7 +1022,7 @@ class MvnKL(Function):
         L, M, _ = T.shape
         kl = torch.empty(L, dtype=T.dtype, device=T.device)
         ws = torch.empty(L, dtype=torch.float64, device=T.device)
-        call("mvn_kl_fwd", T.dtype, ptr(T), ptr(q), ptr(Lc), ptr(Lu), ptr(kl), ptr(ws), c_i(M), c_i(L))
+        call("mvn_kl_fwd", T.dtype, T, q, Lc, Lu, kl, ws, M, L)
         ctx.save_for_backward(T, q, Lc, Lu)
         return kl
 
@@ -1054,8 +1033,7 @@ class MvnKL(Function):
         L, M, _ = T.shape
         g = _c(g)
         gT, gLc, gLu, gq = torch.empty_like(T), torch.empty_like(T), torch.empty_like(T), torch.empty_like(q)
-        call("mvn_kl_bwd", T.dtype, ptr(g), ptr(T), ptr(q), ptr(Lc), ptr(Lu), ptr(gT), ptr(gq), ptr(gLc), ptr(gLu),
-             c_i(M), c_i(L))
+        call("mvn_kl_bwd", T.dtype, g, T, q, Lc, Lu, gT, gq, gLc, gLu, M, L)
         return gT, gq, gLc, gLu
 
 
@@ -1147,7 +1125,7 @@ def _k7_dense(y, idx, W, V, D, mean, spread, eps, n_var, clamp_min, w_softplus, 
     lib = _cabi.lib()
     suf = "f32" if dt == torch.float32 else "f64"
     name = "poisson" if D is None else "negbin"
-    ws_bytes = int(getattr(lib, f"gpz_{name}_workspace_bytes_{suf}")(c_i(G), c_i(F), c_i(B), c_i(E)))
+    ws_bytes = int(getattr(lib, f"gpz_{name}_workspace_bytes_{suf}")(G, F, B, E))
     ws = torch.empty(ws_bytes // 8 + 1, dtype=torch.float64, device=W.device)
     ll = torch.empty(1, dtype=torch.float64, device=W.device)
     gW = torch.empty_like(W)
@@ -1155,14 +1133,13 @@ def _k7_dense(y, idx, W, V, D, mean, spread, eps, n_var, clamp_min, w_softplus, 
     gD = None if D is None else torch.empty_like(D)
     gmean = torch.empty_like(mean)
     gspread = torch.empty_like(spread)
-    nb_in, nb_out = ((), ()) if D is None else ((ptr(D),), (ptr(gD),))
-    tail = (c_i64(y.shape[1]), ptr(idx), ptr(W), c_i(int(w_softplus)), ptr(V), *nb_in, ptr(mean), ptr(spread), ptr(eps), c_i(G),
-            c_i(F), c_i(B), c_i(E), c_i(int(n_var)), scalar(dt, clamp_min), c_i(int(with_lgamma)), ptr(ll), ptr(gW), ptr(gV), *nb_out,
-            ptr(gmean), ptr(gspread), ptr(ws), c_i64(ws_bytes))
+    nb_in, nb_out = ((), ()) if D is None else ((D,), (gD,))
+    tail = (y.shape[1], idx, W, int(w_softplus), V, *nb_in, mean, spread, eps, G, F, B, E, int(n_var), clamp_min,
+            int(with_lgamma), ll, gW, gV, *nb_out, gmean, gspread, ws, ws_bytes)
     if y_kind:
-        call(f"{name}_fwdbwd_yt", dt, ptr(y), c_i(y_kind), *tail)
+        call(f"{name}_fwdbwd_yt", dt, y, y_kind, *tail)
     else:
-        call(f"{name}_fwdbwd", dt, ptr(y), *tail)
+        call(f"{name}_fwdbwd", dt, y, *tail)
     return gW, gV, gmean, gspread, ll, idx, gD
 
 
@@ -1184,15 +1161,14 @@ def _poisson_csc(y, idx, W, V, mean, spread, eps, n_var, clamp_min, w_softplus, 
     kind = _CSC_KINDS.get(vals.dtype, 0)
     if kind == 0 and vals.dtype != dt:
         vals = vals.to(dt)
-    ws_bytes = int(getattr(_cabi.lib(), "gpz_poisson_csc_workspace_bytes_" + ("f32" if dt == torch.float32 else "f64"))(
-        c_i(G), c_i(F), c_i(B), c_i(E)))
+    suf = "f32" if dt == torch.float32 else "f64"
+    ws_bytes = int(getattr(_cabi.lib(), "gpz_poisson_csc_workspace_bytes_" + suf)(G, F, B, E))
     ws = torch.empty(ws_bytes // 8 + 1, dtype=torch.float64, device=W.device)
     ll = torch.empty(1, dtype=torch.float64, device=W.device)
     gW, gV = torch.empty_like(W), torch.empty(B, dtype=dt, device=W.device)
     gmean, gspread = torch.empty_like(mean), torch.empty_like(spread)
-    call("poisson_fwdbwd_csc", dt, ptr(y.indptr), ptr(y.genes), ptr(_c(vals)), c_i(kind), c_i64(N), ptr(idx), ptr(W),
-         c_i(int(w_softplus)), ptr(V), ptr(mean), ptr(spread), ptr(eps), c_i(G), c_i(F), c_i(B), c_i(E), c_i(int(n_var)),
-         scalar(dt, clamp_min), c_i(int(with_lgamma)), ptr(ll), ptr(gW), ptr(gV), ptr(gmean), ptr(gspread), ptr(ws), c_i64(ws_bytes))
+    call("poisson_fwdbwd_csc", dt, y.indptr, y.genes, _c(vals), kind, N, idx, W, int(w_softplus), V, mean, spread, eps, G, F, B,
+         E, int(n_var), clamp_min, int(with_lgamma), ll, gW, gV, gmean, gspread, ws, ws_bytes)
     return gW, gV, gmean, gspread, ll, idx
 
 
@@ -1212,8 +1188,7 @@ class _PoissonRate(Function):
         if idx is not None:
             idx = _c(idx.to(device=W.device, dtype=torch.int64))
         rate = torch.empty((E, G, B), dtype=dt, device=W.device)
-        call("poisson_rate", dt, ptr(W), c_i(int(w_softplus)), ptr(V), ptr(idx), ptr(F), ptr(rate), c_i(G), c_i(nF), c_i(B),
-             c_i(E))
+        call("poisson_rate", dt, W, int(w_softplus), V, idx, F, rate, G, nF, B, E)
         ctx.save_for_backward(W, V, F, idx, rate)
         ctx.w_softplus = w_softplus
         return rate

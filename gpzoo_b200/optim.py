@@ -51,6 +51,6 @@ class Adam(torch.optim.Optimizer):
                 numel = (ctypes.c_int64 * n)(*[p.numel() for p, _, _ in items])
                 clamp = (ctypes.c_int * n)(*[1 if id(p) in self._clamp_ids else 0 for p, _, _ in items])
                 b1, b2 = group["betas"]
-                _cabi.call("adam_step", dtype, ctypes.c_int(n), P, G, M1, M2, numel, clamp, ctypes.c_double(group["lr"]),
-                           ctypes.c_double(b1), ctypes.c_double(b2), ctypes.c_double(group["eps"]), ctypes.c_int(step))
+                _cabi.call("adam_step", dtype, n, P, G, M1, M2, numel, clamp, float(group["lr"]), float(b1), float(b2),
+                           float(group["eps"]), step)
         return loss

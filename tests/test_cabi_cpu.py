@@ -24,6 +24,105 @@ def test_exports_match_header(lib):
     assert b"success" in lib.gpz_error_string(0)
 
 
+def test_every_prototype_binds(lib):
+    """Each declared symbol gets the header's types: one argtype per parameter (counted here from the raw prototype text) and
+    the C return type; every entry point that takes a stream takes it last, as `call()` appends it."""
+    import ctypes
+    import re
+    from gpzoo_b200 import _cabi
+    txt = open(_cabi.HEADER).read()
+    special = {"gpz_error_string": ctypes.c_char_p, "gpz_launch_count": ctypes.c_longlong}
+    for sym, proto in _cabi.prototypes().items():
+        fn = getattr(lib, sym)
+        plist = re.search(rf"\b{sym}\s*\(([^)]*)\)\s*;", txt).group(1).strip()
+        n = 0 if plist == "void" else plist.count(",") + 1
+        assert len(fn.argtypes) == n == len(proto.params), sym
+        want = special.get(sym, ctypes.c_int64 if "_workspace_bytes_" in sym else ctypes.c_int)
+        assert fn.restype is want, (sym, fn.restype)
+        names = [p.name for p in proto.params]
+        if "stream" in names:
+            assert names.index("stream") == n - 1 and proto.params[-1].ctype == "void*", sym
+    assert lib.gpz_error_string.argtypes == (ctypes.c_int,)
+    assert len(lib.gpz_umma_gemm_f32.argtypes) == 25 and len(lib.gpz_adam_step_f64.argtypes) == 13
+
+
+def test_header_parser_rejects_unknown_types():
+    from gpzoo_b200 import _cabi
+    ok = _cabi.parse_header("/* c */\n#define X 1\nlong long gpz_a(void);\nint gpz_b_f32(void* const* t, const int64_t* n, "
+                            "double x, void* stream);")
+    assert set(ok) == {"gpz_a", "gpz_b_f32"} and ok["gpz_a"].params == ()
+    assert [(p.name, p.ctype) for p in ok["gpz_b_f32"].params] == [("t", "void**"), ("n", "int64_t*"), ("x", "double"),
+                                                                    ("stream", "void*")]
+    with pytest.raises(_cabi.GpzError, match=r"half\*.*gpz_c_f32"):
+        _cabi.parse_header("int gpz_c_f32(const half* x, int n, void* stream);")
+    with pytest.raises(_cabi.GpzError, match=r"unsigned.*gpz_d"):
+        _cabi.parse_header("unsigned gpz_d(void);")
+
+
+@pytest.fixture
+def no_stream(monkeypatch):
+    """`call()` without a CUDA stream.  Every call below fails a check before the library is entered; its sizes are all 0, so
+    even a call that got through would launch nothing and touch no memory."""
+    from gpzoo_b200 import _cabi
+    monkeypatch.setattr(_cabi, "stream", lambda: None)
+
+
+def test_call_checks_argument_count(lib, no_stream):
+    from gpzoo_b200 import _cabi
+    # gpz_tri_op_f32(const float* in, float* out, int M, int L, int mode, void* stream)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_tri_op_f32 takes 5 arguments before the stream, got 6"):
+        _cabi.call("tri_op", torch.float32, None, None, 0, 0, 0, 0)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_tri_op_f32 takes 5 arguments before the stream, got 4"):
+        _cabi.call("tri_op", torch.float32, None, None, 0, 0)
+
+
+def test_call_checks_argument_types(lib, no_stream):
+    from gpzoo_b200 import _cabi
+    f64 = torch.zeros(4, dtype=torch.float64)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_tri_op_f32: parameter in is float\*, got a torch.float64 tensor"):
+        _cabi.call("tri_op", torch.float32, f64, None, 0, 0, 0)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_tri_op_f64: parameter out is double\*, got a torch.float32 tensor"):
+        _cabi.call("tri_op", torch.float64, None, f64.float(), 0, 0, 0)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_chol_inv_f32: parameter info is int\*, got a torch.int64 tensor"):
+        _cabi.call("chol_inv", torch.float32, None, None, None, None, 0, 0, torch.zeros(1, dtype=torch.int64))
+    # void* takes any dtype: these get past the dtype check and stop at the CUDA check
+    for dt in (torch.float16, torch.uint8, torch.int16, torch.float64):
+        with pytest.raises(_cabi.GpzError, match="need CUDA tensors"):
+            _cabi.call("split16", torch.float32, None, 0, 0, 0, torch.zeros(4, dtype=dt), None, None, None, None, None)
+    with pytest.raises(_cabi.GpzError, match="need CUDA tensors"):
+        _cabi.call("tri_op", torch.float32, f64.float(), None, 0, 0, 0)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_tri_op_f32: parameter M \(int\)"):
+        _cabi.call("tri_op", torch.float32, None, None, 0.0, 0, 0)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_tri_op_f32: parameter M is int, got a tensor"):
+        _cabi.call("tri_op", torch.float32, None, None, torch.zeros(()), 0, 0)
+    with pytest.raises(_cabi.GpzError, match=r"gpz_tri_op_f32: parameter in is float\*, got int"):
+        _cabi.call("tri_op", torch.float32, 0, None, 0, 0, 0)
+
+
+def test_literal_call_sites_match_the_header():
+    """Every `call("<literal>", dtype, ...)` in the package names a declared entry point, with one argument per parameter before
+    the stream wherever the arguments are written out."""
+    import ast
+    import glob
+    from gpzoo_b200 import _cabi
+    protos = _cabi.prototypes()
+    root = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpzoo_b200")
+    seen = 0
+    for path in glob.glob(os.path.join(root, "*.py")):
+        for node in ast.walk(ast.parse(open(path).read())):
+            if not (isinstance(node, ast.Call) and getattr(node.func, "id", getattr(node.func, "attr", None)) == "call"
+                    and node.args and isinstance(node.args[0], ast.Constant)):
+                continue
+            seen += 1
+            where = f"{os.path.basename(path)}:{node.lineno}"
+            syms = [f"gpz_{node.args[0].value}_{s}" for s in ("f32", "f64") if f"gpz_{node.args[0].value}_{s}" in protos]
+            assert syms, where
+            if not any(isinstance(a, ast.Starred) for a in node.args):
+                for s in syms:
+                    assert len(node.args) - 2 == len(protos[s].params) - 1, (where, s)
+    assert seen >= 30
+
+
 def test_no_cpu_fallback(lib):
     import gpzoo_b200 as gz
     k = gz.kernels.NSF_RBF(L=2)

@@ -92,7 +92,7 @@ def test_outputs_final_on_the_callers_stream():
     assert torch.equal(snap_lc, Lc_ref) and torch.equal(snap_linv, Linv_ref)
 
 
-def test_failure_in_third_panel_reports_first_bad_column():
+def test_third_panel_failure_reports_first_bad_column():
     from gpzoo_b200 import functional as F
     K = _dense_spd(2, 1024, seed=7)
     K[1, 600, 600] = -5.0                                       # panel 2 (columns 512..767); leading minors up to 600 are fine
@@ -100,7 +100,7 @@ def test_failure_in_third_panel_reports_first_bad_column():
     info = torch.full((2,), -1, dtype=torch.int32, device=DEV)
     Lc, Linv, tmp = torch.empty_like(W), torch.empty_like(W), torch.empty_like(W)
     lo_ws = torch.empty((4,) + tuple(W.shape), dtype=W.dtype, device=DEV)
-    F.call("chol_inv_tc", W.dtype, F.ptr(W), F.ptr(Lc), F.ptr(Linv), F.ptr(tmp), F.ptr(lo_ws), F.c_i(1024), F.c_i(2), F.ptr(info))
+    F.call("chol_inv_tc", W.dtype, W, Lc, Linv, tmp, lo_ws, 1024, 2, info)
     assert info.tolist() == [0, 601]
     with pytest.raises(torch.linalg.LinAlgError, match=r"Batch element 1\).*order 601"):
         _chol_inv(K)

@@ -107,11 +107,10 @@ FP64_FACTORS = (1, 4, 5, 12, 13, 20, 21, 32)                   # across every FM
 FP32_FACTORS = (1, 16, 17, 32)                                 # tensor-core path up to 16, then poisson_kernel2 (FMAX 20, 32)
 
 
-def test_shape_table_covers_every_split():
+def test_shape_table_covers_every_split_and_workspace_size():
     """CPU: the table's labels are what poisson_grid gives, the library agrees, and every kind of split is reached on both paths."""
     import os
     from gpzoo_b200 import _cabi, build
-    from gpzoo_b200._cabi import c_i
     if not os.path.exists(_cabi.LIB_PATH):
         build.build()
     lib = _cabi.lib()
@@ -132,7 +131,7 @@ def test_shape_table_covers_every_split():
         for F in (1, 10, 16, 17, 32):
             for is_f32, suf in ((True, "f32"), (False, "f64")):
                 args = (s["G"], F, s["B"] or s["Ntot"], s["E"])
-                got = getattr(lib, "gpz_poisson_workspace_bytes_" + suf)(*(c_i(v) for v in args))
+                got = getattr(lib, "gpz_poisson_workspace_bytes_" + suf)(*args)
                 assert got == _workspace_bytes(*args, is_f32), (args, suf)
 
 
