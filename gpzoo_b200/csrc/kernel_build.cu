@@ -5,9 +5,11 @@
 //
 //   K[l,i,j] = sigma_l^2 * exp(-0.5 * |x1_i - x2_j|^2 / (ls_l^2 * den)) / den^(p/2),   den = a_l * r2[g1_i, g2_j] + 1
 //
-// (den = 1 without groups), and the Matern-3/2 covariance functor of kernels.py:6-30 (batched_Matern32):
+// (den = 1 without groups), and the Matern covariance functors (no groups), r = |x1_i - x2_j|:
 //
-//   K[l,i,j] = sigma_l^2 (1 + v) exp(-v),   v = sqrt(3) |x1_i - x2_j| / ls_l.
+//   kind 1, Matern-3/2 (kernels.py:6-30, batched_Matern32):  K[l,i,j] = sigma_l^2 (1 + v) exp(-v),            v = sqrt(3) r / ls_l
+//   kind 2, Matern-1/2 (exponential, batched_Matern12):        K[l,i,j] = sigma_l^2 exp(-v),                  v = r / ls_l
+//   kind 3, Matern-5/2 (batched_Matern52):                     K[l,i,j] = sigma_l^2 (1 + v + v^2/3) exp(-v),  v = sqrt(5) r / ls_l
 //  d^2 is a direct sum of squared differences (never |x|^2+|z|^2-2xz), which is
 // what makes fp32 results track the fp64 reference (SURVEY.md §0).  Output layout L x n1 x n2, n2 contiguous.
 // HBM-bound: one pass writes 4*L*n1*n2 bytes; each thread owns 4 consecutive j and streams float4 stores.
@@ -33,19 +35,26 @@ template <typename T> struct KBArgs {
   int n1, n2, D, L, ng;
   T p_half;                         // input_dim / 2
   T jitter;                         // added to K[l,i,i] (add_jitter, utilities.py:407-418); 0 for cross matrices
-  int kind;                         // 0: RBF (squared exponential); 1: Matern-3/2 (kernels.py:6-30), no groups
+  int kind;                         // 0: RBF (squared exponential); 1 / 2 / 3: Matern-3/2 / -1/2 / -5/2, no groups
 };
+
+// s_c[l] of the kernels: -1/(2 ls^2) for the RBF, the factor of r in v for the Matern kinds
+template <typename T, int KIND> __device__ __forceinline__ T kb_coeff(T ls) {
+  return KIND == 1 ? Num<T>::sqrt(T(3)) / ls : KIND == 2 ? T(1) / ls : KIND == 3 ? Num<T>::sqrt(T(5)) / ls : T(-0.5) / (ls * ls);
+}
 
 template <typename T> struct Vec4 { T v[4]; };
 
-template <typename T, bool MG, bool ALIGNED, bool MAT = false>
-__global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_kernel(const KBArgs<T> a, T* __restrict__ out, T* __restrict__ out_lo) {
+// fp64 Matern-1/2: without a register target ptxas settles on 64 registers and spills; 3 CTAs per SM (<= 80 registers) keep
+// it spill-free like Matern-3/2.  A min-blocks value of 0 is no bound at all, so every other instantiation compiles as before.
+template <typename T, bool MG, bool ALIGNED, int KIND = 0>
+__global__ void __launch_bounds__(KB_THREADS, (KIND == 2 && sizeof(T) == 8) ? 3 : 0) kbuild_fwd_kernel(const KBArgs<T> a, T* __restrict__ out, T* __restrict__ out_lo) {
   __shared__ T s_c[KB_LMAX * 8], s_s2[KB_LMAX * 8], s_a[KB_LMAX * 8];
   __shared__ T s_r2[MG ? KB_GMAX * KB_GMAX : 1];
   const int tid = threadIdx.x;
   for (int l = tid; l < a.L; l += KB_THREADS) {
     const T ls = a.ls[l], sg = a.sigma[l];
-    s_c[l] = MAT ? Num<T>::sqrt(T(3)) / ls : T(-0.5) / (ls * ls);
+    s_c[l] = kb_coeff<T, KIND>(ls);
     s_s2[l] = sg * sg;
     if (MG) s_a[l] = a.a[l];
   }
@@ -93,9 +102,14 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_kernel(const KBArgs<T> 
           const T idn = fast_div(T(1), den);
           const T sc = a.p_half == T(1) ? idn : Num<T>::pow(den, -a.p_half);
           val = s2 * Num<T>::exp(c * d2[v] * idn) * sc;
-        } else if (MAT) {
+        } else if (KIND == 1) {
           const T vv = c * Num<T>::sqrt(d2[v]);
           val = s2 * (T(1) + vv) * Num<T>::exp(-vv);
+        } else if (KIND == 2) {
+          val = s2 * Num<T>::exp(-c * Num<T>::sqrt(d2[v]));
+        } else if (KIND == 3) {
+          const T vv = c * Num<T>::sqrt(d2[v]);
+          val = s2 * fma(vv * T(1.0 / 3.0), vv, T(1) + vv) * Num<T>::exp(-vv);
         } else {
           val = s2 * Num<T>::exp(c * d2[v]);
         }
@@ -133,7 +147,7 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_kernel(const KBArgs<T> 
 // in (2^14, 2^15].  4 bytes per entry leave the SM (half of K + lo plane in fp32); each thread owns 8 consecutive j and
 // streams one 16-byte store per plane, row and factor.
 constexpr int KB_VEC8 = 8;
-template <bool MG, bool MAT = false>
+template <bool MG, int KIND = 0>
 __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<float> a, __half* __restrict__ out_h,
                                                                   __half* __restrict__ out_l, float* __restrict__ out_scale) {
   __shared__ float s_c[KB_LMAX * 8], s_s2[KB_LMAX * 8], s_a[KB_LMAX * 8], s_sc[KB_LMAX * 8];
@@ -141,7 +155,7 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
   const int tid = threadIdx.x;
   for (int l = tid; l < a.L; l += KB_THREADS) {
     const float ls = a.ls[l], sg = a.sigma[l];
-    s_c[l] = MAT ? sqrtf(3.f) / ls : -0.5f / (ls * ls);
+    s_c[l] = kb_coeff<float, KIND>(ls);
     s_s2[l] = sg * sg;
     s_sc[l] = gpz_pow2_scale(sg * sg + fabsf(a.jitter));
     if (MG) s_a[l] = a.a[l];
@@ -189,9 +203,14 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
           const float idn = __fdividef(1.f, den);
           const float scd = a.p_half == 1.f ? idn : powf(den, -a.p_half);
           val = s2 * expf(c * d2[v] * idn) * scd;
-        } else if (MAT) {
+        } else if (KIND == 1) {
           const float vv = c * sqrtf(d2[v]);
           val = s2 * (1.f + vv) * expf(-vv);
+        } else if (KIND == 2) {
+          val = s2 * expf(-c * sqrtf(d2[v]));
+        } else if (KIND == 3) {
+          const float vv = c * sqrtf(d2[v]);
+          val = s2 * fmaf(vv * (1.f / 3.f), vv, 1.f + vv) * expf(-vv);
         } else {
           val = s2 * expf(c * d2[v]);
         }
@@ -226,9 +245,14 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
 // One CTA covers KB_ROWS rows x (KB_THREADS*4) columns; the L accumulators live in registers.  The recomputed K uses the MUFU
 // exponential in fp32 (error ~1e-6 relative on entries that only enter sums with a 1e-4 parity tolerance; fp64 stays exact):
 // the kernel is issue-bound, not DRAM-bound, and expf's range reduction was a third of its instructions.
-// Matern-3/2 (MAT): with e = exp(-v), K0 = s2 (1 + v) e and u = G s2 (3 / ls^2) e the same three accumulations apply:
-//   g_sigma += (2/sigma) sum G K0 ;  g_ls += sum u d2 / ls  (= G s2 v^2 e / ls) ;  dK/dx1 = -u (x1 - x2)  (finite at d = 0)
-template <typename T, bool MG, bool ALIGNED, int LMAX, bool MAT = false>
+// Matern kinds: with e = s2 exp(-v) and u the scalar with dK/dx1 = -u (x1 - x2), the same three accumulations apply:
+//   g_sigma += (2/sigma) sum G K0 ;  g_ls += sum G u d2 / ls ;  g_x1 -= sum G u (x1 - x2)
+//   kind 1, Matern-3/2:  K0 = (1 + v) e,            u = (3 / ls^2) e                 (finite at r = 0)
+//   kind 2, Matern-1/2:  K0 = e,                    u = e / (ls r), 0 at r = 0        (the sub-gradient 0 at the cusp)
+//   kind 3, Matern-5/2:  K0 = (1 + v + v^2/3) e,    u = (5 / (3 ls^2)) (1 + v) e     (finite at r = 0)
+// The position gradients stay products of u with the direct differences: |u (x1 - x2)| <= K0 / ls for Matern-1/2, so
+// near-coincident points are harmless (an x1 sum(u) - sum(u x2) form would cancel catastrophically).
+template <typename T, bool MG, bool ALIGNED, int LMAX, int KIND = 0>
 __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2 : 1) kbuild_bwd_kernel(const KBArgs<T> a, const T* __restrict__ G, int l0, int Lc,
                                                                  double* __restrict__ g_x1, T* __restrict__ g_x2,
                                                                  double* __restrict__ g_sigma, double* __restrict__ g_ls,
@@ -240,7 +264,7 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   for (int l = tid; l < Lc; l += KB_THREADS) {
     const T ls = a.ls[l0 + l], sg = a.sigma[l0 + l];
-    s_c[l] = MAT ? Num<T>::sqrt(T(3)) / ls : T(-0.5) / (ls * ls);
+    s_c[l] = kb_coeff<T, KIND>(ls);
     s_s2[l] = sg * sg;
     if (MG) s_a[l] = a.a[l0 + l];
   }
@@ -309,24 +333,37 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
           const T c = s_c[l], s2 = s_s2[l];
 #pragma unroll
           for (int v = 0; v < KB_VEC; ++v) {
-            T k0, idn, ee = T(0);
+            T k0, idn, ee = T(0), ir = T(0);
             if (MG) {
               const T den = fma(s_a[l], r2[v], T(1));
               idn = fast_div(T(1), den);
               const T sc = a.p_half == T(1) ? idn : Num<T>::pow(den, -a.p_half);
               k0 = s2 * fast_exp(c * d2[v] * idn) * sc;
-            } else if (MAT) {
+            } else if (KIND == 1) {
               idn = T(1);
               const T vv = c * Num<T>::sqrt(d2[v]);
               ee = s2 * fast_exp(-vv);
               k0 = (T(1) + vv) * ee;
+            } else if (KIND == 2) {
+              idn = T(1);
+              ir = d2[v] > T(0) ? Num<T>::rsqrt(d2[v]) : T(0);      // 1/r; 0 at r = 0 (a d2 below 1e-38 is 0 under -ftz)
+              ee = s2 * fast_exp(-c * d2[v] * ir);                  // r = d2 / r
+              k0 = ee;
+            } else if (KIND == 3) {
+              idn = T(1);
+              const T vv = c * Num<T>::sqrt(d2[v]);
+              ee = s2 * fast_exp(-vv);
+              ir = T(1) + vv;
+              k0 = fma(vv * T(1.0 / 3.0), vv, ir) * ee;
             } else {
               idn = T(1);
               k0 = s2 * fast_exp(c * d2[v]);
             }
             const T gk = g[l][v] * k0;
-            const T u = MAT ? g[l][v] * ee * c * c       // G s2 exp(-v) 3 / ls^2
-                            : gk * (T(-2) * c) * idn;    // G K0 / (ls^2 den)
+            const T u = KIND == 1 ? g[l][v] * ee * c * c                  // G s2 exp(-v) 3 / ls^2
+                      : KIND == 2 ? gk * c * ir                           // G K0 / (ls r)
+                      : KIND == 3 ? g[l][v] * ee * ir * c * c * T(1.0 / 3.0)  // G s2 (1 + v) exp(-v) 5 / (3 ls^2)
+                                  : gk * (T(-2) * c) * idn;               // G K0 / (ls^2 den)
             acc_s[l] += gk;
             acc_l[l] = fma(u, d2[v], acc_l[l]);          // later divided by ls
             if (MG) acc_a[l] = fma(gk * r2[v], (T(-1) * c * d2[v] * idn - a.p_half) * idn, acc_a[l]);
@@ -404,6 +441,15 @@ __global__ void cdist_kernel(const T* __restrict__ x1, const T* __restrict__ x2,
   out[e] = Num<T>::sqrt(d2);
 }
 
+// kinds 0-3 without groups; the multi-group form is the RBF's only
+inline bool kb_kind_ok(int kind, bool mg) { return mg ? kind == 0 : (kind >= 0 && kind <= 3); }
+
+template <typename T, int KIND>
+void kbuild_fwd_launch(const KBArgs<T>& a, bool al, dim3 grid, T* out, T* out_lo, cudaStream_t st) {
+  if (al) kbuild_fwd_kernel<T, false, true, KIND><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
+  else kbuild_fwd_kernel<T, false, false, KIND><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
+}
+
 template <typename T>
 int kbuild_fwd(const KBArgs<T>& a, T* out, T* out_lo, cudaStream_t st) {
   if (a.D < 1 || a.D > KB_DMAX || a.L < 1 || a.L > KB_LMAX * 8) return GPZ_ERR_UNSUPPORTED;
@@ -413,11 +459,11 @@ int kbuild_fwd(const KBArgs<T>& a, T* out, T* out_lo, cudaStream_t st) {
   const bool al = (a.n2 % KB_VEC == 0) && ((reinterpret_cast<uintptr_t>(out) & 31) == 0) &&
                   ((reinterpret_cast<uintptr_t>(out_lo) & 15) == 0);
   dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
-  if (a.kind != 0 && (a.kind != 1 || mg)) return GPZ_ERR_UNSUPPORTED;       // Matern-3/2 has no multi-group form in the reference
-  if (a.kind == 1) {
-    if (al) kbuild_fwd_kernel<T, false, true, true><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
-    else kbuild_fwd_kernel<T, false, false, true><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
-  } else if (mg) {
+  if (!kb_kind_ok(a.kind, mg)) return GPZ_ERR_UNSUPPORTED;       // the Matern kinds have no multi-group form in the reference
+  if (a.kind == 1) kbuild_fwd_launch<T, 1>(a, al, grid, out, out_lo, st);
+  else if (a.kind == 2) kbuild_fwd_launch<T, 2>(a, al, grid, out, out_lo, st);
+  else if (a.kind == 3) kbuild_fwd_launch<T, 3>(a, al, grid, out, out_lo, st);
+  else if (mg) {
     if (al) kbuild_fwd_kernel<T, true, true><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
     else kbuild_fwd_kernel<T, true, false><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
   } else {
@@ -440,26 +486,32 @@ int kbuild_bwd(const KBArgs<T>& a, const T* G, T* g_x1, T* g_x2, T* g_sigma, T* 
   if (a.n1 > 0 && a.n2 > 0) {
     const bool al = (a.n2 % KB_VEC == 0) && ((reinterpret_cast<uintptr_t>(G) & 31) == 0);
     dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
-    if (a.kind != 0 && (a.kind != 1 || mg)) return GPZ_ERR_UNSUPPORTED;
-    const int lmax = a.kind == 1 ? KB_LMAX : (a.L <= 4 ? 4 : (a.L <= 8 ? 8 : (a.L <= 12 ? 12 : (a.L <= 16 ? 16 : KB_LMAX))));
+    if (!kb_kind_ok(a.kind, mg)) return GPZ_ERR_UNSUPPORTED;
+    const int lmax = a.kind != 0 ? KB_LMAX : (a.L <= 4 ? 4 : (a.L <= 8 ? 8 : (a.L <= 12 ? 12 : (a.L <= 16 ? 16 : KB_LMAX))));
     for (int l0 = 0; l0 < a.L; l0 += lmax) {
       const int Lc = min(lmax, a.L - l0);
       // g_x1/g_x2 accumulate over all l-chunks (atomics), so every chunk launch adds its share
 #define GPZ_KB_LAUNCH(MGV, ALV, LM) \
   kbuild_bwd_kernel<T, MGV, ALV, LM><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a)
+#define GPZ_KB_MATERN(KIND)                                                                                                \
+  do {                                                                                                                     \
+    if (al) kbuild_bwd_kernel<T, false, true, KB_LMAX, KIND><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a);  \
+    else kbuild_bwd_kernel<T, false, false, KB_LMAX, KIND><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a);   \
+  } while (0)
 #define GPZ_KB_DISPATCH(LM)                                   \
   do {                                                        \
     if (mg) { if (al) GPZ_KB_LAUNCH(true, true, LM); else GPZ_KB_LAUNCH(true, false, LM); }     \
     else { if (al) GPZ_KB_LAUNCH(false, true, LM); else GPZ_KB_LAUNCH(false, false, LM); }      \
   } while (0)
-      if (a.kind == 1) {
-        if (al) kbuild_bwd_kernel<T, false, true, KB_LMAX, true><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a);
-        else kbuild_bwd_kernel<T, false, false, KB_LMAX, true><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a);
-      } else if (lmax == 4) GPZ_KB_DISPATCH(4);
+      if (a.kind == 1) GPZ_KB_MATERN(1);
+      else if (a.kind == 2) GPZ_KB_MATERN(2);
+      else if (a.kind == 3) GPZ_KB_MATERN(3);
+      else if (lmax == 4) GPZ_KB_DISPATCH(4);
       else if (lmax == 8) GPZ_KB_DISPATCH(8);
       else if (lmax == 12) GPZ_KB_DISPATCH(12);
       else if (lmax == 16) GPZ_KB_DISPATCH(16);
       else GPZ_KB_DISPATCH(KB_LMAX);
+#undef GPZ_KB_MATERN
 #undef GPZ_KB_DISPATCH
 #undef GPZ_KB_LAUNCH
       GPZ_CHECK_LAUNCH();
@@ -513,8 +565,10 @@ extern "C" int gpz_kernel_build_fwd_h_f32(const float* x1, const float* x2, cons
   if (n2 % KB_VEC8 || (reinterpret_cast<uintptr_t>(out_h) & 15) || (reinterpret_cast<uintptr_t>(out_l) & 15)) return GPZ_ERR_UNSUPPORTED;
   if (n1 == 0 || n2 == 0) return GPZ_OK;
   dim3 grid((unsigned)cdiv(n2, (int64_t)KB_THREADS * KB_VEC8), (unsigned)cdiv(n1, KB_ROWS));
-  if (kind != 0 && (kind != 1 || mg)) return GPZ_ERR_UNSUPPORTED;
-  if (kind == 1) kbuild_fwd_h_kernel<false, true><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
+  if (!kb_kind_ok(kind, mg)) return GPZ_ERR_UNSUPPORTED;
+  if (kind == 1) kbuild_fwd_h_kernel<false, 1><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
+  else if (kind == 2) kbuild_fwd_h_kernel<false, 2><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
+  else if (kind == 3) kbuild_fwd_h_kernel<false, 3><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
   else if (mg) kbuild_fwd_h_kernel<true><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
   else kbuild_fwd_h_kernel<false><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
   GPZ_CHECK_LAUNCH();

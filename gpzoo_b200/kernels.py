@@ -36,7 +36,7 @@ def _flat(p):
 class _RBFBase(nn.Module):
     input_dim = 2
     _batched = False        # True: parameters are per-factor, output keeps the leading L dimension
-    _kind = 0               # covariance functor of the fused kernel build: 0 = RBF, 1 = Matern-3/2
+    _kind = 0               # covariance functor of the fused kernel build: 0 = RBF, 1 / 2 / 3 = Matern-3/2 / -1/2 / -5/2
 
     def _params(self):
         return _flat(self.sigma), _flat(self.lengthscale)
@@ -183,6 +183,27 @@ class batched_Matern32(batched_RBF):
     def forward_distance(self, distance_squared):
         v = (3.0 * distance_squared).sqrt() / self.lengthscale
         return (self.sigma ** 2) * (1 + v) * torch.exp(-v)
+
+
+class batched_Matern12(batched_RBF):
+    """Matern-1/2 (exponential) covariance sigma^2 exp(-v), v = |x - z| / lengthscale, scalar or (L,) parameters: `kind = 2`
+    of gpz_kernel_build_*.  K has a cusp at x == z; the fused backward takes the sub-gradient 0 there (the position gradient
+    of a coincident pair is exactly 0).  The reference has no counterpart of this class."""
+    _kind = 2
+
+    def forward_distance(self, distance_squared):
+        return (self.sigma ** 2) * torch.exp(-distance_squared.sqrt() / self.lengthscale)
+
+
+class batched_Matern52(batched_RBF):
+    """Matern-5/2 covariance sigma^2 (1 + v + v^2/3) exp(-v), v = sqrt(5) |x - z| / lengthscale, scalar or (L,) parameters:
+    `kind = 3` of gpz_kernel_build_*.  K is twice differentiable at x == z, and the fused backward is finite there (the position
+    gradient of a coincident pair is exactly 0).  The reference has no counterpart of this class."""
+    _kind = 3
+
+    def forward_distance(self, distance_squared):
+        v = (5.0 * distance_squared).sqrt() / self.lengthscale
+        return (self.sigma ** 2) * (1 + v + v * v / 3) * torch.exp(-v)
 
 
 class batched_MGGP_RBF(batched_RBF):

@@ -34,7 +34,10 @@ long long gpz_launch_count(void);
  *      out[l,i,j] = sigma_l^2 exp(-0.5 |x1_i-x2_j|^2/(ls_l^2 den))/den^p_half (+ jitter if i==j),
  *      den = a_l r2[g1_i,g2_j] + 1.  Pass a=r2=g1=g2=NULL, ng=0 for the plain RBF.
  *      kind = 0: the RBF forms above; kind = 1: Matern-3/2, kernels.py:6-30 (batched_Matern32),
- *      out[l,i,j] = sigma_l^2 (1 + v) exp(-v), v = sqrt(3) |x1_i-x2_j| / ls_l (no groups; its gradients are finite at |x1-x2| = 0).
+ *      out[l,i,j] = sigma_l^2 (1 + v) exp(-v), v = sqrt(3) |x1_i-x2_j| / ls_l (no groups; its gradients are finite at |x1-x2| = 0);
+ *      kind = 2: Matern-1/2 (exponential), out[l,i,j] = sigma_l^2 exp(-|x1_i-x2_j| / ls_l) (no groups; the backward takes the
+ *      sub-gradient 0 at |x1-x2| = 0); kind = 3: Matern-5/2, out[l,i,j] = sigma_l^2 (1 + v + v^2/3) exp(-v),
+ *      v = sqrt(5) |x1_i-x2_j| / ls_l (no groups).  Other kinds, and kinds 1-3 with groups, return GPZ_ERR_UNSUPPORTED.
  *      out_lo (optional, f32 only): lo = out - tf32_trunc(out), the second operand of the split-TF32 GEMMs. */
 int gpz_kernel_build_fwd_f32(const float* x1, const float* x2, const float* sigma, const float* ls, const float* a,
                              const float* r2, const int64_t* g1, const int64_t* g2, int n1, int n2, int D, int L, int ng, int kind,
