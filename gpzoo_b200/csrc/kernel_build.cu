@@ -1,18 +1,14 @@
-// K1: fused pairwise-distance + exp kernel-matrix build and its backward.
+// K1: fused pairwise-distance + covariance kernel-matrix build and its backward.
 //
 // Replaces  torch.cdist(X,Z)**2 -> expand(L) -> /l^2 -> exp -> *sigma^2   (kernels.py:114-130, 141-155)
-// and the multi-group form with group-distance scaling                   (kernels.py:172-191, 204-228):
-//
-//   K[l,i,j] = sigma_l^2 * exp(-0.5 * |x1_i - x2_j|^2 / (ls_l^2 * den)) / den^(p/2),   den = a_l * r2[g1_i, g2_j] + 1
-//
-// (den = 1 without groups), and the Matern covariance functors (no groups), r = |x1_i - x2_j|:
-//
-//   kind 1, Matern-3/2 (kernels.py:6-30, batched_Matern32):  K[l,i,j] = sigma_l^2 (1 + v) exp(-v),            v = sqrt(3) r / ls_l
-//   kind 2, Matern-1/2 (exponential, batched_Matern12):        K[l,i,j] = sigma_l^2 exp(-v),                  v = r / ls_l
-//   kind 3, Matern-5/2 (batched_Matern52):                     K[l,i,j] = sigma_l^2 (1 + v + v^2/3) exp(-v),  v = sqrt(5) r / ls_l
-//  d^2 is a direct sum of squared differences (never |x|^2+|z|^2-2xz), which is
+// and the multi-group form with group-distance scaling (kernels.py:172-191, 204-228); the covariance kinds and their formulas are
+// listed once, with their code, in the block below.
+// d^2 is a direct sum of squared differences (never |x|^2+|z|^2-2xz), which is
 // what makes fp32 results track the fp64 reference (SURVEY.md §0).  Output layout L x n1 x n2, n2 contiguous.
 // HBM-bound: one pass writes 4*L*n1*n2 bytes; each thread owns 4 consecutive j and streams float4 stores.
+#include <climits>
+#include <type_traits>
+
 #include "common.cuh"
 #include "gpzoo_b200.h"
 #include "umma_gemm.h"
@@ -38,9 +34,133 @@ template <typename T> struct KBArgs {
   int kind;                         // 0: RBF (squared exponential); 1 / 2 / 3: Matern-3/2 / -1/2 / -5/2, no groups
 };
 
+// ---- The covariance kinds.  Everything kind-specific lives in this block: a kind is added here and in the host dispatch
+// (kb_dispatch_kind), nowhere else.  r = |x1_i - x2_j|, d2 = r^2:
+//
+//   kind 0, RBF:  K[l,i,j] = sigma_l^2 exp(-0.5 d2 / (ls_l^2 den)) / den^(p/2),  den = a_l r2[g1_i, g2_j] + 1 with groups,
+//                 den = 1 without (p/2 = p_half, input_dim / 2)
+//   kind 1, Matern-3/2 (kernels.py:6-30, batched_Matern32):  K[l,i,j] = sigma_l^2 (1 + v) exp(-v),            v = sqrt(3) r / ls_l
+//   kind 2, Matern-1/2 (exponential, batched_Matern12):        K[l,i,j] = sigma_l^2 exp(-v),                  v = r / ls_l
+//   kind 3, Matern-5/2 (batched_Matern52):                     K[l,i,j] = sigma_l^2 (1 + v + v^2/3) exp(-v),  v = sqrt(5) r / ls_l
+//
+// Only the RBF has a multi-group form (as in the reference).  The backward needs K0 (K without jitter) and the slope u with
+// dK/dx1 = -u (x1 - x2); with e = sigma^2 exp(-v) for the Matern kinds:
+//   kind 0:  u = K0 / (ls^2 den)
+//   kind 1:  K0 = (1 + v) e,            u = (3 / ls^2) e                 (finite at r = 0)
+//   kind 2:  K0 = e,                    u = e / (ls r), 0 at r = 0        (the sub-gradient 0 at the cusp)
+//   kind 3:  K0 = (1 + v + v^2/3) e,    u = (5 / (3 ls^2)) (1 + v) e     (finite at r = 0)
+
 // s_c[l] of the kernels: -1/(2 ls^2) for the RBF, the factor of r in v for the Matern kinds
 template <typename T, int KIND> __device__ __forceinline__ T kb_coeff(T ls) {
   return KIND == 1 ? Num<T>::sqrt(T(3)) / ls : KIND == 2 ? T(1) / ls : KIND == 3 ? Num<T>::sqrt(T(5)) / ls : T(-0.5) / (ls * ls);
+}
+
+// forward: K without jitter, exact functions; c = kb_coeff(ls_l), s2 = sigma_l^2; a_l and r2 are used with groups only
+template <typename T, bool MG, int KIND>
+__device__ __forceinline__ T kb_value(T c, T s2, T a_l, T r2, T d2, T p_half) {
+  if (MG) {
+    // one reciprocal per entry (MUFU.RCP in fp32: the two IEEE divisions held the multi-group build at 20 % of HBM peak)
+    const T den = fma(a_l, r2, T(1));
+    const T idn = fast_div(T(1), den);
+    const T sc = p_half == T(1) ? idn : Num<T>::pow(den, -p_half);
+    return s2 * Num<T>::exp(c * d2 * idn) * sc;
+  } else if (KIND == 1) {
+    const T vv = c * Num<T>::sqrt(d2);
+    return s2 * (T(1) + vv) * Num<T>::exp(-vv);
+  } else if (KIND == 2) {
+    return s2 * Num<T>::exp(-c * Num<T>::sqrt(d2));
+  } else if (KIND == 3) {
+    const T vv = c * Num<T>::sqrt(d2);
+    return s2 * fma(vv * T(1.0 / 3.0), vv, T(1) + vv) * Num<T>::exp(-vv);
+  }
+  return s2 * Num<T>::exp(c * d2);
+}
+
+// backward: K0, u times the upstream gradient g, and (groups) idn = 1/den.  The recomputed K uses the MUFU exponential in fp32
+// (error ~1e-6 relative on entries that only enter sums with a 1e-4 parity tolerance; fp64 stays exact): the backward is
+// issue-bound, not DRAM-bound, and expf's range reduction was a third of its instructions.
+template <typename T> struct KBTerms { T k0, u, idn; };
+template <typename T, bool MG, int KIND>
+__device__ __forceinline__ KBTerms<T> kb_terms(T c, T s2, T a_l, T r2, T d2, T p_half, T g) {
+  T k0, idn = T(1), ee = T(0), ir = T(0);
+  if (MG) {
+    const T den = fma(a_l, r2, T(1));
+    idn = fast_div(T(1), den);
+    const T sc = p_half == T(1) ? idn : Num<T>::pow(den, -p_half);
+    k0 = s2 * fast_exp(c * d2 * idn) * sc;
+  } else if (KIND == 1) {
+    const T vv = c * Num<T>::sqrt(d2);
+    ee = s2 * fast_exp(-vv);
+    k0 = (T(1) + vv) * ee;
+  } else if (KIND == 2) {
+    ir = d2 > T(0) ? Num<T>::rsqrt(d2) : T(0);      // 1/r; 0 at r = 0 (a d2 below 1e-38 is 0 under -ftz)
+    ee = s2 * fast_exp(-c * d2 * ir);               // r = d2 / r
+    k0 = ee;
+  } else if (KIND == 3) {
+    const T vv = c * Num<T>::sqrt(d2);
+    ee = s2 * fast_exp(-vv);
+    ir = T(1) + vv;
+    k0 = fma(vv * T(1.0 / 3.0), vv, ir) * ee;
+  } else {
+    k0 = s2 * fast_exp(c * d2);
+  }
+  const T gk = g * k0;
+  const T u = KIND == 1 ? g * ee * c * c                        // G s2 exp(-v) 3 / ls^2
+            : KIND == 2 ? gk * c * ir                           // G K0 / (ls r)
+            : KIND == 3 ? g * ee * ir * c * c * T(1.0 / 3.0)    // G s2 (1 + v) exp(-v) 5 / (3 ls^2)
+                        : gk * (T(-2) * c) * idn;               // G K0 / (ls^2 den)
+  return {k0, u, idn};
+}
+
+// ---- Tile pieces shared by the kernels.
+
+// factors l0 .. l0 + n - 1 into shared memory (s_c = kb_coeff, s_s2 = sigma^2, s_a with groups) and, with groups, the r^2
+// table; tid = threadIdx.x, the caller synchronises
+template <typename T, bool MG, int KIND>
+__device__ __forceinline__ void kb_stage(const KBArgs<T>& a, int tid, int l0, int n, T* s_c, T* s_s2, T* s_a, T* s_r2) {
+  for (int l = tid; l < n; l += KB_THREADS) {
+    const T ls = a.ls[l0 + l], sg = a.sigma[l0 + l];
+    s_c[l] = kb_coeff<T, KIND>(ls);
+    s_s2[l] = sg * sg;
+    if (MG) s_a[l] = a.a[l0 + l];
+  }
+  if (MG) for (int e = tid; e < a.ng * a.ng; e += KB_THREADS) s_r2[e] = a.r2[e];
+}
+
+// the thread's columns j0 .. j0 + nv - 1 (points and groups; zeros past nv and past D)
+template <typename T, bool MG, int VEC>
+__device__ __forceinline__ void kb_load_cols(const KBArgs<T>& a, int64_t j0, int nv, T (&xj)[KB_DMAX][VEC], int (&gj)[VEC]) {
+#pragma unroll
+  for (int v = 0; v < VEC; ++v) {
+#pragma unroll
+    for (int d = 0; d < KB_DMAX; ++d) xj[d][v] = (v < nv && d < a.D) ? a.x2[(j0 + v) * a.D + d] : T(0);
+    gj[v] = (MG && v < nv) ? (int)a.g2[j0 + v] : 0;
+  }
+}
+
+// squared distances of row i to the thread's columns
+template <typename T, int VEC>
+__device__ __forceinline__ void kb_row_d2(const KBArgs<T>& a, int i, const T (&xj)[KB_DMAX][VEC], T (&d2)[VEC]) {
+#pragma unroll
+  for (int v = 0; v < VEC; ++v) d2[v] = T(0);
+#pragma unroll
+  for (int d = 0; d < KB_DMAX; ++d) {
+    if (d < a.D) {
+      const T xi = a.x1[(int64_t)i * a.D + d];
+#pragma unroll
+      for (int v = 0; v < VEC; ++v) { const T df = xi - xj[d][v]; d2[v] = fma(df, df, d2[v]); }
+    }
+  }
+}
+
+// group r^2 of row i and the thread's columns (groups only)
+template <typename T, bool MG, int VEC>
+__device__ __forceinline__ void kb_row_r2(const KBArgs<T>& a, int i, const T* s_r2, const int (&gj)[VEC], T (&r2)[VEC]) {
+  if (MG) {
+    const int gi = (int)a.g1[i];
+#pragma unroll
+    for (int v = 0; v < VEC; ++v) r2[v] = s_r2[gi * a.ng + gj[v]];
+  }
 }
 
 template <typename T> struct Vec4 { T v[4]; };
@@ -52,13 +172,7 @@ __global__ void __launch_bounds__(KB_THREADS, (KIND == 2 && sizeof(T) == 8) ? 3 
   __shared__ T s_c[KB_LMAX * 8], s_s2[KB_LMAX * 8], s_a[KB_LMAX * 8];
   __shared__ T s_r2[MG ? KB_GMAX * KB_GMAX : 1];
   const int tid = threadIdx.x;
-  for (int l = tid; l < a.L; l += KB_THREADS) {
-    const T ls = a.ls[l], sg = a.sigma[l];
-    s_c[l] = kb_coeff<T, KIND>(ls);
-    s_s2[l] = sg * sg;
-    if (MG) s_a[l] = a.a[l];
-  }
-  if (MG) for (int e = tid; e < a.ng * a.ng; e += KB_THREADS) s_r2[e] = a.r2[e];
+  kb_stage<T, MG, KIND>(a, tid, 0, a.L, s_c, s_s2, s_a, s_r2);
   __syncthreads();
 
   const int64_t j0 = ((int64_t)blockIdx.x * KB_THREADS + tid) * KB_VEC;
@@ -66,53 +180,18 @@ __global__ void __launch_bounds__(KB_THREADS, (KIND == 2 && sizeof(T) == 8) ? 3 
   const int nv = (int)min((int64_t)KB_VEC, a.n2 - j0);
   T xj[KB_DMAX][KB_VEC];
   int gj[KB_VEC];
-#pragma unroll
-  for (int v = 0; v < KB_VEC; ++v) {
-#pragma unroll
-    for (int d = 0; d < KB_DMAX; ++d) xj[d][v] = (v < nv && d < a.D) ? a.x2[(j0 + v) * a.D + d] : T(0);
-    gj[v] = (MG && v < nv) ? (int)a.g2[j0 + v] : 0;
-  }
+  kb_load_cols<T, MG>(a, j0, nv, xj, gj);
   const int i0 = blockIdx.y * KB_ROWS, i1 = min(i0 + KB_ROWS, a.n1);
   for (int i = i0; i < i1; ++i) {
     T d2[KB_VEC], r2[KB_VEC];
-#pragma unroll
-    for (int v = 0; v < KB_VEC; ++v) d2[v] = T(0);
-#pragma unroll
-    for (int d = 0; d < KB_DMAX; ++d) {
-      if (d < a.D) {
-        const T xi = a.x1[(int64_t)i * a.D + d];
-#pragma unroll
-        for (int v = 0; v < KB_VEC; ++v) { const T df = xi - xj[d][v]; d2[v] = fma(df, df, d2[v]); }
-      }
-    }
-    if (MG) {
-      const int gi = (int)a.g1[i];
-#pragma unroll
-      for (int v = 0; v < KB_VEC; ++v) r2[v] = s_r2[gi * a.ng + gj[v]];
-    }
+    kb_row_d2(a, i, xj, d2);
+    kb_row_r2<T, MG>(a, i, s_r2, gj, r2);
     for (int l = 0; l < a.L; ++l) {
       const T c = s_c[l], s2 = s_s2[l];
       Vec4<T> k;
 #pragma unroll
       for (int v = 0; v < KB_VEC; ++v) {
-        T val;
-        if (MG) {
-          // one reciprocal per entry (MUFU.RCP in fp32: the two IEEE divisions held the multi-group build at 20 % of HBM peak)
-          const T den = fma(s_a[l], r2[v], T(1));
-          const T idn = fast_div(T(1), den);
-          const T sc = a.p_half == T(1) ? idn : Num<T>::pow(den, -a.p_half);
-          val = s2 * Num<T>::exp(c * d2[v] * idn) * sc;
-        } else if (KIND == 1) {
-          const T vv = c * Num<T>::sqrt(d2[v]);
-          val = s2 * (T(1) + vv) * Num<T>::exp(-vv);
-        } else if (KIND == 2) {
-          val = s2 * Num<T>::exp(-c * Num<T>::sqrt(d2[v]));
-        } else if (KIND == 3) {
-          const T vv = c * Num<T>::sqrt(d2[v]);
-          val = s2 * fma(vv * T(1.0 / 3.0), vv, T(1) + vv) * Num<T>::exp(-vv);
-        } else {
-          val = s2 * Num<T>::exp(c * d2[v]);
-        }
+        T val = kb_value<T, MG, KIND>(c, s2, MG ? s_a[l] : T(0), MG ? r2[v] : T(0), d2[v], a.p_half);
         if (a.jitter != T(0) && (int64_t)i == j0 + v) val += a.jitter;
         k.v[v] = val;
       }
@@ -152,6 +231,7 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
                                                                   __half* __restrict__ out_l, float* __restrict__ out_scale) {
   __shared__ float s_c[KB_LMAX * 8], s_s2[KB_LMAX * 8], s_a[KB_LMAX * 8], s_sc[KB_LMAX * 8];
   __shared__ float s_r2[MG ? KB_GMAX * KB_GMAX : 1];
+  // kb_stage's loop with s_sc and out_scale: written out, since a per-factor hook inside kb_stage reschedules the multi-group kernel
   const int tid = threadIdx.x;
   for (int l = tid; l < a.L; l += KB_THREADS) {
     const float ls = a.ls[l], sg = a.sigma[l];
@@ -168,52 +248,18 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
   if (j0 >= a.n2) return;                        // n2 % 8 == 0 (checked by the host): whole vectors only
   float xj[KB_DMAX][KB_VEC8];
   int gj[KB_VEC8];
-#pragma unroll
-  for (int v = 0; v < KB_VEC8; ++v) {
-#pragma unroll
-    for (int d = 0; d < KB_DMAX; ++d) xj[d][v] = d < a.D ? a.x2[(j0 + v) * a.D + d] : 0.f;
-    gj[v] = MG ? (int)a.g2[j0 + v] : 0;
-  }
+  kb_load_cols<float, MG>(a, j0, KB_VEC8, xj, gj);
   const int i0 = blockIdx.y * KB_ROWS, i1 = min(i0 + KB_ROWS, a.n1);
   for (int i = i0; i < i1; ++i) {
     float d2[KB_VEC8], r2[KB_VEC8];
-#pragma unroll
-    for (int v = 0; v < KB_VEC8; ++v) d2[v] = 0.f;
-#pragma unroll
-    for (int d = 0; d < KB_DMAX; ++d) {
-      if (d < a.D) {
-        const float xi = a.x1[(int64_t)i * a.D + d];
-#pragma unroll
-        for (int v = 0; v < KB_VEC8; ++v) { const float df = xi - xj[d][v]; d2[v] = fmaf(df, df, d2[v]); }
-      }
-    }
-    if (MG) {
-      const int gi = (int)a.g1[i];
-#pragma unroll
-      for (int v = 0; v < KB_VEC8; ++v) r2[v] = s_r2[gi * a.ng + gj[v]];
-    }
+    kb_row_d2(a, i, xj, d2);
+    kb_row_r2<float, MG>(a, i, s_r2, gj, r2);
     for (int l = 0; l < a.L; ++l) {
       const float c = s_c[l], s2 = s_s2[l], sc = s_sc[l];
       float k[KB_VEC8];
 #pragma unroll
       for (int v = 0; v < KB_VEC8; ++v) {
-        float val;
-        if (MG) {
-          const float den = fmaf(s_a[l], r2[v], 1.f);
-          const float idn = __fdividef(1.f, den);
-          const float scd = a.p_half == 1.f ? idn : powf(den, -a.p_half);
-          val = s2 * expf(c * d2[v] * idn) * scd;
-        } else if (KIND == 1) {
-          const float vv = c * sqrtf(d2[v]);
-          val = s2 * (1.f + vv) * expf(-vv);
-        } else if (KIND == 2) {
-          val = s2 * expf(-c * sqrtf(d2[v]));
-        } else if (KIND == 3) {
-          const float vv = c * sqrtf(d2[v]);
-          val = s2 * fmaf(vv * (1.f / 3.f), vv, 1.f + vv) * expf(-vv);
-        } else {
-          val = s2 * expf(c * d2[v]);
-        }
+        float val = kb_value<float, MG, KIND>(c, s2, MG ? s_a[l] : 0.f, MG ? r2[v] : 0.f, d2[v], a.p_half);
         if (a.jitter != 0.f && (int64_t)i == j0 + v) val += a.jitter;
         k[v] = val * sc;
       }
@@ -237,19 +283,12 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
   }
 }
 
-// Backward: given G = dLoss/dK (L x n1 x n2) recompute K and reduce
-//   g_sigma[l] += (2/sigma_l) sum G K0                       (K0 without jitter)
-//   g_ls[l]    += sum G K0 d2 / (ls^3 den)
+// Backward: given G = dLoss/dK (L x n1 x n2) recompute K0 (K without jitter) and, with u from kb_terms, reduce
+//   g_sigma[l] += (2/sigma_l) sum G K0
+//   g_ls[l]    += sum G u d2 / ls
 //   g_a[l]     += sum G K0 (0.5 d2/(ls^2 den^2) - p_half/den) r2             (MG)
-//   g_x1[i,:]  -= sum_{l,j} G K0 (x1_i - x2_j)/(ls^2 den) ;  g_x2[j,:] += same
-// One CTA covers KB_ROWS rows x (KB_THREADS*4) columns; the L accumulators live in registers.  The recomputed K uses the MUFU
-// exponential in fp32 (error ~1e-6 relative on entries that only enter sums with a 1e-4 parity tolerance; fp64 stays exact):
-// the kernel is issue-bound, not DRAM-bound, and expf's range reduction was a third of its instructions.
-// Matern kinds: with e = s2 exp(-v) and u the scalar with dK/dx1 = -u (x1 - x2), the same three accumulations apply:
-//   g_sigma += (2/sigma) sum G K0 ;  g_ls += sum G u d2 / ls ;  g_x1 -= sum G u (x1 - x2)
-//   kind 1, Matern-3/2:  K0 = (1 + v) e,            u = (3 / ls^2) e                 (finite at r = 0)
-//   kind 2, Matern-1/2:  K0 = e,                    u = e / (ls r), 0 at r = 0        (the sub-gradient 0 at the cusp)
-//   kind 3, Matern-5/2:  K0 = (1 + v + v^2/3) e,    u = (5 / (3 ls^2)) (1 + v) e     (finite at r = 0)
+//   g_x1[i,:]  -= sum_{l,j} G u (x1_i - x2_j) ;  g_x2[j,:] += same
+// One CTA covers KB_ROWS rows x (KB_THREADS*4) columns; the L accumulators live in registers.
 // The position gradients stay products of u with the direct differences: |u (x1 - x2)| <= K0 / ls for Matern-1/2, so
 // near-coincident points are harmless (an x1 sum(u) - sum(u x2) form would cancel catastrophically).
 template <typename T, bool MG, bool ALIGNED, int LMAX, int KIND = 0>
@@ -262,25 +301,14 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
   __shared__ double s_red[32];
   __shared__ T s_row[KB_ROWS][KB_DMAX][KB_THREADS / 32];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int l = tid; l < Lc; l += KB_THREADS) {
-    const T ls = a.ls[l0 + l], sg = a.sigma[l0 + l];
-    s_c[l] = kb_coeff<T, KIND>(ls);
-    s_s2[l] = sg * sg;
-    if (MG) s_a[l] = a.a[l0 + l];
-  }
-  if (MG) for (int e = tid; e < a.ng * a.ng; e += KB_THREADS) s_r2[e] = a.r2[e];
+  kb_stage<T, MG, KIND>(a, tid, l0, Lc, s_c, s_s2, s_a, s_r2);
   __syncthreads();
 
   const int64_t j0 = ((int64_t)blockIdx.x * KB_THREADS + tid) * KB_VEC;
   const int nv = j0 < a.n2 ? (int)min((int64_t)KB_VEC, a.n2 - j0) : 0;
   T xj[KB_DMAX][KB_VEC];
   int gj[KB_VEC];
-#pragma unroll
-  for (int v = 0; v < KB_VEC; ++v) {
-#pragma unroll
-    for (int d = 0; d < KB_DMAX; ++d) xj[d][v] = (v < nv && d < a.D) ? a.x2[(j0 + v) * a.D + d] : T(0);
-    gj[v] = (MG && v < nv) ? (int)a.g2[j0 + v] : 0;
-  }
+  kb_load_cols<T, MG>(a, j0, nv, xj, gj);
   T acc_s[LMAX], acc_l[LMAX], acc_a[MG ? LMAX : 1];
 #pragma unroll
   for (int l = 0; l < LMAX; ++l) { acc_s[l] = T(0); acc_l[l] = T(0); if (MG) acc_a[l] = T(0); }
@@ -292,7 +320,7 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
 
   const int i0 = blockIdx.y * KB_ROWS, i1 = min(i0 + KB_ROWS, a.n1);
   for (int i = i0; i < i1; ++i) {
-    T df[KB_DMAX][KB_VEC], d2[KB_VEC], r2[KB_VEC], w[KB_VEC];   // w = sum_l G K0 /(ls^2 den)
+    T df[KB_DMAX][KB_VEC], d2[KB_VEC], r2[KB_VEC], w[KB_VEC];   // w = sum_l G u
 #pragma unroll
     for (int v = 0; v < KB_VEC; ++v) { d2[v] = T(0); w[v] = T(0); r2[v] = T(0); }
 #pragma unroll
@@ -301,11 +329,7 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
 #pragma unroll
       for (int v = 0; v < KB_VEC; ++v) { df[d][v] = xi - xj[d][v]; d2[v] = fma(df[d][v], df[d][v], d2[v]); }
     }
-    if (MG) {
-      const int gi = (int)a.g1[i];
-#pragma unroll
-      for (int v = 0; v < KB_VEC; ++v) r2[v] = s_r2[gi * a.ng + gj[v]];
-    }
+    kb_row_r2<T, MG>(a, i, s_r2, gj, r2);
     if (nv > 0) {
       // phase 1: issue every load of this row (one 16-byte vector per factor) before any is used
       T g[LMAX][KB_VEC];
@@ -333,41 +357,12 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
           const T c = s_c[l], s2 = s_s2[l];
 #pragma unroll
           for (int v = 0; v < KB_VEC; ++v) {
-            T k0, idn, ee = T(0), ir = T(0);
-            if (MG) {
-              const T den = fma(s_a[l], r2[v], T(1));
-              idn = fast_div(T(1), den);
-              const T sc = a.p_half == T(1) ? idn : Num<T>::pow(den, -a.p_half);
-              k0 = s2 * fast_exp(c * d2[v] * idn) * sc;
-            } else if (KIND == 1) {
-              idn = T(1);
-              const T vv = c * Num<T>::sqrt(d2[v]);
-              ee = s2 * fast_exp(-vv);
-              k0 = (T(1) + vv) * ee;
-            } else if (KIND == 2) {
-              idn = T(1);
-              ir = d2[v] > T(0) ? Num<T>::rsqrt(d2[v]) : T(0);      // 1/r; 0 at r = 0 (a d2 below 1e-38 is 0 under -ftz)
-              ee = s2 * fast_exp(-c * d2[v] * ir);                  // r = d2 / r
-              k0 = ee;
-            } else if (KIND == 3) {
-              idn = T(1);
-              const T vv = c * Num<T>::sqrt(d2[v]);
-              ee = s2 * fast_exp(-vv);
-              ir = T(1) + vv;
-              k0 = fma(vv * T(1.0 / 3.0), vv, ir) * ee;
-            } else {
-              idn = T(1);
-              k0 = s2 * fast_exp(c * d2[v]);
-            }
-            const T gk = g[l][v] * k0;
-            const T u = KIND == 1 ? g[l][v] * ee * c * c                  // G s2 exp(-v) 3 / ls^2
-                      : KIND == 2 ? gk * c * ir                           // G K0 / (ls r)
-                      : KIND == 3 ? g[l][v] * ee * ir * c * c * T(1.0 / 3.0)  // G s2 (1 + v) exp(-v) 5 / (3 ls^2)
-                                  : gk * (T(-2) * c) * idn;               // G K0 / (ls^2 den)
+            const KBTerms<T> t = kb_terms<T, MG, KIND>(c, s2, MG ? s_a[l] : T(0), r2[v], d2[v], a.p_half, g[l][v]);
+            const T gk = g[l][v] * t.k0;
             acc_s[l] += gk;
-            acc_l[l] = fma(u, d2[v], acc_l[l]);          // later divided by ls
-            if (MG) acc_a[l] = fma(gk * r2[v], (T(-1) * c * d2[v] * idn - a.p_half) * idn, acc_a[l]);
-            w[v] += u;
+            acc_l[l] = fma(t.u, d2[v], acc_l[l]);          // later divided by ls
+            if (MG) acc_a[l] = fma(gk * r2[v], (T(-1) * c * d2[v] * t.idn - a.p_half) * t.idn, acc_a[l]);
+            w[v] += t.u;
           }
         }
       }
@@ -441,81 +436,82 @@ __global__ void cdist_kernel(const T* __restrict__ x1, const T* __restrict__ x2,
   out[e] = Num<T>::sqrt(d2);
 }
 
-// kinds 0-3 without groups; the multi-group form is the RBF's only
-inline bool kb_kind_ok(int kind, bool mg) { return mg ? kind == 0 : (kind >= 0 && kind <= 3); }
+// ---- Host dispatch: runtime values -> the compile-time parameters of the kernels.  Every instantiated kernel is reached here.
+template <int V> using kb_int = std::integral_constant<int, V>;
 
-template <typename T, int KIND>
-void kbuild_fwd_launch(const KBArgs<T>& a, bool al, dim3 grid, T* out, T* out_lo, cudaStream_t st) {
-  if (al) kbuild_fwd_kernel<T, false, true, KIND><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
-  else kbuild_fwd_kernel<T, false, false, KIND><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
+// (kind, groups) -> f(std::bool_constant<MG>, kb_int<KIND>) for the five supported forms: the RBF with and without groups and
+// the three Matern kinds (which have no multi-group form in the reference); GPZ_ERR_UNSUPPORTED for anything else
+template <typename F> int kb_dispatch_kind(int kind, bool mg, F&& f) {
+  if (mg) return kind == 0 ? f(std::true_type{}, kb_int<0>{}) : GPZ_ERR_UNSUPPORTED;
+  switch (kind) {
+    case 0: return f(std::false_type{}, kb_int<0>{});
+    case 1: return f(std::false_type{}, kb_int<1>{});
+    case 2: return f(std::false_type{}, kb_int<2>{});
+    case 3: return f(std::false_type{}, kb_int<3>{});
+    default: return GPZ_ERR_UNSUPPORTED;
+  }
+}
+
+template <typename F> int kb_dispatch_aligned(bool al, F&& f) { return al ? f(std::true_type{}) : f(std::false_type{}); }
+
+// factors per backward launch: the RBF's register accumulators are sized to L (4 / 8 / 12 / 16, else KB_LMAX);
+// the Matern kinds always take KB_LMAX
+template <int KIND, typename F> int kb_dispatch_lmax(int L, F&& f) {
+  if constexpr (KIND != 0) return f(kb_int<KB_LMAX>{});
+  else if (L <= 4) return f(kb_int<4>{});
+  else if (L <= 8) return f(kb_int<8>{});
+  else if (L <= 12) return f(kb_int<12>{});
+  else if (L <= 16) return f(kb_int<16>{});
+  else return f(kb_int<KB_LMAX>{});
+}
+
+// sizes every entry point supports: 1 <= D <= KB_DMAX, 1 <= L <= l_max, and 1..KB_GMAX groups when there are groups
+template <typename T> bool kb_sizes_ok(const KBArgs<T>& a, int l_max) {
+  return a.D >= 1 && a.D <= KB_DMAX && a.L >= 1 && a.L <= l_max && (a.g1 == nullptr || (a.ng >= 1 && a.ng <= KB_GMAX));
 }
 
 template <typename T>
 int kbuild_fwd(const KBArgs<T>& a, T* out, T* out_lo, cudaStream_t st) {
-  if (a.D < 1 || a.D > KB_DMAX || a.L < 1 || a.L > KB_LMAX * 8) return GPZ_ERR_UNSUPPORTED;
-  const bool mg = a.g1 != nullptr;
-  if (mg && (a.ng < 1 || a.ng > KB_GMAX)) return GPZ_ERR_UNSUPPORTED;
+  if (!kb_sizes_ok(a, KB_LMAX * 8)) return GPZ_ERR_UNSUPPORTED;
   if (a.n1 == 0 || a.n2 == 0) return GPZ_OK;
   const bool al = (a.n2 % KB_VEC == 0) && ((reinterpret_cast<uintptr_t>(out) & 31) == 0) &&
                   ((reinterpret_cast<uintptr_t>(out_lo) & 15) == 0);
-  dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
-  if (!kb_kind_ok(a.kind, mg)) return GPZ_ERR_UNSUPPORTED;       // the Matern kinds have no multi-group form in the reference
-  if (a.kind == 1) kbuild_fwd_launch<T, 1>(a, al, grid, out, out_lo, st);
-  else if (a.kind == 2) kbuild_fwd_launch<T, 2>(a, al, grid, out, out_lo, st);
-  else if (a.kind == 3) kbuild_fwd_launch<T, 3>(a, al, grid, out, out_lo, st);
-  else if (mg) {
-    if (al) kbuild_fwd_kernel<T, true, true><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
-    else kbuild_fwd_kernel<T, true, false><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
-  } else {
-    if (al) kbuild_fwd_kernel<T, false, true><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
-    else kbuild_fwd_kernel<T, false, false><<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
-  }
-  GPZ_CHECK_LAUNCH();
-  return GPZ_OK;
+  const dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
+  return kb_dispatch_kind(a.kind, a.g1 != nullptr, [&](auto mg, auto kind) {
+    return kb_dispatch_aligned(al, [&](auto aligned) {
+      kbuild_fwd_kernel<T, decltype(mg)::value, decltype(aligned)::value, decltype(kind)::value>
+          <<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
+      GPZ_CHECK_LAUNCH();
+      return GPZ_OK;
+    });
+  });
 }
 
 template <typename T>
 int kbuild_bwd(const KBArgs<T>& a, const T* G, T* g_x1, T* g_x2, T* g_sigma, T* g_ls, T* g_a, double* ws, cudaStream_t st) {
-  if (a.D < 1 || a.D > KB_DMAX || a.L < 1) return GPZ_ERR_UNSUPPORTED;
-  const bool mg = a.g1 != nullptr;
-  if (mg && (a.ng < 1 || a.ng > KB_GMAX)) return GPZ_ERR_UNSUPPORTED;
+  if (!kb_sizes_ok(a, INT_MAX)) return GPZ_ERR_UNSUPPORTED;
   const int n1D = a.n1 * a.D;
   GPZ_CUDA(cudaMemsetAsync(ws, 0, sizeof(double) * (3 * (size_t)a.L + n1D), st));
   if (g_x2) GPZ_CUDA(cudaMemsetAsync(g_x2, 0, sizeof(T) * a.n2 * a.D, st));
   double* w_sigma = ws; double* w_ls = ws + a.L; double* w_a = ws + 2 * a.L; double* w_x1 = ws + 3 * a.L;
   if (a.n1 > 0 && a.n2 > 0) {
     const bool al = (a.n2 % KB_VEC == 0) && ((reinterpret_cast<uintptr_t>(G) & 31) == 0);
-    dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
-    if (!kb_kind_ok(a.kind, mg)) return GPZ_ERR_UNSUPPORTED;
-    const int lmax = a.kind != 0 ? KB_LMAX : (a.L <= 4 ? 4 : (a.L <= 8 ? 8 : (a.L <= 12 ? 12 : (a.L <= 16 ? 16 : KB_LMAX))));
-    for (int l0 = 0; l0 < a.L; l0 += lmax) {
-      const int Lc = min(lmax, a.L - l0);
-      // g_x1/g_x2 accumulate over all l-chunks (atomics), so every chunk launch adds its share
-#define GPZ_KB_LAUNCH(MGV, ALV, LM) \
-  kbuild_bwd_kernel<T, MGV, ALV, LM><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a)
-#define GPZ_KB_MATERN(KIND)                                                                                                \
-  do {                                                                                                                     \
-    if (al) kbuild_bwd_kernel<T, false, true, KB_LMAX, KIND><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a);  \
-    else kbuild_bwd_kernel<T, false, false, KB_LMAX, KIND><<<grid, KB_THREADS, 0, st>>>(a, G, l0, Lc, w_x1, g_x2, w_sigma, w_ls, w_a);   \
-  } while (0)
-#define GPZ_KB_DISPATCH(LM)                                   \
-  do {                                                        \
-    if (mg) { if (al) GPZ_KB_LAUNCH(true, true, LM); else GPZ_KB_LAUNCH(true, false, LM); }     \
-    else { if (al) GPZ_KB_LAUNCH(false, true, LM); else GPZ_KB_LAUNCH(false, false, LM); }      \
-  } while (0)
-      if (a.kind == 1) GPZ_KB_MATERN(1);
-      else if (a.kind == 2) GPZ_KB_MATERN(2);
-      else if (a.kind == 3) GPZ_KB_MATERN(3);
-      else if (lmax == 4) GPZ_KB_DISPATCH(4);
-      else if (lmax == 8) GPZ_KB_DISPATCH(8);
-      else if (lmax == 12) GPZ_KB_DISPATCH(12);
-      else if (lmax == 16) GPZ_KB_DISPATCH(16);
-      else GPZ_KB_DISPATCH(KB_LMAX);
-#undef GPZ_KB_MATERN
-#undef GPZ_KB_DISPATCH
-#undef GPZ_KB_LAUNCH
-      GPZ_CHECK_LAUNCH();
-    }
+    const dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
+    const int rc = kb_dispatch_kind(a.kind, a.g1 != nullptr, [&](auto mg, auto kind) {
+      return kb_dispatch_lmax<decltype(kind)::value>(a.L, [&](auto lmax) {
+        return kb_dispatch_aligned(al, [&](auto aligned) {
+          constexpr int LMAX = decltype(lmax)::value;
+          // g_x1/g_x2 accumulate over all l-chunks (atomics), so every chunk launch adds its share
+          for (int l0 = 0; l0 < a.L; l0 += LMAX) {
+            kbuild_bwd_kernel<T, decltype(mg)::value, decltype(aligned)::value, LMAX, decltype(kind)::value>
+                <<<grid, KB_THREADS, 0, st>>>(a, G, l0, min(LMAX, a.L - l0), w_x1, g_x2, w_sigma, w_ls, w_a);
+            GPZ_CHECK_LAUNCH();
+          }
+          return GPZ_OK;
+        });
+      });
+    });
+    if (rc != GPZ_OK) return rc;
   }
   const int tot = max(a.L, n1D);
   kbuild_bwd_finalize_kernel<T><<<(unsigned)cdiv(tot, 256), 256, 0, st>>>(ws, a.sigma, a.ls, a.L, n1D, g_sigma, g_ls, g_a, g_x1);
@@ -558,19 +554,15 @@ extern "C" int gpz_kernel_build_fwd_h_f32(const float* x1, const float* x2, cons
                                           const float* r2, const int64_t* g1, const int64_t* g2, int n1, int n2, int D, int L,
                                           int ng, int kind, float p_half, float jitter, void* out_h, void* out_l,
                                           float* out_scale, void* stream) {
-  KBArgs<float> k{x1, x2, sigma, ls, a, r2, g1, g2, n1, n2, D, L, ng, p_half, jitter, kind};
-  if (D < 1 || D > KB_DMAX || L < 1 || L > KB_LMAX * 8) return GPZ_ERR_UNSUPPORTED;
-  const bool mg = g1 != nullptr;
-  if (mg && (ng < 1 || ng > KB_GMAX)) return GPZ_ERR_UNSUPPORTED;
+  const KBArgs<float> k{x1, x2, sigma, ls, a, r2, g1, g2, n1, n2, D, L, ng, p_half, jitter, kind};
+  if (!kb_sizes_ok(k, KB_LMAX * 8)) return GPZ_ERR_UNSUPPORTED;
   if (n2 % KB_VEC8 || (reinterpret_cast<uintptr_t>(out_h) & 15) || (reinterpret_cast<uintptr_t>(out_l) & 15)) return GPZ_ERR_UNSUPPORTED;
   if (n1 == 0 || n2 == 0) return GPZ_OK;
-  dim3 grid((unsigned)cdiv(n2, (int64_t)KB_THREADS * KB_VEC8), (unsigned)cdiv(n1, KB_ROWS));
-  if (!kb_kind_ok(kind, mg)) return GPZ_ERR_UNSUPPORTED;
-  if (kind == 1) kbuild_fwd_h_kernel<false, 1><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
-  else if (kind == 2) kbuild_fwd_h_kernel<false, 2><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
-  else if (kind == 3) kbuild_fwd_h_kernel<false, 3><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
-  else if (mg) kbuild_fwd_h_kernel<true><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
-  else kbuild_fwd_h_kernel<false><<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
-  GPZ_CHECK_LAUNCH();
-  return GPZ_OK;
+  const dim3 grid((unsigned)cdiv(n2, (int64_t)KB_THREADS * KB_VEC8), (unsigned)cdiv(n1, KB_ROWS));
+  return kb_dispatch_kind(kind, g1 != nullptr, [&](auto mg, auto kd) {
+    kbuild_fwd_h_kernel<decltype(mg)::value, decltype(kd)::value>
+        <<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
+    GPZ_CHECK_LAUNCH();
+    return GPZ_OK;
+  });
 }

@@ -313,6 +313,21 @@ def _check_kernel_args(x1, x2, sigma, ls, a, r2, g1, g2):
     return a, r2, g1, g2
 
 
+def _kernel_args(x1, x2, sigma, ls, a, r2, g1, g2, check=True):
+    """The leading arguments of every gpz_kernel_build_* call: ((x1, x2, sigma, ls, a, r2, g1, g2), (n1, n2, D, L, ng)), with
+    a = r2 = g1 = g2 = None and ng = 0 when there are no groups (g1 None).  `check` makes the tensors contiguous and runs
+    `_check_kernel_args`; the backward passes check=False, its tensors being the ones its forward returned from here."""
+    if check:
+        x1, x2, sigma, ls = _c(x1), _c(x2), _c(sigma), _c(ls)
+        a, r2, g1, g2 = _check_kernel_args(x1, x2, sigma, ls, a, r2, g1, g2)
+        if g1 is not None:
+            a, r2, g1, g2 = _c(a), _c(r2), _c(g1), _c(g2)
+    if g1 is None:
+        a = r2 = g2 = None
+    n1, D = x1.shape
+    return (x1, x2, sigma, ls, a, r2, g1, g2), (n1, x2.shape[0], D, sigma.numel(), 0 if g1 is None else r2.shape[0])
+
+
 class KernelBuild(Function):
     """K[l,i,j] = sigma_l^2 exp(-0.5 |x1_i-x2_j|^2/(ls_l^2 den)) / den^p_half (+ jitter on i==j).
 
@@ -320,22 +335,13 @@ class KernelBuild(Function):
 
     @staticmethod
     def forward(ctx, x1, x2, sigma, ls, a, r2, g1, g2, p_half, jitter, want_lo=False, kind=0):
-        x1, x2, sigma, ls = _c(x1), _c(x2), _c(sigma), _c(ls)
+        t, (n1, n2, D, L, ng) = _kernel_args(x1, x2, sigma, ls, a, r2, g1, g2)
         dt = x1.dtype
-        a, r2, g1, g2 = _check_kernel_args(x1, x2, sigma, ls, a, r2, g1, g2)
-        n1, D = x1.shape
-        n2 = x2.shape[0]
-        L = sigma.numel()
-        mg = g1 is not None
-        if mg:
-            a, r2, g1, g2 = _c(a), _c(r2), _c(g1), _c(g2)
         out = torch.empty((L, n1, n2), dtype=dt, device=x1.device)
         want_lo = bool(want_lo) and dt == torch.float32
         out_lo = torch.empty_like(out) if want_lo else None
-        call("kernel_build_fwd", dt, x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
-             g2 if mg else None, n1, n2, D, L, r2.shape[0] if mg else 0, int(kind), p_half, jitter, out, out_lo)
-        ctx.save_for_backward(x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
-                              g2 if mg else None)
+        call("kernel_build_fwd", dt, *t, n1, n2, D, L, ng, int(kind), p_half, jitter, out, out_lo)
+        ctx.save_for_backward(*t)
         ctx.p_half = p_half
         ctx.kind = int(kind)
         ctx.want_lo = want_lo
@@ -350,27 +356,23 @@ class KernelBuild(Function):
     def backward(ctx, G, *unused):
         if G is None:
             return (None,) * 12
-        x1, x2, sigma, ls, a, r2, g1, g2 = ctx.saved_tensors
-        grads = _kernel_build_bwd(x1, x2, sigma, ls, a, r2, g1, g2, ctx.p_half, getattr(ctx, "kind", 0), ctx.needs_input_grad[:2], G)
+        grads = _kernel_build_bwd(*ctx.saved_tensors, ctx.p_half, ctx.kind, ctx.needs_input_grad[:2], G)
         return grads + (None,) * 7
 
 
 def _kernel_build_bwd(x1, x2, sigma, ls, a, r2, g1, g2, p_half, kind, need, G):
     """(dL/dx1, dL/dx2, dL/dsigma, dL/dlengthscale, dL/da) from dL/dK on the current stream (csrc/kernel_build.cu)."""
+    t, (n1, n2, D, L, ng) = _kernel_args(x1, x2, sigma, ls, a, r2, g1, g2, check=False)
+    x1, x2, sigma, ls, a, _, g1, _ = t
     dt = x1.dtype
     G = _c(G)
-    n1, D = x1.shape
-    n2 = x2.shape[0]
-    L = sigma.numel()
-    mg = g1 is not None
     g_x1 = torch.empty_like(x1) if need[0] else None
     g_x2 = torch.empty_like(x2) if need[1] else None
     g_sigma = torch.empty_like(sigma)
     g_ls = torch.empty_like(ls)
-    g_a = torch.empty_like(a) if mg else None
+    g_a = torch.empty_like(a) if g1 is not None else None
     ws = torch.empty(3 * L + n1 * D, dtype=torch.float64, device=x1.device)
-    call("kernel_build_bwd", dt, x1, x2, sigma, ls, a, r2, g1, g2, n1, n2, D, L, r2.shape[0] if mg else 0, int(kind), p_half, G,
-         g_x1, g_x2, g_sigma, g_ls, g_a, ws)
+    call("kernel_build_bwd", dt, *t, n1, n2, D, L, ng, int(kind), p_half, G, g_x1, g_x2, g_sigma, g_ls, g_a, ws)
     return g_x1, g_x2, g_sigma, g_ls, g_a
 
 
@@ -393,28 +395,18 @@ class KernelBuildH(Function):
 
     @staticmethod
     def forward(ctx, x1, x2, sigma, ls, a, r2, g1, g2, p_half, jitter, kind=0, box=None):
-        x1, x2, sigma, ls = _c(x1), _c(x2), _c(sigma), _c(ls)
         dt = x1.dtype
         assert dt == torch.float32
-        a, r2, g1, g2 = _check_kernel_args(x1, x2, sigma, ls, a, r2, g1, g2)
-        n1, D = x1.shape
-        n2 = x2.shape[0]
-        L = sigma.numel()
-        mg = g1 is not None
-        if mg:
-            a, r2, g1, g2 = _c(a), _c(r2), _c(g1), _c(g2)
+        t, (n1, n2, D, L, ng) = _kernel_args(x1, x2, sigma, ls, a, r2, g1, g2)
         Kh, Kl = _plane_pair(L, n1, n2, x1.device)
         sK = torch.empty(L, dtype=dt, device=x1.device)
-        call("kernel_build_fwd_h", dt, x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
-             g2 if mg else None, n1, n2, D, L, r2.shape[0] if mg else 0, int(kind), p_half, jitter, Kh, Kl, sK)
-        ctx.save_for_backward(x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None,
-                              g2 if mg else None)
+        call("kernel_build_fwd_h", dt, *t, n1, n2, D, L, ng, int(kind), p_half, jitter, Kh, Kl, sK)
+        ctx.save_for_backward(*t)
         ctx.p_half = p_half
         ctx.kind = int(kind)
         ctx.box = box
         if box is not None:
-            box.args = (x1, x2, sigma, ls, a if mg else None, r2 if mg else None, g1 if mg else None, g2 if mg else None,
-                        p_half, int(kind), tuple(ctx.needs_input_grad[:2]))
+            box.args = (*t, p_half, int(kind), tuple(ctx.needs_input_grad[:2]))
         handle = torch.empty(1, dtype=dt, device=x1.device).expand(L, n1, n2)
         ctx.set_materialize_grads(False)      # otherwise autograd zero-fills "gradients" for the fp16 planes (2 x 0.67 GB)
         ctx.mark_non_differentiable(Kh, Kl, sK)

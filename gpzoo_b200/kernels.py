@@ -48,22 +48,17 @@ class _RBFBase(nn.Module):
         sigma, ls = self._params()
         dt = X.dtype
         sigma, ls = sigma.to(dt), ls.to(dt)
+        if groupsX is not None:     # (a, r^2 table, groups of X, groups of Z, p_half)
+            group = (self._group_coeff().to(dt), _r2_table(self.embedding, dt).to(X.device), groupsX, groupsZ,
+                     0.5 * float(self.input_dim))
+        else:
+            group = (None, None, None, None, 1.0)
         if want_h:      # split-FP16 planes for the tensor-core predict: (stand-in for K, Kh, Kl, scale), leading L kept
             box = F.KernelBuildBox()       # lets the consumer of the planes launch this build's backward early (functional.py)
-            if groupsX is not None:
-                out = F.KernelBuildH.apply(X, Z, sigma, ls, self._group_coeff().to(dt), _r2_table(self.embedding, dt).to(X.device),
-                                           groupsX, groupsZ, 0.5 * float(self.input_dim), float(jitter), 0, box)
-            else:
-                out = F.KernelBuildH.apply(X, Z, sigma, ls, None, None, None, None, 1.0, float(jitter), self._kind, box)
+            out = F.KernelBuildH.apply(X, Z, sigma, ls, *group, float(jitter), self._kind, box)
             out[0]._gpz_box = box
             return out
-        if groupsX is not None:
-            a = self._group_coeff().to(dt)
-            r2 = _r2_table(self.embedding, dt).to(X.device)
-            K = F.KernelBuild.apply(X, Z, sigma, ls, a, r2, groupsX, groupsZ, 0.5 * float(self.input_dim), float(jitter),
-                                    want_lo)
-        else:
-            K = F.KernelBuild.apply(X, Z, sigma, ls, None, None, None, None, 1.0, float(jitter), want_lo, self._kind)
+        K = F.KernelBuild.apply(X, Z, sigma, ls, *group, float(jitter), want_lo, self._kind)
         if want_lo and isinstance(K, tuple):          # (K, K_lo): lo part for the split-TF32 tensor-core GEMMs
             return K if self._batched else (K[0][0], K[1][0])
         if want_lo:
@@ -80,6 +75,19 @@ class _RBFBase(nn.Module):
         """sigma^2 exp(-0.5 d^2 / l^2) on a precomputed squared-distance tensor (kernels.py:128-130).
         Element-wise convenience kept for API compatibility; not on the fused hot path."""
         return (self.sigma ** 2) * torch.exp(-0.5 * distance_squared / (self.lengthscale ** 2))
+
+
+class _MultiGroup:
+    """forward of the multi-group kernels: points carry group labels (groupsX, groupsZ); diag=True is sigma^2, whatever the
+    groups."""
+    _input_dim_from_X = False       # True: p = X.shape[-1] on every call (batched_MGGP_RBF) instead of input_dim
+
+    def forward(self, X, Z, groupsX, groupsZ, diag=False, _jitter=0.0, _want_lo=False, _want_h=False):
+        if diag:
+            return self._diag(X)
+        if self._input_dim_from_X:
+            self.input_dim = X.shape[-1]
+        return self._build(X, Z, groupsX, groupsZ, jitter=_jitter, want_lo=_want_lo, want_h=_want_h)
 
 
 class RBF(_RBFBase):
@@ -108,7 +116,7 @@ class NSF_RBF(RBF):
         self.lengthscale = nn.Parameter(lengthscale * torch.ones((L, 1, 1)))
 
 
-class MGGP_RBF(RBF):
+class MGGP_RBF(_MultiGroup, RBF):
     """Multi-group RBF, scalar parameters, coefficient a = group_diff_param (kernels.py:158-191)."""
 
     def __init__(self, sigma=1.0, lengthscale=2.0, group_diff_param=1.0, n_groups=2, device="cpu"):
@@ -122,13 +130,8 @@ class MGGP_RBF(RBF):
     def _group_coeff(self):
         return _flat(self.group_diff_param)
 
-    def forward(self, X, Z, groupsX, groupsZ, diag=False, _jitter=0.0, _want_lo=False, _want_h=False):
-        if diag:
-            return self._diag(X)
-        return self._build(X, Z, groupsX, groupsZ, jitter=_jitter, want_lo=_want_lo, want_h=_want_h)
 
-
-class MGGP_NSF_RBF(NSF_RBF):
+class MGGP_NSF_RBF(_MultiGroup, NSF_RBF):
     """Per-factor multi-group RBF, a = group_diff_param**2 (kernels.py:194-228)."""
 
     def __init__(self, sigma=1.0, lengthscale=2.0, group_diff_param=1.0, n_groups=2, L=10, device="cpu"):
@@ -142,11 +145,6 @@ class MGGP_NSF_RBF(NSF_RBF):
 
     def _group_coeff(self):
         return _flat(self.group_diff_param) ** 2
-
-    def forward(self, X, Z, groupsX, groupsZ, diag=False, _jitter=0.0, _want_lo=False, _want_h=False):
-        if diag:
-            return self._diag(X)
-        return self._build(X, Z, groupsX, groupsZ, jitter=_jitter, want_lo=_want_lo, want_h=_want_h)
 
 
 class batched_RBF(_RBFBase):
@@ -206,8 +204,9 @@ class batched_Matern52(batched_RBF):
         return (self.sigma ** 2) * (1 + v + v * v / 3) * torch.exp(-v)
 
 
-class batched_MGGP_RBF(batched_RBF):
+class batched_MGGP_RBF(_MultiGroup, batched_RBF):
     """kernels.py:62-104: a = |group_diff_param|, p = X.shape[-1]."""
+    _input_dim_from_X = True
 
     def __init__(self, sigma=1.0, lengthscale=1.0, group_diff_param=1.0, n_groups=10):
         super().__init__(sigma, lengthscale)
@@ -221,9 +220,3 @@ class batched_MGGP_RBF(batched_RBF):
     def _group_coeff(self):
         n = self._params()[0].numel()
         return torch.abs(_flat(self.group_diff_param)).expand(n)
-
-    def forward(self, X, Z, groupsX, groupsZ, diag=False, _jitter=0.0, _want_lo=False, _want_h=False):
-        if diag:
-            return self._diag(X)
-        self.input_dim = X.shape[-1]
-        return self._build(X, Z, groupsX, groupsZ, jitter=_jitter, want_lo=_want_lo, want_h=_want_h)
