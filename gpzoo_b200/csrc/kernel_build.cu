@@ -49,6 +49,11 @@ template <typename T> struct KBArgs {
 //   kind 1:  K0 = (1 + v) e,            u = (3 / ls^2) e                 (finite at r = 0)
 //   kind 2:  K0 = e,                    u = e / (ls r), 0 at r = 0        (the sub-gradient 0 at the cusp)
 //   kind 3:  K0 = (1 + v + v^2/3) e,    u = (5 / (3 ls^2)) (1 + v) e     (finite at r = 0)
+//
+// ARD (per-dimension lengthscales ls[l,d], no groups): every kind is evaluated at unit lengthscale on the scaled squared
+// distance s2 = sum_d (x1_d - x2_d)^2 / ls[l,d]^2, which takes the place of d2 above.  With u from kb_terms at unit lengthscale
+// (dK/ds2 = -u/2):  dK/dx1_d = -u (x1_d - x2_d) / ls_d^2,  dK/dls_d = u (x1_d - x2_d)^2 / ls_d^3.  Equal ls[l,d] give the
+// isotropic kernel.
 
 // s_c[l] of the kernels: -1/(2 ls^2) for the RBF, the factor of r in v for the Matern kinds
 template <typename T, int KIND> __device__ __forceinline__ T kb_coeff(T ls) {
@@ -114,12 +119,24 @@ __device__ __forceinline__ KBTerms<T> kb_terms(T c, T s2, T a_l, T r2, T d2, T p
 
 // ---- Tile pieces shared by the kernels.
 
+// ARD: 1/ls[l,d]^2 of factors l0 .. l0 + n - 1 into s_il2[l * KB_DMAX + d], 0 past D (a.ls is L x D)
+template <typename T>
+__device__ __forceinline__ void kb_stage_il2(const KBArgs<T>& a, int tid, int l0, int n, T* s_il2) {
+  for (int e = tid; e < n * KB_DMAX; e += KB_THREADS) {
+    const int l = e / KB_DMAX, d = e % KB_DMAX;
+    const T ls = d < a.D ? a.ls[(int64_t)(l0 + l) * a.D + d] : T(1);
+    s_il2[e] = d < a.D ? T(1) / (ls * ls) : T(0);
+  }
+}
+
 // factors l0 .. l0 + n - 1 into shared memory (s_c = kb_coeff, s_s2 = sigma^2, s_a with groups) and, with groups, the r^2
-// table; tid = threadIdx.x, the caller synchronises
-template <typename T, bool MG, int KIND>
-__device__ __forceinline__ void kb_stage(const KBArgs<T>& a, int tid, int l0, int n, T* s_c, T* s_s2, T* s_a, T* s_r2) {
+// table, with ARD s_il2 (kb_coeff then at unit lengthscale); tid = threadIdx.x, the caller synchronises
+template <typename T, bool MG, int KIND, bool ARD = false>
+__device__ __forceinline__ void kb_stage(const KBArgs<T>& a, int tid, int l0, int n, T* s_c, T* s_s2, T* s_a, T* s_r2,
+                                         T* s_il2 = nullptr) {
+  if (ARD) kb_stage_il2(a, tid, l0, n, s_il2);
   for (int l = tid; l < n; l += KB_THREADS) {
-    const T ls = a.ls[l0 + l], sg = a.sigma[l0 + l];
+    const T ls = ARD ? T(1) : a.ls[l0 + l], sg = a.sigma[l0 + l];
     s_c[l] = kb_coeff<T, KIND>(ls);
     s_s2[l] = sg * sg;
     if (MG) s_a[l] = a.a[l0 + l];
@@ -153,6 +170,32 @@ __device__ __forceinline__ void kb_row_d2(const KBArgs<T>& a, int i, const T (&x
   }
 }
 
+// ARD: per-dimension squared differences of row i to the thread's columns (0 past D, where x2's columns are 0 as well)
+template <typename T, int VEC>
+__device__ __forceinline__ void kb_row_sq(const KBArgs<T>& a, int i, const T (&xj)[KB_DMAX][VEC], T (&sq)[KB_DMAX][VEC]) {
+#pragma unroll
+  for (int d = 0; d < KB_DMAX; ++d) {
+    const T xi = d < a.D ? a.x1[(int64_t)i * a.D + d] : T(0);
+#pragma unroll
+    for (int v = 0; v < VEC; ++v) { const T df = xi - xj[d][v]; sq[d][v] = df * df; }
+  }
+}
+
+// ARD: scaled squared distances s2 = sum_d sq_d il2_d of one factor (il2 = s_il2 + l * KB_DMAX).  KB_DMAX terms whatever D
+// (sq and il2 are 0 past D): a switch on D per factor, measured, made the Matern kinds' forward slower still
+template <typename T, int VEC>
+__device__ __forceinline__ void kb_scaled_d2(const T* il2, const T (&sq)[KB_DMAX][VEC], T (&s2)[VEC]) {
+  T w[KB_DMAX];
+#pragma unroll
+  for (int d = 0; d < KB_DMAX; ++d) w[d] = il2[d];
+#pragma unroll
+  for (int v = 0; v < VEC; ++v) {
+    s2[v] = sq[0][v] * w[0];
+#pragma unroll
+    for (int d = 1; d < KB_DMAX; ++d) s2[v] = fma(sq[d][v], w[d], s2[v]);
+  }
+}
+
 // group r^2 of row i and the thread's columns (groups only)
 template <typename T, bool MG, int VEC>
 __device__ __forceinline__ void kb_row_r2(const KBArgs<T>& a, int i, const T* s_r2, const int (&gj)[VEC], T (&r2)[VEC]) {
@@ -167,12 +210,15 @@ template <typename T> struct Vec4 { T v[4]; };
 
 // fp64 Matern-1/2: without a register target ptxas settles on 64 registers and spills; 3 CTAs per SM (<= 80 registers) keep
 // it spill-free like Matern-3/2.  A min-blocks value of 0 is no bound at all, so every other instantiation compiles as before.
-template <typename T, bool MG, bool ALIGNED, int KIND = 0>
-__global__ void __launch_bounds__(KB_THREADS, (KIND == 2 && sizeof(T) == 8) ? 3 : 0) kbuild_fwd_kernel(const KBArgs<T> a, T* __restrict__ out, T* __restrict__ out_lo) {
+// ARD: per-dimension lengthscales (see the kinds block); the row keeps its per-dimension squared differences, s2 per factor.
+// Those take ~20 more registers, and the 3-CTA bound made the fp64 ARD Matern-1/2 spill, so ARD has no bound.
+template <typename T, bool MG, bool ALIGNED, int KIND = 0, bool ARD = false>
+__global__ void __launch_bounds__(KB_THREADS, (KIND == 2 && sizeof(T) == 8 && !ARD) ? 3 : 0) kbuild_fwd_kernel(const KBArgs<T> a, T* __restrict__ out, T* __restrict__ out_lo) {
   __shared__ T s_c[KB_LMAX * 8], s_s2[KB_LMAX * 8], s_a[KB_LMAX * 8];
   __shared__ T s_r2[MG ? KB_GMAX * KB_GMAX : 1];
+  __shared__ __align__(16) T s_il2[ARD ? KB_LMAX * 8 * KB_DMAX : 1];
   const int tid = threadIdx.x;
-  kb_stage<T, MG, KIND>(a, tid, 0, a.L, s_c, s_s2, s_a, s_r2);
+  kb_stage<T, MG, KIND, ARD>(a, tid, 0, a.L, s_c, s_s2, s_a, s_r2, s_il2);
   __syncthreads();
 
   const int64_t j0 = ((int64_t)blockIdx.x * KB_THREADS + tid) * KB_VEC;
@@ -183,11 +229,13 @@ __global__ void __launch_bounds__(KB_THREADS, (KIND == 2 && sizeof(T) == 8) ? 3 
   kb_load_cols<T, MG>(a, j0, nv, xj, gj);
   const int i0 = blockIdx.y * KB_ROWS, i1 = min(i0 + KB_ROWS, a.n1);
   for (int i = i0; i < i1; ++i) {
-    T d2[KB_VEC], r2[KB_VEC];
-    kb_row_d2(a, i, xj, d2);
+    T d2[KB_VEC], r2[KB_VEC], sq[ARD ? KB_DMAX : 1][KB_VEC];
+    if constexpr (ARD) kb_row_sq(a, i, xj, sq);
+    else kb_row_d2(a, i, xj, d2);
     kb_row_r2<T, MG>(a, i, s_r2, gj, r2);
     for (int l = 0; l < a.L; ++l) {
       const T c = s_c[l], s2 = s_s2[l];
+      if constexpr (ARD) kb_scaled_d2(s_il2 + l * KB_DMAX, sq, d2);
       Vec4<T> k;
 #pragma unroll
       for (int v = 0; v < KB_VEC; ++v) {
@@ -226,15 +274,17 @@ __global__ void __launch_bounds__(KB_THREADS, (KIND == 2 && sizeof(T) == 8) ? 3 
 // in (2^14, 2^15].  4 bytes per entry leave the SM (half of K + lo plane in fp32); each thread owns 8 consecutive j and
 // streams one 16-byte store per plane, row and factor.
 constexpr int KB_VEC8 = 8;
-template <bool MG, int KIND = 0>
+template <bool MG, int KIND = 0, bool ARD = false>
 __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<float> a, __half* __restrict__ out_h,
                                                                   __half* __restrict__ out_l, float* __restrict__ out_scale) {
   __shared__ float s_c[KB_LMAX * 8], s_s2[KB_LMAX * 8], s_a[KB_LMAX * 8], s_sc[KB_LMAX * 8];
   __shared__ float s_r2[MG ? KB_GMAX * KB_GMAX : 1];
+  __shared__ __align__(16) float s_il2[ARD ? KB_LMAX * 8 * KB_DMAX : 1];
   // kb_stage's loop with s_sc and out_scale: written out, since a per-factor hook inside kb_stage reschedules the multi-group kernel
   const int tid = threadIdx.x;
+  if (ARD) kb_stage_il2(a, tid, 0, a.L, s_il2);
   for (int l = tid; l < a.L; l += KB_THREADS) {
-    const float ls = a.ls[l], sg = a.sigma[l];
+    const float ls = ARD ? 1.f : a.ls[l], sg = a.sigma[l];
     s_c[l] = kb_coeff<float, KIND>(ls);
     s_s2[l] = sg * sg;
     s_sc[l] = gpz_pow2_scale(sg * sg + fabsf(a.jitter));
@@ -251,11 +301,13 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
   kb_load_cols<float, MG>(a, j0, KB_VEC8, xj, gj);
   const int i0 = blockIdx.y * KB_ROWS, i1 = min(i0 + KB_ROWS, a.n1);
   for (int i = i0; i < i1; ++i) {
-    float d2[KB_VEC8], r2[KB_VEC8];
-    kb_row_d2(a, i, xj, d2);
+    float d2[KB_VEC8], r2[KB_VEC8], sq[ARD ? KB_DMAX : 1][KB_VEC8];
+    if constexpr (ARD) kb_row_sq(a, i, xj, sq);
+    else kb_row_d2(a, i, xj, d2);
     kb_row_r2<float, MG>(a, i, s_r2, gj, r2);
     for (int l = 0; l < a.L; ++l) {
       const float c = s_c[l], s2 = s_s2[l], sc = s_sc[l];
+      if constexpr (ARD) kb_scaled_d2(s_il2 + l * KB_DMAX, sq, d2);
       float k[KB_VEC8];
 #pragma unroll
       for (int v = 0; v < KB_VEC8; ++v) {
@@ -291,7 +343,9 @@ __global__ void __launch_bounds__(KB_THREADS) kbuild_fwd_h_kernel(const KBArgs<f
 // One CTA covers KB_ROWS rows x (KB_THREADS*4) columns; the L accumulators live in registers.
 // The position gradients stay products of u with the direct differences: |u (x1 - x2)| <= K0 / ls for Matern-1/2, so
 // near-coincident points are harmless (an x1 sum(u) - sum(u x2) form would cancel catastrophically).
-template <typename T, bool MG, bool ALIGNED, int LMAX, int KIND = 0>
+// ARD: u at unit lengthscale on s2; g_ls (L x D) += sum G u (x1_d - x2_d)^2 (later divided by ls_d^3), and the position
+// weights are per dimension, w_d = sum_l G u / ls[l,d]^2.
+template <typename T, bool MG, bool ALIGNED, int LMAX, int KIND = 0, bool ARD = false>
 __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2 : 1) kbuild_bwd_kernel(const KBArgs<T> a, const T* __restrict__ G, int l0, int Lc,
                                                                  double* __restrict__ g_x1, T* __restrict__ g_x2,
                                                                  double* __restrict__ g_sigma, double* __restrict__ g_ls,
@@ -300,8 +354,9 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
   __shared__ T s_r2[MG ? KB_GMAX * KB_GMAX : 1];
   __shared__ double s_red[32];
   __shared__ T s_row[KB_ROWS][KB_DMAX][KB_THREADS / 32];
+  __shared__ __align__(16) T s_il2[ARD ? LMAX * KB_DMAX : 1];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  kb_stage<T, MG, KIND>(a, tid, l0, Lc, s_c, s_s2, s_a, s_r2);
+  kb_stage<T, MG, KIND, ARD>(a, tid, l0, Lc, s_c, s_s2, s_a, s_r2, s_il2);
   __syncthreads();
 
   const int64_t j0 = ((int64_t)blockIdx.x * KB_THREADS + tid) * KB_VEC;
@@ -312,6 +367,13 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
   T acc_s[LMAX], acc_l[LMAX], acc_a[MG ? LMAX : 1];
 #pragma unroll
   for (int l = 0; l < LMAX; ++l) { acc_s[l] = T(0); acc_l[l] = T(0); if (MG) acc_a[l] = T(0); }
+  T acc_d[ARD ? LMAX : 1][KB_DMAX];                    // ARD: sum G u (x1_d - x2_d)^2 per factor and dimension
+  if constexpr (ARD) {
+#pragma unroll
+    for (int l = 0; l < LMAX; ++l)
+#pragma unroll
+      for (int d = 0; d < KB_DMAX; ++d) acc_d[l][d] = T(0);
+  }
   T gx2[KB_DMAX][KB_VEC];
 #pragma unroll
   for (int d = 0; d < KB_DMAX; ++d)
@@ -321,8 +383,15 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
   const int i0 = blockIdx.y * KB_ROWS, i1 = min(i0 + KB_ROWS, a.n1);
   for (int i = i0; i < i1; ++i) {
     T df[KB_DMAX][KB_VEC], d2[KB_VEC], r2[KB_VEC], w[KB_VEC];   // w = sum_l G u
+    T wd[KB_DMAX][KB_VEC];                                       // ARD: w_d = sum_l G u / ls[l,d]^2
 #pragma unroll
     for (int v = 0; v < KB_VEC; ++v) { d2[v] = T(0); w[v] = T(0); r2[v] = T(0); }
+    if constexpr (ARD) {
+#pragma unroll
+      for (int d = 0; d < KB_DMAX; ++d)
+#pragma unroll
+        for (int v = 0; v < KB_VEC; ++v) wd[d][v] = T(0);
+    }
 #pragma unroll
     for (int d = 0; d < KB_DMAX; ++d) {
       const T xi = d < a.D ? a.x1[(int64_t)i * a.D + d] : T(0);
@@ -353,7 +422,26 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
       // phase 2: recompute K and accumulate
 #pragma unroll
       for (int l = 0; l < LMAX; ++l) {
-        if (l < Lc) {
+        if constexpr (ARD) {
+          if (l >= Lc) continue;
+          // the squared differences are formed again per factor: kept per row, their registers made the fp32 kernels spill
+          T il2[KB_DMAX];
+#pragma unroll
+          for (int d = 0; d < KB_DMAX; ++d) il2[d] = s_il2[l * KB_DMAX + d];
+#pragma unroll
+          for (int v = 0; v < KB_VEC; ++v) {
+            T s2d = df[0][v] * il2[0] * df[0][v];
+#pragma unroll
+            for (int d = 1; d < KB_DMAX; ++d) s2d = fma(df[d][v] * il2[d], df[d][v], s2d);
+            const KBTerms<T> t = kb_terms<T, false, KIND>(s_c[l], s_s2[l], T(0), T(0), s2d, a.p_half, g[l][v]);
+            acc_s[l] = fma(g[l][v], t.k0, acc_s[l]);
+#pragma unroll
+            for (int d = 0; d < KB_DMAX; ++d) {
+              acc_d[l][d] = fma(t.u * df[d][v], df[d][v], acc_d[l][d]);
+              wd[d][v] = fma(t.u, il2[d], wd[d][v]);
+            }
+          }
+        } else if (l < Lc) {
           const T c = s_c[l], s2 = s_s2[l];
 #pragma unroll
           for (int v = 0; v < KB_VEC; ++v) {
@@ -373,7 +461,10 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
       if (d < a.D) {
         T r = T(0);
 #pragma unroll
-        for (int v = 0; v < KB_VEC; ++v) { r = fma(w[v], df[d][v], r); gx2[d][v] = fma(w[v], df[d][v], gx2[d][v]); }
+        for (int v = 0; v < KB_VEC; ++v) {
+          const T wv = ARD ? wd[d][v] : w[v];
+          r = fma(wv, df[d][v], r); gx2[d][v] = fma(wv, df[d][v], gx2[d][v]);
+        }
         r = warp_sum(r);
         if (lane == 0) s_row[i - i0][d][warp] = r;
       }
@@ -400,14 +491,35 @@ __global__ void __launch_bounds__(KB_THREADS, (sizeof(T) == 4 && LMAX <= 12) ? 2
     if (l < Lc) {                                   // uniform across the block
       double v = block_sum<double>((double)acc_s[l], s_red);
       if (tid == 0) atomicAdd(g_sigma + l0 + l, v);
-      v = block_sum<double>((double)acc_l[l], s_red);
-      if (tid == 0) atomicAdd(g_ls + l0 + l, v);
-      if (MG) {
-        v = block_sum<double>((double)acc_a[l], s_red);
-        if (tid == 0) atomicAdd(g_a + l0 + l, v);
+      if constexpr (ARD) {
+#pragma unroll
+        for (int d = 0; d < KB_DMAX; ++d) {
+          if (d < a.D) {
+            v = block_sum<double>((double)acc_d[l][d], s_red);
+            if (tid == 0) atomicAdd(g_ls + (int64_t)(l0 + l) * a.D + d, v);
+          }
+        }
+      } else {
+        v = block_sum<double>((double)acc_l[l], s_red);
+        if (tid == 0) atomicAdd(g_ls + l0 + l, v);
+        if (MG) {
+          v = block_sum<double>((double)acc_a[l], s_red);
+          if (tid == 0) atomicAdd(g_a + l0 + l, v);
+        }
       }
     }
   }
+}
+
+// ARD: g_sigma = 2 S/sigma, g_ls[l,d] = Sl[l,d]/ls[l,d]^3 (LD = L * D entries), g_x1 = ws_x1
+template <typename T>
+__global__ void kbuild_bwd_ard_finalize_kernel(const double* __restrict__ ws, const T* __restrict__ sigma, const T* __restrict__ ls,
+                                               int L, int LD, int n1D, T* __restrict__ g_sigma, T* __restrict__ g_ls,
+                                               T* __restrict__ g_x1) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < L) g_sigma[e] = (T)(2.0 * ws[e] / (double)sigma[e]);
+  if (e < LD) { const double l = (double)ls[e]; g_ls[e] = (T)(ws[L + e] / (l * l * l)); }
+  if (g_x1 != nullptr && e < n1D) g_x1[e] = (T)ws[L + LD + e];
 }
 
 // double accumulators -> outputs:  g_sigma = 2 S/sigma, g_ls = Sl/ls, g_a = Sa, g_x1 = ws_x1
@@ -439,15 +551,17 @@ __global__ void cdist_kernel(const T* __restrict__ x1, const T* __restrict__ x2,
 // ---- Host dispatch: runtime values -> the compile-time parameters of the kernels.  Every instantiated kernel is reached here.
 template <int V> using kb_int = std::integral_constant<int, V>;
 
-// (kind, groups) -> f(std::bool_constant<MG>, kb_int<KIND>) for the five supported forms: the RBF with and without groups and
-// the three Matern kinds (which have no multi-group form in the reference); GPZ_ERR_UNSUPPORTED for anything else
-template <typename F> int kb_dispatch_kind(int kind, bool mg, F&& f) {
-  if (mg) return kind == 0 ? f(std::true_type{}, kb_int<0>{}) : GPZ_ERR_UNSUPPORTED;
+// (kind, groups, ARD) -> f(std::bool_constant<MG>, kb_int<KIND>, std::bool_constant<ARD>) for the nine supported forms: the
+// RBF with and without groups, the three Matern kinds (which have no multi-group form in the reference), and the four kinds
+// with per-dimension lengthscales (no groups); GPZ_ERR_UNSUPPORTED for anything else
+template <typename F> int kb_dispatch_kind(int kind, bool mg, bool ard, F&& f) {
+  if (mg) return kind == 0 && !ard ? f(std::true_type{}, kb_int<0>{}, std::false_type{}) : GPZ_ERR_UNSUPPORTED;
+  const auto with_ard = [&](auto kd) { return ard ? f(std::false_type{}, kd, std::true_type{}) : f(std::false_type{}, kd, std::false_type{}); };
   switch (kind) {
-    case 0: return f(std::false_type{}, kb_int<0>{});
-    case 1: return f(std::false_type{}, kb_int<1>{});
-    case 2: return f(std::false_type{}, kb_int<2>{});
-    case 3: return f(std::false_type{}, kb_int<3>{});
+    case 0: return with_ard(kb_int<0>{});
+    case 1: return with_ard(kb_int<1>{});
+    case 2: return with_ard(kb_int<2>{});
+    case 3: return with_ard(kb_int<3>{});
     default: return GPZ_ERR_UNSUPPORTED;
   }
 }
@@ -455,9 +569,12 @@ template <typename F> int kb_dispatch_kind(int kind, bool mg, F&& f) {
 template <typename F> int kb_dispatch_aligned(bool al, F&& f) { return al ? f(std::true_type{}) : f(std::false_type{}); }
 
 // factors per backward launch: the RBF's register accumulators are sized to L (4 / 8 / 12 / 16, else KB_LMAX);
-// the Matern kinds always take KB_LMAX
-template <int KIND, typename F> int kb_dispatch_lmax(int L, F&& f) {
-  if constexpr (KIND != 0) return f(kb_int<KB_LMAX>{});
+// the Matern kinds always take KB_LMAX.  ARD keeps 1 + KB_DMAX accumulators per factor: with 3 factors the fp32 kernels (two
+// CTAs per SM, <= 128 registers) use 120-127 registers and do not spill; with 4 the Matern-3/2 and -5/2 ones spilled 8 B
+constexpr int KB_LMAX_ARD = 3;
+template <int KIND, bool ARD, typename F> int kb_dispatch_lmax(int L, F&& f) {
+  if constexpr (ARD) return f(kb_int<KB_LMAX_ARD>{});
+  else if constexpr (KIND != 0) return f(kb_int<KB_LMAX>{});
   else if (L <= 4) return f(kb_int<4>{});
   else if (L <= 8) return f(kb_int<8>{});
   else if (L <= 12) return f(kb_int<12>{});
@@ -470,16 +587,17 @@ template <typename T> bool kb_sizes_ok(const KBArgs<T>& a, int l_max) {
   return a.D >= 1 && a.D <= KB_DMAX && a.L >= 1 && a.L <= l_max && (a.g1 == nullptr || (a.ng >= 1 && a.ng <= KB_GMAX));
 }
 
+// ard: a.ls holds L x D per-dimension lengthscales (no groups)
 template <typename T>
-int kbuild_fwd(const KBArgs<T>& a, T* out, T* out_lo, cudaStream_t st) {
+int kbuild_fwd(const KBArgs<T>& a, T* out, T* out_lo, cudaStream_t st, bool ard = false) {
   if (!kb_sizes_ok(a, KB_LMAX * 8)) return GPZ_ERR_UNSUPPORTED;
   if (a.n1 == 0 || a.n2 == 0) return GPZ_OK;
   const bool al = (a.n2 % KB_VEC == 0) && ((reinterpret_cast<uintptr_t>(out) & 31) == 0) &&
                   ((reinterpret_cast<uintptr_t>(out_lo) & 15) == 0);
   const dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
-  return kb_dispatch_kind(a.kind, a.g1 != nullptr, [&](auto mg, auto kind) {
+  return kb_dispatch_kind(a.kind, a.g1 != nullptr, ard, [&](auto mg, auto kind, auto ardc) {
     return kb_dispatch_aligned(al, [&](auto aligned) {
-      kbuild_fwd_kernel<T, decltype(mg)::value, decltype(aligned)::value, decltype(kind)::value>
+      kbuild_fwd_kernel<T, decltype(mg)::value, decltype(aligned)::value, decltype(kind)::value, decltype(ardc)::value>
           <<<grid, KB_THREADS, 0, st>>>(a, out, out_lo);
       GPZ_CHECK_LAUNCH();
       return GPZ_OK;
@@ -487,23 +605,40 @@ int kbuild_fwd(const KBArgs<T>& a, T* out, T* out_lo, cudaStream_t st) {
   });
 }
 
+// fp16-plane forward (fp32 arithmetic): see kbuild_fwd_h_kernel
+int kbuild_fwd_h(const KBArgs<float>& a, void* out_h, void* out_l, float* out_scale, cudaStream_t st, bool ard = false) {
+  if (!kb_sizes_ok(a, KB_LMAX * 8)) return GPZ_ERR_UNSUPPORTED;
+  if (a.n2 % KB_VEC8 || (reinterpret_cast<uintptr_t>(out_h) & 15) || (reinterpret_cast<uintptr_t>(out_l) & 15)) return GPZ_ERR_UNSUPPORTED;
+  if (a.n1 == 0 || a.n2 == 0) return GPZ_OK;
+  const dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC8), (unsigned)cdiv(a.n1, KB_ROWS));
+  return kb_dispatch_kind(a.kind, a.g1 != nullptr, ard, [&](auto mg, auto kd, auto ardc) {
+    kbuild_fwd_h_kernel<decltype(mg)::value, decltype(kd)::value, decltype(ardc)::value>
+        <<<grid, KB_THREADS, 0, st>>>(a, (__half*)out_h, (__half*)out_l, out_scale);
+    GPZ_CHECK_LAUNCH();
+    return GPZ_OK;
+  });
+}
+
+// ws: 3 L + n1 D doubles (sigma, ls, a, x1 sums); with ard L + L D + n1 D (sigma, the L x D ls sums, x1)
 template <typename T>
-int kbuild_bwd(const KBArgs<T>& a, const T* G, T* g_x1, T* g_x2, T* g_sigma, T* g_ls, T* g_a, double* ws, cudaStream_t st) {
+int kbuild_bwd(const KBArgs<T>& a, const T* G, T* g_x1, T* g_x2, T* g_sigma, T* g_ls, T* g_a, double* ws, cudaStream_t st,
+               bool ard = false) {
   if (!kb_sizes_ok(a, INT_MAX)) return GPZ_ERR_UNSUPPORTED;
-  const int n1D = a.n1 * a.D;
-  GPZ_CUDA(cudaMemsetAsync(ws, 0, sizeof(double) * (3 * (size_t)a.L + n1D), st));
+  const int n1D = a.n1 * a.D, nls = ard ? a.L * a.D : a.L;
+  GPZ_CUDA(cudaMemsetAsync(ws, 0, sizeof(double) * ((ard ? 1 : 2) * (size_t)a.L + nls + n1D), st));
   if (g_x2) GPZ_CUDA(cudaMemsetAsync(g_x2, 0, sizeof(T) * a.n2 * a.D, st));
-  double* w_sigma = ws; double* w_ls = ws + a.L; double* w_a = ws + 2 * a.L; double* w_x1 = ws + 3 * a.L;
+  double* w_sigma = ws; double* w_ls = ws + a.L; double* w_a = ws + 2 * a.L;
+  double* w_x1 = ard ? ws + a.L + nls : ws + 3 * a.L;
   if (a.n1 > 0 && a.n2 > 0) {
     const bool al = (a.n2 % KB_VEC == 0) && ((reinterpret_cast<uintptr_t>(G) & 31) == 0);
     const dim3 grid((unsigned)cdiv(a.n2, (int64_t)KB_THREADS * KB_VEC), (unsigned)cdiv(a.n1, KB_ROWS));
-    const int rc = kb_dispatch_kind(a.kind, a.g1 != nullptr, [&](auto mg, auto kind) {
-      return kb_dispatch_lmax<decltype(kind)::value>(a.L, [&](auto lmax) {
+    const int rc = kb_dispatch_kind(a.kind, a.g1 != nullptr, ard, [&](auto mg, auto kind, auto ardc) {
+      return kb_dispatch_lmax<decltype(kind)::value, decltype(ardc)::value>(a.L, [&](auto lmax) {
         return kb_dispatch_aligned(al, [&](auto aligned) {
           constexpr int LMAX = decltype(lmax)::value;
           // g_x1/g_x2 accumulate over all l-chunks (atomics), so every chunk launch adds its share
           for (int l0 = 0; l0 < a.L; l0 += LMAX) {
-            kbuild_bwd_kernel<T, decltype(mg)::value, decltype(aligned)::value, LMAX, decltype(kind)::value>
+            kbuild_bwd_kernel<T, decltype(mg)::value, decltype(aligned)::value, LMAX, decltype(kind)::value, decltype(ardc)::value>
                 <<<grid, KB_THREADS, 0, st>>>(a, G, l0, min(LMAX, a.L - l0), w_x1, g_x2, w_sigma, w_ls, w_a);
             GPZ_CHECK_LAUNCH();
           }
@@ -513,8 +648,9 @@ int kbuild_bwd(const KBArgs<T>& a, const T* G, T* g_x1, T* g_x2, T* g_sigma, T* 
     });
     if (rc != GPZ_OK) return rc;
   }
-  const int tot = max(a.L, n1D);
-  kbuild_bwd_finalize_kernel<T><<<(unsigned)cdiv(tot, 256), 256, 0, st>>>(ws, a.sigma, a.ls, a.L, n1D, g_sigma, g_ls, g_a, g_x1);
+  const int tot = max(nls, n1D);
+  if (ard) kbuild_bwd_ard_finalize_kernel<T><<<(unsigned)cdiv(tot, 256), 256, 0, st>>>(ws, a.sigma, a.ls, a.L, nls, n1D, g_sigma, g_ls, g_x1);
+  else kbuild_bwd_finalize_kernel<T><<<(unsigned)cdiv(tot, 256), 256, 0, st>>>(ws, a.sigma, a.ls, a.L, n1D, g_sigma, g_ls, g_a, g_x1);
   GPZ_CHECK_LAUNCH();
   return GPZ_OK;
 }
@@ -538,6 +674,18 @@ using namespace gpz;
     KBArgs<T> k{x1, x2, sigma, ls, a, r2, g1, g2, n1, n2, D, L, ng, p_half, T(0), kind};                           \
     return kbuild_bwd<T>(k, G, g_x1, g_x2, g_sigma, g_ls, g_a, ws, (cudaStream_t)stream);                          \
   }                                                                                                                \
+  extern "C" int gpz_kernel_build_ard_fwd_##SUF(const T* x1, const T* x2, const T* sigma, const T* ls, int n1,     \
+                                                int n2, int D, int L, int kind, T jitter, T* out, T* out_lo,       \
+                                                void* stream) {                                                    \
+    KBArgs<T> k{x1, x2, sigma, ls, nullptr, nullptr, nullptr, nullptr, n1, n2, D, L, 0, T(1), jitter, kind};       \
+    return kbuild_fwd<T>(k, out, out_lo, (cudaStream_t)stream, true);                                              \
+  }                                                                                                                \
+  extern "C" int gpz_kernel_build_ard_bwd_##SUF(const T* x1, const T* x2, const T* sigma, const T* ls, int n1,     \
+                                                int n2, int D, int L, int kind, const T* G, T* g_x1, T* g_x2,      \
+                                                T* g_sigma, T* g_ls, double* ws, void* stream) {                   \
+    KBArgs<T> k{x1, x2, sigma, ls, nullptr, nullptr, nullptr, nullptr, n1, n2, D, L, 0, T(1), T(0), kind};         \
+    return kbuild_bwd<T>(k, G, g_x1, g_x2, g_sigma, g_ls, nullptr, ws, (cudaStream_t)stream, true);                \
+  }                                                                                                                \
   extern "C" int gpz_cdist_##SUF(const T* x1, const T* x2, T* out, int n1, int n2, int D, void* stream) {          \
     const int64_t total = (int64_t)n1 * n2;                                                                        \
     if (total == 0) return GPZ_OK;                                                                                 \
@@ -549,20 +697,17 @@ using namespace gpz;
 GPZ_KB_IMPL(f32, float)
 GPZ_KB_IMPL(f64, double)
 
-// fp16-plane forward (fp32 arithmetic): see kbuild_fwd_h_kernel
 extern "C" int gpz_kernel_build_fwd_h_f32(const float* x1, const float* x2, const float* sigma, const float* ls, const float* a,
                                           const float* r2, const int64_t* g1, const int64_t* g2, int n1, int n2, int D, int L,
                                           int ng, int kind, float p_half, float jitter, void* out_h, void* out_l,
                                           float* out_scale, void* stream) {
   const KBArgs<float> k{x1, x2, sigma, ls, a, r2, g1, g2, n1, n2, D, L, ng, p_half, jitter, kind};
-  if (!kb_sizes_ok(k, KB_LMAX * 8)) return GPZ_ERR_UNSUPPORTED;
-  if (n2 % KB_VEC8 || (reinterpret_cast<uintptr_t>(out_h) & 15) || (reinterpret_cast<uintptr_t>(out_l) & 15)) return GPZ_ERR_UNSUPPORTED;
-  if (n1 == 0 || n2 == 0) return GPZ_OK;
-  const dim3 grid((unsigned)cdiv(n2, (int64_t)KB_THREADS * KB_VEC8), (unsigned)cdiv(n1, KB_ROWS));
-  return kb_dispatch_kind(kind, g1 != nullptr, [&](auto mg, auto kd) {
-    kbuild_fwd_h_kernel<decltype(mg)::value, decltype(kd)::value>
-        <<<grid, KB_THREADS, 0, (cudaStream_t)stream>>>(k, (__half*)out_h, (__half*)out_l, out_scale);
-    GPZ_CHECK_LAUNCH();
-    return GPZ_OK;
-  });
+  return kbuild_fwd_h(k, out_h, out_l, out_scale, (cudaStream_t)stream);
+}
+
+extern "C" int gpz_kernel_build_ard_fwd_h_f32(const float* x1, const float* x2, const float* sigma, const float* ls, int n1,
+                                              int n2, int D, int L, int kind, float jitter, void* out_h, void* out_l,
+                                              float* out_scale, void* stream) {
+  const KBArgs<float> k{x1, x2, sigma, ls, nullptr, nullptr, nullptr, nullptr, n1, n2, D, L, 0, 1.f, jitter, kind};
+  return kbuild_fwd_h(k, out_h, out_l, out_scale, (cudaStream_t)stream, true);
 }

@@ -300,6 +300,12 @@ def _check_kernel_args(x1, x2, sigma, ls, a, r2, g1, g2):
     for name, t in (("x2", x2), ("sigma", sigma), ("lengthscale", ls), ("group coefficient", a), ("group r^2 table", r2)):
         if t is not None and (t.dtype != x1.dtype or t.device != x1.device):
             raise _cabi.GpzError(f"kernel build: {name} is {t.dtype} on {t.device}, expected {x1.dtype} on {x1.device}")
+    if ls.dim() == 2:           # per-dimension (ARD) lengthscales: L x D, no groups
+        if tuple(ls.shape) != (sigma.numel(), x1.shape[1]):
+            raise _cabi.GpzError(f"kernel build: ARD lengthscale is {tuple(ls.shape)}, expected (L, D) = "
+                                 f"{(sigma.numel(), x1.shape[1])}")
+        if g1 is not None:
+            raise _cabi.GpzError("kernel build: per-dimension (ARD) lengthscales have no multi-group form")
     if g1 is not None:
         g1 = g1.to(device=x1.device, dtype=torch.int64)
         g2 = g2.to(device=x1.device, dtype=torch.int64)
@@ -315,8 +321,10 @@ def _check_kernel_args(x1, x2, sigma, ls, a, r2, g1, g2):
 
 def _kernel_args(x1, x2, sigma, ls, a, r2, g1, g2, check=True):
     """The leading arguments of every gpz_kernel_build_* call: ((x1, x2, sigma, ls, a, r2, g1, g2), (n1, n2, D, L, ng)), with
-    a = r2 = g1 = g2 = None and ng = 0 when there are no groups (g1 None).  `check` makes the tensors contiguous and runs
-    `_check_kernel_args`; the backward passes check=False, its tensors being the ones its forward returned from here."""
+    a = r2 = g1 = g2 = None and ng = 0 when there are no groups (g1 None).  A 2-D ls (L x D) selects the per-dimension (ARD)
+    calls gpz_kernel_build_ard_*, which take (x1, x2, sigma, ls) and the sizes without ng.  `check` makes the tensors
+    contiguous and runs `_check_kernel_args`; the backward passes check=False, its tensors being the ones its forward returned
+    from here."""
     if check:
         x1, x2, sigma, ls = _c(x1), _c(x2), _c(sigma), _c(ls)
         a, r2, g1, g2 = _check_kernel_args(x1, x2, sigma, ls, a, r2, g1, g2)
@@ -329,7 +337,8 @@ def _kernel_args(x1, x2, sigma, ls, a, r2, g1, g2, check=True):
 
 
 class KernelBuild(Function):
-    """K[l,i,j] = sigma_l^2 exp(-0.5 |x1_i-x2_j|^2/(ls_l^2 den)) / den^p_half (+ jitter on i==j).
+    """K[l,i,j] = sigma_l^2 exp(-0.5 |x1_i-x2_j|^2/(ls_l^2 den)) / den^p_half (+ jitter on i==j); the other kinds and, for an
+    L x D ls, per-dimension lengthscales as in include/gpzoo_b200.h.
 
     Replaces kernels.py:114-130 / 141-155 / 172-191 / 204-228 (+ utilities.py:407-418 add_jitter)."""
 
@@ -340,7 +349,10 @@ class KernelBuild(Function):
         out = torch.empty((L, n1, n2), dtype=dt, device=x1.device)
         want_lo = bool(want_lo) and dt == torch.float32
         out_lo = torch.empty_like(out) if want_lo else None
-        call("kernel_build_fwd", dt, *t, n1, n2, D, L, ng, int(kind), p_half, jitter, out, out_lo)
+        if ls.dim() == 2:
+            call("kernel_build_ard_fwd", dt, *t[:4], n1, n2, D, L, int(kind), jitter, out, out_lo)
+        else:
+            call("kernel_build_fwd", dt, *t, n1, n2, D, L, ng, int(kind), p_half, jitter, out, out_lo)
         ctx.save_for_backward(*t)
         ctx.p_half = p_half
         ctx.kind = int(kind)
@@ -371,6 +383,10 @@ def _kernel_build_bwd(x1, x2, sigma, ls, a, r2, g1, g2, p_half, kind, need, G):
     g_sigma = torch.empty_like(sigma)
     g_ls = torch.empty_like(ls)
     g_a = torch.empty_like(a) if g1 is not None else None
+    if ls.dim() == 2:
+        ws = torch.empty(L + L * D + n1 * D, dtype=torch.float64, device=x1.device)
+        call("kernel_build_ard_bwd", dt, x1, x2, sigma, ls, n1, n2, D, L, int(kind), G, g_x1, g_x2, g_sigma, g_ls, ws)
+        return g_x1, g_x2, g_sigma, g_ls, None
     ws = torch.empty(3 * L + n1 * D, dtype=torch.float64, device=x1.device)
     call("kernel_build_bwd", dt, *t, n1, n2, D, L, ng, int(kind), p_half, G, g_x1, g_x2, g_sigma, g_ls, g_a, ws)
     return g_x1, g_x2, g_sigma, g_ls, g_a
@@ -400,7 +416,10 @@ class KernelBuildH(Function):
         t, (n1, n2, D, L, ng) = _kernel_args(x1, x2, sigma, ls, a, r2, g1, g2)
         Kh, Kl = _plane_pair(L, n1, n2, x1.device)
         sK = torch.empty(L, dtype=dt, device=x1.device)
-        call("kernel_build_fwd_h", dt, *t, n1, n2, D, L, ng, int(kind), p_half, jitter, Kh, Kl, sK)
+        if ls.dim() == 2:
+            call("kernel_build_ard_fwd_h", dt, *t[:4], n1, n2, D, L, int(kind), jitter, Kh, Kl, sK)
+        else:
+            call("kernel_build_fwd_h", dt, *t, n1, n2, D, L, ng, int(kind), p_half, jitter, Kh, Kl, sK)
         ctx.save_for_backward(*t)
         ctx.p_half = p_half
         ctx.kind = int(kind)

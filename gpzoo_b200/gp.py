@@ -374,6 +374,9 @@ class VNNGP(_SparseGPBase):
 
     def moments(self, X, groupsX=None):
         dt = X.dtype
+        if getattr(self.kernel, "_ard", False):
+            raise NotImplementedError("VNNGP's fused neighbour kernel takes one lengthscale per factor; "
+                                      f"{type(self.kernel).__name__} (per-dimension lengthscales) is not supported")
         if getattr(self.kernel, "_kind", 0) != 0:
             raise NotImplementedError("VNNGP's fused neighbour kernel evaluates the RBF cross-covariance; "
                                       f"{type(self.kernel).__name__} is not supported")

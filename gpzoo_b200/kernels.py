@@ -204,6 +204,84 @@ class batched_Matern52(batched_RBF):
         return (self.sigma ** 2) * (1 + v + v * v / 3) * torch.exp(-v)
 
 
+class _ARDBase(_RBFBase):
+    """Per-dimension (ARD) lengthscales: the covariance of `_kind` at unit lengthscale on the scaled squared distance
+    s2 = sum_d (x_d - z_d)^2 / lengthscale[l, d]^2 (gpz_kernel_build_ard_*).  `sigma` is a scalar or (L,); `lengthscale` is
+    (D,) or (L, D), its last axis always the input dimension (a scalar is broadcast to (dim,)).  Equal lengthscales along D
+    give the isotropic kernel of the same kind.  There is no multi-group form, and VNNGP refuses these kernels."""
+    _ard = True
+
+    def __init__(self, sigma=1.0, lengthscale=2.0, dim=2):
+        super().__init__()
+        dt = torch.get_default_dtype()
+        sigma = torch.as_tensor(sigma, dtype=dt)
+        ls = torch.as_tensor(lengthscale, dtype=dt)
+        if ls.dim() == 0:
+            ls = ls.expand(dim).clone()
+        if sigma.dim() > 1 or ls.dim() > 2:
+            raise ValueError(f"{type(self).__name__}: sigma must be a scalar or (L,) and lengthscale (D,) or (L, D); got "
+                             f"{tuple(sigma.shape)} and {tuple(ls.shape)}")
+        self.sigma = nn.Parameter(sigma)
+        self.lengthscale = nn.Parameter(ls)
+        self._params()
+
+    @property
+    def input_dim(self):
+        return self.lengthscale.shape[-1]
+
+    @property
+    def _batched(self):
+        return self.sigma.dim() > 0 or self.lengthscale.dim() == 2
+
+    def _params(self):
+        """(sigma (L,), lengthscale (L, D))."""
+        s, l = _flat(self.sigma), self.lengthscale
+        Ls = s.numel() if self.sigma.dim() > 0 else None
+        Ll = l.shape[0] if l.dim() == 2 else None
+        if Ls is not None and Ll is not None and Ls != Ll:
+            raise ValueError(f"{type(self).__name__}: sigma has L = {Ls} factors, lengthscale has L = {Ll}")
+        L = Ls or Ll or 1
+        return s.expand(L), l.reshape(-1, l.shape[-1]).expand(L, -1)
+
+    def _diag(self, X):
+        s2 = self._params()[0] ** 2
+        return s2[:, None].expand(-1, X.size(0)) if self._batched else s2.reshape(()).expand(X.size(0))
+
+    def forward(self, X, Z, diag=False, _jitter=0.0, _want_lo=False, _want_h=False):
+        D = self.lengthscale.shape[-1]
+        for name, t in (("X", X), ("Z", Z)):
+            if t.dim() != 2 or t.shape[-1] != D:
+                raise ValueError(f"{type(self).__name__}: {name} is {tuple(t.shape)}, expected (n, {D}) for its lengthscale's D")
+        if diag:
+            return self._diag(X)
+        return self._build(X, Z, jitter=_jitter, want_lo=_want_lo, want_h=_want_h)
+
+    def forward_distance(self, distance_squared):
+        raise NotImplementedError(f"{type(self).__name__}: a summed squared distance has lost the per-dimension differences "
+                                  "that per-dimension lengthscales scale")
+
+
+class batched_ARD_RBF(_ARDBase):
+    """RBF sigma^2 exp(-s2 / 2) with per-dimension lengthscales (`kind = 0` of gpz_kernel_build_ard_*)."""
+    _kind = 0
+
+
+class batched_ARD_Matern12(_ARDBase):
+    """Matern-1/2 sigma^2 exp(-r), r = sqrt(s2), with per-dimension lengthscales (`kind = 2`); the backward takes the
+    sub-gradient 0 at r = 0."""
+    _kind = 2
+
+
+class batched_ARD_Matern32(_ARDBase):
+    """Matern-3/2 sigma^2 (1 + v) exp(-v), v = sqrt(3 s2), with per-dimension lengthscales (`kind = 1`)."""
+    _kind = 1
+
+
+class batched_ARD_Matern52(_ARDBase):
+    """Matern-5/2 sigma^2 (1 + v + v^2/3) exp(-v), v = sqrt(5 s2), with per-dimension lengthscales (`kind = 3`)."""
+    _kind = 3
+
+
 class batched_MGGP_RBF(_MultiGroup, batched_RBF):
     """kernels.py:62-104: a = |group_diff_param|, p = X.shape[-1]."""
     _input_dim_from_X = True

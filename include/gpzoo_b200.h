@@ -55,6 +55,26 @@ int gpz_kernel_build_bwd_f64(const double* x1, const double* x2, const double* s
                              const double* r2, const int64_t* g1, const int64_t* g2, int n1, int n2, int D, int L, int ng, int kind,
                              double p_half, const double* G, double* g_x1, double* g_x2, double* g_sigma, double* g_ls,
                              double* g_a, double* ws, void* stream);
+/* ---- K1 with per-dimension (ARD) lengthscales, every kind, no groups (csrc/kernel_build.cu):
+ *      ls is L x D (row-major); s2 = sum_d (x1_i,d - x2_j,d)^2 / ls[l,d]^2, r = sqrt(s2);
+ *      kind = 0: out[l,i,j] = sigma_l^2 exp(-s2/2); kind = 1: sigma_l^2 (1 + v) exp(-v), v = sqrt(3) r;
+ *      kind = 2: sigma_l^2 exp(-r) (the backward takes the sub-gradient 0 at r = 0); kind = 3: sigma_l^2 (1 + v + v^2/3) exp(-v),
+ *      v = sqrt(5) r; (+ jitter if i==j).  Equal ls[l,d] = ls_l give gpz_kernel_build_fwd of the same kind.
+ *      Kinds outside 0-3, D outside 1-4 and L outside the limits of the isotropic calls return GPZ_ERR_UNSUPPORTED.
+ *      out_lo and the fwd_h planes and out_scale (sigma_l^2 + |jitter| in (2^14, 2^15]) are as in the isotropic calls.
+ *      bwd: g_ls is L x D; g_x1/g_x2 may be NULL; ws: L + L*D + n1*D doubles of scratch. */
+int gpz_kernel_build_ard_fwd_f32(const float* x1, const float* x2, const float* sigma, const float* ls, int n1, int n2, int D,
+                                 int L, int kind, float jitter, float* out, float* out_lo, void* stream);
+int gpz_kernel_build_ard_fwd_f64(const double* x1, const double* x2, const double* sigma, const double* ls, int n1, int n2, int D,
+                                 int L, int kind, double jitter, double* out, double* out_lo, void* stream);
+int gpz_kernel_build_ard_fwd_h_f32(const float* x1, const float* x2, const float* sigma, const float* ls, int n1, int n2, int D,
+                                   int L, int kind, float jitter, void* out_h, void* out_l, float* out_scale, void* stream);
+int gpz_kernel_build_ard_bwd_f32(const float* x1, const float* x2, const float* sigma, const float* ls, int n1, int n2, int D,
+                                 int L, int kind, const float* G, float* g_x1, float* g_x2, float* g_sigma, float* g_ls,
+                                 double* ws, void* stream);
+int gpz_kernel_build_ard_bwd_f64(const double* x1, const double* x2, const double* sigma, const double* ls, int n1, int n2, int D,
+                                 int L, int kind, const double* G, double* g_x1, double* g_x2, double* g_sigma, double* g_ls,
+                                 double* ws, void* stream);
 /* kernels.py:118,123-124 (return_distance=True): Euclidean distances n1 x n2 */
 int gpz_cdist_f32(const float* x1, const float* x2, float* out, int n1, int n2, int D, void* stream);
 int gpz_cdist_f64(const double* x1, const double* x2, double* out, int n1, int n2, int D, void* stream);
