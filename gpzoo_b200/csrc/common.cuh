@@ -72,6 +72,22 @@ template <typename T> __device__ inline T sigmoid(T x) { return T(1) / (T(1) + N
 // d softplus / dx with the same threshold rule
 template <typename T> __device__ inline T softplus_grad(T x) { return x > T(20) ? T(1) : sigmoid(x); }
 
+// 16-byte vector loads of an FMAX-long shared-memory row (FMAX is a multiple of 4, rows are 16-byte aligned)
+template <int FMAX> __device__ __forceinline__ void load_row(const float* p, float (&o)[FMAX]) {
+#pragma unroll
+  for (int i = 0; i < FMAX / 4; ++i) {
+    const float4 v = reinterpret_cast<const float4*>(p)[i];
+    o[4 * i] = v.x; o[4 * i + 1] = v.y; o[4 * i + 2] = v.z; o[4 * i + 3] = v.w;
+  }
+}
+template <int FMAX> __device__ __forceinline__ void load_row(const double* p, double (&o)[FMAX]) {
+#pragma unroll
+  for (int i = 0; i < FMAX / 2; ++i) {
+    const double2 v = reinterpret_cast<const double2*>(p)[i];
+    o[2 * i] = v.x; o[2 * i + 1] = v.y;
+  }
+}
+
 template <typename T> __device__ inline T warp_sum(T v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

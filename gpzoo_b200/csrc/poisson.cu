@@ -47,22 +47,6 @@ template <typename T> struct NegBinArgs : PoissonArgs<T> {
 };
 template <typename T, bool NB> using K7Args = typename std::conditional<NB, NegBinArgs<T>, PoissonArgs<T>>::type;
 
-// 16-byte vector loads of an FMAX-long shared-memory row (FMAX is a multiple of 4, rows are 16-byte aligned)
-template <int FMAX> __device__ __forceinline__ void load_row(const float* p, float (&o)[FMAX]) {
-#pragma unroll
-  for (int i = 0; i < FMAX / 4; ++i) {
-    const float4 v = reinterpret_cast<const float4*>(p)[i];
-    o[4 * i] = v.x; o[4 * i + 1] = v.y; o[4 * i + 2] = v.z; o[4 * i + 3] = v.w;
-  }
-}
-template <int FMAX> __device__ __forceinline__ void load_row(const double* p, double (&o)[FMAX]) {
-#pragma unroll
-  for (int i = 0; i < FMAX / 2; ++i) {
-    const double2 v = reinterpret_cast<const double2*>(p)[i];
-    o[2 * i] = v.x; o[2 * i + 1] = v.y;
-  }
-}
-
 // ---- negative-binomial helpers ----------------------------------------------------------------------------------------------
 // log1p(q) for q >= 0.  fp32: the series to q^5 below 1/32 (truncation < 5e-9 relative; 1 + q would lose q's low bits),
 // __log2f(1 + q) above; fp64: the exact function.

@@ -1154,6 +1154,48 @@ def _k7_dense(y, idx, W, V, D, mean, spread, eps, n_var, clamp_min, w_softplus, 
     return gW, gV, gmean, gspread, ll, idx, gD
 
 
+class GaussianLL(Function):
+    """sum_{g,n} E_q[log N(y_gn | bias_g + sum_f W_gf F_fn, softplus(noise_g)^2)] under q(F) = N(mean, v), in closed form (no
+    samples), with the gradients w.r.t. W, bias, noise, mean and spread from the same pass over y (K7-G, csrc/gaussian.cu).
+    spread[f] is a variance (v = clamp(spread, clamp_min)) for f < n_var and a std-dev (v = spread^2) otherwise.
+    y: dense G x N of any float or integer dtype (converted on the device to the compute dtype); idx: optional minibatch
+    indices, y is read as y[:, idx]."""
+
+    @staticmethod
+    def forward(ctx, y, idx, W, bias, noise, mean, spread, n_var, clamp_min):
+        if isinstance(y, SparseCounts):
+            raise NotImplementedError(
+                "the Gaussian likelihood has no sparse kernel yet: y enters only linearly and through sum y^2, so a sparse path "
+                "is possible, but it is not built; pass y.to_dense()")
+        W, bias, noise, mean, spread = _c(W), _c(bias), _c(noise), _c(mean), _c(spread)
+        dt = W.dtype
+        G, F = W.shape
+        B = mean.shape[1]
+        y = _c(y if y.dtype == dt else y.to(dt))
+        assert y.shape[0] == G and mean.shape[0] == F and spread.shape == mean.shape
+        assert bias.shape == (G,) and noise.shape == (G,) and bias.dtype == dt and noise.dtype == dt
+        if idx is not None:
+            idx = _c(idx.to(device=W.device, dtype=torch.int64))
+        else:
+            assert y.shape[1] == B
+        suf = "f32" if dt == torch.float32 else "f64"
+        ws_bytes = int(getattr(_cabi.lib(), "gpz_gaussian_workspace_bytes_" + suf)(G, F, B))
+        ws = torch.empty(ws_bytes // 8 + 1, dtype=torch.float64, device=W.device)
+        ll = torch.empty(1, dtype=torch.float64, device=W.device)
+        gW, gbias, gnoise = torch.empty_like(W), torch.empty_like(bias), torch.empty_like(noise)
+        gmean, gspread = torch.empty_like(mean), torch.empty_like(spread)
+        call("gaussian_fwdbwd", dt, y, y.shape[1], idx, W, bias, noise, mean, spread, G, F, B, int(n_var), clamp_min, ll, gW, gbias,
+             gnoise, gmean, gspread, ws, ws_bytes)
+        ctx.save_for_backward(gW, gbias, gnoise, gmean, gspread)
+        return ll.to(dt).reshape(())
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        gW, gbias, gnoise, gmean, gspread = ctx.saved_tensors
+        return None, None, g * gW, g * gbias, g * gnoise, g * gmean, g * gspread, None, None
+
+
 _CSC_KINDS = {torch.uint8: 1, torch.int16: 2, torch.int32: 3}      # count_kind of gpz_poisson_fwdbwd_csc_* (0 = the compute type)
 
 

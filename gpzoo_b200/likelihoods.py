@@ -32,6 +32,13 @@ def _kl_of(m):
     return m["kl"] if m.get("kl") is not None else F.MvnKL.apply(m["T"], m["q"], m["Lc"], m["Lu"])
 
 
+def _gp_moments(gp, X, idx, kwargs):
+    """The fused ELBOs' GP moments at the minibatch X[idx], with the multi-group labels `groupsX` when given (their KL: `_kl_of`)."""
+    Xb = X if idx is None else X[idx]
+    gX = kwargs.get("groupsX")
+    return gp.moments(Xb, gX) if gX is not None else gp.moments(Xb)
+
+
 def _gp_call(gp, X, verbose, kwargs):
     # keywords, as the reference calls its priors (likelihoods.py:81, 111): MGGP_SVGP.forward(X, groupsX, verbose) and
     # MGGP_WSVGP.forward(X, verbose, **args) both take groupsX by name
@@ -127,9 +134,7 @@ class _FusedPoissonMixin(_PoissonCounts):
         eps: optional E x L x B standard-normal draw (else drawn from the global RNG on the device);
         kl_weight: data-parallel ranks pass 1/world_size so that the all-reduced sum counts the KL once."""
         gp = self._gp()
-        Xb = X if idx is None else X[idx]
-        gX = kwargs.get("groupsX")
-        m = gp.moments(Xb, gX) if gX is not None else gp.moments(Xb)
+        m = _gp_moments(gp, X, idx, kwargs)
         mean, var = m["mean"], m["var"]
         if eps is None:
             eps = torch.randn((E,) + tuple(mean.shape), dtype=mean.dtype, device=mean.device)
@@ -386,3 +391,85 @@ class Hybrid_NSF2_NB(_NegBinCounts, Hybrid_NSF2):
     def __init__(self, gp, prior, y, L=10, T=10):
         super().__init__(gp, prior, y, L=L, T=T)
         self._init_dispersion(y.shape[0])
+
+
+# ------------------------------------------------------------------------------------------------
+# Gaussian factor models: real-valued loadings, one noise and one intercept per gene
+# ------------------------------------------------------------------------------------------------
+class _GaussianFactors:
+    """y_g ~ N(bias_g + W_g F, s_g^2), s = softplus(noise) (G; initialised to log(e - 1): s = 1), W real (G x L, torch.randn), bias
+    zeros (G).  `elbo` runs the fused K7-G call (functional.GaussianLL), whose expectation over q(F) is exact: it draws no samples.
+    The loadings are real, so the training loops do not clamp them (`clamp_loadings`).  In data-parallel training W, bias and
+    noise are shared gradients: include model.W, model.bias, model.noise in distributed.FlatGradReducer's list."""
+
+    clamp_loadings = False
+
+    def _init_params(self, G, L):
+        self.W = nn.Parameter(torch.randn((G, L)))
+        self.bias = nn.Parameter(torch.zeros(G))            # not data-dependent: every data-parallel rank starts from the same value
+        self.noise = nn.Parameter(torch.full((G,), math.log(math.e - 1.0)))
+
+    def _ll(self, y, idx, mean, spread, n_var, clamp_min):
+        dt = mean.dtype
+        return F.GaussianLL.apply(y, idx, self.W.to(dt), self.bias.to(dt), self.noise.to(dt), mean, spread, n_var, clamp_min)
+
+    def _pY(self, Fs):
+        """Normal(bias + W F_e, s) over the E x G x B loc, materialised on the library's GEMM (compatibility path)."""
+        dt = Fs.dtype
+        loc = F.matmul(self.W.to(dt), Fs.contiguous()) + self.bias.to(dt)[:, None]
+        scale = torch.nn.functional.softplus(self.noise.to(dt))[:, None]
+        return distributions.Normal(loc, scale, validate_args=False)
+
+
+class RSF(_GaussianFactors, nn.Module):
+    """Real-valued spatial factorization: GP factors with real loadings and a Gaussian likelihood with one noise per gene.
+    Takes every prior NSF2 takes (SVGP, VNNGP, MGGP_SVGP with groupsX, WSVGP)."""
+
+    def __init__(self, gp, y, L=10):
+        super().__init__()
+        G, N = y.shape
+        self.prior = gp
+        self._init_params(G, L)
+
+    def elbo(self, X, y, idx=None, E=1, eps=None, kl_weight=1.0, return_parts=False, **kwargs):
+        """ELBO = sum_{g,n} E_q[log N(y | bias + W F, s^2)] - kl_weight sum_l KL(qU_l || pU_l), the expectation in closed form.
+
+        X: N x D (all spots); idx: optional minibatch indices; y: G x N real values (dense).  E and eps are accepted so that the
+        training loops can call it, and ignored: no samples are drawn.  kl_weight: data-parallel ranks pass 1/world_size."""
+        gp = self.prior
+        m = _gp_moments(gp, X, idx, kwargs)
+        mean, var = m["mean"], m["var"]
+        ll = self._ll(y, idx, mean, var, mean.shape[0], gp.clamp_min)
+        kl = _kl_of(m).to(mean.dtype)
+        out = ll - kl_weight * kl.sum()
+        if return_parts:
+            return out, dict(ll=ll, kl=kl, mean=mean, var=var)
+        return out
+
+    def forward(self, X, E=10, verbose=False, eps=None, **kwargs):
+        qF, qU, pU = _gp_call(self.prior, X, verbose, kwargs)
+        return self._pY(_sample(qF, E, eps)), qF, qU, pU
+
+    def forward_batched(self, X, idx, E=10, verbose=False, eps=None, **kwargs):
+        qF, qU, pU = _gp_call(self.prior, X[idx], verbose, kwargs)
+        return self._pY(_sample(qF, E, eps)), qF, qU, pU
+
+
+class FA(_GaussianFactors, nn.Module):
+    """Factor analysis: non-spatial factors (a GaussianPrior) with real loadings and one noise per gene."""
+
+    def __init__(self, prior, y, L=10):
+        super().__init__()
+        G, N = y.shape
+        self.prior = prior
+        self._init_params(G, L)
+
+    def elbo(self, y, idx=None, E=10, eps=None, **kwargs):
+        """sum_{g,n} E_q[log N(y | bias + W F, s^2)] - sum KL(qF || pF), the expectation in closed form (E and eps are ignored)."""
+        qF, pF = self.prior() if idx is None else self.prior.forward_batched(idx)
+        ll = self._ll(y, idx, qF.loc, qF.scale, 0, 0.0)
+        return ll - distributions.kl_divergence(qF, pF).sum()
+
+    def forward(self, E=10, eps=None, **kwargs):
+        qF, pF = self.prior()
+        return self._pY(_sample(qF, E, eps)), qF, pF

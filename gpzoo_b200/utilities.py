@@ -73,6 +73,14 @@ def _step(model, optimizer, elbo_fn, clamp_W):
     return loss.detach()
 
 
+def _clamped(model, names):
+    """The loadings the loops keep >= 0 after each step (utilities.py:523-524, 623): none for models with real-valued loadings
+    (`clamp_loadings = False`: RSF, FA)."""
+    if not getattr(model, "clamp_loadings", True):
+        return ()
+    return [w for w in (getattr(model, n, None) for n in names) if w is not None]
+
+
 def _finish(losses):
     F.check_cholesky_info()
     return [float(v) for v in torch.stack(losses).cpu()] if losses else []
@@ -92,27 +100,28 @@ def _sample_idx(N, batch_size, device):
 
 
 def train_batched(model, optimizer, X, y, device=None, steps=200, E=20, batch_size=1000, **kwargs):
-    """Minibatch loop (utilities.py:600-631), including the W >= 0 clamp after each update."""
+    """Minibatch loop (utilities.py:600-631), including the W >= 0 clamp after each update (not for real-valued loadings)."""
+    clamp = _clamped(model, ("W",))
     losses = []
     for _ in range(steps):
         idx = _sample_idx(X.shape[0], batch_size, X.device)
         kw = dict(kwargs)
         if "groupsX" in kw:
             kw["groupsX"] = kw["groupsX"][idx]
-        losses.append(_step(model, optimizer, lambda: model.elbo(X, y, idx=idx, E=E, **kw), (model.W,)))
+        losses.append(_step(model, optimizer, lambda: model.elbo(X, y, idx=idx, E=E, **kw), clamp))
     return _finish(losses)
 
 
 def train_hybrid(model, optimizer, X, y, device=None, steps=200, E=20, **kwargs):
     """utilities.py:531-563 (two KL terms; W, W2 clamped)."""
-    ws = [w for w in (getattr(model, "W", None), getattr(model, "W2", None)) if w is not None]
+    ws = _clamped(model, ("W", "W2"))
     losses = [_step(model, optimizer, lambda: model.elbo(X, y, E=E, **kwargs), ws) for _ in range(steps)]
     return _finish(losses)
 
 
 def train_hybrid_batched(model, optimizer, X, y, device=None, steps=200, E=20, batch_size=1000, **kwargs):
     """utilities.py:498-529; uses the y*log(rate)-rate form of the log-likelihood (utilities.py:507)."""
-    ws = [w for w in (getattr(model, "W", None), getattr(model, "W2", None)) if w is not None]
+    ws = _clamped(model, ("W", "W2"))
     losses = []
     for _ in range(steps):
         idx = _sample_idx(X.shape[0], batch_size, X.device)

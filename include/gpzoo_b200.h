@@ -252,6 +252,25 @@ int gpz_negbin_fwdbwd_yt_f32(const void* y, int y_kind, int64_t y_ld, const int6
                              const float* V, const float* D, const float* mean, const float* spread, const float* eps, int G, int F,
                              int B, int E, int n_var, float clamp_min, int with_lgamma, double* ll, float* gW, float* gV, float* gD,
                              float* gmean, float* gspread, void* ws, int64_t ws_bytes, void* stream);
+/* K7-G: the Gaussian factor model of RSF / FA (csrc/gaussian.cu), y_gn ~ N(bias_g + sum_f W_gf F_fn, s_g^2), s = softplus(noise),
+ *   real-valued y (G x Ntot, row stride y_ld), real loadings W (G x F), bias and raw noise (G).  The expectation over
+ *   q(F) = N(mean, v) is exact, so there are no samples:
+ *   ll = sum_{g,n} [ -1/2 log 2 pi - log s_g - (y_gn - bias_g - sum_f W_gf mean_fn)^2 / (2 s_g^2) ] - 1/2 sum_{g,f} W_gf^2 V_f / s_g^2,
+ *   V_f = sum_n v_fn.  spread as gpz_poisson_fwdbwd_* (v = max(spread, clamp_min) for f < n_var, spread^2 otherwise); idx (B or
+ *   NULL) gathers y[:, idx]; nothing is rescaled by Ntot / B.  Outputs: ll (one double), gW, gbias, gnoise (G x F, G, G), gmean,
+ *   gspread (F x B).  y is read once and nothing of size G x B is written; partials are summed in a fixed order (no atomics).
+ *   1 <= F <= 32, 0 <= n_var <= F, and y_ld >= B without idx; GPZ_ERR_UNSUPPORTED otherwise.  ws sized by
+ *   gpz_gaussian_workspace_bytes_*. */
+int64_t gpz_gaussian_workspace_bytes_f32(int G, int F, int B);
+int64_t gpz_gaussian_workspace_bytes_f64(int G, int F, int B);
+int gpz_gaussian_fwdbwd_f32(const float* y, int64_t y_ld, const int64_t* idx, const float* W, const float* bias, const float* noise,
+                            const float* mean, const float* spread, int G, int F, int B, int n_var, float clamp_min, double* ll,
+                            float* gW, float* gbias, float* gnoise, float* gmean, float* gspread, void* ws, int64_t ws_bytes,
+                            void* stream);
+int gpz_gaussian_fwdbwd_f64(const double* y, int64_t y_ld, const int64_t* idx, const double* W, const double* bias,
+                            const double* noise, const double* mean, const double* spread, int G, int F, int B, int n_var,
+                            double clamp_min, double* ll, double* gW, double* gbias, double* gnoise, double* gmean,
+                            double* gspread, void* ws, int64_t ws_bytes, void* stream);
 /* the digamma and lgamma of the K7-NB kernels (x > 0), element-wise over n doubles on the device */
 int gpz_digamma_f64(const double* x, double* out, int64_t n, void* stream);
 int gpz_lgamma_f64(const double* x, double* out, int64_t n, void* stream);
